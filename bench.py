@@ -2,6 +2,7 @@
 """bench.py -- GKR prover throughput (gates/s) and sumcheck ms/proof on B200, beside the CPU reference.
 
   python bench.py --gpus N --steps K --warmup W            our arm (CUDA, through the C ABI)
+      [--dump-outputs DIR]                                 + the transcript of the last timed proof as DIR/transcript.npy
   python bench.py --impl reference --gpus N --steps K ...  the reference's CPU prover on the host cores
 
 One step = one complete GKR proof (evaluate + every phase-1 / phase-2 / Liu sumcheck of every layer +
@@ -161,6 +162,8 @@ def run_ours(args):
     barrier()
     ms_resident = max_over_ranks(e0.elapsed_time(e1)) / args.steps
     launches = prover.last_prove_launches
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, prover.transcript())
     # the same K steps again with a CUDA-event pair around every kernel launch (per-class device time for the
     # roofline object; the event pairs cost a few % so `value` comes from the un-instrumented pass above)
     prover.set_profiling(True)
@@ -454,6 +457,21 @@ class Env:
 
 def sha256_of(tr):
     return hashlib.sha256(np.ascontiguousarray(tr).tobytes()).hexdigest()
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, tr):
+    """--dump-outputs: the transcript of the last timed proof (what a caller reads back with vp_get_transcript) as out_dir/transcript.npy,
+    float32 of shape (len, 16): the 16 little-endian bytes of each F_p^2 element (re, then im). The elements are integers
+    below 2^61 that no float type holds exactly; a byte is exact in float32, and a changed element changes some byte by
+    at least 1, which a comparison with an absolute tolerance below 1 (and no relative one) always catches. Inputs and challenges are fixed (the .pws inputs, challenge seed 3396), so
+    two builds run with the same arguments can be compared file for file."""
+    rows = np.ascontiguousarray(tr).view(np.uint8).reshape(len(tr), 16).astype(np.float32)
+    assert rows.nbytes <= DUMP_LIMIT_BYTES, rows.nbytes   # 64 B per element, 3 elements per round: ~350k sumcheck rounds to reach it
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "transcript.npy"), rows)
 
 
 def golden_full(name):
@@ -864,7 +882,13 @@ def main():
     ap.add_argument("--no-extras", action="store_true", help="skip the C1/C2 side measurements and the CPU sample")
     ap.add_argument("--extras-deadline", type=float, default=900.0,
                     help="seconds the legs after the timed regions may take before rank 0 prints the line without them")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the transcript of the last timed proof to DIR/transcript.npy (see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what the GPU arm computed; the reference arm has no dump")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3
     # The contract is ONE JSON line on stdout. Libraries write there too (NCCL prints its version banner on stdout at

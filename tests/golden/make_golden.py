@@ -7,6 +7,7 @@
   small_*            hand-written / seeded-random .pws circuits covering every gate type the parser
                      emits, operand swaps (Sub->AntiSub, Naab->AntiNaab), the Not fall-through quirk,
                      empty and single-element dad subsets, layers of size 1
+  random_pws_<seed>  seeded random .pws circuits (random_pws), stored without the .pws
 
 For each case it stores  <name>.pws.xz (except sha256_64, already here), <name>.transcript.txt.xz
 (lines "TAG real img", the prover->verifier messages and received challenges in emission order) and
@@ -167,6 +168,9 @@ def main():
     run_case("small_random_a", random_pws(1, 200, 150), keep_circuit=True)
     run_case("small_random_b", random_pws(2, 333, 600), keep_circuit=True)
     run_case("small_random_c", random_pws(3, 260, 60), keep_circuit=True)
+    # test_loader_and_oracle_match_live_reference_on_random_pws regenerates these .pws files from the seed
+    for seed, n_in, n_gates in [(11, 200, 450), (12, 257, 900), (13, 511, 200), (14, 300, 90)]:
+        run_case(f"random_pws_{seed}", random_pws(seed, n_in, n_gates), keep_pws=False, keep_circuit=True)
 
 
 if __name__ == "__main__":

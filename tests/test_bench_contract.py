@@ -1,9 +1,11 @@
-"""CPU checks of bench.py's contract: the reference arm prints exactly one JSON line with the agreed keys, and our
-arm refuses to run without a CUDA device (the product has no CPU path)."""
+"""Checks of bench.py's contract: the reference arm prints exactly one JSON line with the agreed keys, our arm refuses to
+run without a CUDA device (the product has no CPU path), and --dump-outputs writes the timed proof's transcript."""
 import json
 import os
 import subprocess
 import sys
+
+import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -32,6 +34,44 @@ def test_our_arm_needs_a_gpu():
     assert r.returncode != 0
     assert "no CUDA device" in (r.stderr + r.stdout)
     assert not [l for l in r.stdout.splitlines() if l.startswith("{")]   # no number without a GPU
+
+
+def test_steps_must_be_positive():
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "0"], capture_output=True, text=True, timeout=600)
+    assert r.returncode != 0 and "--steps must be at least 1" in r.stderr
+    assert not [l for l in r.stdout.splitlines() if l.startswith("{")]
+
+
+def test_dump_outputs_keeps_every_bit(tmp_path):
+    """--dump-outputs stores field elements as float32 bytes: exact, and any changed element differs by >= 1 somewhere"""
+    import numpy as np
+    sys.path.insert(0, ROOT)
+    import bench
+    P = (1 << 61) - 1
+    rng = np.random.default_rng(5)
+    tr = np.zeros(1000, [("re", "<u8"), ("im", "<u8")])
+    tr["re"] = rng.integers(0, P, len(tr), dtype=np.uint64)
+    tr["im"] = rng.integers(0, P, len(tr), dtype=np.uint64)
+    tr[0] = (P - 1, 0)
+    bench.dump_outputs(str(tmp_path / "out"), tr)
+    d = np.load(tmp_path / "out" / "transcript.npy")
+    assert d.dtype == np.float32 and d.shape == (len(tr), 16)
+    assert (d.astype(np.uint8).view(tr.dtype).ravel() == tr).all()
+
+
+@pytest.mark.gpu
+def test_dump_outputs_is_the_proof_of_the_timed_circuit(tmp_path, B, O, sha_circuit):
+    """bench.py --dump-outputs on a small workload: one JSON line, and the dumped transcript is the oracle's proof of the same
+    circuit (SHA256_64 x 2) with the same challenges"""
+    import numpy as np
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "2", "--warmup", "3", "--instances", "2",
+                        "--no-extras", "--dump-outputs", str(tmp_path)], capture_output=True, text=True, timeout=900)
+    assert r.returncode == 0, r.stderr[-2000:]
+    assert len([l for l in r.stdout.splitlines() if l.strip()]) == 1, r.stdout[-2000:]
+    assert json.loads(r.stdout)["steps"] == 2
+    got = np.load(tmp_path / "transcript.npy").astype(np.uint8).view(B.F_DTYPE).ravel()
+    want, _, _ = O.OracleCircuit(sha_circuit.replicate(2).expand().flat()).prove()
+    assert (got["re"] == want["re"]).all() and (got["im"] == want["im"]).all()
 
 
 _GUARD_SCRIPT = r'''

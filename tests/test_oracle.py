@@ -469,30 +469,18 @@ def test_fft_gkr_oracle_verifier_rejects_a_wrong_message(O):
     assert add(ev(bad, (0, 0)), ev(bad, (1, 0))) != prev
 
 
-# ------------------------------------------------------------------ live differential check (this container only)
+# ------------------------------------------------------------------ seeded random .pws circuits
 @pytest.mark.parametrize("seed,n_in,n_gates", [(11, 200, 450), (12, 257, 900), (13, 511, 200), (14, 300, 90)])
 def test_loader_and_oracle_match_live_reference_on_random_pws(B, O, seed, n_in, n_gates):
-    """Where the unmodified reference is built (oracle/_ref/ref_dump, this container): a fresh seeded random .pws goes
-    through the reference's loader + prover + verifier and through this repo's loader + C oracle; circuit dump and
-    transcript must be byte-identical. (tools/diff_reference_campaign.py ran 400 more seeds: 0 mismatches.)"""
-    mg = _make_golden()
-    if not os.path.exists(mg.REF_DUMP):
-        pytest.skip("oracle/_ref/ref_dump not built (needs /root/reference)")
-    import tempfile
-    pws = mg.random_pws(seed, n_in, n_gates)
-    with tempfile.TemporaryDirectory() as td:
-        path = os.path.join(td, "c.pws")
-        with open(path, "wb") as f:
-            f.write(pws)
-        r = subprocess.run([mg.REF_DUMP, path, os.path.join(td, "c")], capture_output=True, text=True)
-        if "VERIFY 1" not in r.stdout:
-            pytest.skip("the reference aborts on this circuit (its own heap corruption on 1-gate layers)")
-        want_tr = open(os.path.join(td, "c.transcript.txt")).read()
-        want_cb = open(os.path.join(td, "c.circuit.bin"), "rb").read()
-    circ = B.Circuit.from_pws_text(pws)
-    assert H.circuit_dump(circ) == want_cb
+    """A seeded random .pws (make_golden.random_pws, regenerated here from the seed) through this repo's loader + C oracle:
+    circuit dump and transcript byte-identical to what the unmodified reference's loader + prover + verifier wrote for the
+    same file (golden random_pws_<seed>.*, make_golden.py). (tools/diff_reference_campaign.py ran 400 more seeds against
+    the live reference: 0 mismatches.)"""
+    name = f"random_pws_{seed}"
+    circ = B.Circuit.from_pws_text(_make_golden().random_pws(seed, n_in, n_gates))
+    assert H.circuit_dump(circ) == H.golden_bytes(name + ".circuit.bin.xz")
     tr, ch, _ = O.OracleCircuit(circ.flat()).prove()
-    assert H.transcript_text(circ, tr, ch) == want_tr
+    assert H.transcript_text(circ, tr, ch) == H.golden_bytes(name + ".transcript.txt.xz").decode()
 
 
 # ------------------------------------------------------------------ Fiat-Shamir challenge source == the reference's own class
