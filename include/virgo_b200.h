@@ -271,10 +271,52 @@ int vp_fft_gkr(int device, int lg_size, const vp_F* rnd, size_t n_rnd, vp_F* lay
  * and returns the transcript and, optionally, the challenges it drew (usual layout, unused slots zero);
  * vp_fs_challenges recomputes them from a transcript alone; vp_verify_fs = vp_fs_challenges + vp_verify (fail_code 7:
  * a non-canonical transcript element). Not parity-bound to the reference (it has no such mode); pinned against the
- * oracle's restatement of transcriptCache. */
+ * oracle's restatement of transcriptCache.
+ * The seed MUST be a digest of the statement (circuit, inputs, outputs): this mode absorbs nothing else, so with a seed
+ * that does not commit to them a prover can fix a transcript first and pick inputs that pass the input-layer check
+ * afterwards, and the verifier never learns the outputs. vp_prove_fs_bound / vp_verify_fs_bound below derive the seed
+ * from the statement; vp_prove_fs(ctx, statement) is the same proof.
+ * On an unsharded context the whole proof is queued on the device (the transcript cache is a device buffer, every
+ * round's challenge is drawn inside the sumcheck phase kernel); sharded contexts draw on the host between rounds. */
 int vp_prove_fs(vp_ctx* ctx, const uint8_t seed[32], vp_F* transcript, size_t transcript_cap, vp_F* challenges, size_t challenges_cap);
 int vp_fs_challenges(const vp_circuit* c, const uint8_t seed[32], const vp_F* transcript, size_t n, vp_F* challenges, size_t cap);
 int vp_verify_fs(vp_ctx* ctx, const uint8_t seed[32], const vp_F* transcript, size_t n, int* accept, int* fail_code, int* fail_layer);
+
+/* ------------------------------------------------------------------ statement-bound Fiat-Shamir proofs
+ * Every integer is little-endian; H = SHA3-256 (FIPS 202).
+ * Vector root R(bytes): zero-pad bytes to 64 * 2^k bytes, 2^k the smallest power of two >= max(1, ceil(len / 64)); leaf j =
+ *   H(64-byte block j); array-heap Merkle tree with node = H(left | right), leaves at nodes 2^k .. 2^(k+1) - 1, root = node 1
+ *   (one leaf: the root is that leaf's hash).
+ * Inputs root  = R over circuitValue[0] as the prover holds it (instances * layer_size(0) canonical elements, 16 bytes
+ *   {re, im} each, after vp_set_inputs' reading rules). Outputs root = R over circuitValue[n-1] (instances * layer_size(n-1)).
+ * Circuit digest = R(circuit_bytes), from what vp_circuit_export_layer / vp_circuit_export_dad return:
+ *   "VPCIRC01" | u64 n_layers | u64 instances | u64 layer_size(i), i = 0..n-1 |
+ *   for i = 1..n-1, every template gate, packed 34 bytes: u8 ty, u8 is_assert, i32 l, u32 u, u32 v, u32 lv, u64 c.re, u64 c.im |
+ *   for i = 1..n-1, s = 0..i-1: u64 dad_size(i, s) | u32 dad_id[dad_size(i, s)].
+ *   Layer 0 contributes its size only (its values are bound by the inputs root). A replicated circuit is hashed as its
+ *   template + K: vp_circuit_expand of it is another circuit object with another digest.
+ * Statement = H("VPSTMT01" | circuit digest | u64 n_inputs | inputs root | u64 n_outputs | outputs root | context[32]) (152
+ *   bytes); context = 32 caller-chosen bytes (application tag, session id; may be zero).
+ * vp_prove_fs_bound(ctx, context) is, by definition, vp_prove_fs(ctx, statement).
+ * vp_statement_digest: the four digests of the context's resident inputs (the circuit is evaluated first if needed);
+ *   circuit / inputs / outputs may be NULL. The circuit digest is computed once per context (on the device, from bytes
+ *   serialised on the host) and kept.
+ * vp_prove_fs_bound: the proof; transcript / challenges as vp_prove_fs; statement (may be NULL) = the seed it used.
+ * vp_verify_fs_bound: the verifier's side, from its own circuit and resident inputs and the CLAIMED outputs (n_outputs =
+ *   instances * layer_size(n-1) canonical elements, else VP_ERR_ARG): computes the statement, the challenges
+ *   (vp_fs_challenges), checks Vres == MLE(outputs)(r_out) (fail_code 8), then vp_verify's checks. fail_code 7: a
+ *   non-canonical transcript element.
+ * vp_fs_round_stamps: %globaltimer stamps (ns) of block 0 in the last device Fiat-Shamir proof, 4 per sumcheck round in
+ *   proof order {round start, own fold work done, polynomial reduced (after the grid barrier), challenge drawn};
+ *   *n_rounds = the number of rounds; out may be NULL (cap >= 4 * rounds otherwise).
+ * Sharded contexts: all of these return VP_ERR_ARG. */
+int vp_statement_digest(vp_ctx* ctx, const uint8_t context[32], uint8_t circuit[32], uint8_t inputs[32], uint8_t outputs[32],
+                        uint8_t statement[32]);
+int vp_prove_fs_bound(vp_ctx* ctx, const uint8_t context[32], vp_F* transcript, size_t cap, vp_F* challenges, size_t ch_cap,
+                      uint8_t statement[32]);
+int vp_verify_fs_bound(vp_ctx* ctx, const uint8_t context[32], const vp_F* outputs, size_t n_outputs, const vp_F* transcript, size_t n,
+                       int* accept, int* fail_code, int* fail_layer);
+int vp_fs_round_stamps(vp_ctx* ctx, unsigned long long* out, size_t cap, size_t* n_rounds);
 
 /* Self-test of the device-only arithmetic paths of csrc/field.cuh (inline-PTX carry chains, mul.wide / mad.wide):
    runs one routine on n caller-provided operand triples and returns the results, so that tests can feed edge values

@@ -130,6 +130,11 @@ def _declare(L):
     L.vp_prove_fs.argtypes = [vp, C.c_char_p, vp, C.c_size_t, vp, C.c_size_t]
     L.vp_fs_challenges.argtypes = [vp, C.c_char_p, vp, C.c_size_t, vp, C.c_size_t]
     L.vp_verify_fs.argtypes = [vp, C.c_char_p, vp, C.c_size_t, C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(C.c_int)]
+    L.vp_statement_digest.argtypes = [vp, C.c_char_p, vp, vp, vp, vp]
+    L.vp_prove_fs_bound.argtypes = [vp, C.c_char_p, vp, C.c_size_t, vp, C.c_size_t, vp]
+    L.vp_verify_fs_bound.argtypes = [vp, C.c_char_p, vp, C.c_size_t, vp, C.c_size_t, C.POINTER(C.c_int), C.POINTER(C.c_int),
+                                     C.POINTER(C.c_int)]
+    L.vp_fs_round_stamps.argtypes = [vp, vp, C.c_size_t, C.POINTER(C.c_size_t)]
     L.vp_get_transcript.argtypes = [vp, vp, C.c_size_t]
     L.vp_last_prove_ms.argtypes = [vp]
     L.vp_last_prove_ms.restype = C.c_float
@@ -167,6 +172,13 @@ def _ck(rc):
 
 def _ptr(a):
     return a.ctypes.data_as(C.c_void_p) if a is not None else None
+
+
+def _context(context):
+    context = bytes(context)
+    if len(context) != 32:
+        raise ValueError("a Fiat-Shamir context is 32 bytes")
+    return context
 
 
 def fe(re, im=0):
@@ -678,6 +690,38 @@ class Prover:
         a, c, l = C.c_int(0), C.c_int(0), C.c_int(0)
         _ck(lib().vp_verify_fs(self.h, bytes(seed32), _ptr(tr), len(tr), C.byref(a), C.byref(c), C.byref(l)))
         return bool(a.value), c.value, l.value
+
+    def statement_digest(self, context=bytes(32)):
+        """the statement of the resident inputs (include/virgo_b200.h) -> dict(circuit, inputs, outputs, statement), 32 bytes each"""
+        out = [np.zeros(32, np.uint8) for _ in range(4)]
+        _ck(lib().vp_statement_digest(self.h, _context(context), *[_ptr(x) for x in out]))
+        return dict(zip(("circuit", "inputs", "outputs", "statement"), (x.tobytes() for x in out)))
+
+    def prove_fs_bound(self, context=bytes(32)):
+        """statement-bound Fiat-Shamir proof -> (transcript, challenges, statement); == prove_fs(statement)"""
+        tr = np.zeros(self.circuit.transcript_len, F_DTYPE)
+        ch = np.zeros(self.circuit.challenge_count, F_DTYPE)
+        st = np.zeros(32, np.uint8)
+        _ck(lib().vp_prove_fs_bound(self.h, _context(context), _ptr(tr), len(tr), _ptr(ch), len(ch), _ptr(st)))
+        return tr, ch, st.tobytes()
+
+    def verify_fs_bound(self, context, outputs, transcript):
+        """(accept, fail_code, fail_layer) of a statement-bound proof for the claimed outputs and this context's inputs"""
+        out = np.ascontiguousarray(outputs, dtype=F_DTYPE)
+        tr = np.ascontiguousarray(transcript, dtype=F_DTYPE)
+        a, c, l = C.c_int(0), C.c_int(0), C.c_int(0)
+        _ck(lib().vp_verify_fs_bound(self.h, _context(context), _ptr(out), len(out), _ptr(tr), len(tr), C.byref(a), C.byref(c),
+                                     C.byref(l)))
+        return bool(a.value), c.value, l.value
+
+    def fs_round_stamps(self):
+        """block 0's %globaltimer stamps (ns) per round of the last device Fiat-Shamir proof: [rounds, 4] = round start, own
+        fold work done, polynomial reduced, challenge drawn"""
+        n = C.c_size_t()
+        _ck(lib().vp_fs_round_stamps(self.h, None, 0, C.byref(n)))
+        out = np.zeros(4 * max(n.value, 1), np.uint64)
+        _ck(lib().vp_fs_round_stamps(self.h, _ptr(out), len(out), C.byref(n)))
+        return out[:4 * n.value].reshape(n.value, 4)
 
     def input_range(self):
         """instances [first, end) whose witness this rank uploads (everything on an unsharded context)"""

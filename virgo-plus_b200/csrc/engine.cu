@@ -26,6 +26,7 @@
 #include "../host/proof_io.h"
 #include "../host/fiat_shamir.h"
 #include "kernels.cuh"
+#include "fs_device.cuh"
 #include "pc_commit.h"
 
 using namespace vp;
@@ -1030,6 +1031,25 @@ struct Engine {
     bool use_phase_kernel = true;
     void prove_all();
     void prove_fs(const uint8_t seed[32], F* tr_out, F* ch_out);
+    // Fiat-Shamir mode on the device (fs_device.cuh): the pool, the per-round stamps and the statement digest's buffers
+    DBuf<uint64_t> d_fs_pool;
+    DBuf<unsigned long long> d_fs_stamps;
+    size_t fs_rounds = 0;                  // rounds of the last device FS proof (4 stamps each)
+    DBuf<uint64_t> d_stmt;                 // {circuit, inputs, outputs, statement} digests, 4 words each
+    DBuf<uint64_t> d_root_scratch;
+    DBuf<F> d_fs_outputs;                  // vp_verify_fs_bound: the claimed outputs
+    bool circuit_digest_ready = false;
+    int cap_phase_fs = 0;
+    void fs_alloc();
+    void fs_begin();
+    void statement_async(const uint8_t context[32], const F* d_outputs);
+    void circuit_digest_async();
+    void prove_fs_device(const uint8_t* seed, F* tr_out, F* ch_out);
+    void launch_phase_kernel_fs(const SumcheckPlan& P, uint32_t ci, F* keep, const F* at_init, uint32_t tr_rounds, size_t stamp_round);
+    void fs_absorb_draw(uint32_t tr_begin, uint32_t n_store, uint32_t ci_begin, uint32_t n_draw) {
+        k_fs_absorb_draw<<<1, 32, 0, stream>>>(d_fs_pool.p, d_tr.p, tr_begin, n_store, d_chal.p, ci_begin, n_draw);
+        ++launches;
+    }
     std::vector<F> h_chal;   // host copy of the challenges: the pass kernel gets their limbs through its parameters
     void set_chal(uint32_t idx, const vp_F* v, size_t cnt = 1) {
         // the limb arithmetic needs canonical challenges (split31 would silently drop the top bits of anything else)
@@ -1108,6 +1128,7 @@ void Engine::build(const Circuit& circ, int dev, int world_, int rank_, const ui
     cap_dot = occ_cap(k_dot_eq);
     cap_comb = occ_cap(k_combine_phase2);
     cap_phase = occ_cap(k_sumcheck_phase);
+    cap_phase_fs = occ_cap(k_sumcheck_phase_fs);
     dfs_enable_smem();
     cap_dfs = std::min({occ_cap(k_phase_dfs<true, DFS_VREAL>, DFS_THREADS, DFS_DYN_SMEM), occ_cap(k_phase_dfs<false, DFS_VREAL>, DFS_THREADS, DFS_DYN_SMEM),
                         occ_cap(k_phase_dfs<true, DFS_PLAIN>, DFS_THREADS, DFS_DYN_SMEM), occ_cap(k_phase_dfs<false, DFS_PLAIN>, DFS_THREADS, DFS_DYN_SMEM)});
@@ -1130,7 +1151,7 @@ void Engine::build(const Circuit& circ, int dev, int world_, int rank_, const ui
         CK(cudaDeviceGetAttribute(&coop, cudaDevAttrCooperativeLaunch, dev));
         if (!coop) throw CudaError{"device does not support cooperative launches"};
     }
-    max_grid = std::max({cap_round, cap_round1, cap_un, cap_dot, cap_phase, cap_dfs});  // sizes the block-partials buffer
+    max_grid = std::max({cap_round, cap_round1, cap_un, cap_dot, cap_phase, cap_phase_fs, cap_dfs});  // sizes the block-partials buffer
 
     // challenge / transcript index maps (draw order of verifier.cpp, see circuit.cpp draw_challenges)
     L.resize(n);
@@ -2640,6 +2661,165 @@ void Engine::prove_fs(const uint8_t seed[32], F* tr_out, F* ch_out) {
     }
 }
 
+// ---- Fiat-Shamir mode on the device (fs_device.cuh): the order of prove_fs, with the transcript cache in a device pool;
+// the host only enqueues. One synchronisation for the assert flag after evaluate, one at the end for the copies.
+void Engine::fs_alloc() {
+    if (d_fs_pool.p) return;
+    d_fs_pool.alloc(1 + 4 + 2 * ((size_t)n + 4));   // the longest run of stores between two draws: claim_u + claims_v
+    size_t rounds = 0;
+    for (int i = 1; i < n; ++i) rounds += (size_t)(2 * C.bit_length(i - 1) + std::max(L[i].max_dad_bl, 0));
+    d_fs_stamps.alloc(4 * std::max<size_t>(rounds, 1));
+    d_stmt.alloc(16);
+}
+void Engine::fs_begin() {
+    leave();
+    fs_alloc();
+    CK(cudaMemsetAsync(d_chal.p, 0, (n_chal + 1) * sizeof(F), stream));   // unused challenge slots are zero
+    h_chal.assign(n_chal, f_zero());
+    evaluate();
+    check_assert_flag();
+}
+
+// one cooperative launch of k_sumcheck_phase_fs over P (unsharded: the whole phase)
+void Engine::launch_phase_kernel_fs(const SumcheckPlan& P, uint32_t ci, F* keep, const F* at_init, uint32_t tr_rounds, size_t stamp_round) {
+    PhaseArgs a;
+    for (int b = 0; b < 2; ++b) { a.bufV[b] = bufV[b].p; a.bufM[b] = bufM[b].p; a.bufA[b] = bufA[b].p; }
+    a.rounds = d_rdev.p + P.rdev_begin;
+    a.tabs = d_tabs.p;
+    a.cols = d_cols.p;
+    a.fins = d_fins.p + P.fin_begin;
+    a.n_rounds = (uint32_t)P.rounds;
+    a.n_fin = P.n_fin;
+    a.fin_buf = (uint32_t)P.fin_buf;
+    a.tail_work = tail_work;
+    a.round_base = 0;
+    a.at_init = at_init;
+    a.chal = d_chal.p + ci;
+    a.add_term = scal(SC_ADD_TERM);
+    a.claims = d_claims.p;
+    a.out_poly = d_tr.p + tr_rounds;
+    a.transcript = d_tr.p;
+    a.keep = keep;
+    a.partials = d_partials.p;
+    FsPhaseArgs f;
+    f.pool = d_fs_pool.p;
+    f.chal = d_chal.p + ci;
+    f.stamps = d_fs_stamps.p + 4 * stamp_round;
+    const int grid = P.max_work > tail_work ? grid_for(P.max_work, cap_phase_fs) : 1;
+    void* args[] = {&a, &f};
+    size_t h = prof_begin(KC_ROUND_FOLD);
+    CK(cudaLaunchCooperativeKernel((const void*)k_sumcheck_phase_fs, dim3(grid), dim3(256), args, 0, stream));
+    prof_end(h, P.bytes);
+    ++launches;
+}
+
+// The circuit digest R(circuit_bytes) (include/virgo_b200.h), serialised on the host once per context and hashed on the device.
+void Engine::circuit_digest_async() {
+    if (circuit_digest_ready) return;
+    std::vector<uint8_t> b;
+    auto put = [&](const void* q, size_t len) { const uint8_t* c = static_cast<const uint8_t*>(q); b.insert(b.end(), c, c + len); };
+    auto u64 = [&](uint64_t x) { put(&x, 8); };
+    size_t total = 8 + 16 + 8 * (size_t)n;
+    for (int i = 1; i < n; ++i) {
+        total += 34 * C.layers[i].size;
+        for (int s = 0; s < i; ++s) total += 8 + 4 * C.layers[i].dadId[s].size();
+    }
+    b.reserve(total + 64);
+    put("VPCIRC01", 8);
+    u64((uint64_t)n);
+    u64(C.instances);
+    for (int i = 0; i < n; ++i) u64(C.layers[i].size);
+    for (int i = 1; i < n; ++i) {
+        const Layer& T = C.layers[i];
+        for (uint64_t g = 0; g < T.size; ++g) {
+            const uint8_t ty = T.ty[g], as = T.is_assert.empty() ? 0 : T.is_assert[g];
+            const int32_t l = T.l[g];
+            const uint32_t u = T.u[g], v = T.v[g], lv = T.lv[g];
+            const F c = T.c.empty() ? f_zero() : T.c[g];
+            put(&ty, 1); put(&as, 1); put(&l, 4); put(&u, 4); put(&v, 4); put(&lv, 4); put(&c.re, 8); put(&c.im, 8);
+        }
+    }
+    for (int i = 1; i < n; ++i)
+        for (int s = 0; s < i; ++s) {
+            u64(C.layers[i].dadSize[s]);
+            put(C.layers[i].dadId[s].data(), 4 * C.layers[i].dadId[s].size());
+        }
+    b.resize((b.size() + 63) / 64 * 64, 0);   // whole leaves (R pads with zeros anyway)
+    DBuf<uint64_t> words, scratch;
+    words.alloc(b.size() / 8);
+    CK(cudaMemcpyAsync(words.p, b.data(), b.size(), cudaMemcpyHostToDevice, stream));
+    scratch.alloc(pc_vector_root_scratch(words.n) / 8);
+    launches += (uint64_t)pc_vector_root(words.p, words.n, scratch.p, reinterpret_cast<uint8_t*>(d_stmt.p), stream);
+    CK(cudaStreamSynchronize(stream));   // (the host bytes and the scratch go out of scope)
+    circuit_digest_ready = true;
+}
+
+// inputs root (circuitValue[0]), outputs root (d_outputs, or circuitValue[n-1]) and the statement, which seeds the pool
+void Engine::statement_async(const uint8_t context[32], const F* d_outputs) {
+    circuit_digest_async();
+    const size_t n_in = C.layer_size(0), n_out = C.layer_size(n - 1);
+    const size_t need = std::max(pc_vector_root_scratch(2 * n_in), pc_vector_root_scratch(2 * n_out)) / 8;
+    if (d_root_scratch.n < need) d_root_scratch.alloc(need);
+    uint8_t* roots = reinterpret_cast<uint8_t*>(d_stmt.p);
+    launches += (uint64_t)pc_vector_root(reinterpret_cast<const uint64_t*>(val[0].p), 2 * n_in, d_root_scratch.p, roots + 32, stream);
+    launches += (uint64_t)pc_vector_root(reinterpret_cast<const uint64_t*>(d_outputs ? d_outputs : val[n - 1].p), 2 * n_out, d_root_scratch.p,
+                                         roots + 64, stream);
+    FsContext cx;
+    memcpy(cx.w, context, 32);
+    k_fs_statement<<<1, 32, 0, stream>>>(d_stmt.p, (uint64_t)n_in, (uint64_t)n_out, cx, d_fs_pool.p, d_stmt.p + 12);
+    ++launches;
+}
+
+// The proof in the order of prove_fs (host/fiat_shamir.h). seed != null: the pool starts with it; null: statement_async
+// seeded it. The transcript and the challenges come back in one copy each.
+void Engine::prove_fs_device(const uint8_t* seed, F* tr_out, F* ch_out) {
+    if (seed) {
+        uint64_t h[5] = {4, 0, 0, 0, 0};
+        memcpy(h + 1, seed, 32);
+        CK(cudaMemcpyAsync(d_fs_pool.p, h, sizeof h, cudaMemcpyHostToDevice, stream));
+    }
+    size_t sr = 0;   // stamp slot of the next phase's first round
+    fs_absorb_draw(0, 0, ci_out, (uint32_t)C.bit_length(n - 1));
+    do_vres();
+    uint32_t tr_prev = tr_vres;   // the message stored before the next layer's assert_random: Vres, then claim_liu
+    for (int i = n - 1; i >= 1; --i) {
+        LayerDev& D = L[i];
+        const int m = D.max_dad_bl;
+        cur_layer = i;
+        fs_absorb_draw(tr_prev, 1, D.ci_assert, 1);
+        do_init_phase1(i);
+        launch_phase_kernel_fs(D.ph1.planB, D.ci_ru, scal(SC_VU), nullptr, D.tr_p1, sr);
+        sr += (size_t)D.ph1.planB.rounds;
+        if (m != -1) {
+            fs_absorb_draw(D.tr_claim_u, 1, 0, 0);
+            do_init_phase2(i);
+            launch_phase_kernel_fs(D.ph2.planB, D.ci_rv, nullptr, scal(SC_UNARY), D.tr_p2, sr);
+            sr += (size_t)D.ph2.planB.rounds;
+            fs_absorb_draw(D.tr_claims_v, (uint32_t)i, D.ci_sig, (uint32_t)n);
+        } else
+            fs_absorb_draw(D.tr_claim_u, 1, D.ci_sig, (uint32_t)n);
+        do_init_liu(i, true);
+        launch_phase_kernel_fs(D.ph3.planB, D.ci_rliu, nullptr, nullptr, D.tr_liu, sr);
+        sr += (size_t)D.ph3.planB.rounds;
+        tr_prev = D.tr_claim_liu;
+    }
+    do_input_mle();
+    fs_rounds = sr;
+    std::vector<F> ch(n_chal);
+    CK(cudaMemcpyAsync(tr_out, d_tr.p, n_tr * sizeof(F), cudaMemcpyDeviceToHost, stream));
+    CK(cudaMemcpyAsync(ch.data(), d_chal.p, n_chal * sizeof(F), cudaMemcpyDeviceToHost, stream));
+    CK(cudaStreamSynchronize(stream));
+    CK(cudaGetLastError());
+    h_chal = ch;   // a later vp_verify / vp_prove on this context sees the challenges the proof used
+    if (ch_out) memcpy(ch_out, ch.data(), n_chal * sizeof(F));
+    proof_size = 0;
+    for (int i = n - 1; i >= 1; --i) {
+        const int pb = C.bit_length(i - 1), m = L[i].max_dad_bl;
+        proof_size += (uint64_t)(2 * pb + (m != -1 ? m : 0)) * 3 * sizeof(F) + sizeof(F);
+        if (m != -1) proof_size += (uint64_t)i * sizeof(F);
+    }
+}
+
 // The challenges of a Fiat-Shamir transcript, recomputed from the messages alone (what a verifier does first), in the
 // usual challenge layout (vp_draw_challenges order; unused slots zero).
 static void fs_challenges(const Circuit& C, const uint8_t seed[32], const F* tr, F* ch, size_t n_chal) {
@@ -3562,7 +3742,11 @@ extern "C" int vp_prove_fs(vp_ctx* ctx, const uint8_t seed[32], vp_F* transcript
     if (!e.inputs_loaded) return fail(VP_ERR_ARG, "vp_prove_fs: inputs not loaded");
     const uint64_t l0 = e.launches;
     CK(cudaEventRecord(e.ev0, e.stream));
-    e.prove_fs(seed, reinterpret_cast<F*>(transcript), reinterpret_cast<F*>(challenges));
+    if (e.world == 1) {   // the whole proof queued on the device; sharded contexts keep the host loop
+        e.fs_begin();
+        e.prove_fs_device(seed, reinterpret_cast<F*>(transcript), reinterpret_cast<F*>(challenges));
+    } else
+        e.prove_fs(seed, reinterpret_cast<F*>(transcript), reinterpret_cast<F*>(challenges));
     CK(cudaEventRecord(e.ev1, e.stream));
     CK(cudaStreamSynchronize(e.stream));
     CK(cudaEventElapsedTime(&e.last_ms, e.ev0, e.ev1));
@@ -3594,6 +3778,117 @@ extern "C" int vp_verify_fs(vp_ctx* ctx, const uint8_t seed[32], const vp_F* tra
     fs_challenges(e.C, seed, reinterpret_cast<const F*>(transcript), ch.data(), e.n_chal);
     e.set_chal(0, reinterpret_cast<const vp_F*>(ch.data()), e.n_chal);
     *accept = e.verify(reinterpret_cast<const F*>(transcript), fail_code, fail_layer);
+    return VP_OK;
+    API_END
+}
+// ---- statement-bound Fiat-Shamir proofs (unsharded contexts)
+static bool fs_canonical(const vp_F* x, size_t n) {
+    for (size_t i = 0; i < n; ++i)
+        if (x[i].re >= P || x[i].im >= P) return false;
+    return true;
+}
+static void copy_digest(const uint64_t* h, uint8_t* out) { if (out) memcpy(out, h, 32); }
+extern "C" int vp_statement_digest(vp_ctx* ctx, const uint8_t context[32], uint8_t circuit[32], uint8_t inputs[32], uint8_t outputs[32],
+                                   uint8_t statement[32]) {
+    if (!ctx || !context || !statement) return fail(VP_ERR_ARG, "null argument");
+    API_BEGIN
+    Engine& e = ctx->e;
+    ScopedTimer t(e);
+    if (e.world != 1) return fail(VP_ERR_ARG, "vp_statement_digest: sharded contexts are not supported");
+    if (!e.inputs_loaded) return fail(VP_ERR_ARG, "vp_statement_digest: inputs not loaded");
+    e.leave();
+    e.fs_alloc();
+    if (!e.evaluated) e.evaluate();
+    e.statement_async(context, nullptr);
+    uint64_t h[16];
+    CK(cudaMemcpyAsync(h, e.d_stmt.p, sizeof h, cudaMemcpyDeviceToHost, e.stream));
+    CK(cudaStreamSynchronize(e.stream));
+    copy_digest(h, circuit);
+    copy_digest(h + 4, inputs);
+    copy_digest(h + 8, outputs);
+    copy_digest(h + 12, statement);
+    return VP_OK;
+    API_END
+}
+extern "C" int vp_prove_fs_bound(vp_ctx* ctx, const uint8_t context[32], vp_F* transcript, size_t cap, vp_F* challenges, size_t ch_cap,
+                                 uint8_t statement[32]) {
+    if (!ctx || !context || !transcript) return fail(VP_ERR_ARG, "null argument");
+    API_BEGIN
+    Engine& e = ctx->e;
+    ScopedTimer t(e);
+    if (e.world != 1) return fail(VP_ERR_ARG, "vp_prove_fs_bound: sharded contexts are not supported");
+    if (cap < e.n_tr) return fail(VP_ERR_ARG, "transcript buffer too small (%zu < %zu)", cap, e.n_tr);
+    if (challenges && ch_cap < e.n_chal) return fail(VP_ERR_ARG, "challenge buffer too small (%zu < %zu)", ch_cap, e.n_chal);
+    if (!e.inputs_loaded) return fail(VP_ERR_ARG, "vp_prove_fs_bound: inputs not loaded");
+    const uint64_t l0 = e.launches;
+    CK(cudaEventRecord(e.ev0, e.stream));
+    e.fs_begin();
+    e.statement_async(context, nullptr);
+    e.prove_fs_device(nullptr, reinterpret_cast<F*>(transcript), reinterpret_cast<F*>(challenges));
+    CK(cudaEventRecord(e.ev1, e.stream));
+    uint64_t h[4];
+    CK(cudaMemcpyAsync(h, e.d_stmt.p + 12, sizeof h, cudaMemcpyDeviceToHost, e.stream));
+    CK(cudaStreamSynchronize(e.stream));
+    copy_digest(h, statement);
+    CK(cudaEventElapsedTime(&e.last_ms, e.ev0, e.ev1));
+    e.last_launches = e.launches - l0;
+    return VP_OK;
+    API_END
+}
+extern "C" int vp_verify_fs_bound(vp_ctx* ctx, const uint8_t context[32], const vp_F* outputs, size_t n_outputs, const vp_F* transcript,
+                                  size_t n, int* accept, int* fail_code, int* fail_layer) {
+    if (!ctx || !context || !outputs || !transcript || !accept) return fail(VP_ERR_ARG, "null argument");
+    API_BEGIN
+    Engine& e = ctx->e;
+    cudaSetDevice(e.device);
+    if (e.world != 1) return fail(VP_ERR_ARG, "vp_verify_fs_bound: sharded contexts are not supported");
+    if (!e.inputs_loaded) return fail(VP_ERR_ARG, "vp_verify_fs_bound: inputs not loaded");
+    if (n != e.n_tr) return fail(VP_ERR_ARG, "expected a transcript of %zu field elements, got %zu", e.n_tr, n);
+    const size_t n_out = e.C.layer_size(e.n - 1);
+    if (n_outputs != n_out) return fail(VP_ERR_ARG, "expected %zu outputs, got %zu", n_out, n_outputs);
+    if (!fs_canonical(outputs, n_outputs)) return fail(VP_ERR_ARG, "an output is not canonical (components must be < p)");
+    auto reject = [&](int code) { *accept = 0; if (fail_code) *fail_code = code; if (fail_layer) *fail_layer = 0; return VP_OK; };
+    if (!fs_canonical(transcript, n)) return reject(7);
+    e.leave();
+    e.fs_alloc();
+    if (e.d_fs_outputs.n < n_out) e.d_fs_outputs.alloc(n_out);
+    CK(cudaMemcpyAsync(e.d_fs_outputs.p, outputs, n_out * sizeof(F), cudaMemcpyHostToDevice, e.stream));
+    {   // circuitValue[0] from the resident inputs: the verifier does not evaluate the circuit
+        const uint32_t S0 = (uint32_t)e.C.layers[0].size, b0 = e.k_lo * S0, e0 = e.k_hi * S0;
+        k_load_inputs<<<cdiv(std::max<uint32_t>(e0 - b0, 1), 256), 256, 0, e.stream>>>(e.d_inputs.p, e.val[0].p, b0, e0);
+        ++e.launches;
+    }
+    e.statement_async(context, e.d_fs_outputs.p);
+    uint64_t h[4];
+    CK(cudaMemcpyAsync(h, e.d_stmt.p + 12, sizeof h, cudaMemcpyDeviceToHost, e.stream));
+    CK(cudaStreamSynchronize(e.stream));
+    uint8_t stmt[32];
+    memcpy(stmt, h, 32);
+    std::vector<F> ch(e.n_chal);
+    fs_challenges(e.C, stmt, reinterpret_cast<const F*>(transcript), ch.data(), e.n_chal);
+    e.set_chal(0, reinterpret_cast<const vp_F*>(ch.data()), e.n_chal);
+    // the claim chain starts from Vres: it must be the MLE of the claimed outputs at r_out
+    e.run_eq(e.eqb_out, 2);
+    if (e.d_vf_out.n < 1) e.d_vf_out.alloc(2);
+    e.run_dot_eq(e.d_fs_outputs.p, (uint32_t)e.C.layers[e.n - 1].size, e.eqtab(2, e.C.bit_length(e.n - 1)), e.d_vf_out.p);
+    F mle;
+    CK(cudaMemcpyAsync(&mle, e.d_vf_out.p, sizeof mle, cudaMemcpyDeviceToHost, e.stream));
+    CK(cudaStreamSynchronize(e.stream));
+    if (!f_eq(mle, reinterpret_cast<const F*>(transcript)[e.tr_vres])) return reject(8);
+    *accept = e.verify(reinterpret_cast<const F*>(transcript), fail_code, fail_layer);
+    return VP_OK;
+    API_END
+}
+extern "C" int vp_fs_round_stamps(vp_ctx* ctx, unsigned long long* out, size_t cap, size_t* n_rounds) {
+    if (!ctx || !n_rounds) return fail(VP_ERR_ARG, "null argument");
+    API_BEGIN
+    Engine& e = ctx->e;
+    cudaSetDevice(e.device);
+    *n_rounds = e.fs_rounds;
+    if (out && e.fs_rounds) {
+        if (cap < 4 * e.fs_rounds) return fail(VP_ERR_ARG, "stamp buffer too small (%zu < %zu)", cap, 4 * e.fs_rounds);
+        CK(cudaMemcpy(out, e.d_fs_stamps.p, 4 * e.fs_rounds * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
+    }
     return VP_OK;
     API_END
 }

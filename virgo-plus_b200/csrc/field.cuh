@@ -43,6 +43,7 @@ struct alignas(16) F {
 VP_HD u64 fp_red1(u64 x) { return x >= P ? x - P : x; }          // x < 2p  ->  [0,p)
 VP_HD u64 fp_fold(u64 x) { return (x & P) + (x >> 61); }         // any u64 -> [0, p + 7], same class
 VP_HD u64 fp_canon(u64 x) { return fp_red1(fp_fold(x)); }        // any u64 < 2^64 - 2^61 -> [0,p)
+VP_HD u64 fp_mod(u64 x) { return fp_red1(fp_fold(fp_fold(x))); }  // any u64 -> x % p (a Fiat-Shamir digest word)
 VP_HD u64 fp_add(u64 a, u64 b) { return fp_red1(a + b); }
 VP_HD u64 fp_sub(u64 a, u64 b) { return fp_red1(a + (P - b)); }
 VP_HD u64 fp_neg(u64 a) { return a ? P - a : 0; }

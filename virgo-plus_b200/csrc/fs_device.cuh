@@ -1,0 +1,204 @@
+// Fiat-Shamir mode on the device (DESIGN.md section 7): the transcript cache of host/fiat_shamir.h (FsCache, the reference's
+// transcriptCache) restated as a small device buffer, so that a whole Fiat-Shamir proof is queued on one stream without a
+// host round trip per round.
+//
+// Pool layout (FS_POOL words): pool[0] = number of message words held, pool[1 ..] = the bytes of FsCache::pool as
+// little-endian words. Everything FsCache stores is a whole number of words (the 32-byte seed / digest, 16-byte field
+// elements), so the pool is a word array. Only one thread at a time touches it: the kernels below run in stream order and
+// inside k_sumcheck_phase_fs only thread 0 of block 0 does.
+#pragma once
+#include "kernels.cuh"
+#include "keccak.cuh"
+
+namespace vp {
+
+// store(x): 16 bytes {re, im}
+VP_D void fs_store(uint64_t* pool, const F& x) {
+    const uint64_t n = pool[0];
+    pool[1 + n] = x.re;
+    pool[2 + n] = x.im;
+    pool[0] = n + 2;
+}
+// random(): hash the pool, the digest becomes the pool, the challenge is the first two digest words mod p
+VP_D F fs_draw(uint64_t* pool) {
+    uint64_t d[4];
+    sha3_256_words(pool + 1, (uint32_t)pool[0], d);
+#pragma unroll
+    for (int k = 0; k < 4; ++k) pool[1 + k] = d[k];
+    pool[0] = 4;
+    return F{fp_mod(d[0]), fp_mod(d[1])};
+}
+
+// Between phases (one warp, lane 0 hashes): store transcript[tr_begin .. + n_store), then draw chal[ci_begin .. + n_draw)
+// (host/fiat_shamir.h: Vres / claim_u / claims_v / claim_liu, then r_out / assert_random / sig).
+__global__ void k_fs_absorb_draw(uint64_t* pool, const F* __restrict__ transcript, uint32_t tr_begin, uint32_t n_store, F* chal,
+                                 uint32_t ci_begin, uint32_t n_draw) {
+    const uint64_t n0 = pool[0];
+    __syncwarp();
+    for (uint32_t k = threadIdx.x; k < n_store; k += 32) {
+        const F x = transcript[tr_begin + k];
+        pool[1 + n0 + 2 * k] = x.re;
+        pool[2 + n0 + 2 * k] = x.im;
+    }
+    __syncwarp();
+    if (threadIdx.x != 0) return;
+    pool[0] = n0 + 2ull * n_store;
+    for (uint32_t k = 0; k < n_draw; ++k) st_f(chal + ci_begin + k, fs_draw(pool));
+}
+
+// The statement (include/virgo_b200.h): H("VPSTMT01" | circuit | u64 n_inputs | inputs root | u64 n_outputs | outputs root |
+// context[32]), 152 bytes. roots = {circuit, inputs, outputs} digests, 4 words each. Seeds the pool with it and copies it to
+// `out` (4 words).
+struct FsContext { uint64_t w[4]; };
+__global__ void k_fs_statement(const uint64_t* __restrict__ roots, uint64_t n_inputs, uint64_t n_outputs, FsContext ctx, uint64_t* pool,
+                               uint64_t* out) {
+    if (threadIdx.x != 0) return;
+    uint64_t m[19];
+    m[0] = 0x3130544d54535056ull;   // "VPSTMT01"
+#pragma unroll
+    for (int k = 0; k < 4; ++k) { m[1 + k] = roots[k]; m[6 + k] = roots[4 + k]; m[11 + k] = roots[8 + k]; m[15 + k] = ctx.w[k]; }
+    m[5] = n_inputs;
+    m[10] = n_outputs;
+    uint64_t d[4];
+    sha3_256_words(m, 19, d);
+#pragma unroll
+    for (int k = 0; k < 4; ++k) { pool[1 + k] = d[k]; out[k] = d[k]; }
+    pool[0] = 4;
+}
+
+// ------------------------------------------------------------------ K6f: a Fiat-Shamir sumcheck phase in ONE launch
+// k_sumcheck_phase with the challenges drawn inside: after round j's grid barrier block 0 reduces the partials, writes
+// (a, b, c) to the transcript, stores them in the pool and draws the round's challenge into chal[j - 1]; a second grid
+// barrier then releases the other blocks into round j + 1's fold, which needs that challenge. The tail rounds (block 0
+// alone) store and draw the same way behind a block barrier. The final claims are written like k_sumcheck_phase writes
+// them; storing them is the next k_fs_absorb_draw's job.
+// stamps (4 per round, block 0, %globaltimer): round start, own fold work done, polynomial reduced (grid rounds: after the
+// barrier), challenge drawn. The next round's start minus "drawn" is the release barrier.
+struct FsPhaseArgs {
+    uint64_t* pool;
+    F* chal;                     // = PhaseArgs::chal, writable
+    unsigned long long* stamps;  // 4 * n_rounds, may be null
+};
+VP_D void fs_stamp(unsigned long long* s, uint32_t j, int k) {
+    if (!s) return;
+    unsigned long long t;
+    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
+    s[4 * (j - 1) + k] = t;
+}
+
+__global__ void __launch_bounds__(256, 2) k_sumcheck_phase_fs(PhaseArgs p, FsPhaseArgs f) {
+    namespace cg = cooperative_groups;
+    cg::grid_group grid = cg::this_grid();
+    __shared__ F smem[3 * 32];
+    __shared__ uint32_t s_wend[128];
+    const uint32_t gtid = blockIdx.x * blockDim.x + threadIdx.x, gstride = gridDim.x * blockDim.x;
+    const bool stamp = blockIdx.x == 0 && threadIdx.x == 0;
+    F at = p.at_init ? *p.at_init : f_zero();  // add_term: meaningful in block 0 / thread 0 only
+    uint32_t j = 1;
+    // ---- grid rounds
+    for (; j <= p.n_rounds; ++j) {
+        const RoundDev R = p.rounds[j - 1];
+        if (R.work <= p.tail_work) break;
+        if (stamp) fs_stamp(f.stamps, j, 0);
+        const bool fold = j >= 2;
+        __syncthreads();
+        for (uint32_t i = threadIdx.x; i < R.n_tabs; i += blockDim.x) s_wend[i] = p.tabs[R.tab_begin + i].work_end;
+        __syncthreads();
+        const uint32_t ib = R.in_buf, ob = ib ^ 1;
+        const bool scale = j >= 2;
+        const F prev = scale ? ld_f_cg(f.chal + j - 2) : f_zero();   // drawn by block 0 in this launch: bypass L1
+        const FoldK rk = make_foldk(prev);
+        RoundAcc acc;
+        racc_init(acc);
+        if (fold) round_work<true, false>(acc, p.tabs + R.tab_begin, R.n_tabs, s_wend, p.bufV[ib], p.bufM[ib], p.bufA[ib],
+                                          p.bufV[ob], p.bufM[ob], p.bufA[ob], rk, gtid, gstride);
+        else round_work<false, false>(acc, p.tabs + R.tab_begin, R.n_tabs, s_wend, p.bufV[ib], p.bufM[ib], p.bufA[ib],
+                                      p.bufV[ob], p.bufM[ob], p.bufA[ob], rk, gtid, gstride);
+        F v[3];
+        racc_finish(acc, v);
+        block_sum<3>(v, smem);
+        F* part = p.partials + (size_t)(j & 1) * gridDim.x * 3;
+        if (threadIdx.x == 0) {
+            st_f(part + (size_t)blockIdx.x * 3 + 0, v[0]);
+            st_f(part + (size_t)blockIdx.x * 3 + 1, v[1]);
+            st_f(part + (size_t)blockIdx.x * 3 + 2, v[2]);
+            if (blockIdx.x == 0)
+                at = collapse_update<false>(at, p.cols + R.col_begin, R.n_cols, p.bufV[ib], p.bufM[ib], p.bufA[ib], fold,
+                                            scale, prev, rk, p.claims);
+        }
+        if (stamp) fs_stamp(f.stamps, j, 1);
+        grid.sync();
+        if (blockIdx.x == 0) {
+            F t[3] = {f_zero(), f_zero(), f_zero()};
+            for (uint32_t b = threadIdx.x; b < gridDim.x; b += blockDim.x) {
+                t[0] = f_add(t[0], ld_one<false>(part + (size_t)b * 3 + 0));
+                t[1] = f_add(t[1], ld_one<false>(part + (size_t)b * 3 + 1));
+                t[2] = f_add(t[2], ld_one<false>(part + (size_t)b * 3 + 2));
+            }
+            block_sum<3>(t, smem);
+            if (threadIdx.x == 0) {
+                const F o[3] = {t[0], f_sub(t[1], at), f_add(t[2], at)};
+                F* out = p.out_poly + 3 * (j - 1);
+                fs_stamp(f.stamps, j, 2);
+                for (int k = 0; k < 3; ++k) { st_f(out + k, o[k]); fs_store(f.pool, o[k]); }
+                st_f(f.chal + j - 1, fs_draw(f.pool));
+                fs_stamp(f.stamps, j, 3);
+            }
+        }
+        grid.sync();   // release: round j + 1 folds with the challenge just drawn
+    }
+    if (blockIdx.x != 0) return;
+    // ---- tail rounds: block 0 alone
+    for (; j <= p.n_rounds; ++j) {
+        const RoundDev R = p.rounds[j - 1];
+        if (stamp) fs_stamp(f.stamps, j, 0);
+        const bool fold = j >= 2;
+        __syncthreads();   // (also publishes the previous round's challenge to the block)
+        for (uint32_t i = threadIdx.x; i < R.n_tabs; i += blockDim.x) s_wend[i] = p.tabs[R.tab_begin + i].work_end;
+        __syncthreads();
+        const uint32_t ib = R.in_buf, ob = ib ^ 1;
+        const bool scale = j >= 2;
+        const F prev = scale ? ld_f_cg(f.chal + j - 2) : f_zero();
+        const FoldK rk = make_foldk(prev);
+        RoundAcc acc;
+        racc_init(acc);
+        if (fold) round_work<true, false>(acc, p.tabs + R.tab_begin, R.n_tabs, s_wend, p.bufV[ib], p.bufM[ib], p.bufA[ib],
+                                          p.bufV[ob], p.bufM[ob], p.bufA[ob], rk, threadIdx.x, blockDim.x);
+        else round_work<false, false>(acc, p.tabs + R.tab_begin, R.n_tabs, s_wend, p.bufV[ib], p.bufM[ib], p.bufA[ib],
+                                      p.bufV[ob], p.bufM[ob], p.bufA[ob], rk, threadIdx.x, blockDim.x);
+        F v[3];
+        racc_finish(acc, v);
+        if (stamp) fs_stamp(f.stamps, j, 1);
+        block_sum<3>(v, smem);
+        if (threadIdx.x == 0) {
+            at = collapse_update<false>(at, p.cols + R.col_begin, R.n_cols, p.bufV[ib], p.bufM[ib], p.bufA[ib], fold, scale, prev,
+                                        rk, p.claims);
+            const F o[3] = {v[0], f_sub(v[1], at), f_add(v[2], at)};
+            F* out = p.out_poly + 3 * (j - 1);
+            fs_stamp(f.stamps, j, 2);
+            for (int k = 0; k < 3; ++k) { st_f(out + k, o[k]); fs_store(f.pool, o[k]); }
+            st_f(f.chal + j - 1, fs_draw(f.pool));
+            fs_stamp(f.stamps, j, 3);
+        }
+    }
+    __syncthreads();  // the last round's table writes, the claims of collapsed tables and the last challenge
+    if (threadIdx.x == 0) st_f(p.add_term, at);
+    // ---- final claims (prover.cpp:494-521)
+    const F* V = p.bufV[p.fin_buf];
+    for (uint32_t i = threadIdx.x; i < p.n_fin; i += blockDim.x) {
+        const FinDesc fd = p.fins[i];
+        F c;
+        if (fd.from_claim >= 0) c = ld_one<false>(p.claims + fd.from_claim);
+        else {
+            const F v0 = fd.n_vals >= 1 ? ld_one<false>(V + fd.in_off) : f_zero();
+            if (p.n_rounds >= 1) {
+                const F v1 = fd.n_vals >= 2 ? ld_one<false>(V + fd.in_off + 1) : f_zero();
+                c = f_fold(v0, v1, ld_f_cg(f.chal + p.n_rounds - 1));
+            } else c = v0;
+        }
+        st_f(p.transcript + fd.out_idx, c);
+        if (p.keep && i == 0) st_f(p.keep, c);
+    }
+}
+
+}  // namespace vp

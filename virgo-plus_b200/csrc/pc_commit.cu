@@ -21,6 +21,7 @@
 // All arithmetic is the canonical F_{p^2} arithmetic of field.cuh: exact, hence bit-identical to the reference's
 // packed-AVX FFT whatever the butterfly order.
 #include "pc_commit.h"
+#include "keccak.cuh"
 
 #include <algorithm>
 #include <stdexcept>
@@ -263,55 +264,8 @@ __global__ void __launch_bounds__(256) k_pc_interleave(const F* __restrict__ eva
     for (uint32_t i = threadIdx.x; i < (2 * PC_SLICES) << PC_VOW_LEAVES_LOG; i += blockDim.x) pc_st(o + i, sh[i]);
 }
 
-// ---- SHA3-256 of a 64-byte block (my_hhash.h:27-33 -> XKCP SHA3_256; FIPS 202): one Keccak-f[1600] permutation
-__constant__ uint64_t PC_KECCAK_RC[24] = {
-    0x0000000000000001ULL, 0x0000000000008082ULL, 0x800000000000808aULL, 0x8000000080008000ULL, 0x000000000000808bULL,
-    0x0000000080000001ULL, 0x8000000080008081ULL, 0x8000000000008009ULL, 0x000000000000008aULL, 0x0000000000000088ULL,
-    0x0000000080008009ULL, 0x000000008000000aULL, 0x000000008000808bULL, 0x800000000000008bULL, 0x8000000000008089ULL,
-    0x8000000000008003ULL, 0x8000000000008002ULL, 0x8000000000000080ULL, 0x000000000000800aULL, 0x800000008000000aULL,
-    0x8000000080008081ULL, 0x8000000000008080ULL, 0x0000000080000001ULL, 0x8000000080008008ULL};
-VP_D uint64_t pc_rotl(uint64_t x, int n) { return (x << n) | (x >> (64 - n)); }
-// msg: 8 words in, digest: words 0..3 out
-VP_D void pc_sha3_64(const uint64_t (&msg)[8], uint64_t (&dig)[4]) {
-    uint64_t a[25];
-#pragma unroll
-    for (int i = 0; i < 25; ++i) a[i] = 0;
-#pragma unroll
-    for (int i = 0; i < 8; ++i) a[i] = msg[i];
-    a[8] = 0x06ULL;                      // domain suffix + first pad bit right after the 64 message bytes
-    a[16] = 0x8000000000000000ULL;       // last pad bit in the last byte of the 136-byte rate
-#pragma unroll 1
-    for (int round = 0; round < 24; ++round) {
-        uint64_t c0 = a[0] ^ a[5] ^ a[10] ^ a[15] ^ a[20], c1 = a[1] ^ a[6] ^ a[11] ^ a[16] ^ a[21],
-                 c2 = a[2] ^ a[7] ^ a[12] ^ a[17] ^ a[22], c3 = a[3] ^ a[8] ^ a[13] ^ a[18] ^ a[23],
-                 c4 = a[4] ^ a[9] ^ a[14] ^ a[19] ^ a[24];
-        const uint64_t d0 = c4 ^ pc_rotl(c1, 1), d1 = c0 ^ pc_rotl(c2, 1), d2 = c1 ^ pc_rotl(c3, 1), d3 = c2 ^ pc_rotl(c4, 1),
-                       d4 = c3 ^ pc_rotl(c0, 1);
-#pragma unroll
-        for (int j = 0; j < 25; j += 5) { a[j] ^= d0; a[j + 1] ^= d1; a[j + 2] ^= d2; a[j + 3] ^= d3; a[j + 4] ^= d4; }
-        // rho + pi
-        uint64_t b[25];
-        b[0] = a[0];
-        b[10] = pc_rotl(a[1], 1);   b[7] = pc_rotl(a[10], 3);   b[11] = pc_rotl(a[7], 6);   b[17] = pc_rotl(a[11], 10);
-        b[18] = pc_rotl(a[17], 15); b[3] = pc_rotl(a[18], 21);  b[5] = pc_rotl(a[3], 28);   b[16] = pc_rotl(a[5], 36);
-        b[8] = pc_rotl(a[16], 45);  b[21] = pc_rotl(a[8], 55);  b[24] = pc_rotl(a[21], 2);  b[4] = pc_rotl(a[24], 14);
-        b[15] = pc_rotl(a[4], 27);  b[23] = pc_rotl(a[15], 41); b[19] = pc_rotl(a[23], 56); b[13] = pc_rotl(a[19], 8);
-        b[12] = pc_rotl(a[13], 25); b[2] = pc_rotl(a[12], 43);  b[20] = pc_rotl(a[2], 62);  b[14] = pc_rotl(a[20], 18);
-        b[22] = pc_rotl(a[14], 39); b[9] = pc_rotl(a[22], 61);  b[6] = pc_rotl(a[9], 20);   b[1] = pc_rotl(a[6], 44);
-        // chi
-#pragma unroll
-        for (int j = 0; j < 25; j += 5) {
-            a[j] = b[j] ^ (~b[j + 1] & b[j + 2]);
-            a[j + 1] = b[j + 1] ^ (~b[j + 2] & b[j + 3]);
-            a[j + 2] = b[j + 2] ^ (~b[j + 3] & b[j + 4]);
-            a[j + 3] = b[j + 3] ^ (~b[j + 4] & b[j]);
-            a[j + 4] = b[j + 4] ^ (~b[j] & b[j + 1]);
-        }
-        a[0] ^= PC_KECCAK_RC[round];
-    }
-#pragma unroll
-    for (int i = 0; i < 4; ++i) dig[i] = a[i];
-}
+// ---- SHA3-256 of a 64-byte block (my_hhash.h:27-33 -> XKCP SHA3_256; FIPS 202): one Keccak-f[1600] permutation (keccak.cuh)
+VP_D void pc_sha3_64(const uint64_t (&msg)[8], uint64_t (&dig)[4]) { sha3_256_64(msg, dig); }
 
 // fri.cpp:97-126: leaf i = chain over the slices; slice 64 (the mask) is all zero for the GKR prover's zero mask
 __global__ void __launch_bounds__(128) k_pc_leaf_hash(const F* __restrict__ l_eval, uint32_t log_N, uint64_t* __restrict__ leaf, int mask_is_zero) {
@@ -610,16 +564,78 @@ static void pc_merkle(PcCommit* p, const F* eval, uint64_t* tree, cudaStream_t s
     pc_tree_levels(p, tree, half, st);
 }
 // the inner nodes of an array heap whose n_leaves (a power of two >= 2) leaves are in place
-static void pc_tree_levels(PcCommit* p, uint64_t* tree, uint32_t n_leaves, cudaStream_t st) {
+static int pc_tree_levels_raw(uint64_t* tree, uint32_t n_leaves, cudaStream_t st) {
+    int launches = 0;
     uint32_t lvl = n_leaves / 2;
     for (; lvl > 128; lvl >>= 1) {
         k_pc_merkle_level<<<(lvl + 127) / 128, 128, 0, st>>>(tree, lvl);
-        ++p->launches;
+        ++launches;
     }
     if (lvl >= 1) {
         k_pc_merkle_top<<<1, 128, 0, st>>>(tree, lvl);
-        ++p->launches;
+        ++launches;
     }
+    return launches;
+}
+static void pc_tree_levels(PcCommit* p, uint64_t* tree, uint32_t n_leaves, cudaStream_t st) {
+    p->launches += (uint64_t)pc_tree_levels_raw(tree, n_leaves, st);
+}
+
+// ---- Merkle root of a word vector (the statement digest, see pc_commit.h): leaf j = H(words [8j, 8j + 8)), zero past the
+// end. One thread per leaf; a block of 128 leaves then climbs min(7, log2 leaves) levels in shared memory and leaves its
+// subtree root at its place in the array heap, so that k_pc_merkle_level / k_pc_merkle_top only see the upper levels
+// (a tree of 2^21 leaves: 8 launches instead of 16). The per-level hashes are the same ones either way.
+__global__ void __launch_bounds__(128) k_pc_vec_leaves(const uint64_t* __restrict__ words, size_t n_words, uint32_t log_leaves,
+                                                       uint32_t climb, uint64_t* __restrict__ tree) {
+    __shared__ uint64_t sh[128][4];
+    const uint32_t t = threadIdx.x, width = 1u << climb;
+    const size_t leaf = (size_t)blockIdx.x * width + t;
+    if (t < width) {
+        uint64_t msg[8], h[4];
+#pragma unroll
+        for (int k = 0; k < 8; ++k) {
+            const size_t w = leaf * 8 + (size_t)k;
+            msg[k] = w < n_words ? words[w] : 0;
+        }
+        pc_sha3_64(msg, h);
+#pragma unroll
+        for (int k = 0; k < 4; ++k) sh[t][k] = h[k];
+    }
+    __syncthreads();
+    for (uint32_t w = width / 2; w >= 1; w >>= 1) {
+        uint64_t msg[8], h[4];
+        if (t < w) {
+#pragma unroll
+            for (int k = 0; k < 4; ++k) { msg[k] = sh[2 * t][k]; msg[4 + k] = sh[2 * t + 1][k]; }
+            pc_sha3_64(msg, h);
+        }
+        __syncthreads();
+        if (t < w)
+#pragma unroll
+            for (int k = 0; k < 4; ++k) sh[t][k] = h[k];
+        __syncthreads();
+    }
+    if (t < 4) tree[(((size_t)1 << (log_leaves - climb)) + blockIdx.x) * 4 + t] = sh[0][t];
+}
+
+static uint32_t pc_vector_log_leaves(size_t n_words) {
+    uint32_t k = 0;
+    while (((size_t)8 << k) < n_words) ++k;
+    return k;
+}
+size_t pc_vector_root_scratch(size_t n_words) {   // nodes 0 .. 2^(k - climb + 1) - 1 of the heap: the leaf level itself is never stored
+    const uint32_t k = pc_vector_log_leaves(n_words);
+    return (size_t)64 << (k - std::min<uint32_t>(k, 7));
+}
+int pc_vector_root(const uint64_t* d_words, size_t n_words, uint64_t* d_scratch, uint8_t* d_root, cudaStream_t st) {
+    const uint32_t k = pc_vector_log_leaves(n_words), climb = std::min<uint32_t>(k, 7);
+    if (k - climb > 31) throw std::runtime_error("vector root: more than 2^38 leaves");
+    const size_t blocks = (size_t)1 << (k - climb);
+    k_pc_vec_leaves<<<(unsigned)blocks, 128, 0, st>>>(d_words, n_words, k, climb, d_scratch);
+    int launches = 1 + pc_tree_levels_raw(d_scratch, (uint32_t)blocks, st);
+    PCK(cudaGetLastError());
+    PCK(cudaMemcpyAsync(d_root, d_scratch + 4, 32, cudaMemcpyDeviceToDevice, st));
+    return launches;
 }
 
 float pc_commit(PcCommit* p, const F* d_array, size_t n_valid, cudaStream_t st, uint8_t root[32]) {

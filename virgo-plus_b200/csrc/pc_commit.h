@@ -48,4 +48,12 @@ void pc_fri_export(PcCommit* p, cudaStream_t stream, int lvl, F* code, uint8_t* 
 void pc_export_interleaved(PcCommit* p, cudaStream_t stream, int which, F* out);
 uint64_t pc_launches(const PcCommit* p);
 
+// Merkle root R of a vector of n_words little-endian words on the device (the statement digest of the Fiat-Shamir mode,
+// include/virgo_b200.h): the words zero-padded to 2^k 64-byte leaves (2^k the smallest power of two >= max(1, ceil(n_words /
+// 8))), leaf j = SHA3-256(block j), an array-heap tree with node = SHA3-256(left | right), root = node 1 (with one leaf: that
+// leaf's hash). d_scratch: pc_vector_root_scratch(n_words) bytes; the 32-byte root goes to d_root (device). Asynchronous on
+// `st`; returns the number of kernel launches.
+size_t pc_vector_root_scratch(size_t n_words);
+int pc_vector_root(const uint64_t* d_words, size_t n_words, uint64_t* d_scratch, uint8_t* d_root, cudaStream_t st);
+
 }  // namespace vp
