@@ -318,6 +318,22 @@ int vp_verify_fs_bound(vp_ctx* ctx, const uint8_t context[32], const vp_F* outpu
                        int* accept, int* fail_code, int* fail_layer);
 int vp_fs_round_stamps(vp_ctx* ctx, unsigned long long* out, size_t cap, size_t* n_rounds);
 
+/* B independent statement-bound proofs over this context's circuit (template + K, as the context was created), in one pass.
+ * inputs: B * vp_circuit_num_inputs values, statement-major, read with vp_circuit_set_inputs' rules (0 <= x < p; others VP_ERR_ARG).
+ * contexts: B * 32 bytes. transcripts: B * n_tr (cap >= that), statement-major; challenges (may be NULL): B * n_chal;
+ * statements (may be NULL): B * 32 bytes.
+ * Proof b is, bit for bit, vp_prove_fs_bound on this circuit with inputs b and context b.
+ * The context's resident inputs, values, transcript and challenges are not changed.
+ * VP_ERR_ASSERT: an is_assert gate is non-zero in some statement; vp_last_error names the first such b.
+ * Sharded contexts: VP_ERR_ARG.
+ * The statements share the circuit's wiring, plans and digest and one sequence of launches: every kernel of the proof runs
+ * all B statements at once (statement b in blockIdx.z), so the launch count does not grow with B (the sumcheck phase
+ * kernel, a cooperative launch, runs in chunks of statements when B exceeds the blocks that can be co-resident). The
+ * per-statement buffers live in a slab kept on the context for the next call (grown when needed, freed by vp_destroy).
+ * vp_last_prove_ms / vp_last_prove_launches describe the batch; vp_fs_round_stamps are statement 0's. */
+int vp_prove_fs_bound_batch(vp_ctx* ctx, size_t B, const uint64_t* inputs, size_t n_inputs, const uint8_t* contexts,
+                            vp_F* transcripts, size_t cap, vp_F* challenges, size_t ch_cap, uint8_t* statements);
+
 /* Self-test of the device-only arithmetic paths of csrc/field.cuh (inline-PTX carry chains, mul.wide / mad.wide):
    runs one routine on n caller-provided operand triples and returns the results, so that tests can feed edge values
    (0, 1, p-1, p, limb boundaries) and compare with big-integer arithmetic.  op: 0 weak fold a + c*(b-a); 1 the same for

@@ -135,6 +135,7 @@ def _declare(L):
     L.vp_verify_fs_bound.argtypes = [vp, C.c_char_p, vp, C.c_size_t, vp, C.c_size_t, C.POINTER(C.c_int), C.POINTER(C.c_int),
                                      C.POINTER(C.c_int)]
     L.vp_fs_round_stamps.argtypes = [vp, vp, C.c_size_t, C.POINTER(C.c_size_t)]
+    L.vp_prove_fs_bound_batch.argtypes = [vp, C.c_size_t, vp, C.c_size_t, vp, vp, C.c_size_t, vp, C.c_size_t, vp]
     L.vp_get_transcript.argtypes = [vp, vp, C.c_size_t]
     L.vp_last_prove_ms.argtypes = [vp]
     L.vp_last_prove_ms.restype = C.c_float
@@ -704,6 +705,35 @@ class Prover:
         st = np.zeros(32, np.uint8)
         _ck(lib().vp_prove_fs_bound(self.h, _context(context), _ptr(tr), len(tr), _ptr(ch), len(ch), _ptr(st)))
         return tr, ch, st.tobytes()
+
+    def prove_fs_bound_batch(self, inputs, contexts):
+        """B independent statement-bound proofs of this circuit in one pass: inputs [B, n_inputs], contexts B `bytes` of 32
+        or a [B, 32] uint8 array -> (transcripts [B, n_tr], challenges [B, n_chal], statements [B, 32] uint8); proof b ==
+        prove_fs_bound(contexts[b]) after set_inputs(inputs[b]). The resident inputs and values are not changed."""
+        n_in = self.circuit.layer_size(0) * self.circuit.instances
+        inputs = np.asarray(inputs)
+        if inputs.ndim != 2 or inputs.shape[1] != n_in or inputs.shape[0] < 1:
+            raise ValueError(f"inputs must be a [B, {n_in}] array with B >= 1, got shape {inputs.shape}")
+        if inputs.dtype.kind not in "ui":
+            raise ValueError(f"inputs must be integers, got {inputs.dtype}")
+        B = inputs.shape[0]
+        if isinstance(contexts, np.ndarray):
+            if contexts.dtype != np.uint8 or contexts.shape != (B, 32):
+                raise ValueError(f"contexts must be a [{B}, 32] uint8 array, got {contexts.dtype} {contexts.shape}")
+            ctx = np.ascontiguousarray(contexts)
+        else:
+            contexts = list(contexts)
+            if len(contexts) != B:
+                raise ValueError(f"{B} statements need {B} contexts, got {len(contexts)}")
+            ctx = np.frombuffer(b"".join(_context(c) for c in contexts), np.uint8).reshape(B, 32)
+        inputs = np.ascontiguousarray(inputs, dtype=np.uint64)
+        n_tr, n_ch = self.circuit.transcript_len, self.circuit.challenge_count
+        tr = np.zeros((B, n_tr), F_DTYPE)
+        ch = np.zeros((B, n_ch), F_DTYPE)
+        st = np.zeros((B, 32), np.uint8)
+        _ck(lib().vp_prove_fs_bound_batch(self.h, B, _ptr(inputs), inputs.size, _ptr(ctx), _ptr(tr), tr.size, _ptr(ch), ch.size,
+                                          _ptr(st)))
+        return tr, ch, st
 
     def verify_fs_bound(self, context, outputs, transcript):
         """(accept, fail_code, fail_layer) of a statement-bound proof for the claimed outputs and this context's inputs"""

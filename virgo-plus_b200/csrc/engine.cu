@@ -724,6 +724,7 @@ struct XchgLane {
     DBuf<F> d_sc;                        // this rank's partial scalars of the phase in flight (zero between phases)
     DBuf<unsigned int> ticket;
 };
+struct StatementAssert { uint32_t stmt; unsigned int flag; };   // a batch's first statement with a failed assert gate
 struct Engine {
     Circuit C;
     int device = 0;
@@ -1042,12 +1043,46 @@ struct Engine {
     int cap_phase_fs = 0;
     void fs_alloc();
     void fs_begin();
-    void statement_async(const uint8_t context[32], const F* d_outputs);
+    void statement_async(const uint8_t context[32], const F* d_outputs, const uint64_t* d_contexts = nullptr);
     void circuit_digest_async();
     void prove_fs_device(const uint8_t* seed, F* tr_out, F* ch_out);
     void launch_phase_kernel_fs(const SumcheckPlan& P, uint32_t ci, F* keep, const F* at_init, uint32_t tr_rounds, size_t stamp_round);
+    // A batch of statements (vp_prove_fs_bound_batch): the Fiat-Shamir path runs n_stmt statements at once, statement b
+    // in blockIdx.z == b with its working set sstride bytes after statement b - 1's (kernels.cuh, stmt_at). A single proof
+    // is n_stmt = 1, sstride = 0 on the context's own buffers.
+    uint32_t n_stmt = 1;
+    size_t sstride = 0;
+    dim3 sgrid(uint32_t x, uint32_t y = 1) const { return dim3(x, y, n_stmt); }
+    int grid_b(uint32_t work, int cap) const { return grid_for(work, std::max(1, cap / (int)n_stmt)); }   // x-width of one statement
+    void memset_stmts(void* p, size_t bytes) {   // zero `bytes` at p in every statement's working set
+        if (n_stmt == 1) CK(cudaMemsetAsync(p, 0, bytes, stream));
+        else CK(cudaMemset2DAsync(p, sstride, 0, bytes, n_stmt, stream));
+    }
+    void copy_stmts_to_host(void* dst, size_t dpitch, const void* src, size_t bytes) {   // statement b's bytes to dst + b * dpitch
+        if (n_stmt == 1) CK(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToHost, stream));
+        else CK(cudaMemcpy2DAsync(dst, dpitch, src, sstride, bytes, n_stmt, cudaMemcpyDeviceToHost, stream));
+    }
+    // The batch's own buffers, kept for the next batch and grown when needed: per statement a copy of every buffer the
+    // Fiat-Shamir path writes (one slab, `stride` bytes per statement), and the layer values, inputs and the descriptors that
+    // point into them (phase-2 tables: src_val; Liu eq tables: the eq region) for n_stmt * K instances.
+    struct FsSlab {
+        uint32_t cap = 0;                  // statements it holds
+        size_t stride = 0;
+        DBuf<uint8_t> mem;
+        size_t o_buf[6] = {0}, o_chal = 0, o_tr = 0, o_scal = 0, o_claims = 0, o_partials = 0, o_counter = 0, o_rowpart = 0, o_eq = 0,
+               o_hs = 0, o_pool = 0, o_stmt = 0;
+        std::vector<DBuf<F>> val;
+        DBuf<F*> valptr;
+        DBuf<uint64_t> inputs, contexts, root_scratch;
+        std::vector<DBuf<P2Table>> p2_tabs;
+        std::vector<DBuf<EqTab>> liu_eqtabs;
+        std::vector<std::pair<void*, size_t>> views;   // statement 0's buffers in the slab (the context's while swapped)
+    } slab;
+    const uint64_t* d_circuit_digest = nullptr;   // the context's circuit digest (d_stmt[0 .. 4), shared by a batch)
+    void slab_reserve(uint32_t B);
+    void slab_swap();   // exchanges the context's buffers with the slab's (an involution)
     void fs_absorb_draw(uint32_t tr_begin, uint32_t n_store, uint32_t ci_begin, uint32_t n_draw) {
-        k_fs_absorb_draw<<<1, 32, 0, stream>>>(d_fs_pool.p, d_tr.p, tr_begin, n_store, d_chal.p, ci_begin, n_draw);
+        k_fs_absorb_draw<<<sgrid(1), 32, 0, stream>>>(d_fs_pool.p, d_tr.p, tr_begin, n_store, d_chal.p, ci_begin, n_draw, sstride);
         ++launches;
     }
     std::vector<F> h_chal;   // host copy of the challenges: the pass kernel gets their limbs through its parameters
@@ -1789,24 +1824,26 @@ void Engine::load_inputs_chunked(const uint64_t* host, size_t cnt, bool local) {
     evaluated = false;
 }
 
+// A batch of n_stmt statements (unsharded) is one replicated circuit of n_stmt * K instances here.
 void Engine::evaluate() {
     const uint32_t S0 = (uint32_t)C.layers[0].size;
-    CK(cudaMemsetAsync(d_counter.p + 1, 0, sizeof(unsigned int), stream));
+    memset_stmts(d_counter.p + 1, sizeof(unsigned int));
     const int nc = pending_chunks > 0 ? pending_chunks : 1;
     for (int c = 0; c < nc; ++c) {
-        const uint32_t ca = pending_chunks > 0 ? chunk_lo[c] : k_lo, cb = pending_chunks > 0 ? chunk_hi[c] : k_hi;
+        const uint32_t ca = pending_chunks > 0 ? chunk_lo[c] : k_lo, cb = pending_chunks > 0 ? chunk_hi[c] : k_hi * n_stmt;
         if (pending_chunks > 0) CK(cudaStreamWaitEvent(stream, ev_chunk[c], 0));
         if (cb > ca) {
             k_load_inputs<<<cdiv(std::max<uint32_t>((cb - ca) * S0, 1), 256), 256, 0, stream>>>(d_inputs.p, val[0].p, ca * S0, cb * S0);
             ++launches;
         }
         for (int i = 1; i < n; ++i) {
-            const uint32_t a = std::max(ca, ev_lo[i]), b = std::min(cb, ev_hi[i]);
+            const uint32_t a = std::max(ca, ev_lo[i]), b = std::min(cb, ev_hi[i] * n_stmt);
             if (b <= a) continue;
             const uint32_t gb = a * L[i].S, ge = b * L[i].S, tot = ge - gb;
             size_t h = prof_begin(KC_EVAL);
             k_eval_layer<<<grid_for(std::max<uint32_t>(tot, 1), cap_eval), 256, 0, stream>>>(L[i].G, L[i].S, K, i, d_valptr.p, d_sizes.p,
-                                                                                            val[i].p, d_counter.p + 1, gb, ge, values_real ? 1 : 0);
+                                                                                            val[i].p, d_counter.p + 1, gb, ge, values_real ? 1 : 0,
+                                                                                            sstride);
             prof_end(h, (double)tot * (16.0 + 32.0 + 11.0 / K));  // out + two operand gathers (+ amortised wiring)
             ++launches;
         }
@@ -1818,7 +1855,7 @@ void Engine::evaluate() {
 
 void Engine::run_eq(uint32_t first, uint32_t count) {
     if (!count) return;
-    k_eq_build<<<count, 1024, 0, stream>>>(d_eqb.p + first, d_chal.p, d_eq.p + eq_off);
+    k_eq_build<<<sgrid(count), 1024, 0, stream>>>(d_eqb.p + first, d_chal.p, d_eq.p + eq_off, sstride);
     ++launches;
 }
 
@@ -1827,8 +1864,8 @@ void Engine::run_eq(uint32_t first, uint32_t count) {
 void Engine::run_dot_eq(const F* X, uint32_t S, EqTab eq, F* out, bool local_only) {
     const uint32_t begin = ko_lo * S, end = ko_hi * S;
     F* dst = (world > 1 && !local_only) ? d_send.p : out;
-    k_dot_eq<<<grid_for(std::max<uint32_t>(end - begin, 1), cap_dot), 256, 0, stream>>>(X, begin, end, eq, dst, d_partials.p,
-                                                                                       d_counter.p);
+    k_dot_eq<<<sgrid(grid_b(std::max<uint32_t>(end - begin, 1), cap_dot)), 256, 0, stream>>>(X, begin, end, eq, dst, d_partials.p,
+                                                                                            d_counter.p, sstride);
     ++launches;
     if (world > 1 && !local_only) {
         NCK(g_nccl.AllGather(d_send.p, d_recv.p, 2, /*ncclUint64*/ 5, comm, stream));
@@ -1857,25 +1894,26 @@ void Engine::do_init_phase1(int i) {
     const uint64_t work = (uint64_t)D.p1_items.n * (k1 - k0);
     size_t h = prof_begin(KC_INIT1);
     if (lane_init && K >= 8 && k1 - k0 >= 4 && n <= 64 && !p1_old) {   // template-major: an item of the template x 4 instances per thread
-        dim3 grid(cdiv(std::max<uint32_t>((uint32_t)D.p1_items.n, 1), 256), cdiv(k1 - k0, 4));
+        dim3 grid(cdiv(std::max<uint32_t>((uint32_t)D.p1_items.n, 1), 256), cdiv(k1 - k0, 4), n_stmt);
         k_init_phase1_real_tm<4><<<grid, 256, 0, stream>>>(
             D.p1_items.p, (uint32_t)D.p1_items.n, csr, S_pre, D.S, K, eqtab(0, C.bit_length(i)), d_chal.p + D.ci_assert,
             d_valptr.p, d_sizes.p, D.c.p, val[i - 1].p, bufV[0].p + D.ph1.tab_off[0], bufM[0].p + D.ph1.tab_off[0],
-            bufA[0].p + D.ph1.tab_off[0], d_rowpart.p, D.p1_nslots, direct_v ? 0 : 1, (uint32_t)i, D.ph1.maps[0], k0, k1);
+            bufA[0].p + D.ph1.tab_off[0], d_rowpart.p, D.p1_nslots, direct_v ? 0 : 1, (uint32_t)i, D.ph1.maps[0], k0, k1, sstride);
     } else if (lane_init && work < 0xffffffffull && n <= 64)
-        k_init_phase1_real<<<grid_for((uint32_t)std::min<uint64_t>(work, 0xffffffffu), cap_p1il), 256, 0, stream>>>(
+        k_init_phase1_real<<<sgrid(grid_b((uint32_t)std::min<uint64_t>(work, 0xffffffffu), cap_p1il)), 256, 0, stream>>>(
             D.p1_items.p, (uint32_t)D.p1_items.n, csr, S_pre, D.S, K, eqtab(0, C.bit_length(i)), d_chal.p + D.ci_assert,
             d_valptr.p, d_sizes.p, D.c.p, val[i - 1].p, bufV[0].p + D.ph1.tab_off[0], bufM[0].p + D.ph1.tab_off[0],
-            bufA[0].p + D.ph1.tab_off[0], d_rowpart.p, D.p1_nslots, D.ph1.maps[0], direct_v ? 0 : 1, k0, k1, (uint32_t)i);
+            bufA[0].p + D.ph1.tab_off[0], d_rowpart.p, D.p1_nslots, D.ph1.maps[0], direct_v ? 0 : 1, k0, k1, (uint32_t)i, sstride);
     else
-    k_init_phase1<<<grid_for((uint32_t)std::min<uint64_t>(work, 0xffffffffu), cap_p1), 256, 0, stream>>>(
+    k_init_phase1<<<sgrid(grid_b((uint32_t)std::min<uint64_t>(work, 0xffffffffu), cap_p1)), 256, 0, stream>>>(
         D.p1_items.p, (uint32_t)D.p1_items.n, csr, S_pre, D.S, K, eqtab(0, C.bit_length(i)), d_chal.p + D.ci_assert,
         d_valptr.p, d_sizes.p, D.c.p, val[i - 1].p, bufV[0].p + D.ph1.tab_off[0], bufM[0].p + D.ph1.tab_off[0],
-        bufA[0].p + D.ph1.tab_off[0], d_rowpart.p, D.p1_nslots, D.ph1.maps[0], direct_v ? 0 : 1, k0, k1);
+        bufA[0].p + D.ph1.tab_off[0], d_rowpart.p, D.p1_nslots, D.ph1.maps[0], direct_v ? 0 : 1, k0, k1, sstride);
     if (D.p1_long.n && k1 > k0) {
-        k_combine_phase1<<<grid_for((uint32_t)(D.p1_long.n * (k1 - k0)), cap_comb), 256, 0, stream>>>(
+        k_combine_phase1<<<sgrid(grid_b((uint32_t)(D.p1_long.n * (k1 - k0)), cap_comb)), 256, 0, stream>>>(
             D.p1_long.p, (uint32_t)D.p1_long.n, S_pre, K, val[i - 1].p, bufV[0].p + D.ph1.tab_off[0],
-            bufM[0].p + D.ph1.tab_off[0], bufA[0].p + D.ph1.tab_off[0], d_rowpart.p, D.p1_nslots, D.ph1.maps[0], direct_v ? 0 : 1, k0, k1);
+            bufM[0].p + D.ph1.tab_off[0], bufA[0].p + D.ph1.tab_off[0], d_rowpart.p, D.p1_nslots, D.ph1.maps[0], direct_v ? 0 : 1, k0, k1,
+            sstride);
         ++launches;
     }
     // per output this rank holds: V read + 3 table writes; per gate it visits: one gathered operand
@@ -1903,21 +1941,21 @@ void Engine::do_init_phase2(int i) {
             const uint32_t ng = (D.S >> eqg.fh) + 2, nu = (S_pre >> equ.fh) + 2;
             if (K >= 8 && (uint64_t)ng * nu <= 64 && (uint64_t)K * ng * nu <= d_hs.n && !getenv_no_hs) {
                 H = HsTab{d_hs.p, ng, nu};
-                k_p2_hs<<<grid_for(K * ng * nu, cap_dot), 256, 0, stream>>>(eqg, equ, D.S, S_pre, K, ng, nu, d_hs.p);
+                k_p2_hs<<<sgrid(grid_b(K * ng * nu, cap_dot)), 256, 0, stream>>>(eqg, equ, D.S, S_pre, K, ng, nu, d_hs.p, sstride);
                 ++launches;
             }
-            k_init_phase2_v2<<<grid_for((uint32_t)work, cap_p2v2), 256, 0, stream>>>(
+            k_init_phase2_v2<<<sgrid(grid_b((uint32_t)work, cap_p2v2)), 256, 0, stream>>>(
                 D.p2_items.p, (uint32_t)D.p2_items.n, D.p2_tabs.p, csr, S_pre, D.S, K, eqg, equ, d_chal.p + D.ci_assert,
-                Vu, bufV[0].p, bufM[0].p, bufA[0].p, d_rowpart.p, D.p2_nslots, kk0, kk1, H);
+                Vu, bufV[0].p, bufM[0].p, bufA[0].p, d_rowpart.p, D.p2_nslots, kk0, kk1, H, sstride);
         }
         else
-        k_init_phase2<<<grid_for((uint32_t)std::min<uint64_t>(work, 0xffffffffu), cap_p2), 256, 0, stream>>>(
+        k_init_phase2<<<sgrid(grid_b((uint32_t)std::min<uint64_t>(work, 0xffffffffu), cap_p2)), 256, 0, stream>>>(
             D.p2_items.p, (uint32_t)D.p2_items.n, D.p2_tabs.p, csr, S_pre, D.S, K, eqg, equ, d_chal.p + D.ci_assert,
-            Vu, bufV[0].p, bufM[0].p, bufA[0].p, d_rowpart.p, D.p2_nslots, kk0, kk1);
+            Vu, bufV[0].p, bufM[0].p, bufA[0].p, d_rowpart.p, D.p2_nslots, kk0, kk1, sstride);
         if (D.p2_long.n && kk1 > kk0) {
-            k_combine_phase2<<<grid_for((uint32_t)(D.p2_long.n * (kk1 - kk0)), cap_comb), 256, 0, stream>>>(
+            k_combine_phase2<<<sgrid(grid_b((uint32_t)(D.p2_long.n * (kk1 - kk0)), cap_comb)), 256, 0, stream>>>(
                 D.p2_long.p, (uint32_t)D.p2_long.n, D.p2_tabs.p, K, bufV[0].p, bufM[0].p, bufA[0].p, d_rowpart.p, D.p2_nslots, kk0,
-                kk1);
+                kk1, sstride);
             ++launches;
         }
         double rows2 = D.p2_out_entries;   // table entries this rank holds
@@ -1931,11 +1969,11 @@ void Engine::do_init_phase2(int i) {
     if (D.n_unary > 0 && k1 > k0) {
         CsrUnary un{D.un_g0.p, D.un_u0.p, D.un_ty.p, D.n_unary};
         const uint64_t tot = (uint64_t)D.n_unary * (k1 - k0);
-        k_phase2_unary<<<grid_for((uint32_t)std::min<uint64_t>(tot, 0xffffffffu), cap_un), 256, 0, stream>>>(
+        k_phase2_unary<<<sgrid(grid_b((uint32_t)std::min<uint64_t>(tot, 0xffffffffu), cap_un)), 256, 0, stream>>>(
             un, S_pre, D.S, K, eqg, equ, d_chal.p + D.ci_assert, Vu, D.c.p, scal(SC_UNARY), d_partials.p,
-            d_counter.p, k0, k1);
+            d_counter.p, k0, k1, sstride);
         ++launches;
-    } else CK(cudaMemsetAsync(scal(SC_UNARY), 0, sizeof(F), stream));
+    } else memset_stmts(scal(SC_UNARY), sizeof(F));
 }
 
 void Engine::do_init_liu(int i, bool write_a) {
@@ -1959,16 +1997,16 @@ void Engine::do_init_liu(int i, bool write_a) {
     }
     if (K >= 8 && lk1 - lk0 >= 8 && !liu_old) {   // template-major: one thread per template entry, a chunk of instances each
         const uint32_t k_chunk = 8;
-        dim3 grid(cdiv(S_pre, 256), cdiv(lk1 - lk0, k_chunk));
+        dim3 grid(cdiv(S_pre, 256), cdiv(lk1 - lk0, k_chunk), n_stmt);
         k_init_liu_tm<<<grid, 256, 0, stream>>>(D.liu_off.p, D.liu_perm.p, D.liu_ent.p, eq_off ? D.liu_eqtabs_b.p : D.liu_eqtabs.p, S_pre, K, k_chunk,
                                                eqtab(reg_u, C.bit_length(i - 1)), d_chal.p + D.ci_sig, val[i - 1].p, bufV[0].p + D.ph3.tab_off[0],
                                                bufM[0].p + D.ph3.tab_off[0], bufA[0].p + D.ph3.tab_off[0], write_a ? 1 : 0, on_lane1 ? 1 : 0, direct_v ? 0 : 1,
-                                               D.ph3.maps[0], lk0, lk1);
+                                               D.ph3.maps[0], lk0, lk1, sstride);
     } else
-    k_init_liu<<<grid_for(std::max<uint32_t>(n_local, 1), cap_liu), 256, 0, stream>>>(
+    k_init_liu<<<sgrid(grid_b(std::max<uint32_t>(n_local, 1), cap_liu)), 256, 0, stream>>>(
         D.liu_off.p, world == 1 ? D.liu_perm.p : nullptr, D.liu_ent.p, eq_off ? D.liu_eqtabs_b.p : D.liu_eqtabs.p, S_pre, K, eqtab(reg_u, C.bit_length(i - 1)), d_chal.p + D.ci_sig, val[i - 1].p,
         bufV[0].p + D.ph3.tab_off[0], bufM[0].p + D.ph3.tab_off[0], bufA[0].p + D.ph3.tab_off[0], D.ph3.maps[0], n_local,
-        write_a ? 1 : 0, on_lane1 ? 1 : 0, direct_v ? 0 : 1);
+        write_a ? 1 : 0, on_lane1 ? 1 : 0, direct_v ? 0 : 1, sstride);
     prof_end(h, (double)n_local * ((write_a ? 64.0 : 48.0) - (direct_v ? 32.0 : 0.0)));
     ++launches;
 }
@@ -2670,14 +2708,125 @@ void Engine::fs_alloc() {
     for (int i = 1; i < n; ++i) rounds += (size_t)(2 * C.bit_length(i - 1) + std::max(L[i].max_dad_bl, 0));
     d_fs_stamps.alloc(4 * std::max<size_t>(rounds, 1));
     d_stmt.alloc(16);
+    d_circuit_digest = d_stmt.p;
 }
 void Engine::fs_begin() {
     leave();
     fs_alloc();
-    CK(cudaMemsetAsync(d_chal.p, 0, (n_chal + 1) * sizeof(F), stream));   // unused challenge slots are zero
-    h_chal.assign(n_chal, f_zero());
+    memset_stmts(d_chal.p, (n_chal + 1) * sizeof(F));   // unused challenge slots are zero
+    if (n_stmt == 1) h_chal.assign(n_chal, f_zero());
     evaluate();
-    check_assert_flag();
+    if (n_stmt == 1) {
+        check_assert_flag();
+        return;
+    }
+    // the first statement with a failed assert gate
+    std::vector<unsigned int> flags(n_stmt);
+    copy_stmts_to_host(flags.data(), sizeof(unsigned int), d_counter.p + 1, sizeof(unsigned int));
+    CK(cudaStreamSynchronize(stream));
+    for (uint32_t b = 0; b < n_stmt; ++b)
+        if (flags[b]) throw StatementAssert{b, flags[b]};
+}
+
+// Batch slab: per statement a copy of every buffer below, in this order, each 256-byte aligned (slab_swap's order).
+void Engine::slab_reserve(uint32_t B) {
+    if (slab.cap >= B) return;
+    size_t off = 0;
+    auto put = [&](size_t bytes) { const size_t o = off; off += (bytes + 255) & ~(size_t)255; return o; };
+    for (int b = 0; b < 2; ++b) {
+        slab.o_buf[3 * b] = put(bufV[b].n * sizeof(F));
+        slab.o_buf[3 * b + 1] = put(bufM[b].n * sizeof(F));
+        slab.o_buf[3 * b + 2] = put(bufA[b].n * sizeof(F));
+    }
+    slab.o_chal = put(d_chal.n * sizeof(F));
+    slab.o_tr = put(d_tr.n * sizeof(F));
+    slab.o_scal = put(d_scal.n * sizeof(F));
+    slab.o_claims = put(d_claims.n * sizeof(F));
+    slab.o_partials = put(d_partials.n * sizeof(F));
+    slab.o_counter = put(d_counter.n * sizeof(unsigned int));
+    slab.o_rowpart = put(d_rowpart.n * sizeof(F));
+    slab.o_eq = put(eq_set_entries * sizeof(F));
+    slab.o_hs = put(d_hs.n * sizeof(F));
+    slab.o_pool = put(d_fs_pool.n * sizeof(uint64_t));
+    slab.o_stmt = put(d_stmt.n * sizeof(uint64_t));
+    slab.cap = 0;
+    slab.stride = off;
+    slab.mem.alloc((size_t)B * off);
+    CK(cudaMemsetAsync(slab.mem.p, 0, (size_t)B * off, stream));   // the grid-sum tickets start at zero
+    slab.val.resize(n);
+    std::vector<F*> h_ptr(n);
+    for (int i = 0; i < n; ++i) {
+        slab.val[i].alloc((size_t)B * C.layer_size(i));
+        h_ptr[i] = slab.val[i].p;
+    }
+    slab.valptr.upload(h_ptr, stream);
+    slab.inputs.alloc((size_t)B * C.layer_size(0));
+    slab.contexts.alloc((size_t)4 * B);
+    // descriptors that point into the context's values / eq tables, rebased on the slab's
+    slab.p2_tabs.resize(n);
+    slab.liu_eqtabs.resize(n);
+    const uintptr_t eq0 = reinterpret_cast<uintptr_t>(d_eq.p), eq1 = reinterpret_cast<uintptr_t>(slab.mem.p + slab.o_eq);
+    for (int i = 1; i < n; ++i) {
+        std::vector<P2Table> t = L[i].h_p2;
+        for (P2Table& x : t)
+            for (int l = 0; l < n; ++l)
+                if (x.src_val == val[l].p) { x.src_val = slab.val[l].p; break; }
+        slab.p2_tabs[i].upload(t, stream);
+        std::vector<EqTab> e(L[i].liu_eqtabs.n);
+        if (!e.empty()) CK(cudaMemcpy(e.data(), L[i].liu_eqtabs.p, e.size() * sizeof(EqTab), cudaMemcpyDeviceToHost));
+        for (EqTab& x : e) {
+            x.f = reinterpret_cast<const F*>(reinterpret_cast<uintptr_t>(x.f) - eq0 + eq1);
+            x.s = reinterpret_cast<const F*>(reinterpret_cast<uintptr_t>(x.s) - eq0 + eq1);
+        }
+        slab.liu_eqtabs[i].upload(e, stream);
+    }
+    // statement 0's views of the slab, in slab_swap's order
+    uint8_t* const m = slab.mem.p;
+    slab.views.clear();
+    for (int b = 0; b < 2; ++b) {
+        slab.views.push_back({m + slab.o_buf[3 * b], bufV[b].n});
+        slab.views.push_back({m + slab.o_buf[3 * b + 1], bufM[b].n});
+        slab.views.push_back({m + slab.o_buf[3 * b + 2], bufA[b].n});
+    }
+    slab.views.push_back({m + slab.o_chal, d_chal.n});
+    slab.views.push_back({m + slab.o_tr, d_tr.n});
+    slab.views.push_back({m + slab.o_scal, d_scal.n});
+    slab.views.push_back({m + slab.o_claims, d_claims.n});
+    slab.views.push_back({m + slab.o_partials, d_partials.n});
+    slab.views.push_back({m + slab.o_counter, d_counter.n});
+    slab.views.push_back({m + slab.o_rowpart, d_rowpart.n});
+    slab.views.push_back({m + slab.o_eq, eq_set_entries});
+    slab.views.push_back({m + slab.o_hs, d_hs.n});
+    slab.views.push_back({m + slab.o_pool, d_fs_pool.n});
+    slab.views.push_back({m + slab.o_stmt, d_stmt.n});
+    CK(cudaStreamSynchronize(stream));   // (the host vectors go out of scope)
+    slab.cap = B;
+}
+
+// Exchanges the buffers of the Fiat-Shamir path with the slab's: statement 0 of the slab takes the context's place. Called
+// twice, it restores the context (FsBatchScope).
+void Engine::slab_swap() {
+    size_t k = 0;
+    auto sw = [&](auto& d) {
+        using T = std::remove_reference_t<decltype(*d.p)>;
+        std::pair<void*, size_t>& v = slab.views[k++];
+        T* const p = d.p;
+        const size_t c = d.n;
+        d.p = static_cast<T*>(v.first);
+        d.n = v.second;
+        v = {p, c};
+    };
+    for (int b = 0; b < 2; ++b) { sw(bufV[b]); sw(bufM[b]); sw(bufA[b]); }
+    sw(d_chal); sw(d_tr); sw(d_scal); sw(d_claims); sw(d_partials); sw(d_counter); sw(d_rowpart); sw(d_eq); sw(d_hs); sw(d_fs_pool);
+    sw(d_stmt);
+    std::swap(val, slab.val);
+    std::swap(d_valptr, slab.valptr);
+    std::swap(d_inputs, slab.inputs);
+    std::swap(d_root_scratch, slab.root_scratch);
+    for (int i = 1; i < n; ++i) {
+        std::swap(L[i].p2_tabs, slab.p2_tabs[i]);
+        std::swap(L[i].liu_eqtabs, slab.liu_eqtabs[i]);
+    }
 }
 
 // one cooperative launch of k_sumcheck_phase_fs over P (unsharded: the whole phase)
@@ -2705,12 +2854,29 @@ void Engine::launch_phase_kernel_fs(const SumcheckPlan& P, uint32_t ci, F* keep,
     f.pool = d_fs_pool.p;
     f.chal = d_chal.p + ci;
     f.stamps = d_fs_stamps.p + 4 * stamp_round;
-    const int grid = P.max_work > tail_work ? grid_for(P.max_work, cap_phase_fs) : 1;
-    void* args[] = {&a, &f};
-    size_t h = prof_begin(KC_ROUND_FOLD);
-    CK(cudaLaunchCooperativeKernel((const void*)k_sumcheck_phase_fs, dim3(grid), dim3(256), args, 0, stream));
-    prof_end(h, P.bytes);
-    ++launches;
+    f.ss = sstride;
+    // a row of gx blocks per statement; the cooperative grid holds at most cap_phase_fs blocks, so a batch larger than
+    // that runs in chunks of statements (row z of a chunk starting at statement s0 is statement s0 + z)
+    const uint32_t rows = std::min<uint32_t>(n_stmt, (uint32_t)cap_phase_fs);
+    const int gx = P.max_work > tail_work ? grid_for(P.max_work, std::max(1, cap_phase_fs / (int)rows)) : 1;
+    for (uint32_t s0 = 0; s0 < n_stmt; s0 += rows) {
+        const uint32_t nz = std::min(rows, n_stmt - s0);
+        PhaseArgs ac = a;
+        FsPhaseArgs fc = f;
+        if (s0) {
+            const size_t d = s0 * sstride;
+            auto sh = [d](auto* q) { return q ? reinterpret_cast<decltype(q)>(reinterpret_cast<uintptr_t>(q) + d) : q; };
+            for (int b = 0; b < 2; ++b) { ac.bufV[b] = sh(a.bufV[b]); ac.bufM[b] = sh(a.bufM[b]); ac.bufA[b] = sh(a.bufA[b]); }
+            ac.at_init = sh(a.at_init); ac.chal = sh(a.chal); ac.add_term = sh(a.add_term); ac.claims = sh(a.claims);
+            ac.out_poly = sh(a.out_poly); ac.transcript = sh(a.transcript); ac.keep = sh(a.keep); ac.partials = sh(a.partials);
+            fc.pool = sh(f.pool); fc.chal = sh(f.chal); fc.stamps = nullptr;
+        }
+        void* args[] = {&ac, &fc};
+        size_t h = prof_begin(KC_ROUND_FOLD);
+        CK(cudaLaunchCooperativeKernel((const void*)k_sumcheck_phase_fs, dim3(gx, 1, nz), dim3(256), args, 0, stream));
+        prof_end(h, P.bytes * nz);
+        ++launches;
+    }
 }
 
 // The circuit digest R(circuit_bytes) (include/virgo_b200.h), serialised on the host once per context and hashed on the device.
@@ -2749,24 +2915,28 @@ void Engine::circuit_digest_async() {
     words.alloc(b.size() / 8);
     CK(cudaMemcpyAsync(words.p, b.data(), b.size(), cudaMemcpyHostToDevice, stream));
     scratch.alloc(pc_vector_root_scratch(words.n) / 8);
-    launches += (uint64_t)pc_vector_root(words.p, words.n, scratch.p, reinterpret_cast<uint8_t*>(d_stmt.p), stream);
+    launches += (uint64_t)pc_vector_root(words.p, words.n, scratch.p, reinterpret_cast<uint8_t*>(const_cast<uint64_t*>(d_circuit_digest)), stream);
     CK(cudaStreamSynchronize(stream));   // (the host bytes and the scratch go out of scope)
     circuit_digest_ready = true;
 }
 
-// inputs root (circuitValue[0]), outputs root (d_outputs, or circuitValue[n-1]) and the statement, which seeds the pool
-void Engine::statement_async(const uint8_t context[32], const F* d_outputs) {
+// inputs root (circuitValue[0]), outputs root (d_outputs, or circuitValue[n-1]) and the statement, which seeds the pool.
+// A batch: the roots of every statement's slice in one pass each, the contexts from d_contexts (4 words per statement).
+void Engine::statement_async(const uint8_t context[32], const F* d_outputs, const uint64_t* d_contexts) {
     circuit_digest_async();
     const size_t n_in = C.layer_size(0), n_out = C.layer_size(n - 1);
-    const size_t need = std::max(pc_vector_root_scratch(2 * n_in), pc_vector_root_scratch(2 * n_out)) / 8;
+    const size_t need = n_stmt * std::max(pc_vector_root_scratch(2 * n_in), pc_vector_root_scratch(2 * n_out)) / 8;
     if (d_root_scratch.n < need) d_root_scratch.alloc(need);
     uint8_t* roots = reinterpret_cast<uint8_t*>(d_stmt.p);
-    launches += (uint64_t)pc_vector_root(reinterpret_cast<const uint64_t*>(val[0].p), 2 * n_in, d_root_scratch.p, roots + 32, stream);
+    launches += (uint64_t)pc_vector_root(reinterpret_cast<const uint64_t*>(val[0].p), 2 * n_in, d_root_scratch.p, roots + 32, stream,
+                                         n_stmt, sstride);
     launches += (uint64_t)pc_vector_root(reinterpret_cast<const uint64_t*>(d_outputs ? d_outputs : val[n - 1].p), 2 * n_out, d_root_scratch.p,
-                                         roots + 64, stream);
+                                         roots + 64, stream, n_stmt, sstride);
     FsContext cx;
-    memcpy(cx.w, context, 32);
-    k_fs_statement<<<1, 32, 0, stream>>>(d_stmt.p, (uint64_t)n_in, (uint64_t)n_out, cx, d_fs_pool.p, d_stmt.p + 12);
+    memset(cx.w, 0, 32);
+    if (context) memcpy(cx.w, context, 32);
+    k_fs_statement<<<sgrid(1), 32, 0, stream>>>(d_circuit_digest, d_stmt.p, (uint64_t)n_in, (uint64_t)n_out, cx, d_contexts, d_fs_pool.p,
+                                                d_stmt.p + 12, sstride);
     ++launches;
 }
 
@@ -2805,13 +2975,13 @@ void Engine::prove_fs_device(const uint8_t* seed, F* tr_out, F* ch_out) {
     }
     do_input_mle();
     fs_rounds = sr;
-    std::vector<F> ch(n_chal);
-    CK(cudaMemcpyAsync(tr_out, d_tr.p, n_tr * sizeof(F), cudaMemcpyDeviceToHost, stream));
-    CK(cudaMemcpyAsync(ch.data(), d_chal.p, n_chal * sizeof(F), cudaMemcpyDeviceToHost, stream));
+    std::vector<F> ch((size_t)n_stmt * n_chal);   // statement-major, like the transcripts
+    copy_stmts_to_host(tr_out, n_tr * sizeof(F), d_tr.p, n_tr * sizeof(F));
+    copy_stmts_to_host(ch.data(), n_chal * sizeof(F), d_chal.p, n_chal * sizeof(F));
     CK(cudaStreamSynchronize(stream));
     CK(cudaGetLastError());
-    h_chal = ch;   // a later vp_verify / vp_prove on this context sees the challenges the proof used
-    if (ch_out) memcpy(ch_out, ch.data(), n_chal * sizeof(F));
+    if (n_stmt == 1) h_chal = ch;   // a later vp_verify / vp_prove on this context sees the challenges the proof used
+    if (ch_out) memcpy(ch_out, ch.data(), ch.size() * sizeof(F));
     proof_size = 0;
     for (int i = n - 1; i >= 1; --i) {
         const int pb = C.bit_length(i - 1), m = L[i].max_dad_bl;
@@ -3831,6 +4001,66 @@ extern "C" int vp_prove_fs_bound(vp_ctx* ctx, const uint8_t context[32], vp_F* t
     CK(cudaStreamSynchronize(e.stream));
     copy_digest(h, statement);
     CK(cudaEventElapsedTime(&e.last_ms, e.ev0, e.ev1));
+    e.last_launches = e.launches - l0;
+    return VP_OK;
+    API_END
+}
+// A batch runs on the context's slab (Engine::FsSlab): the scope swaps the slab in and, on every exit, the context's own
+// buffers and host state back, so that the context's inputs, values, transcript and challenges are untouched.
+struct FsBatchScope {
+    Engine& e;
+    std::vector<F> h_chal;
+    bool evaluated;
+    int pending_chunks;
+    FsBatchScope(Engine& e_, uint32_t B) : e(e_), h_chal(e_.h_chal), evaluated(e_.evaluated), pending_chunks(e_.pending_chunks) {
+        e.slab_reserve(B);
+        e.slab_swap();
+        e.n_stmt = B;
+        e.sstride = e.slab.stride;
+        e.pending_chunks = 0;
+    }
+    ~FsBatchScope() {
+        e.slab_swap();
+        e.n_stmt = 1;
+        e.sstride = 0;
+        e.h_chal.swap(h_chal);
+        e.evaluated = evaluated;
+        e.pending_chunks = pending_chunks;
+    }
+};
+extern "C" int vp_prove_fs_bound_batch(vp_ctx* ctx, size_t B, const uint64_t* inputs, size_t n_inputs, const uint8_t* contexts,
+                                       vp_F* transcripts, size_t cap, vp_F* challenges, size_t ch_cap, uint8_t* statements) {
+    if (!ctx || !inputs || !contexts || !transcripts) return fail(VP_ERR_ARG, "null argument");
+    API_BEGIN
+    Engine& e = ctx->e;
+    ScopedTimer t(e);
+    if (e.world != 1) return fail(VP_ERR_ARG, "vp_prove_fs_bound_batch: sharded contexts are not supported");
+    if (B == 0 || B > 65535) return fail(VP_ERR_ARG, "batch size %zu is not in [1, 65535]", B);
+    const size_t n_in = e.C.layer_size(0);
+    if (n_inputs != B * n_in) return fail(VP_ERR_ARG, "expected %zu inputs (%zu statements of %zu), got %zu", B * n_in, B, n_in, n_inputs);
+    if (cap < B * e.n_tr) return fail(VP_ERR_ARG, "transcript buffer too small (%zu < %zu)", cap, B * e.n_tr);
+    if (challenges && ch_cap < B * e.n_chal) return fail(VP_ERR_ARG, "challenge buffer too small (%zu < %zu)", ch_cap, B * e.n_chal);
+    for (size_t i = 0; i < n_inputs; ++i)
+        if (inputs[i] >= P) return fail(VP_ERR_ARG, "input %zu of statement %zu is not < p", i % n_in, i / n_in);
+    e.leave();
+    e.fs_alloc();
+    e.circuit_digest_async();
+    const uint64_t l0 = e.launches;
+    try {
+        FsBatchScope scope(e, (uint32_t)B);
+        CK(cudaEventRecord(e.ev0, e.stream));
+        CK(cudaMemcpyAsync(e.d_inputs.p, inputs, n_inputs * sizeof(uint64_t), cudaMemcpyHostToDevice, e.stream));
+        CK(cudaMemcpyAsync(e.slab.contexts.p, contexts, 32 * B, cudaMemcpyHostToDevice, e.stream));
+        e.fs_begin();
+        e.statement_async(nullptr, nullptr, e.slab.contexts.p);
+        e.prove_fs_device(nullptr, reinterpret_cast<F*>(transcripts), reinterpret_cast<F*>(challenges));
+        CK(cudaEventRecord(e.ev1, e.stream));
+        if (statements) e.copy_stmts_to_host(statements, 32, e.d_stmt.p + 12, 32);
+        CK(cudaStreamSynchronize(e.stream));
+        CK(cudaEventElapsedTime(&e.last_ms, e.ev0, e.ev1));
+    } catch (const StatementAssert& a) {
+        return fail(VP_ERR_ASSERT, "statement %u: assert gate violated in layer %u", a.stmt, a.flag - 1);
+    }
     e.last_launches = e.launches - l0;
     return VP_OK;
     API_END

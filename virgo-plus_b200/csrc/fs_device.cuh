@@ -6,6 +6,9 @@
 // little-endian words. Everything FsCache stores is a whole number of words (the 32-byte seed / digest, 16-byte field
 // elements), so the pool is a word array. Only one thread at a time touches it: the kernels below run in stream order and
 // inside k_sumcheck_phase_fs only thread 0 of block 0 does.
+// A batch of B statements (vp_prove_fs_bound_batch) gives every statement its own pool, transcript and challenges, `ss`
+// bytes apart (kernels.cuh, stmt_at); statement b runs in blockIdx.z == b: one warp per statement in the kernels between
+// phases, one row of blocks per statement in the phase kernel.
 #pragma once
 #include "kernels.cuh"
 #include "keccak.cuh"
@@ -32,7 +35,8 @@ VP_D F fs_draw(uint64_t* pool) {
 // Between phases (one warp, lane 0 hashes): store transcript[tr_begin .. + n_store), then draw chal[ci_begin .. + n_draw)
 // (host/fiat_shamir.h: Vres / claim_u / claims_v / claim_liu, then r_out / assert_random / sig).
 __global__ void k_fs_absorb_draw(uint64_t* pool, const F* __restrict__ transcript, uint32_t tr_begin, uint32_t n_store, F* chal,
-                                 uint32_t ci_begin, uint32_t n_draw) {
+                                 uint32_t ci_begin, uint32_t n_draw, size_t ss) {
+    pool = stmt_at(pool, ss); transcript = stmt_at(transcript, ss); chal = stmt_at(chal, ss);
     const uint64_t n0 = pool[0];
     __syncwarp();
     for (uint32_t k = threadIdx.x; k < n_store; k += 32) {
@@ -47,16 +51,23 @@ __global__ void k_fs_absorb_draw(uint64_t* pool, const F* __restrict__ transcrip
 }
 
 // The statement (include/virgo_b200.h): H("VPSTMT01" | circuit | u64 n_inputs | inputs root | u64 n_outputs | outputs root |
-// context[32]), 152 bytes. roots = {circuit, inputs, outputs} digests, 4 words each. Seeds the pool with it and copies it to
-// `out` (4 words).
+// context[32]), 152 bytes. circuit: its digest (4 words, shared by a batch); roots = {-, inputs, outputs} digests, 4 words
+// each. The context is `ctx`, or ctxs[4b ..] for statement b when ctxs is not null. Seeds the pool with the statement and
+// copies it to `out` (4 words).
 struct FsContext { uint64_t w[4]; };
-__global__ void k_fs_statement(const uint64_t* __restrict__ roots, uint64_t n_inputs, uint64_t n_outputs, FsContext ctx, uint64_t* pool,
-                               uint64_t* out) {
+__global__ void k_fs_statement(const uint64_t* __restrict__ circuit, const uint64_t* __restrict__ roots, uint64_t n_inputs,
+                               uint64_t n_outputs, FsContext ctx, const uint64_t* __restrict__ ctxs, uint64_t* pool, uint64_t* out,
+                               size_t ss) {
     if (threadIdx.x != 0) return;
+    roots = stmt_at(roots, ss); pool = stmt_at(pool, ss); out = stmt_at(out, ss);
+    if (ctxs) {
+#pragma unroll
+        for (int k = 0; k < 4; ++k) ctx.w[k] = ctxs[4 * (size_t)blockIdx.z + k];
+    }
     uint64_t m[19];
     m[0] = 0x3130544d54535056ull;   // "VPSTMT01"
 #pragma unroll
-    for (int k = 0; k < 4; ++k) { m[1 + k] = roots[k]; m[6 + k] = roots[4 + k]; m[11 + k] = roots[8 + k]; m[15 + k] = ctx.w[k]; }
+    for (int k = 0; k < 4; ++k) { m[1 + k] = circuit[k]; m[6 + k] = roots[4 + k]; m[11 + k] = roots[8 + k]; m[15 + k] = ctx.w[k]; }
     m[5] = n_inputs;
     m[10] = n_outputs;
     uint64_t d[4];
@@ -74,10 +85,13 @@ __global__ void k_fs_statement(const uint64_t* __restrict__ roots, uint64_t n_in
 // them; storing them is the next k_fs_absorb_draw's job.
 // stamps (4 per round, block 0, %globaltimer): round start, own fold work done, polynomial reduced (grid rounds: after the
 // barrier), challenge drawn. The next round's start minus "drawn" is the release barrier.
+// A batch runs a gridDim.x x B grid: row blockIdx.z is statement b, its block x == 0 reduces the row's partials and draws
+// the statement's challenge, and one grid barrier serves all rows. Stamps are those of row 0.
 struct FsPhaseArgs {
     uint64_t* pool;
     F* chal;                     // = PhaseArgs::chal, writable
     unsigned long long* stamps;  // 4 * n_rounds, may be null
+    size_t ss;                   // bytes between two statements' working sets (0: one statement)
 };
 VP_D void fs_stamp(unsigned long long* s, uint32_t j, int k) {
     if (!s) return;
@@ -92,41 +106,48 @@ __global__ void __launch_bounds__(256, 2) k_sumcheck_phase_fs(PhaseArgs p, FsPha
     __shared__ F smem[3 * 32];
     __shared__ uint32_t s_wend[128];
     const uint32_t gtid = blockIdx.x * blockDim.x + threadIdx.x, gstride = gridDim.x * blockDim.x;
+    const size_t ss = f.ss;
+    uint64_t* const pool = stmt_at(f.pool, ss);
+    F* const chal = stmt_at(f.chal, ss);
+    F* const claims = stmt_at(p.claims, ss);
+    unsigned long long* const stamps = blockIdx.z == 0 ? f.stamps : nullptr;
     const bool stamp = blockIdx.x == 0 && threadIdx.x == 0;
-    F at = p.at_init ? *p.at_init : f_zero();  // add_term: meaningful in block 0 / thread 0 only
+    F at = p.at_init ? *stmt_at(p.at_init, ss) : f_zero();  // add_term: meaningful in block 0 / thread 0 only
     uint32_t j = 1;
     // ---- grid rounds
     for (; j <= p.n_rounds; ++j) {
         const RoundDev R = p.rounds[j - 1];
         if (R.work <= p.tail_work) break;
-        if (stamp) fs_stamp(f.stamps, j, 0);
+        if (stamp) fs_stamp(stamps, j, 0);
         const bool fold = j >= 2;
         __syncthreads();
         for (uint32_t i = threadIdx.x; i < R.n_tabs; i += blockDim.x) s_wend[i] = p.tabs[R.tab_begin + i].work_end;
         __syncthreads();
         const uint32_t ib = R.in_buf, ob = ib ^ 1;
         const bool scale = j >= 2;
-        const F prev = scale ? ld_f_cg(f.chal + j - 2) : f_zero();   // drawn by block 0 in this launch: bypass L1
+        const F prev = scale ? ld_f_cg(chal + j - 2) : f_zero();   // drawn by block 0 in this launch: bypass L1
         const FoldK rk = make_foldk(prev);
         RoundAcc acc;
         racc_init(acc);
-        if (fold) round_work<true, false>(acc, p.tabs + R.tab_begin, R.n_tabs, s_wend, p.bufV[ib], p.bufM[ib], p.bufA[ib],
-                                          p.bufV[ob], p.bufM[ob], p.bufA[ob], rk, gtid, gstride);
-        else round_work<false, false>(acc, p.tabs + R.tab_begin, R.n_tabs, s_wend, p.bufV[ib], p.bufM[ib], p.bufA[ib],
-                                      p.bufV[ob], p.bufM[ob], p.bufA[ob], rk, gtid, gstride);
+        if (fold) round_work<true, false>(acc, p.tabs + R.tab_begin, R.n_tabs, s_wend, stmt_at(p.bufV[ib], ss), stmt_at(p.bufM[ib], ss),
+                                          stmt_at(p.bufA[ib], ss), stmt_at(p.bufV[ob], ss), stmt_at(p.bufM[ob], ss),
+                                          stmt_at(p.bufA[ob], ss), rk, gtid, gstride);
+        else round_work<false, false>(acc, p.tabs + R.tab_begin, R.n_tabs, s_wend, stmt_at(p.bufV[ib], ss), stmt_at(p.bufM[ib], ss),
+                                      stmt_at(p.bufA[ib], ss), stmt_at(p.bufV[ob], ss), stmt_at(p.bufM[ob], ss),
+                                      stmt_at(p.bufA[ob], ss), rk, gtid, gstride);
         F v[3];
         racc_finish(acc, v);
         block_sum<3>(v, smem);
-        F* part = p.partials + (size_t)(j & 1) * gridDim.x * 3;
+        F* part = stmt_at(p.partials, ss) + (size_t)(j & 1) * gridDim.x * 3;
         if (threadIdx.x == 0) {
             st_f(part + (size_t)blockIdx.x * 3 + 0, v[0]);
             st_f(part + (size_t)blockIdx.x * 3 + 1, v[1]);
             st_f(part + (size_t)blockIdx.x * 3 + 2, v[2]);
             if (blockIdx.x == 0)
-                at = collapse_update<false>(at, p.cols + R.col_begin, R.n_cols, p.bufV[ib], p.bufM[ib], p.bufA[ib], fold,
-                                            scale, prev, rk, p.claims);
+                at = collapse_update<false>(at, p.cols + R.col_begin, R.n_cols, stmt_at(p.bufV[ib], ss), stmt_at(p.bufM[ib], ss),
+                                            stmt_at(p.bufA[ib], ss), fold, scale, prev, rk, claims);
         }
-        if (stamp) fs_stamp(f.stamps, j, 1);
+        if (stamp) fs_stamp(stamps, j, 1);
         grid.sync();
         if (blockIdx.x == 0) {
             F t[3] = {f_zero(), f_zero(), f_zero()};
@@ -138,11 +159,11 @@ __global__ void __launch_bounds__(256, 2) k_sumcheck_phase_fs(PhaseArgs p, FsPha
             block_sum<3>(t, smem);
             if (threadIdx.x == 0) {
                 const F o[3] = {t[0], f_sub(t[1], at), f_add(t[2], at)};
-                F* out = p.out_poly + 3 * (j - 1);
-                fs_stamp(f.stamps, j, 2);
-                for (int k = 0; k < 3; ++k) { st_f(out + k, o[k]); fs_store(f.pool, o[k]); }
-                st_f(f.chal + j - 1, fs_draw(f.pool));
-                fs_stamp(f.stamps, j, 3);
+                F* out = stmt_at(p.out_poly, ss) + 3 * (j - 1);
+                fs_stamp(stamps, j, 2);
+                for (int k = 0; k < 3; ++k) { st_f(out + k, o[k]); fs_store(pool, o[k]); }
+                st_f(chal + j - 1, fs_draw(pool));
+                fs_stamp(stamps, j, 3);
             }
         }
         grid.sync();   // release: round j + 1 folds with the challenge just drawn
@@ -151,53 +172,56 @@ __global__ void __launch_bounds__(256, 2) k_sumcheck_phase_fs(PhaseArgs p, FsPha
     // ---- tail rounds: block 0 alone
     for (; j <= p.n_rounds; ++j) {
         const RoundDev R = p.rounds[j - 1];
-        if (stamp) fs_stamp(f.stamps, j, 0);
+        if (stamp) fs_stamp(stamps, j, 0);
         const bool fold = j >= 2;
         __syncthreads();   // (also publishes the previous round's challenge to the block)
         for (uint32_t i = threadIdx.x; i < R.n_tabs; i += blockDim.x) s_wend[i] = p.tabs[R.tab_begin + i].work_end;
         __syncthreads();
         const uint32_t ib = R.in_buf, ob = ib ^ 1;
         const bool scale = j >= 2;
-        const F prev = scale ? ld_f_cg(f.chal + j - 2) : f_zero();
+        const F prev = scale ? ld_f_cg(chal + j - 2) : f_zero();
         const FoldK rk = make_foldk(prev);
         RoundAcc acc;
         racc_init(acc);
-        if (fold) round_work<true, false>(acc, p.tabs + R.tab_begin, R.n_tabs, s_wend, p.bufV[ib], p.bufM[ib], p.bufA[ib],
-                                          p.bufV[ob], p.bufM[ob], p.bufA[ob], rk, threadIdx.x, blockDim.x);
-        else round_work<false, false>(acc, p.tabs + R.tab_begin, R.n_tabs, s_wend, p.bufV[ib], p.bufM[ib], p.bufA[ib],
-                                      p.bufV[ob], p.bufM[ob], p.bufA[ob], rk, threadIdx.x, blockDim.x);
+        if (fold) round_work<true, false>(acc, p.tabs + R.tab_begin, R.n_tabs, s_wend, stmt_at(p.bufV[ib], ss), stmt_at(p.bufM[ib], ss),
+                                          stmt_at(p.bufA[ib], ss), stmt_at(p.bufV[ob], ss), stmt_at(p.bufM[ob], ss),
+                                          stmt_at(p.bufA[ob], ss), rk, threadIdx.x, blockDim.x);
+        else round_work<false, false>(acc, p.tabs + R.tab_begin, R.n_tabs, s_wend, stmt_at(p.bufV[ib], ss), stmt_at(p.bufM[ib], ss),
+                                      stmt_at(p.bufA[ib], ss), stmt_at(p.bufV[ob], ss), stmt_at(p.bufM[ob], ss),
+                                      stmt_at(p.bufA[ob], ss), rk, threadIdx.x, blockDim.x);
         F v[3];
         racc_finish(acc, v);
-        if (stamp) fs_stamp(f.stamps, j, 1);
+        if (stamp) fs_stamp(stamps, j, 1);
         block_sum<3>(v, smem);
         if (threadIdx.x == 0) {
-            at = collapse_update<false>(at, p.cols + R.col_begin, R.n_cols, p.bufV[ib], p.bufM[ib], p.bufA[ib], fold, scale, prev,
-                                        rk, p.claims);
+            at = collapse_update<false>(at, p.cols + R.col_begin, R.n_cols, stmt_at(p.bufV[ib], ss), stmt_at(p.bufM[ib], ss),
+                                        stmt_at(p.bufA[ib], ss), fold, scale, prev, rk, claims);
             const F o[3] = {v[0], f_sub(v[1], at), f_add(v[2], at)};
-            F* out = p.out_poly + 3 * (j - 1);
-            fs_stamp(f.stamps, j, 2);
-            for (int k = 0; k < 3; ++k) { st_f(out + k, o[k]); fs_store(f.pool, o[k]); }
-            st_f(f.chal + j - 1, fs_draw(f.pool));
-            fs_stamp(f.stamps, j, 3);
+            F* out = stmt_at(p.out_poly, ss) + 3 * (j - 1);
+            fs_stamp(stamps, j, 2);
+            for (int k = 0; k < 3; ++k) { st_f(out + k, o[k]); fs_store(pool, o[k]); }
+            st_f(chal + j - 1, fs_draw(pool));
+            fs_stamp(stamps, j, 3);
         }
     }
     __syncthreads();  // the last round's table writes, the claims of collapsed tables and the last challenge
-    if (threadIdx.x == 0) st_f(p.add_term, at);
+    if (threadIdx.x == 0) st_f(stmt_at(p.add_term, ss), at);
     // ---- final claims (prover.cpp:494-521)
-    const F* V = p.bufV[p.fin_buf];
+    const F* V = stmt_at(p.bufV[p.fin_buf], ss);
+    F* const transcript = stmt_at(p.transcript, ss);
     for (uint32_t i = threadIdx.x; i < p.n_fin; i += blockDim.x) {
         const FinDesc fd = p.fins[i];
         F c;
-        if (fd.from_claim >= 0) c = ld_one<false>(p.claims + fd.from_claim);
+        if (fd.from_claim >= 0) c = ld_one<false>(claims + fd.from_claim);
         else {
             const F v0 = fd.n_vals >= 1 ? ld_one<false>(V + fd.in_off) : f_zero();
             if (p.n_rounds >= 1) {
                 const F v1 = fd.n_vals >= 2 ? ld_one<false>(V + fd.in_off + 1) : f_zero();
-                c = f_fold(v0, v1, ld_f_cg(f.chal + p.n_rounds - 1));
+                c = f_fold(v0, v1, ld_f_cg(chal + p.n_rounds - 1));
             } else c = v0;
         }
-        st_f(p.transcript + fd.out_idx, c);
-        if (p.keep && i == 0) st_f(p.keep, c);
+        st_f(transcript + fd.out_idx, c);
+        if (p.keep && i == 0) st_f(stmt_at(p.keep, ss), c);
     }
 }
 

@@ -52,6 +52,16 @@ struct EqTab {
 };
 VP_D F eq_at(const EqTab& t, uint32_t idx) { return f_mul(ld_f(t.f + (idx & t.mask)), ld_f(t.s + (idx >> t.fh))); }
 
+// ------------------------------------------------------------------ statements of a batch (vp_prove_fs_bound_batch)
+// The Fiat-Shamir kernels run B independent statements of one circuit at once, statement b in blockIdx.z == b. Every
+// per-statement buffer of statement b (tables, challenges, transcript, claims, scalars, eq tables, partial sums, pool)
+// sits `ss` bytes after statement b - 1's: stmt_at shifts a statement-0 pointer to this block's statement. Layer values
+// are instance-major over the B * K instances instead (statement b, instance k = global instance b * K + k). A single
+// proof is the batch of one: blockIdx.z == 0, and every shift is zero.
+template <class T>
+VP_D T* stmt_at(T* p, size_t ss) { return reinterpret_cast<T*>(reinterpret_cast<uintptr_t>(p) + (size_t)blockIdx.z * ss); }
+VP_D EqTab stmt_at(EqTab t, size_t ss) { t.f = stmt_at(t.f, ss); t.s = stmt_at(t.s, ss); return t; }
+
 // ------------------------------------------------------------------ sharding of a table over G GPUs
 // A table is cut into blocks of 2^m consecutive entries and every rank holds a CONTIGUOUS run of blocks, i.e. the
 // entries [lo, hi) (multiples of 2^m), stored from local index 0. Rounds 1..m of a sumcheck pair entries inside one
@@ -136,7 +146,9 @@ struct EqBuild {
 };
 
 __global__ void __launch_bounds__(1024) k_eq_build(const EqBuild* __restrict__ descs, const F* __restrict__ chal,
-                                                    F* __restrict__ eqbuf) {
+                                                    F* __restrict__ eqbuf, size_t ss) {
+    chal = stmt_at(chal, ss);
+    eqbuf = stmt_at(eqbuf, ss);
     const EqBuild d = descs[blockIdx.x];
     F* T = eqbuf + d.out_off;
     if (threadIdx.x == 0) T[0] = d.scale_idx >= 0 ? chal[d.scale_idx] : f_one();
@@ -175,12 +187,12 @@ struct GateArrays {          // one template layer (one instance)
 };
 
 // prover.cpp:38-90. Thread per gate of the replicated layer: g = k*S + g0.
-// vals[l] = device pointer of circuitValue[l]; sizes[l] = template size S_l.
+// vals[l] = device pointer of circuitValue[l]; sizes[l] = template size S_l. A batch of statements is evaluated as one
+// replicated layer of B * K instances; a failed assert of instance k raises the flag of statement k / K (flags ss bytes apart).
 __global__ void __launch_bounds__(256) k_eval_layer(GateArrays G, uint32_t S, uint32_t K, int layer,
                                                      F* const* __restrict__ vals, const uint32_t* __restrict__ sizes,
                                                      F* __restrict__ out, unsigned int* __restrict__ assert_fail,
-                                                     uint32_t g_begin, uint32_t g_end, int real_only) {
-    (void)K;
+                                                     uint32_t g_begin, uint32_t g_end, int real_only, size_t ss) {
     const uint32_t S_pre = sizes[layer - 1];
     const F* __restrict__ pre = vals[layer - 1];
     for (uint32_t g = g_begin + blockIdx.x * blockDim.x + threadIdx.x; g < g_end; g += gridDim.x * blockDim.x) {
@@ -225,7 +237,8 @@ __global__ void __launch_bounds__(256) k_eval_layer(GateArrays G, uint32_t S, ui
             default: r = f_zero(); break;
         }
         st_f(out + g, r);
-        if ((tyb & TY_ASSERT_BIT) && !f_is_zero(r)) atomicExch(assert_fail, 1u + (unsigned)layer);
+        if ((tyb & TY_ASSERT_BIT) && !f_is_zero(r))
+            atomicExch(reinterpret_cast<unsigned int*>(reinterpret_cast<uintptr_t>(assert_fail) + (size_t)(k / K) * ss), 1u + (unsigned)layer);
     }
 }
 
@@ -306,8 +319,11 @@ k_init_phase1(const RowItem* __restrict__ items, uint32_t n_items, CsrP1 csr, ui
               EqTab eqg, const F* __restrict__ assert_r, F* const* __restrict__ vals, const uint32_t* __restrict__ sizes,
               const F* __restrict__ cst, const F* __restrict__ Vpre, F* __restrict__ tV, F* __restrict__ tM,
               F* __restrict__ tA, F* __restrict__ partial, uint32_t n_slots, ShardMap sm, int write_v, uint32_t k_begin,
-              uint32_t k_end) {
-    (void)K;
+              uint32_t k_end, size_t ss) {
+    const size_t kz = (size_t)blockIdx.z * K;   // this statement's first global instance
+    eqg = stmt_at(eqg, ss); assert_r = stmt_at(assert_r, ss);
+    tV = stmt_at(tV, ss); tM = stmt_at(tM, ss); tA = stmt_at(tA, ss); partial = stmt_at(partial, ss);
+    Vpre += kz * S_pre;
     const uint64_t total = (uint64_t)n_items * (k_end - k_begin);
     for (uint64_t w = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; w < total; w += (uint64_t)gridDim.x * blockDim.x) {
         const uint32_t kq = (uint32_t)(w / n_items), it = (uint32_t)(w - (uint64_t)kq * n_items), k = k_begin + kq;
@@ -322,7 +338,7 @@ k_init_phase1(const RowItem* __restrict__ items, uint32_t n_items, CsrP1 csr, ui
             F beta = eq_at(eqg, k * S_cur + g0);
             if (tyl & TY_ASSERT_BIT) beta = f_mul(beta, *assert_r);
             F Vv = f_zero();
-            if (l >= 0) Vv = ld_f(vals[l] + (size_t)k * sizes[l] + csr.v0[e]);
+            if (l >= 0) Vv = ld_f(vals[l] + (kz + k) * sizes[l] + csr.v0[e]);
             p1_gate(tyl, beta, Vv, cst, g0, M, A);
         }
         const uint32_t slot = I.cnt_slot >> 8;
@@ -366,11 +382,17 @@ k_init_phase1_real(const RowItem* __restrict__ items, uint32_t n_items, CsrP1 cs
                    EqTab eqg, const F* __restrict__ assert_r, F* const* __restrict__ vals, const uint32_t* __restrict__ sizes,
                    const F* __restrict__ cst, const F* __restrict__ Vpre, F* __restrict__ tV, F* __restrict__ tM,
                    F* __restrict__ tA, F* __restrict__ partial, uint32_t n_slots, ShardMap sm, int write_v, uint32_t k_begin,
-                   uint32_t k_end, uint32_t n_src) {
-    (void)K;
+                   uint32_t k_end, uint32_t n_src, size_t ss) {
+    const size_t kz = (size_t)blockIdx.z * K;   // this statement's first global instance
+    eqg = stmt_at(eqg, ss); assert_r = stmt_at(assert_r, ss);
+    tV = stmt_at(tV, ss); tM = stmt_at(tM, ss); tA = stmt_at(tA, ss); partial = stmt_at(partial, ss);
+    Vpre += kz * S_pre;
     __shared__ const u64* s_vals[64];
     __shared__ uint32_t s_sizes[64];
-    for (uint32_t i = threadIdx.x; i < min(n_src, 64u); i += blockDim.x) { s_vals[i] = reinterpret_cast<const u64*>(vals[i]); s_sizes[i] = sizes[i]; }
+    for (uint32_t i = threadIdx.x; i < min(n_src, 64u); i += blockDim.x) {
+        s_vals[i] = reinterpret_cast<const u64*>(vals[i] + kz * sizes[i]);
+        s_sizes[i] = sizes[i];
+    }
     __syncthreads();
     const uint32_t total = n_items * (k_end - k_begin);   // < 2^32 (host check)
     for (uint32_t w = blockIdx.x * blockDim.x + threadIdx.x; w < total; w += gridDim.x * blockDim.x) {
@@ -456,11 +478,17 @@ k_init_phase1_real_tm(const RowItem* __restrict__ items, uint32_t n_items, CsrP1
                       EqTab eqg, const F* __restrict__ assert_r, F* const* __restrict__ vals, const uint32_t* __restrict__ sizes,
                       const F* __restrict__ cst, const F* __restrict__ Vpre, F* __restrict__ tV, F* __restrict__ tM,
                       F* __restrict__ tA, F* __restrict__ partial, uint32_t n_slots, int write_v, uint32_t n_src, ShardMap sm,
-                      uint32_t k_begin, uint32_t k_end) {
-    (void)K;
+                      uint32_t k_begin, uint32_t k_end, size_t ss) {
+    const size_t kz = (size_t)blockIdx.z * K;   // this statement's first global instance
+    eqg = stmt_at(eqg, ss); assert_r = stmt_at(assert_r, ss);
+    tV = stmt_at(tV, ss); tM = stmt_at(tM, ss); tA = stmt_at(tA, ss); partial = stmt_at(partial, ss);
+    Vpre += kz * S_pre;
     __shared__ const u64* s_vals[64];
     __shared__ uint32_t s_sizes[64];
-    for (uint32_t i = threadIdx.x; i < min(n_src, 64u); i += blockDim.x) { s_vals[i] = reinterpret_cast<const u64*>(vals[i]); s_sizes[i] = sizes[i]; }
+    for (uint32_t i = threadIdx.x; i < min(n_src, 64u); i += blockDim.x) {
+        s_vals[i] = reinterpret_cast<const u64*>(vals[i] + kz * sizes[i]);
+        s_sizes[i] = sizes[i];
+    }
     __syncthreads();
     const uint32_t it = blockIdx.x * blockDim.x + threadIdx.x;
     if (it >= n_items) return;
@@ -535,8 +563,9 @@ k_init_phase1_real_tm(const RowItem* __restrict__ items, uint32_t n_items, CsrP1
 __global__ void __launch_bounds__(256)
 k_combine_phase1(const LongRow* __restrict__ rows, uint32_t n_rows, uint32_t S_pre, uint32_t K, const F* __restrict__ Vpre,
                  F* __restrict__ tV, F* __restrict__ tM, F* __restrict__ tA, const F* __restrict__ partial, uint32_t n_slots,
-                 ShardMap sm, int write_v, uint32_t k_begin, uint32_t k_end) {
-    (void)K;
+                 ShardMap sm, int write_v, uint32_t k_begin, uint32_t k_end, size_t ss) {
+    tV = stmt_at(tV, ss); tM = stmt_at(tM, ss); tA = stmt_at(tA, ss); partial = stmt_at(partial, ss);
+    Vpre += (size_t)blockIdx.z * K * S_pre;
     const uint64_t total = (uint64_t)n_rows * (k_end - k_begin);
     for (uint64_t w = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; w < total; w += (uint64_t)gridDim.x * blockDim.x) {
         const uint32_t kq = (uint32_t)(w / n_rows), j = (uint32_t)(w - (uint64_t)kq * n_rows), k = k_begin + kq;
@@ -591,7 +620,10 @@ __global__ void __launch_bounds__(256)
 k_init_phase2(const RowItem* __restrict__ items, uint32_t n_items, const P2Table* __restrict__ tabs, CsrP2 csr,
               uint32_t S_pre, uint32_t S_cur, uint32_t K, EqTab eqg, EqTab equ, const F* __restrict__ assert_r,
               const F* __restrict__ Vu_ptr, F* __restrict__ tV, F* __restrict__ tM, F* __restrict__ tA,
-              F* __restrict__ partial, uint32_t n_slots, uint32_t kk_begin, uint32_t kk_end) {
+              F* __restrict__ partial, uint32_t n_slots, uint32_t kk_begin, uint32_t kk_end, size_t ss) {
+    const size_t kz = (size_t)blockIdx.z * K;   // this statement's first global instance
+    eqg = stmt_at(eqg, ss); equ = stmt_at(equ, ss); assert_r = stmt_at(assert_r, ss); Vu_ptr = stmt_at(Vu_ptr, ss);
+    tV = stmt_at(tV, ss); tM = stmt_at(tM, ss); tA = stmt_at(tA, ss); partial = stmt_at(partial, ss);
     __shared__ F s_cM[12], s_cA[12];
     if (threadIdx.x == 0) make_p2_coef(*Vu_ptr, s_cM, s_cA);
     __syncthreads();
@@ -615,7 +647,7 @@ k_init_phase2(const RowItem* __restrict__ items, uint32_t n_items, const P2Table
         const uint32_t slot = I.cnt_slot >> 8;
         if (slot == 0) {
             const uint32_t o = T.tab_off + loc;
-            st_f(tV + o, ld_f(T.src_val + (size_t)k * T.src_S + T.dadId[I.row]));
+            st_f(tV + o, ld_f(T.src_val + (kz + k) * T.src_S + T.dadId[I.row]));
             st_f(tM + o, M);
             st_f(tA + o, A);
         } else {
@@ -663,7 +695,9 @@ struct HsTab {
     const F* hs;           // null: not used (too many distinct factors per instance, e.g. one huge instance)
     uint32_t ng, nu;
 };
-__global__ void k_p2_hs(EqTab eqg, EqTab equ, uint32_t S_cur, uint32_t S_pre, uint32_t K, uint32_t ng, uint32_t nu, F* __restrict__ hs) {
+__global__ void k_p2_hs(EqTab eqg, EqTab equ, uint32_t S_cur, uint32_t S_pre, uint32_t K, uint32_t ng, uint32_t nu, F* __restrict__ hs,
+                        size_t ss) {
+    eqg = stmt_at(eqg, ss); equ = stmt_at(equ, ss); hs = stmt_at(hs, ss);
     const uint32_t ig_max = (K * S_cur - 1) >> eqg.fh, iu_max = (K * S_pre - 1) >> equ.fh;   // last second-half entries in use
     const uint32_t per = ng * nu, total = K * per;
     for (uint32_t w = blockIdx.x * blockDim.x + threadIdx.x; w < total; w += gridDim.x * blockDim.x) {
@@ -677,8 +711,10 @@ __global__ void __launch_bounds__(256, 4)
 k_init_phase2_v2(const RowItem* __restrict__ items, uint32_t n_items, const P2Table* __restrict__ tabs, CsrP2 csr,
                  uint32_t S_pre, uint32_t S_cur, uint32_t K, EqTab eqg, EqTab equ, const F* __restrict__ assert_r,
                  const F* __restrict__ Vu_ptr, F* __restrict__ tV, F* __restrict__ tM, F* __restrict__ tA,
-                 F* __restrict__ partial, uint32_t n_slots, uint32_t kk_begin, uint32_t kk_end, HsTab H) {
-    const F Vu = *Vu_ptr;
+                 F* __restrict__ partial, uint32_t n_slots, uint32_t kk_begin, uint32_t kk_end, HsTab H, size_t ss) {
+    // this statement's buffers are zo entries on: one offset instead of ten shifted pointers (those would spill here)
+    const size_t zo = (size_t)blockIdx.z * (ss / sizeof(F));
+    const F Vu = Vu_ptr[zo];
     const uint32_t total = n_items * (kk_end - kk_begin);   // < 2^32 (host check)
     for (uint32_t w = blockIdx.x * blockDim.x + threadIdx.x; w < total; w += gridDim.x * blockDim.x) {
         const uint32_t kq = w / n_items, it = w - kq * n_items, kk = kk_begin + kq, k = K - 1 - kk;
@@ -694,13 +730,14 @@ k_init_phase2_v2(const RowItem* __restrict__ items, uint32_t n_items, const P2Ta
             if (H.hs) {
                 const uint32_t ig = k * S_cur + g0, iu = k * S_pre + u0;
                 const uint32_t i = (ig >> eqg.fh) - ((k * S_cur) >> eqg.fh), j = (iu >> equ.fh) - ((k * S_pre) >> equ.fh);
-                const F ff = f_mul_w(ld_f(eqg.f + (ig & eqg.mask)), ld_f(equ.f + (iu & equ.mask)));
-                t = f_mul_w(ff, ld_f(H.hs + (k * H.ng + i) * H.nu + j));
-                if (tyb & TY_ASSERT_BIT) t = f_mul(t, *assert_r);
+                const F ff = f_mul_w(ld_f(eqg.f + zo + (ig & eqg.mask)), ld_f(equ.f + zo + (iu & equ.mask)));
+                t = f_mul_w(ff, ld_f(H.hs + zo + (k * H.ng + i) * H.nu + j));
+                if (tyb & TY_ASSERT_BIT) t = f_mul(t, assert_r[zo]);
             } else {
-                F bg = eq_at_weak(eqg, k * S_cur + g0);
-                if (tyb & TY_ASSERT_BIT) bg = f_mul(bg, *assert_r);
-                t = f_mul_w(bg, eq_at_weak(equ, k * S_pre + u0));
+                const EqTab g{eqg.f + zo, eqg.s + zo, eqg.fh, eqg.mask}, u{equ.f + zo, equ.s + zo, equ.fh, equ.mask};
+                F bg = eq_at_weak(g, k * S_cur + g0);
+                if (tyb & TY_ASSERT_BIT) bg = f_mul(bg, assert_r[zo]);
+                t = f_mul_w(bg, eq_at_weak(u, k * S_pre + u0));
             }
             p2_accumulate(tyb & 0x7f, t, S0, S1, SA);
         }
@@ -708,11 +745,11 @@ k_init_phase2_v2(const RowItem* __restrict__ items, uint32_t n_items, const P2Ta
         const uint32_t slot = I.cnt_slot >> 8;
         if (slot == 0) {
             const uint32_t o = T.tab_off + loc;
-            st_f(tV + o, ld_f(T.src_val + (size_t)k * T.src_S + T.dadId[I.row]));
-            st_f(tM + o, M);
-            st_f(tA + o, A);
+            st_f(tV + zo + o, ld_f(T.src_val + ((size_t)blockIdx.z * K + k) * T.src_S + T.dadId[I.row]));
+            st_f(tM + zo + o, M);
+            st_f(tA + zo + o, A);
         } else {
-            F* dst = partial + 2 * ((size_t)kk * n_slots + (slot - 1));
+            F* dst = partial + zo + 2 * ((size_t)kk * n_slots + (slot - 1));
             st_f(dst, M);
             st_f(dst + 1, A);
         }
@@ -722,7 +759,9 @@ k_init_phase2_v2(const RowItem* __restrict__ items, uint32_t n_items, const P2Ta
 __global__ void __launch_bounds__(256)
 k_combine_phase2(const LongRow* __restrict__ rows, uint32_t n_rows, const P2Table* __restrict__ tabs, uint32_t K,
                  F* __restrict__ tV, F* __restrict__ tM, F* __restrict__ tA, const F* __restrict__ partial, uint32_t n_slots,
-                 uint32_t kk_begin, uint32_t kk_end) {
+                 uint32_t kk_begin, uint32_t kk_end, size_t ss) {
+    const size_t kz = (size_t)blockIdx.z * K;   // this statement's first global instance
+    tV = stmt_at(tV, ss); tM = stmt_at(tM, ss); tA = stmt_at(tA, ss); partial = stmt_at(partial, ss);
     const uint64_t total = (uint64_t)n_rows * (kk_end - kk_begin);
     for (uint64_t w = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; w < total; w += (uint64_t)gridDim.x * blockDim.x) {
         const uint32_t kq = (uint32_t)(w / n_rows), j = (uint32_t)(w - (uint64_t)kq * n_rows), kk = kk_begin + kq, k = K - 1 - kk;
@@ -737,7 +776,7 @@ k_combine_phase2(const LongRow* __restrict__ rows, uint32_t n_rows, const P2Tabl
             A = f_add(A, ld_f_cg(src + 1));
         }
         const uint32_t o = T.tab_off + loc;
-        st_f(tV + o, ld_f(T.src_val + (size_t)k * T.src_S + T.dadId[R.row]));
+        st_f(tV + o, ld_f(T.src_val + (kz + k) * T.src_S + T.dadId[R.row]));
         st_f(tM + o, M);
         st_f(tA + o, A);
     }
@@ -758,17 +797,20 @@ struct CsrUnary {
 __global__ void __launch_bounds__(256)
 k_phase2_unary(CsrUnary un, uint32_t S_pre, uint32_t S_cur, uint32_t K, EqTab eqg, EqTab equ,
                const F* __restrict__ assert_r, const F* __restrict__ Vu_ptr, const F* __restrict__ cst,
-               F* __restrict__ dst, F* partials, unsigned int* counter, uint32_t k_begin, uint32_t k_end) {
+               F* __restrict__ dst, F* partials, unsigned int* counter, uint32_t k_begin, uint32_t k_end, size_t ss) {
     __shared__ F smem[32];
-    const F Vu = *Vu_ptr;
+    // this statement's eq tables are zo entries on; the outputs are shifted after the loop (fewer live registers)
+    const size_t zo = (size_t)blockIdx.z * (ss / sizeof(F));
+    const EqTab g{eqg.f + zo, eqg.s + zo, eqg.fh, eqg.mask}, u{equ.f + zo, equ.s + zo, equ.fh, equ.mask};
+    const F Vu = Vu_ptr[zo];
     const uint64_t total = (uint64_t)un.n * (k_end - k_begin);
     F acc[1] = {f_zero()};
     for (uint64_t w = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; w < total; w += (uint64_t)gridDim.x * blockDim.x) {
         const uint32_t k = k_begin + (uint32_t)(w / un.n), j = (uint32_t)(w % un.n);
         const uint32_t g0 = un.g0[j], tyb = un.ty[j], ty = tyb & 0x7f;
-        F bg = eq_at(eqg, k * S_cur + g0);
-        if (tyb & TY_ASSERT_BIT) bg = f_mul(bg, *assert_r);
-        const F tmp = f_mul(bg, eq_at(equ, k * S_pre + un.u0[j]));
+        F bg = eq_at(g, k * S_cur + g0);
+        if (tyb & TY_ASSERT_BIT) bg = f_mul(bg, assert_r[zo]);
+        const F tmp = f_mul(bg, eq_at(u, k * S_pre + un.u0[j]));
         F coef;
         switch (ty) {
             case T_ADDC: coef = f_add(cst[g0], Vu); break;
@@ -778,7 +820,7 @@ k_phase2_unary(CsrUnary un, uint32_t S_pre, uint32_t S_cur, uint32_t K, EqTab eq
         }
         acc[0] = f_add(acc[0], f_mul(tmp, coef));
     }
-    if (grid_sum<1>(acc, smem, partials, counter) && threadIdx.x == 0) st_f(dst, acc[0]);
+    if (grid_sum<1>(acc, smem, stmt_at(partials, ss), stmt_at(counter, ss)) && threadIdx.x == 0) st_f(stmt_at(dst, ss), acc[0]);
 }
 
 // ------------------------------------------------------------------ K5: Liu table init
@@ -793,7 +835,10 @@ __global__ void __launch_bounds__(256)
 k_init_liu(const uint32_t* __restrict__ off, const uint32_t* __restrict__ perm, const LiuEntry* __restrict__ ent, const EqTab* __restrict__ eqs,
            uint32_t S_pre, uint32_t K, EqTab equ, const F* __restrict__ s0_ptr, const F* __restrict__ Vpre,
            F* __restrict__ tV, F* __restrict__ tM, F* __restrict__ tA, ShardMap sm, uint32_t n_local, int write_a,
-           int equ_scaled, int write_v) {
+           int equ_scaled, int write_v, size_t ss) {
+    equ = stmt_at(equ, ss); s0_ptr = stmt_at(s0_ptr, ss);
+    tV = stmt_at(tV, ss); tM = stmt_at(tM, ss); tA = stmt_at(tA, ss);
+    Vpre += (size_t)blockIdx.z * K * S_pre;
     const uint32_t n = S_pre * K;
     const F s0 = *s0_ptr;
     for (uint32_t loc0 = blockIdx.x * blockDim.x + threadIdx.x; loc0 < n_local; loc0 += gridDim.x * blockDim.x) {
@@ -809,7 +854,7 @@ k_init_liu(const uint32_t* __restrict__ off, const uint32_t* __restrict__ perm, 
         if (!equ_scaled) M = f_mul(M, s0);
         for (uint32_t e = off[u0]; e < off[u0 + 1]; ++e) {   // the running sum rides as the addend of each product's reduction
             const LiuEntry E = ent[e];
-            M = eq_at_acc_w(eqs[E.eq_id], (K - 1 - k) * E.D + E.slot0, M);
+            M = eq_at_acc_w(stmt_at(eqs[E.eq_id], ss), (K - 1 - k) * E.D + E.slot0, M);
         }
         if (write_v) st_f(tV + loc, ld_f(Vpre + u));   // unsharded whole-proof mode reads V straight from circuitValue
         st_f(tM + loc, f_strict(M));
@@ -827,33 +872,36 @@ __global__ void __launch_bounds__(256)
 k_init_liu_tm(const uint32_t* __restrict__ off, const uint32_t* __restrict__ perm, const LiuEntry* __restrict__ ent, const EqTab* __restrict__ eqs,
               uint32_t S_pre, uint32_t K, uint32_t k_chunk, EqTab equ, const F* __restrict__ s0_ptr, const F* __restrict__ Vpre,
               F* __restrict__ tV, F* __restrict__ tM, F* __restrict__ tA, int write_a, int equ_scaled, int write_v, ShardMap sm,
-              uint32_t k_begin, uint32_t k_end) {
+              uint32_t k_begin, uint32_t k_end, size_t ss) {
     const uint32_t x = blockIdx.x * blockDim.x + threadIdx.x;
     if (x >= S_pre) return;
+    // this statement's buffers are zo entries on, its values vz: two offsets instead of six shifted pointers (registers)
+    const size_t zo = (size_t)blockIdx.z * (ss / sizeof(F)), vz = (size_t)blockIdx.z * K * S_pre;
     const uint32_t u0 = perm ? perm[x] : x;
     const uint32_t eb = off[u0], n_terms = off[u0 + 1] - eb;
     const uint32_t k0 = k_begin + blockIdx.y * k_chunk, k1 = min(k_end, k0 + k_chunk);   // sharded: the instances the rank's rows touch
-    const F s0 = *s0_ptr;
+    const F s0 = s0_ptr[zo];
     // the first two scattered terms live in registers (most entries have at most two)
     LiuEntry E0{0, 0, 0}, E1{0, 0, 0};
-    EqTab T0 = equ, T1 = equ;
-    if (n_terms >= 1) { E0 = ent[eb]; T0 = eqs[E0.eq_id]; }
-    if (n_terms >= 2) { E1 = ent[eb + 1]; T1 = eqs[E1.eq_id]; }
+    const EqTab eu{equ.f + zo, equ.s + zo, equ.fh, equ.mask};
+    EqTab T0 = eu, T1 = eu;
+    if (n_terms >= 1) { E0 = ent[eb]; T0 = stmt_at(eqs[E0.eq_id], ss); }
+    if (n_terms >= 2) { E1 = ent[eb + 1]; T1 = stmt_at(eqs[E1.eq_id], ss); }
     for (uint32_t k = k0; k < k1; ++k) {
         const uint32_t u = k * S_pre + u0, kk = K - 1 - k;
         uint32_t loc;
         if (!shard_local(sm, u, loc)) continue;   // (sharded) a row of another rank
-        F M = eq_at_weak(equ, u);
+        F M = eq_at_weak(eu, u);
         if (!equ_scaled) M = f_mul(M, s0);
         if (n_terms >= 1) M = eq_at_acc_w(T0, kk * E0.D + E0.slot0, M);
         if (n_terms >= 2) M = eq_at_acc_w(T1, kk * E1.D + E1.slot0, M);
         for (uint32_t q = 2; q < n_terms; ++q) {
             const LiuEntry E = ent[eb + q];
-            M = eq_at_acc_w(eqs[E.eq_id], kk * E.D + E.slot0, M);
+            M = eq_at_acc_w(stmt_at(eqs[E.eq_id], ss), kk * E.D + E.slot0, M);
         }
-        if (write_v) st_f(tV + loc, ld_f(Vpre + u));
-        st_f(tM + loc, f_strict(M));
-        if (write_a) st_f(tA + loc, f_zero());
+        if (write_v) st_f(tV + zo + loc, ld_f(Vpre + vz + u));
+        st_f(tM + zo + loc, f_strict(M));
+        if (write_a) st_f(tA + zo + loc, f_zero());
     }
 }
 
@@ -2019,8 +2067,11 @@ __global__ void __launch_bounds__(256) k_xchg(XchgArgs p) {
 // ------------------------------------------------------------------ K8 / K9: MLE evaluation = dot with eq
 // prover.cpp:99-129 (Vres) and :532-540 (inner_prod against eq(r_liu,.), verifier.cpp:368-369).
 __global__ void __launch_bounds__(256)
-k_dot_eq(const F* __restrict__ X, uint32_t begin, uint32_t n, EqTab eq, F* __restrict__ out, F* partials, unsigned int* counter) {
+k_dot_eq(const F* __restrict__ X, uint32_t begin, uint32_t n, EqTab eq, F* __restrict__ out, F* partials, unsigned int* counter,
+         size_t ss) {
     __shared__ F smem[32];
+    X += (size_t)blockIdx.z * n;   // statement b's slice of the layer (a batch lays the statements' layers end to end)
+    eq = stmt_at(eq, ss); out = stmt_at(out, ss); partials = stmt_at(partials, ss); counter = stmt_at(counter, ss);
     Acc acc = acc_zero();
     F run = f_zero();
     int pending = 0;

@@ -287,7 +287,9 @@ __global__ void __launch_bounds__(128) k_pc_leaf_hash(const F* __restrict__ l_ev
     o[0] = h[0]; o[1] = h[1]; o[2] = h[2]; o[3] = h[3];
 }
 // merkle_tree.cpp:39-50: one level of the array heap: node lvl + i = H(node 2(lvl + i) | node 2(lvl + i) + 1)
-__global__ void __launch_bounds__(128) k_pc_merkle_level(uint64_t* __restrict__ tree, uint32_t lvl) {
+// (blockIdx.y: one of several trees, tree_stride words apart)
+__global__ void __launch_bounds__(128) k_pc_merkle_level(uint64_t* __restrict__ tree, uint32_t lvl, size_t tree_stride) {
+    tree += blockIdx.y * tree_stride;
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= lvl) return;
     const uint64_t* c = tree + (size_t)(2 * (lvl + i)) * 4;
@@ -299,7 +301,8 @@ __global__ void __launch_bounds__(128) k_pc_merkle_level(uint64_t* __restrict__ 
     o[0] = h[0]; o[1] = h[1]; o[2] = h[2]; o[3] = h[3];
 }
 // the top of the tree (levels of <= 128 nodes) in one block
-__global__ void __launch_bounds__(128) k_pc_merkle_top(uint64_t* __restrict__ tree, uint32_t first_lvl) {
+__global__ void __launch_bounds__(128) k_pc_merkle_top(uint64_t* __restrict__ tree, uint32_t first_lvl, size_t tree_stride) {
+    tree += blockIdx.y * tree_stride;
     for (uint32_t lvl = first_lvl; lvl >= 1; lvl >>= 1) {
         const uint32_t i = threadIdx.x;
         if (i < lvl) {
@@ -563,16 +566,17 @@ static void pc_merkle(PcCommit* p, const F* eval, uint64_t* tree, cudaStream_t s
     ++p->launches;
     pc_tree_levels(p, tree, half, st);
 }
-// the inner nodes of an array heap whose n_leaves (a power of two >= 2) leaves are in place
-static int pc_tree_levels_raw(uint64_t* tree, uint32_t n_leaves, cudaStream_t st) {
+// the inner nodes of an array heap whose n_leaves (a power of two >= 2) leaves are in place (n_trees such heaps,
+// tree_stride words apart, in the same launches)
+static int pc_tree_levels_raw(uint64_t* tree, uint32_t n_leaves, cudaStream_t st, uint32_t n_trees = 1, size_t tree_stride = 0) {
     int launches = 0;
     uint32_t lvl = n_leaves / 2;
     for (; lvl > 128; lvl >>= 1) {
-        k_pc_merkle_level<<<(lvl + 127) / 128, 128, 0, st>>>(tree, lvl);
+        k_pc_merkle_level<<<dim3((lvl + 127) / 128, n_trees), 128, 0, st>>>(tree, lvl, tree_stride);
         ++launches;
     }
     if (lvl >= 1) {
-        k_pc_merkle_top<<<1, 128, 0, st>>>(tree, lvl);
+        k_pc_merkle_top<<<dim3(1, n_trees), 128, 0, st>>>(tree, lvl, tree_stride);
         ++launches;
     }
     return launches;
@@ -586,8 +590,10 @@ static void pc_tree_levels(PcCommit* p, uint64_t* tree, uint32_t n_leaves, cudaS
 // subtree root at its place in the array heap, so that k_pc_merkle_level / k_pc_merkle_top only see the upper levels
 // (a tree of 2^21 leaves: 8 launches instead of 16). The per-level hashes are the same ones either way.
 __global__ void __launch_bounds__(128) k_pc_vec_leaves(const uint64_t* __restrict__ words, size_t n_words, uint32_t log_leaves,
-                                                       uint32_t climb, uint64_t* __restrict__ tree) {
+                                                       uint32_t climb, uint64_t* __restrict__ tree, size_t tree_stride) {
     __shared__ uint64_t sh[128][4];
+    words += blockIdx.y * n_words;   // vector blockIdx.y of a batch: the vectors lie end to end, each tree tree_stride words
+    tree += blockIdx.y * tree_stride;
     const uint32_t t = threadIdx.x, width = 1u << climb;
     const size_t leaf = (size_t)blockIdx.x * width + t;
     if (t < width) {
@@ -627,14 +633,17 @@ size_t pc_vector_root_scratch(size_t n_words) {   // nodes 0 .. 2^(k - climb + 1
     const uint32_t k = pc_vector_log_leaves(n_words);
     return (size_t)64 << (k - std::min<uint32_t>(k, 7));
 }
-int pc_vector_root(const uint64_t* d_words, size_t n_words, uint64_t* d_scratch, uint8_t* d_root, cudaStream_t st) {
+int pc_vector_root(const uint64_t* d_words, size_t n_words, uint64_t* d_scratch, uint8_t* d_root, cudaStream_t st, uint32_t n_vec,
+                   size_t root_stride) {
     const uint32_t k = pc_vector_log_leaves(n_words), climb = std::min<uint32_t>(k, 7);
     if (k - climb > 31) throw std::runtime_error("vector root: more than 2^38 leaves");
-    const size_t blocks = (size_t)1 << (k - climb);
-    k_pc_vec_leaves<<<(unsigned)blocks, 128, 0, st>>>(d_words, n_words, k, climb, d_scratch);
-    int launches = 1 + pc_tree_levels_raw(d_scratch, (uint32_t)blocks, st);
+    if (n_vec < 1 || n_vec > 65535) throw std::runtime_error("vector root: 1 to 65535 vectors per pass");
+    const size_t blocks = (size_t)1 << (k - climb), tree_words = pc_vector_root_scratch(n_words) / 8;
+    k_pc_vec_leaves<<<dim3((unsigned)blocks, n_vec), 128, 0, st>>>(d_words, n_words, k, climb, d_scratch, tree_words);
+    int launches = 1 + pc_tree_levels_raw(d_scratch, (uint32_t)blocks, st, n_vec, tree_words);
     PCK(cudaGetLastError());
-    PCK(cudaMemcpyAsync(d_root, d_scratch + 4, 32, cudaMemcpyDeviceToDevice, st));
+    if (n_vec == 1) PCK(cudaMemcpyAsync(d_root, d_scratch + 4, 32, cudaMemcpyDeviceToDevice, st));
+    else PCK(cudaMemcpy2DAsync(d_root, root_stride, d_scratch + 4, tree_words * 8, 32, n_vec, cudaMemcpyDeviceToDevice, st));
     return launches;
 }
 

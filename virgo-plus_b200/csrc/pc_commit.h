@@ -53,7 +53,10 @@ uint64_t pc_launches(const PcCommit* p);
 // 8))), leaf j = SHA3-256(block j), an array-heap tree with node = SHA3-256(left | right), root = node 1 (with one leaf: that
 // leaf's hash). d_scratch: pc_vector_root_scratch(n_words) bytes; the 32-byte root goes to d_root (device). Asynchronous on
 // `st`; returns the number of kernel launches.
+// n_vec > 1: the roots of n_vec vectors of n_words words each, lying end to end from d_words, in the same launches;
+// d_scratch holds n_vec * pc_vector_root_scratch(n_words) bytes and root v goes to d_root + v * root_stride bytes.
 size_t pc_vector_root_scratch(size_t n_words);
-int pc_vector_root(const uint64_t* d_words, size_t n_words, uint64_t* d_scratch, uint8_t* d_root, cudaStream_t st);
+int pc_vector_root(const uint64_t* d_words, size_t n_words, uint64_t* d_scratch, uint8_t* d_root, cudaStream_t st, uint32_t n_vec = 1,
+                   size_t root_stride = 0);
 
 }  // namespace vp
