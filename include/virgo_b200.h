@@ -333,6 +333,31 @@ int vp_fs_round_stamps(vp_ctx* ctx, unsigned long long* out, size_t cap, size_t*
  * vp_last_prove_ms / vp_last_prove_launches describe the batch; vp_fs_round_stamps are statement 0's. */
 int vp_prove_fs_bound_batch(vp_ctx* ctx, size_t B, const uint64_t* inputs, size_t n_inputs, const uint8_t* contexts,
                             vp_F* transcripts, size_t cap, vp_F* challenges, size_t ch_cap, uint8_t* statements);
+/* The output layers of the last successful vp_prove_fs_bound_batch: B * (instances * layer_size(n-1)) elements, statement-major
+ * (what a verifier passes to vp_verify_fs_bound(_batch) as the claimed outputs). Valid until the next batch call on the
+ * context (vp_prove_fs_bound_batch or vp_verify_fs_bound_batch). VP_ERR_ARG: no batch has run, the last batch failed,
+ * or cap is too small. */
+int vp_last_batch_outputs(vp_ctx* ctx, vp_F* out, size_t cap);
+/* B statement-bound proofs of this context's circuit checked in one pass. inputs / contexts as vp_prove_fs_bound_batch;
+ * outputs: B * (instances * layer_size(n-1)) claimed outputs, statement-major; transcripts: B * n_tr, statement-major.
+ * accept / fail_code / fail_layer: B entries each (fail_code / fail_layer may be NULL); challenges (may be NULL, ch_cap >=
+ * B * n_chal): statement-major.
+ * Verdict b is, exactly, (accept, fail_code, fail_layer) of vp_verify_fs_bound(context b, outputs b, transcript b) on a
+ * context whose resident inputs are inputs b, and challenges b are what vp_fs_challenges derives from statement b and
+ * transcript b. A non-canonical transcript element rejects that statement alone (code 7, layer 0; its challenges are
+ * zero). VP_ERR_ARG: B not in [1, 65535], a count that does not match B, an input >= p or a non-canonical output
+ * (vp_last_error names the statement), a sharded context.
+ * The context's resident inputs, values, transcript and challenges are not changed (vp_verify_fs_bound, in contrast,
+ * leaves the proof's challenges resident).
+ * On the device: one upload, the roots and statements of all B statements (as in the batch prover), every challenge
+ * replayed from the transcripts by one warp per statement (k_fs_replay), then the verifier's O(#gates) sums, the
+ * outputs' MLE at r_out and the input MLE of every statement, one sequence of launches for all B (the launch count
+ * does not grow with B); one read-back of the sums and the challenges, then the round checks on the host. Memory: the
+ * batch prover's slab for B statements (vp_prove_fs_bound_batch), plus the verifier's sums per statement.
+ * vp_last_prove_ms / vp_last_prove_launches describe the call. */
+int vp_verify_fs_bound_batch(vp_ctx* ctx, size_t B, const uint64_t* inputs, size_t n_inputs, const uint8_t* contexts,
+                             const vp_F* outputs, size_t n_outputs, const vp_F* transcripts, size_t n_tr,
+                             int* accept, int* fail_code, int* fail_layer, vp_F* challenges, size_t ch_cap);
 
 /* Self-test of the device-only arithmetic paths of csrc/field.cuh (inline-PTX carry chains, mul.wide / mad.wide):
    runs one routine on n caller-provided operand triples and returns the results, so that tests can feed edge values

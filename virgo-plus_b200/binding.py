@@ -136,6 +136,9 @@ def _declare(L):
                                      C.POINTER(C.c_int)]
     L.vp_fs_round_stamps.argtypes = [vp, vp, C.c_size_t, C.POINTER(C.c_size_t)]
     L.vp_prove_fs_bound_batch.argtypes = [vp, C.c_size_t, vp, C.c_size_t, vp, vp, C.c_size_t, vp, C.c_size_t, vp]
+    L.vp_last_batch_outputs.argtypes = [vp, vp, C.c_size_t]
+    L.vp_verify_fs_bound_batch.argtypes = [vp, C.c_size_t, vp, C.c_size_t, vp, vp, C.c_size_t, vp, C.c_size_t, vp, vp, vp, vp,
+                                           C.c_size_t]
     L.vp_get_transcript.argtypes = [vp, vp, C.c_size_t]
     L.vp_last_prove_ms.argtypes = [vp]
     L.vp_last_prove_ms.restype = C.c_float
@@ -706,10 +709,8 @@ class Prover:
         _ck(lib().vp_prove_fs_bound(self.h, _context(context), _ptr(tr), len(tr), _ptr(ch), len(ch), _ptr(st)))
         return tr, ch, st.tobytes()
 
-    def prove_fs_bound_batch(self, inputs, contexts):
-        """B independent statement-bound proofs of this circuit in one pass: inputs [B, n_inputs], contexts B `bytes` of 32
-        or a [B, 32] uint8 array -> (transcripts [B, n_tr], challenges [B, n_chal], statements [B, 32] uint8); proof b ==
-        prove_fs_bound(contexts[b]) after set_inputs(inputs[b]). The resident inputs and values are not changed."""
+    def _batch_statements(self, inputs, contexts):
+        """checked (inputs [B, n_inputs] uint64, contexts [B, 32] uint8) of a batch call"""
         n_in = self.circuit.layer_size(0) * self.circuit.instances
         inputs = np.asarray(inputs)
         if inputs.ndim != 2 or inputs.shape[1] != n_in or inputs.shape[0] < 1:
@@ -726,14 +727,48 @@ class Prover:
             if len(contexts) != B:
                 raise ValueError(f"{B} statements need {B} contexts, got {len(contexts)}")
             ctx = np.frombuffer(b"".join(_context(c) for c in contexts), np.uint8).reshape(B, 32)
-        inputs = np.ascontiguousarray(inputs, dtype=np.uint64)
+        return np.ascontiguousarray(inputs, dtype=np.uint64), ctx
+
+    def _n_outputs(self):
+        return self.circuit.layer_size(self.circuit.n_layers - 1) * self.circuit.instances
+
+    def prove_fs_bound_batch(self, inputs, contexts, return_outputs=False):
+        """B independent statement-bound proofs of this circuit in one pass: inputs [B, n_inputs], contexts B `bytes` of 32
+        or a [B, 32] uint8 array -> (transcripts [B, n_tr], challenges [B, n_chal], statements [B, 32] uint8), and with
+        return_outputs the statements' output layers [B, n_outputs] as well; proof b == prove_fs_bound(contexts[b]) after
+        set_inputs(inputs[b]). The resident inputs and values are not changed."""
+        inputs, ctx = self._batch_statements(inputs, contexts)
+        B = inputs.shape[0]
         n_tr, n_ch = self.circuit.transcript_len, self.circuit.challenge_count
         tr = np.zeros((B, n_tr), F_DTYPE)
         ch = np.zeros((B, n_ch), F_DTYPE)
         st = np.zeros((B, 32), np.uint8)
         _ck(lib().vp_prove_fs_bound_batch(self.h, B, _ptr(inputs), inputs.size, _ptr(ctx), _ptr(tr), tr.size, _ptr(ch), ch.size,
                                           _ptr(st)))
-        return tr, ch, st
+        if not return_outputs:
+            return tr, ch, st
+        out = np.zeros((B, self._n_outputs()), F_DTYPE)
+        _ck(lib().vp_last_batch_outputs(self.h, _ptr(out), out.size))
+        return tr, ch, st, out
+
+    def verify_fs_bound_batch(self, inputs, contexts, outputs, transcripts, return_challenges=False):
+        """B statement-bound proofs checked in one pass: inputs and contexts as prove_fs_bound_batch, the claimed outputs
+        [B, n_outputs] and the transcripts [B, n_tr] (F_DTYPE) -> (accept bool[B], fail_code int32[B], fail_layer int32[B]),
+        and with return_challenges the challenges [B, n_chal]; verdict b == verify_fs_bound(contexts[b], outputs[b],
+        transcripts[b]) after set_inputs(inputs[b]). The resident inputs, values and challenges are not changed."""
+        inputs, ctx = self._batch_statements(inputs, contexts)
+        B = inputs.shape[0]
+        for name, a, n in (("outputs", outputs, self._n_outputs()), ("transcripts", transcripts, self.circuit.transcript_len)):
+            if not isinstance(a, np.ndarray) or a.dtype != F_DTYPE or a.shape != (B, n):
+                raise ValueError(f"{name} must be a [{B}, {n}] field-element array, got "
+                                 f"{getattr(a, 'dtype', type(a))} {getattr(a, 'shape', None)}")
+        out, tr = np.ascontiguousarray(outputs), np.ascontiguousarray(transcripts)
+        acc, code, layer = np.zeros(B, np.int32), np.zeros(B, np.int32), np.zeros(B, np.int32)
+        ch = np.zeros((B, self.circuit.challenge_count), F_DTYPE) if return_challenges else None
+        _ck(lib().vp_verify_fs_bound_batch(self.h, B, _ptr(inputs), inputs.size, _ptr(ctx), _ptr(out), out.size, _ptr(tr), tr.size,
+                                           _ptr(acc), _ptr(code), _ptr(layer), _ptr(ch), 0 if ch is None else ch.size))
+        res = (acc.astype(bool), code, layer)
+        return res + (ch,) if return_challenges else res
 
     def verify_fs_bound(self, context, outputs, transcript):
         """(accept, fail_code, fail_layer) of a statement-bound proof for the claimed outputs and this context's inputs"""

@@ -1020,6 +1020,12 @@ struct Engine {
     // verifier (SURVEY 8(f) N2): O(#gates) sums on the device, protocol checks on the host
     void verify_prepare(int i);
     int verify(const F* tr, int* fail_code, int* fail_layer);
+    // the device half of verify: out_total sums per statement (vf_layout), queued into out (partials: vf_max_b * VF_GX * 2)
+    uint32_t vf_out_total = 0, vf_max_b = 1;
+    void vf_layout();
+    void verify_sums_async(F* out, F* partial);
+    // the host half: the protocol driver on one transcript, its sums and its challenges
+    int verify_check(const F* tr, const F* out, const F* chal, int* fail_code, int* fail_layer) const;
     DBuf<F> d_vf_partial, d_vf_out, d_vf_gather;
     static constexpr uint32_t VF_GX = 64;
     DBuf<ChainDesc> d_chains;
@@ -1038,7 +1044,9 @@ struct Engine {
     size_t fs_rounds = 0;                  // rounds of the last device FS proof (4 stamps each)
     DBuf<uint64_t> d_stmt;                 // {circuit, inputs, outputs, statement} digests, 4 words each
     DBuf<uint64_t> d_root_scratch;
-    DBuf<F> d_fs_outputs;                  // vp_verify_fs_bound: the claimed outputs
+    DBuf<F> d_fs_outputs;                  // vp_verify_fs_bound(_batch): the claimed outputs, statements end to end
+    DBuf<FsStep> d_fs_steps;               // vp_verify_fs_bound_batch: the store / draw order of a transcript (k_fs_replay)
+    void fs_replay_table();
     bool circuit_digest_ready = false;
     int cap_phase_fs = 0;
     void fs_alloc();
@@ -1071,6 +1079,7 @@ struct Engine {
         DBuf<uint8_t> mem;
         size_t o_buf[6] = {0}, o_chal = 0, o_tr = 0, o_scal = 0, o_claims = 0, o_partials = 0, o_counter = 0, o_rowpart = 0, o_eq = 0,
                o_hs = 0, o_pool = 0, o_stmt = 0;
+        size_t o_vf = 0, vf_entries = 0;   // vp_verify_fs_bound_batch: the verifier's sums and partial sums (0: none yet)
         std::vector<DBuf<F>> val;
         DBuf<F*> valptr;
         DBuf<uint64_t> inputs, contexts, root_scratch;
@@ -1079,7 +1088,8 @@ struct Engine {
         std::vector<std::pair<void*, size_t>> views;   // statement 0's buffers in the slab (the context's while swapped)
     } slab;
     const uint64_t* d_circuit_digest = nullptr;   // the context's circuit digest (d_stmt[0 .. 4), shared by a batch)
-    void slab_reserve(uint32_t B);
+    uint32_t batch_outputs = 0;   // statements of the last successful vp_prove_fs_bound_batch, whose outputs are in slab.val[n-1]
+    void slab_reserve(uint32_t B, size_t vf_entries = 0);
     void slab_swap();   // exchanges the context's buffers with the slab's (an involution)
     void fs_absorb_draw(uint32_t tr_begin, uint32_t n_store, uint32_t ci_begin, uint32_t n_draw) {
         k_fs_absorb_draw<<<sgrid(1), 32, 0, stream>>>(d_fs_pool.p, d_tr.p, tr_begin, n_store, d_chal.p, ci_begin, n_draw, sstride);
@@ -2369,6 +2379,51 @@ void Engine::verify_prepare(int i) {
     D.vf_ready = true;
 }
 
+// Where each layer's sums go: L[i].vf_out; vf_out_total entries per statement, the last two being the input MLE and (a
+// batch only) the claimed outputs' MLE at r_out.
+void Engine::vf_layout() {
+    uint32_t out_total = 0, max_b = 1;
+    for (int i = 1; i < n; ++i) {
+        verify_prepare(i);
+        L[i].vf_out = out_total;
+        out_total += 2u * ((uint32_t)L[i].vf_key.size() + L[i].n_vf_liu);
+        max_b = std::max<uint32_t>(max_b, std::max<uint32_t>((uint32_t)L[i].vf_key.size(), L[i].n_vf_liu));
+    }
+    vf_out_total = out_total + 2;
+    vf_max_b = max_b;
+}
+
+// All O(#gates) sums of every layer and the input MLE into out (vf_out_total entries), with the challenges in d_chal and
+// circuitValue[0] loaded. A batch: every statement's sums at once, statement b's out and partial sstride bytes apart; the
+// x-width of a bucket shrinks with the batch (as grid_b does) so that a large batch does not launch B x VF_GX blocks.
+void Engine::verify_sums_async(F* out, F* partial) {
+    const uint32_t gx = std::max<uint32_t>(1, VF_GX / n_stmt);
+    for (int i = n - 1; i >= 1; --i) {
+        LayerDev& D = L[i];
+        const uint32_t S_pre = (uint32_t)C.layers[i - 1].size, nb = (uint32_t)D.vf_key.size();
+        const int pb = C.bit_length(i - 1), m = D.max_dad_bl;
+        run_eq(D.eqb_g, 2);
+        run_eq(D.eqb_u, 2);
+        if (m != -1) run_eq(D.eqb_v, 2);
+        if (nb) {
+            k_verify_sums<<<sgrid(gx, nb), 256, 0, stream>>>(D.vf_buckets.p, D.vf_gates.p, D.vf_assert.p, D.c.p, S_pre, D.S, K,
+                                                           eqtab(0, C.bit_length(i)), eqtab(1, pb), eqtab(6 + (uint32_t)n, std::max(m, 0)),
+                                                           d_chal.p + D.ci_assert, partial, ko_lo, ko_hi, sstride);
+            k_verify_reduce<<<sgrid(nb), 64, 0, stream>>>(partial, gx, out + D.vf_out, sstride);
+            launches += 2;
+        }
+        run_eq(D.eqb_u1, 2);                 // sig[0] * eq(r_u, .)
+        run_eq(D.eqb_rl, 2);                 // eq(r_liu, .)
+        run_eq(D.eqb_liu, D.n_eqb_liu);      // sig[j - pre] * eq(r_v[j], .)
+        k_verify_gr<<<sgrid(gx, D.n_vf_liu), 256, 0, stream>>>(D.vf_liu.p, D.liu_eqtabs.p, eqtab(3 + (uint32_t)n, pb),
+                                                              eqtab(7 + (uint32_t)n, pb), S_pre, K, partial, ko_lo, ko_hi, sstride);
+        k_verify_reduce<<<sgrid(D.n_vf_liu), 64, 0, stream>>>(partial, gx, out + D.vf_out + 2 * nb, sstride);
+        launches += 2;
+    }
+    run_eq(eqb_in, 2);
+    run_dot_eq(val[0].p, (uint32_t)C.layers[0].size, eqtab(2, C.bit_length(0)), out + vf_out_total - 2, /*local_only=*/true);
+}
+
 // verifier::verify (verifier.cpp:134-337) on a host transcript; challenges = the stream set by vp_set_challenges /
 // vp_prove. Returns 1 (accept) or 0 with the failing check: 1 phase-1 round, 2 phase-2 round, 3 final value of the
 // layer, 4 Liu round, 5 Liu final, 6 input layer -- the codes of the CPU oracle's verifier (tests compare them).
@@ -2379,47 +2434,17 @@ int Engine::verify(const F* tr, int* fail_code, int* fail_layer) {
     if (h_chal.size() < n_chal) throw CudaError{"vp_verify: challenges not set"};
     if (active) throw CudaError{"vp_verify: lanes not joined"};
     // ---- device: all O(#gates) sums, every layer, results in one buffer
-    uint32_t out_total = 0, max_b = 1;
-    for (int i = 1; i < n; ++i) {
-        verify_prepare(i);
-        L[i].vf_out = out_total;
-        out_total += 2u * ((uint32_t)L[i].vf_key.size() + L[i].n_vf_liu);
-        max_b = std::max<uint32_t>(max_b, std::max<uint32_t>((uint32_t)L[i].vf_key.size(), L[i].n_vf_liu));
-    }
-    out_total += 2;   // input MLE
+    vf_layout();
+    const uint32_t out_total = vf_out_total;
     if (d_vf_out.n < out_total) d_vf_out.alloc(out_total);
-    if (d_vf_partial.n < (size_t)max_b * VF_GX * 2) d_vf_partial.alloc((size_t)max_b * VF_GX * 2);
+    if (d_vf_partial.n < (size_t)vf_max_b * VF_GX * 2) d_vf_partial.alloc((size_t)vf_max_b * VF_GX * 2);
     {   // circuitValue[0] from the resident inputs (the verifier does not evaluate the circuit)
         const uint32_t S0 = (uint32_t)C.layers[0].size, b0 = k_lo * S0, e0 = k_hi * S0;   // the inputs this rank holds
         k_load_inputs<<<cdiv(std::max<uint32_t>(e0 - b0, 1), 256), 256, 0, stream>>>(d_inputs.p, val[0].p, b0, e0);
         ++launches;
     }
     CK(cudaMemsetAsync(d_vf_out.p, 0, (size_t)out_total * sizeof(F), stream));
-    for (int i = n - 1; i >= 1; --i) {
-        LayerDev& D = L[i];
-        const uint32_t S_pre = (uint32_t)C.layers[i - 1].size, nb = (uint32_t)D.vf_key.size();
-        const int pb = C.bit_length(i - 1), m = D.max_dad_bl;
-        run_eq(D.eqb_g, 2);
-        run_eq(D.eqb_u, 2);
-        if (m != -1) run_eq(D.eqb_v, 2);
-        if (nb) {
-            k_verify_sums<<<dim3(VF_GX, nb), 256, 0, stream>>>(D.vf_buckets.p, D.vf_gates.p, D.vf_assert.p, D.c.p, S_pre, D.S, K,
-                                                              eqtab(0, C.bit_length(i)), eqtab(1, pb),
-                                                              eqtab(6 + (uint32_t)n, std::max(m, 0)), d_chal.p + D.ci_assert,
-                                                              d_vf_partial.p, ko_lo, ko_hi);
-            k_verify_reduce<<<nb, 64, 0, stream>>>(d_vf_partial.p, VF_GX, d_vf_out.p + D.vf_out);
-            launches += 2;
-        }
-        run_eq(D.eqb_u1, 2);                 // sig[0] * eq(r_u, .)
-        run_eq(D.eqb_rl, 2);                 // eq(r_liu, .)
-        run_eq(D.eqb_liu, D.n_eqb_liu);      // sig[j - pre] * eq(r_v[j], .)
-        k_verify_gr<<<dim3(VF_GX, D.n_vf_liu), 256, 0, stream>>>(D.vf_liu.p, D.liu_eqtabs.p, eqtab(3 + (uint32_t)n, pb),
-                                                                  eqtab(7 + (uint32_t)n, pb), S_pre, K, d_vf_partial.p, ko_lo, ko_hi);
-        k_verify_reduce<<<D.n_vf_liu, 64, 0, stream>>>(d_vf_partial.p, VF_GX, d_vf_out.p + D.vf_out + 2 * nb);
-        launches += 2;
-    }
-    run_eq(eqb_in, 2);
-    run_dot_eq(val[0].p, (uint32_t)C.layers[0].size, eqtab(2, C.bit_length(0)), d_vf_out.p + out_total - 2, /*local_only=*/true);
+    verify_sums_async(d_vf_out.p, d_vf_partial.p);
     if (world > 1) {
         if (d_vf_gather.n < (size_t)out_total * world) d_vf_gather.alloc((size_t)out_total * world);
         NCK(g_nccl.AllGather(d_vf_out.p, d_vf_gather.p, (size_t)out_total * 2, /*ncclUint64*/ 5, comm, stream));
@@ -2429,8 +2454,12 @@ int Engine::verify(const F* tr, int* fail_code, int* fail_layer) {
     std::vector<F> out(out_total);
     CK(cudaMemcpyAsync(out.data(), d_vf_out.p, (size_t)out_total * sizeof(F), cudaMemcpyDeviceToHost, stream));
     CK(cudaStreamSynchronize(stream));
+    return verify_check(tr, out.data(), h_chal.data(), fail_code, fail_layer);
+}
 
-    // ---- host: the protocol driver (canonical host arithmetic of field.cuh)
+int Engine::verify_check(const F* tr, const F* out, const F* chal, int* fail_code, int* fail_layer) const {
+    const uint32_t out_total = vf_out_total;
+    // the protocol driver (canonical host arithmetic of field.cuh)
     auto ev = [](const F* q, const F& x) { return f_mul_add(f_mul_add(q[0], x, q[1]), x, q[2]); };   // a x^2 + b x + c
     auto ok_sum = [&](const F* q, const F& claim) { return f_eq(f_add(q[2], f_add(f_add(q[0], q[1]), q[2])), claim); };
 #define VP_FAIL(cd, ly) do { if (fail_code) *fail_code = (cd); if (fail_layer) *fail_layer = (ly); return 0; } while (0)
@@ -2442,7 +2471,7 @@ int Engine::verify(const F* tr, int* fail_code, int* fail_layer) {
     for (int i = n - 1; i >= 1; --i) {
         const LayerDev& D = L[i];
         const int pb = C.bit_length(i - 1), m = D.max_dad_bl;
-        const F* r_u = h_chal.data() + D.ci_ru;
+        const F* r_u = chal + D.ci_ru;
         for (int j = 0; j < pb; ++j, ti += 3) {
             if (!ok_sum(tr + ti, previousSum)) VP_FAIL(1, i);
             previousSum = ev(tr + ti, r_u[j]);
@@ -2451,7 +2480,7 @@ int Engine::verify(const F* tr, int* fail_code, int* fail_layer) {
         claims_v[i].assign(i, f_zero());
         F bv0 = f_one();
         if (m != -1) {
-            const F* r_v = h_chal.data() + D.ci_rv;
+            const F* r_v = chal + D.ci_rv;
             for (int j = 0; j < m; ++j, ti += 3) {
                 if (!ok_sum(tr + ti, previousSum)) VP_FAIL(2, i);
                 previousSum = ev(tr + ti, r_v[j]);
@@ -2461,7 +2490,7 @@ int Engine::verify(const F* tr, int* fail_code, int* fail_layer) {
         }
         // getFinalValue (verifier.cpp:115-132) from the bucket sums
         F cl[4] = {f_zero(), f_zero(), f_zero(), f_zero()}, bias = f_zero(), res = f_zero();
-        const F* o = out.data() + D.vf_out;
+        const F* o = out + D.vf_out;
         const F one_m_cu = f_sub(f_one(), claim_u);
         for (size_t b = 0; b < D.vf_key.size(); ++b) {
             const uint32_t key = D.vf_key[b];
@@ -2496,8 +2525,8 @@ int Engine::verify(const F* tr, int* fail_code, int* fail_layer) {
         if (!f_eq(previousSum, res)) VP_FAIL(3, i);
         // verifyLiu
         const int pre = i - 1;
-        const F* sig = h_chal.data() + D.ci_sig;
-        const F* r_liu = h_chal.data() + D.ci_rliu;
+        const F* sig = chal + D.ci_sig;
+        const F* r_liu = chal + D.ci_rliu;
         previousSum = f_mul(sig[0], claim_u);
         // verifier.cpp:281-284 tests `~dadBitLength`, which is also true for an EMPTY subset (dadBitLength == INT_MIN there,
         // circuit.cpp:73): the claim the prover sent for it (0 if honest) counts, so a non-zero one is caught here
@@ -2729,8 +2758,11 @@ void Engine::fs_begin() {
 }
 
 // Batch slab: per statement a copy of every buffer below, in this order, each 256-byte aligned (slab_swap's order).
-void Engine::slab_reserve(uint32_t B) {
-    if (slab.cap >= B) return;
+void Engine::slab_reserve(uint32_t B, size_t vf_entries) {
+    if (slab.cap >= B && slab.vf_entries >= vf_entries) return;
+    vf_entries = std::max(vf_entries, slab.vf_entries);
+    B = std::max(B, slab.cap);
+    batch_outputs = 0;   // (the values are reallocated)
     size_t off = 0;
     auto put = [&](size_t bytes) { const size_t o = off; off += (bytes + 255) & ~(size_t)255; return o; };
     for (int b = 0; b < 2; ++b) {
@@ -2749,6 +2781,8 @@ void Engine::slab_reserve(uint32_t B) {
     slab.o_hs = put(d_hs.n * sizeof(F));
     slab.o_pool = put(d_fs_pool.n * sizeof(uint64_t));
     slab.o_stmt = put(d_stmt.n * sizeof(uint64_t));
+    slab.o_vf = put(vf_entries * sizeof(F));
+    slab.vf_entries = vf_entries;
     slab.cap = 0;
     slab.stride = off;
     slab.mem.alloc((size_t)B * off);
@@ -2988,6 +3022,33 @@ void Engine::prove_fs_device(const uint8_t* seed, F* tr_out, F* ch_out) {
         proof_size += (uint64_t)(2 * pb + (m != -1 ? m : 0)) * 3 * sizeof(F) + sizeof(F);
         if (m != -1) proof_size += (uint64_t)i * sizeof(F);
     }
+}
+
+// The store / draw order of prove_fs_device (and of fs_challenges below) as k_fs_replay's steps, built once per context.
+void Engine::fs_replay_table() {
+    if (d_fs_steps.p) return;
+    std::vector<FsStep> st;
+    auto rounds = [&](uint32_t tr0, uint32_t ci0, int cnt) {
+        for (int j = 0; j < cnt; ++j) st.push_back(FsStep{tr0 + 3u * (uint32_t)j, 3, ci0 + (uint32_t)j, 1});
+    };
+    st.push_back(FsStep{0, 0, ci_out, (uint32_t)C.bit_length(n - 1)});
+    uint32_t tr_prev = tr_vres;
+    for (int i = n - 1; i >= 1; --i) {
+        const LayerDev& D = L[i];
+        const int pb = C.bit_length(i - 1), m = D.max_dad_bl;
+        st.push_back(FsStep{tr_prev, 1, D.ci_assert, 1});
+        rounds(D.tr_p1, D.ci_ru, pb);
+        if (m != -1) {
+            st.push_back(FsStep{D.tr_claim_u, 1, 0, 0});
+            rounds(D.tr_p2, D.ci_rv, m);
+            st.push_back(FsStep{D.tr_claims_v, (uint32_t)i, D.ci_sig, (uint32_t)n});
+        } else
+            st.push_back(FsStep{D.tr_claim_u, 1, D.ci_sig, (uint32_t)n});
+        rounds(D.tr_liu, D.ci_rliu, pb);
+        tr_prev = D.tr_claim_liu;
+    }
+    d_fs_steps.upload(st, stream);
+    CK(cudaStreamSynchronize(stream));   // (the host vector goes out of scope)
 }
 
 // The challenges of a Fiat-Shamir transcript, recomputed from the messages alone (what a verifier does first), in the
@@ -4012,8 +4073,9 @@ struct FsBatchScope {
     std::vector<F> h_chal;
     bool evaluated;
     int pending_chunks;
-    FsBatchScope(Engine& e_, uint32_t B) : e(e_), h_chal(e_.h_chal), evaluated(e_.evaluated), pending_chunks(e_.pending_chunks) {
-        e.slab_reserve(B);
+    FsBatchScope(Engine& e_, uint32_t B, size_t vf_entries = 0)
+        : e(e_), h_chal(e_.h_chal), evaluated(e_.evaluated), pending_chunks(e_.pending_chunks) {
+        e.slab_reserve(B, vf_entries);
         e.slab_swap();
         e.n_stmt = B;
         e.sstride = e.slab.stride;
@@ -4045,6 +4107,7 @@ extern "C" int vp_prove_fs_bound_batch(vp_ctx* ctx, size_t B, const uint64_t* in
     e.leave();
     e.fs_alloc();
     e.circuit_digest_async();
+    e.batch_outputs = 0;
     const uint64_t l0 = e.launches;
     try {
         FsBatchScope scope(e, (uint32_t)B);
@@ -4062,6 +4125,107 @@ extern "C" int vp_prove_fs_bound_batch(vp_ctx* ctx, size_t B, const uint64_t* in
         return fail(VP_ERR_ASSERT, "statement %u: assert gate violated in layer %u", a.stmt, a.flag - 1);
     }
     e.last_launches = e.launches - l0;
+    e.batch_outputs = (uint32_t)B;
+    return VP_OK;
+    API_END
+}
+// The batch's output layers are still in the slab (statement-major: instance-major over B * K instances).
+extern "C" int vp_last_batch_outputs(vp_ctx* ctx, vp_F* out, size_t cap) {
+    if (!ctx || !out) return fail(VP_ERR_ARG, "null argument");
+    API_BEGIN
+    Engine& e = ctx->e;
+    cudaSetDevice(e.device);
+    if (!e.batch_outputs) return fail(VP_ERR_ARG, "vp_last_batch_outputs: no successful vp_prove_fs_bound_batch since the last batch call");
+    const size_t cnt = (size_t)e.batch_outputs * e.C.layer_size(e.n - 1);
+    if (cap < cnt) return fail(VP_ERR_ARG, "output buffer too small (%zu < %zu)", cap, cnt);
+    CK(cudaMemcpyAsync(out, e.slab.val[e.n - 1].p, cnt * sizeof(F), cudaMemcpyDeviceToHost, e.stream));
+    CK(cudaStreamSynchronize(e.stream));
+    return VP_OK;
+    API_END
+}
+extern "C" int vp_verify_fs_bound_batch(vp_ctx* ctx, size_t B, const uint64_t* inputs, size_t n_inputs, const uint8_t* contexts,
+                                        const vp_F* outputs, size_t n_outputs, const vp_F* transcripts, size_t n_tr, int* accept,
+                                        int* fail_code, int* fail_layer, vp_F* challenges, size_t ch_cap) {
+    if (!ctx || !inputs || !contexts || !outputs || !transcripts || !accept) return fail(VP_ERR_ARG, "null argument");
+    API_BEGIN
+    Engine& e = ctx->e;
+    ScopedTimer t(e);
+    if (e.world != 1) return fail(VP_ERR_ARG, "vp_verify_fs_bound_batch: sharded contexts are not supported");
+    if (B == 0 || B > 65535) return fail(VP_ERR_ARG, "batch size %zu is not in [1, 65535]", B);
+    const size_t n_in = e.C.layer_size(0), n_out = e.C.layer_size(e.n - 1);
+    if (n_inputs != B * n_in) return fail(VP_ERR_ARG, "expected %zu inputs (%zu statements of %zu), got %zu", B * n_in, B, n_in, n_inputs);
+    if (n_outputs != B * n_out) return fail(VP_ERR_ARG, "expected %zu outputs (%zu statements of %zu), got %zu", B * n_out, B, n_out, n_outputs);
+    if (n_tr != B * e.n_tr) return fail(VP_ERR_ARG, "expected %zu transcript elements (%zu statements of %zu), got %zu", B * e.n_tr, B, e.n_tr, n_tr);
+    if (challenges && ch_cap < B * e.n_chal) return fail(VP_ERR_ARG, "challenge buffer too small (%zu < %zu)", ch_cap, B * e.n_chal);
+    for (size_t i = 0; i < n_inputs; ++i)
+        if (inputs[i] >= P) return fail(VP_ERR_ARG, "input %zu of statement %zu is not < p", i % n_in, i / n_in);
+    for (size_t i = 0; i < n_outputs; ++i)
+        if (outputs[i].re >= P || outputs[i].im >= P)
+            return fail(VP_ERR_ARG, "output %zu of statement %zu is not canonical (components must be < p)", i % n_out, i / n_out);
+    // a statement with a non-canonical transcript element is rejected (code 7) on its own; its row goes up as zeros
+    const F* tr = reinterpret_cast<const F*>(transcripts);
+    std::vector<uint8_t> bad(B, 0);
+    std::vector<F> clean;
+    for (size_t b = 0; b < B; ++b) bad[b] = !fs_canonical(transcripts + b * e.n_tr, e.n_tr);
+    if (std::find(bad.begin(), bad.end(), 1) != bad.end()) {
+        clean.assign(tr, tr + n_tr);
+        for (size_t b = 0; b < B; ++b)
+            if (bad[b]) std::fill(clean.begin() + b * e.n_tr, clean.begin() + (b + 1) * e.n_tr, f_zero());
+        tr = clean.data();
+    }
+    e.leave();
+    e.fs_alloc();
+    e.circuit_digest_async();
+    e.fs_replay_table();
+    e.vf_layout();
+    e.batch_outputs = 0;
+    const uint32_t out_total = e.vf_out_total;
+    if (e.d_fs_outputs.n < n_outputs) e.d_fs_outputs.alloc(n_outputs);
+    std::vector<F> sums((size_t)B * out_total), ch((size_t)B * e.n_chal);
+    const uint64_t l0 = e.launches;
+    {
+        FsBatchScope scope(e, (uint32_t)B, (size_t)out_total + (size_t)e.vf_max_b * Engine::VF_GX * 2);
+        F* const d_out = reinterpret_cast<F*>(e.slab.mem.p + e.slab.o_vf);
+        F* const d_part = d_out + out_total;
+        CK(cudaEventRecord(e.ev0, e.stream));
+        CK(cudaMemcpyAsync(e.d_inputs.p, inputs, n_inputs * sizeof(uint64_t), cudaMemcpyHostToDevice, e.stream));
+        CK(cudaMemcpyAsync(e.d_fs_outputs.p, outputs, n_outputs * sizeof(F), cudaMemcpyHostToDevice, e.stream));
+        CK(cudaMemcpyAsync(e.slab.contexts.p, contexts, 32 * B, cudaMemcpyHostToDevice, e.stream));
+        CK(cudaMemcpy2DAsync(e.d_tr.p, e.sstride, tr, e.n_tr * sizeof(F), e.n_tr * sizeof(F), B, cudaMemcpyHostToDevice, e.stream));
+        e.memset_stmts(e.d_chal.p, (e.n_chal + 1) * sizeof(F));   // unused challenge slots are zero
+        e.memset_stmts(d_out, (size_t)out_total * sizeof(F));
+        const uint32_t n0 = (uint32_t)(B * n_in);   // circuitValue[0] of every statement, instance-major over B * K
+        k_load_inputs<<<cdiv(n0, 256), 256, 0, e.stream>>>(e.d_inputs.p, e.val[0].p, 0, n0);
+        ++e.launches;
+        e.statement_async(nullptr, e.d_fs_outputs.p, e.slab.contexts.p);
+        k_fs_replay<<<e.sgrid(1), 32, 0, e.stream>>>(e.d_fs_steps.p, (uint32_t)e.d_fs_steps.n, e.d_fs_pool.p, e.d_tr.p, e.d_chal.p, e.sstride);
+        ++e.launches;
+        // the claim chain starts from Vres: the MLE of the claimed outputs at r_out, next to the input MLE
+        e.run_eq(e.eqb_out, 2);
+        e.run_dot_eq(e.d_fs_outputs.p, (uint32_t)e.C.layers[e.n - 1].size, e.eqtab(2, e.C.bit_length(e.n - 1)), d_out + out_total - 1);
+        e.verify_sums_async(d_out, d_part);
+        CK(cudaEventRecord(e.ev1, e.stream));
+        e.copy_stmts_to_host(sums.data(), out_total * sizeof(F), d_out, out_total * sizeof(F));
+        e.copy_stmts_to_host(ch.data(), e.n_chal * sizeof(F), e.d_chal.p, e.n_chal * sizeof(F));
+        CK(cudaStreamSynchronize(e.stream));
+        CK(cudaGetLastError());
+        CK(cudaEventElapsedTime(&e.last_ms, e.ev0, e.ev1));
+    }
+    e.last_launches = e.launches - l0;
+    // the host driver, one statement at a time, in vp_verify_fs_bound's order: code 7, code 8, then vp_verify's checks
+    for (size_t b = 0; b < B; ++b) {
+        int code = 0, layer = 0, ok = 0;
+        const F* tb = tr + b * e.n_tr;
+        const F* sb = sums.data() + b * out_total;
+        if (bad[b]) code = 7;
+        else if (!f_eq(sb[out_total - 1], tb[e.tr_vres])) code = 8;
+        else ok = e.verify_check(tb, sb, ch.data() + b * e.n_chal, &code, &layer);
+        accept[b] = ok;
+        if (fail_code) fail_code[b] = code;
+        if (fail_layer) fail_layer[b] = layer;
+        if (bad[b]) std::fill(ch.begin() + b * e.n_chal, ch.begin() + (b + 1) * e.n_chal, f_zero());
+    }
+    if (challenges) memcpy(challenges, ch.data(), ch.size() * sizeof(F));
     return VP_OK;
     API_END
 }

@@ -32,11 +32,9 @@ VP_D F fs_draw(uint64_t* pool) {
     return F{fp_mod(d[0]), fp_mod(d[1])};
 }
 
-// Between phases (one warp, lane 0 hashes): store transcript[tr_begin .. + n_store), then draw chal[ci_begin .. + n_draw)
-// (host/fiat_shamir.h: Vres / claim_u / claims_v / claim_liu, then r_out / assert_random / sig).
-__global__ void k_fs_absorb_draw(uint64_t* pool, const F* __restrict__ transcript, uint32_t tr_begin, uint32_t n_store, F* chal,
-                                 uint32_t ci_begin, uint32_t n_draw, size_t ss) {
-    pool = stmt_at(pool, ss); transcript = stmt_at(transcript, ss); chal = stmt_at(chal, ss);
+// One warp, lane 0 hashes: store transcript[tr_begin .. + n_store), then draw chal[ci_begin .. + n_draw).
+VP_D void fs_absorb_draw_warp(uint64_t* pool, const F* transcript, uint32_t tr_begin, uint32_t n_store, F* chal, uint32_t ci_begin,
+                              uint32_t n_draw) {
     const uint64_t n0 = pool[0];
     __syncwarp();
     for (uint32_t k = threadIdx.x; k < n_store; k += 32) {
@@ -45,9 +43,31 @@ __global__ void k_fs_absorb_draw(uint64_t* pool, const F* __restrict__ transcrip
         pool[2 + n0 + 2 * k] = x.im;
     }
     __syncwarp();
-    if (threadIdx.x != 0) return;
-    pool[0] = n0 + 2ull * n_store;
-    for (uint32_t k = 0; k < n_draw; ++k) st_f(chal + ci_begin + k, fs_draw(pool));
+    if (threadIdx.x == 0) {
+        pool[0] = n0 + 2ull * n_store;
+        for (uint32_t k = 0; k < n_draw; ++k) st_f(chal + ci_begin + k, fs_draw(pool));
+    }
+    __syncwarp();   // (the next call's lanes read pool[0])
+}
+
+// Between phases (host/fiat_shamir.h: Vres / claim_u / claims_v / claim_liu, then r_out / assert_random / sig).
+__global__ void k_fs_absorb_draw(uint64_t* pool, const F* __restrict__ transcript, uint32_t tr_begin, uint32_t n_store, F* chal,
+                                 uint32_t ci_begin, uint32_t n_draw, size_t ss) {
+    fs_absorb_draw_warp(stmt_at(pool, ss), stmt_at(transcript, ss), tr_begin, n_store, stmt_at(chal, ss), ci_begin, n_draw);
+}
+
+// The verifier's side (vp_verify_fs_bound_batch): every challenge of a transcript recomputed from its messages, in the
+// store / draw order of host/fiat_shamir.h (fs_challenges). The order is a table of steps built once per context: one per
+// sumcheck round (store the 3 coefficients, draw the round's challenge) and one per store / draw run between phases.
+// One warp per statement (blockIdx.z), lane 0 hashes; the pool must hold the statement (k_fs_statement).
+struct FsStep { uint32_t tr_begin, n_store, ci_begin, n_draw; };
+__global__ void k_fs_replay(const FsStep* __restrict__ steps, uint32_t n_steps, uint64_t* pool, const F* __restrict__ transcript, F* chal,
+                            size_t ss) {
+    pool = stmt_at(pool, ss); transcript = stmt_at(transcript, ss); chal = stmt_at(chal, ss);
+    for (uint32_t s = 0; s < n_steps; ++s) {
+        const FsStep st = steps[s];
+        fs_absorb_draw_warp(pool, transcript, st.tr_begin, st.n_store, chal, st.ci_begin, st.n_draw);
+    }
 }
 
 // The statement (include/virgo_b200.h): H("VPSTMT01" | circuit | u64 n_inputs | inputs root | u64 n_outputs | outputs root |

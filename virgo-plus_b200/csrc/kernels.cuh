@@ -2120,6 +2120,8 @@ __global__ void k_sum_ranks(const F* __restrict__ recv, uint32_t G, uint32_t str
 // needs. They are written against the circuit wiring directly (buckets of gates, plain dadId lists) and use only the
 // canonical field routines: none of the prover's tables, CSRs or lazy/weak primitives are involved, so the
 // verifier's accept is an independent check of the prover's messages.
+// A batch (vp_verify_fs_bound_batch) runs statement b in blockIdx.z == b: its eq tables, challenges, partial sums and
+// outputs sit `ss` bytes after statement b - 1's (stmt_at); gates, buckets and Liu segments are shared.
 struct VfGate {          // one template gate in bucket order
     uint32_t g0, u0, lv0;
     uint32_t l_c;        // binary: source layer l; unary: index of the gate's constant (== g0)
@@ -2133,8 +2135,9 @@ struct VfBucket {
 __global__ void __launch_bounds__(256)
 k_verify_sums(const VfBucket* __restrict__ buckets, const VfGate* __restrict__ gates, const uint8_t* __restrict__ is_assert,
               const F* __restrict__ cst, uint32_t S_pre, uint32_t S_cur, uint32_t K, EqTab eqg, EqTab equ, EqTab eqv,
-              const F* __restrict__ assert_r, F* __restrict__ partial, uint32_t k_begin, uint32_t k_end) {
+              const F* __restrict__ assert_r, F* __restrict__ partial, uint32_t k_begin, uint32_t k_end, size_t ss) {
     __shared__ F smem[2 * 32];
+    eqg = stmt_at(eqg, ss); equ = stmt_at(equ, ss); eqv = stmt_at(eqv, ss); assert_r = stmt_at(assert_r, ss); partial = stmt_at(partial, ss);
     const VfBucket B = buckets[blockIdx.y];
     const uint64_t total = (uint64_t)B.cnt * (k_end - k_begin);   // sharded: this rank's slice of the instances
     F acc[2] = {f_zero(), f_zero()};
@@ -2157,8 +2160,9 @@ k_verify_sums(const VfBucket* __restrict__ buckets, const VfGate* __restrict__ g
     }
 }
 // out[bucket * 2 + {0,1}] = sum over the gx partials of the bucket
-__global__ void k_verify_reduce(const F* __restrict__ partial, uint32_t gx, F* __restrict__ out) {
+__global__ void k_verify_reduce(const F* __restrict__ partial, uint32_t gx, F* __restrict__ out, size_t ss) {
     __shared__ F smem[2 * 32];
+    partial = stmt_at(partial, ss); out = stmt_at(out, ss);
     F acc[2] = {f_zero(), f_zero()};
     for (uint32_t b = threadIdx.x; b < gx; b += blockDim.x) {
         acc[0] = f_add(acc[0], partial[((size_t)blockIdx.x * gx + b) * 2]);
@@ -2177,8 +2181,9 @@ struct VfLiuSeg {
 };
 __global__ void __launch_bounds__(256)
 k_verify_gr(const VfLiuSeg* __restrict__ segs, const EqTab* __restrict__ eqs, EqTab eq_g0, EqTab eq_rl, uint32_t S_pre, uint32_t K,
-            F* __restrict__ partial, uint32_t k_begin, uint32_t k_end) {
+            F* __restrict__ partial, uint32_t k_begin, uint32_t k_end, size_t ss) {
     __shared__ F smem[2 * 32];
+    eq_g0 = stmt_at(eq_g0, ss); eq_rl = stmt_at(eq_rl, ss); partial = stmt_at(partial, ss);
     const VfLiuSeg Sg = segs[blockIdx.y];
     // sharded: this rank's slice [k_begin, k_end) of the instances; a subset segment runs in reverse instance order
     const uint64_t w_lo = (uint64_t)Sg.D * (blockIdx.y == 0 ? k_begin : K - k_end), total = (uint64_t)Sg.D * (blockIdx.y == 0 ? k_end : K - k_begin);
@@ -2187,7 +2192,7 @@ k_verify_gr(const VfLiuSeg* __restrict__ segs, const EqTab* __restrict__ eqs, Eq
         if (blockIdx.y == 0) acc[0] = f_add(acc[0], f_mul(eq_at(eq_g0, (uint32_t)w), eq_at(eq_rl, (uint32_t)w)));
         else {
             const uint32_t kk = (uint32_t)(w / Sg.D), g0 = (uint32_t)(w - (uint64_t)kk * Sg.D), k = K - 1 - kk;
-            acc[0] = f_add(acc[0], f_mul(eq_at(eqs[Sg.eq_id], (uint32_t)w), eq_at(eq_rl, k * S_pre + Sg.dadId[g0])));
+            acc[0] = f_add(acc[0], f_mul(eq_at(stmt_at(eqs[Sg.eq_id], ss), (uint32_t)w), eq_at(eq_rl, k * S_pre + Sg.dadId[g0])));
         }
     }
     block_sum<2>(acc, smem);
