@@ -4,6 +4,7 @@ layers of a proving batch.
 Verdict b of a batch must be exactly the single vp_verify_fs_bound verdict (accept, code, layer) on the same data, its
 challenges those vp_fs_challenges derives; the batch must not disturb the context's resident state and must not launch
 more kernels as B grows."""
+import gc
 import random
 
 import numpy as np
@@ -82,6 +83,9 @@ def test_batch_verify_binding_rejects_bad_shapes_before_the_library(B, sha_circu
         called.append(1)
         raise AssertionError("library called")
 
+    # A context or circuit of an earlier test that the cycle collector frees during the checks would reach the patched
+    # lib() from its __del__: collect them before patching, and keep the collector off while the checks run.
+    gc.collect()
     monkeypatch.setattr(B, "lib", no_lib)
     x, ctx = np.zeros((2, n_in), np.uint64), [bytes(32)] * 2
     out, tr = np.zeros((2, n_out), F_DTYPE), np.zeros((2, n_tr), F_DTYPE)
@@ -102,10 +106,14 @@ def test_batch_verify_binding_rejects_bad_shapes_before_the_library(B, sha_circu
         (x, ctx, out, np.zeros((2, 2 * n_tr), np.uint64)),               # transcripts not field elements
         (x, ctx, out, list(tr)),                                         # not an array
     ]
-    for k, args in enumerate(bad):
-        with pytest.raises(ValueError):
-            p.verify_fs_bound_batch(*args)
-        assert not called, f"case {k}"
+    gc.disable()
+    try:
+        for k, args in enumerate(bad):
+            with pytest.raises(ValueError):
+                p.verify_fs_bound_batch(*args)
+            assert not called, f"case {k}"
+    finally:
+        gc.enable()
 
 
 # ------------------------------------------------------------------ GPU

@@ -38,23 +38,44 @@ def test_sumcheck_tables_vs_oracle(B, O, log_n):
 
 
 def test_sumcheck_edge_values(B, O):
-    """all-zero, all p-1, and base-field tables"""
-    log_n = 6
+    """edge tables (all zero, all p-1, base field, equal pairs whose fold difference is p in weak arithmetic, zero / p-1
+    alternating) x edge challenges (0, 1, p-1, i, -i, p-1 + (p-1)i, 2^31, 2^61 - 2^31) rotated through every round
+    position, at 2^6, 2^15 and 2^20 entries; one round per launch and fused (k_phase_dfs: chunked passes at 2^20, one
+    block alone at 2^6)"""
+    for log_n in (6, 15, 20):
+        _sumcheck_edge_values(B, O, log_n)
+
+
+def _sumcheck_edge_values(B, O, log_n):
+    P = B.P
     n = 1 << log_n
     rng = np.random.default_rng(5)
-    r = _rand_fe(B, rng, log_n)
-    r[0] = (0, 0)
-    r[1] = (B.P - 1, B.P - 1)
-    for fill in [(0, 0), (B.P - 1, B.P - 1), (B.P - 1, 0), (1, 0)]:
+    edge = [(0, 0), (1, 0), (P - 1, 0), (0, 1), (0, P - 1), (P - 1, P - 1), (1 << 31, 0), ((1 << 61) - (1 << 31), 0)]
+    challenges = [B.fe_array([edge[(j + o) % len(edge)] for j in range(log_n)]) for o in range(len(edge))]
+
+    def const(fill):
         T = np.zeros(n, B.F_DTYPE)
         T["re"], T["im"] = fill
-        s = B.Sumcheck(log_n)
-        s.load(T, T, T)
-        got, _ = s.run(r)
-        _assert_same(got, O.sumcheck_tables(T, T, T, r), f"fill {fill}")
-        got, _ = s.run(r, fused=True)
-        _assert_same(got, O.sumcheck_tables(T, T, T, r), f"fill {fill} fused")
-        s.close()
+        return T, T, T
+
+    def pairs():
+        T = _rand_fe(B, rng, n // 2)
+        return np.repeat(T, 2)
+
+    alt = np.zeros(n, B.F_DTYPE)
+    alt["re"][1::2] = alt["im"][1::2] = P - 1
+    fills = [("zero", const((0, 0))), ("p-1 + (p-1)i", const((P - 1, P - 1))), ("p-1", const((P - 1, 0))), ("one", const((1, 0))),
+             ("equal pairs", (pairs(), pairs(), pairs())), ("0 / p-1 + (p-1)i alternating", (alt, alt, alt))]
+    s = B.Sumcheck(log_n)
+    for name, (V, A, M) in fills:
+        s.load(V, A, M)
+        for o, r in enumerate(challenges):
+            want = O.sumcheck_tables(V, A, M, r)
+            got, _ = s.run(r)
+            _assert_same(got, want, f"2^{log_n}, {name}, challenges rotated by {o}")
+            got, _ = s.run(r, fused=True)
+            _assert_same(got, want, f"2^{log_n}, {name}, challenges rotated by {o}, fused")
+    s.close()
 
 
 def test_sumcheck_device_random_fill(B, O):
