@@ -61,10 +61,24 @@ def main():
         got4 = B.prove_interactive(p, circ)
         same4 = bool((got4["re"] == want["re"]).all() and (got4["im"] == want["im"]).all())
         size_ok = abs(p.proofSize() * 1024 - 16 * (len(want) - 1 - 1)) < 1e-6 or True
+        # Fiat-Shamir mode on the sharded context (the host-driven loop): the oracle's proof for the same seed, and the
+        # sharded verifier's verdicts on it, on a tampered message and under another seed
+        fs = "-"
+        if name in ("sha256_64 x 3", "random 4x2^5 x 37"):
+            seed = bytes(range(32))
+            tr_fs, ch_fs = p.prove_fs(seed)
+            want_tr, want_ch = oc.prove_fs(seed)
+            eq = lambda a, b: bool((a["re"] == b["re"]).all() and (a["im"] == b["im"]).all())
+            t = tr_fs.copy()
+            t[len(t) // 2]["re"] = (int(t[len(t) // 2]["re"]) + 1) % B.P
+            fs_ok = (eq(tr_fs, want_tr) and eq(ch_fs, want_ch) and p.verify_fs(seed, tr_fs) == (True, 0, 0)
+                     and not p.verify_fs(seed, t)[0] and not p.verify_fs(bytes(32), tr_fs)[0])
+            fs = "OK" if fs_ok else "MISMATCH"
         print(f"[rank {rank}/{world}] {name}: gates {circ.total_gates}, sharded phases {sharded}, transcript {len(got)} "
               f"{'OK' if same and same2 and same3 else 'MISMATCH at ' + str(bad[:8])}, sharded verifier {'OK' if vok else 'MISMATCH'}, "
-              f"interactive {'OK' if same4 else 'MISMATCH at ' + str(np.nonzero((got4['re'] != want['re']) | (got4['im'] != want['im']))[0][:8])}", flush=True)
-        ok_all &= same and same2 and same3 and vok and same4
+              f"interactive {'OK' if same4 else 'MISMATCH at ' + str(np.nonzero((got4['re'] != want['re']) | (got4['im'] != want['im']))[0][:8])}, "
+              f"fiat-shamir {fs}", flush=True)
+        ok_all &= same and same2 and same3 and vok and same4 and fs != "MISMATCH"
         p.close()
         dist.barrier()
     # A batch large enough for the ranks to differ in what they upload (250 instances per rank: on 4 GPUs only some ranks

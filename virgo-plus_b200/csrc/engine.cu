@@ -608,7 +608,8 @@ static void sort_items_by_length(std::vector<RowItem>& items) {
 }
 
 // ------------------------------------------------------------------ per-layer device data
-struct LayerDev {
+// a layer's device state; its transcript and challenge indices are the proof layout's (Engine::build copies them)
+struct LayerDev : LayerLayout {
     uint32_t S = 0;
     DBuf<uint8_t> ty;
     DBuf<int16_t> l;
@@ -640,14 +641,10 @@ struct LayerDev {
     std::vector<int> liu_j;      // source layers j of the eq tables, in eq_id order
     // plans
     PhasePlan ph1, ph2, ph3;
-    int max_dad_bl = -1;
     // eq build descriptor slices (indices into Engine::eq_descs)
     uint32_t eqb_g = 0, eqb_u = 0, eqb_u1 = 0, eqb_g2 = 0, eqb_u2 = 0, eqb_liu = 0, n_eqb_liu = 0;
     DBuf<EqTab> liu_eqtabs, liu_eqtabs_b;   // in eq region set A / B
-    // challenge indices
-    uint32_t ci_ru = 0, ci_assert = 0, ci_rv = 0, ci_sig = 0, ci_rliu = 0, ci_g = 0;
-    // transcript indices
-    uint32_t tr_p1 = 0, tr_claim_u = 0, tr_p2 = 0, tr_claims_v = 0, tr_liu = 0, tr_claim_liu = 0;
+    uint32_t ci_g = 0;   // challenges of the point g of phase 1: r_out (top layer) or r_liu of the layer above
     // verifier sums (vp_verify): gates in bucket order, built on first use
     std::vector<P2Table> h_p2;       // host copy of the phase-2 table descriptors (dadId lists on the device)
     std::vector<int> p2_src;         // source layer of each phase-2 table
@@ -835,8 +832,8 @@ struct Engine {
     uint32_t eq_half_cap = 0;          // entries of one half table
     size_t eq_set_entries = 0;         // entries of one eq region set
     uint32_t eqb_out = 0, eqb_in = 0;
-    uint32_t ci_out = 0, tr_vres = 0, tr_input = 0;
-    size_t n_chal = 0, n_tr = 0;
+    ProofLayout lay;                 // where every message and challenge of a proof sits
+    std::vector<FsEntry> fs_sched;   // the Fiat-Shamir order over lay
 
     // scalars in d_scal
     enum { SC_ADD_TERM = 0, SC_VU = 1, SC_UNARY = 2, SC_N = 4 };
@@ -1035,9 +1032,9 @@ struct Engine {
     void launch_phase_kernel(const SumcheckPlan& P, uint32_t ci, uint32_t round_base, const F* at_init, F* add_term_out,
                              F* claims, F* out_poly, F* keep);
     uint32_t tail_work = 512;
-    bool use_phase_kernel = true;
     void prove_all();
     void prove_fs(const uint8_t seed[32], F* tr_out, F* ch_out);
+    const PhasePlan& fs_phase_init(int i, int phase, F*& keep, const F*& at_init);
     // Fiat-Shamir mode on the device (fs_device.cuh): the pool, the per-round stamps and the statement digest's buffers
     DBuf<uint64_t> d_fs_pool;
     DBuf<unsigned long long> d_fs_stamps;
@@ -1198,40 +1195,21 @@ void Engine::build(const Circuit& circ, int dev, int world_, int rank_, const ui
     }
     max_grid = std::max({cap_round, cap_round1, cap_un, cap_dot, cap_phase, cap_phase_fs, cap_dfs});  // sizes the block-partials buffer
 
-    // challenge / transcript index maps (draw order of verifier.cpp, see circuit.cpp draw_challenges)
+    lay = proof_layout(C);
+    fs_sched = fs_schedule(lay);
     L.resize(n);
-    uint32_t ci = 0, ti = 0;
-    ci_out = ci;
-    ci += (uint32_t)C.bit_length(n - 1);
-    tr_vres = ti++;
     for (int i = n - 1; i >= 1; --i) {
-        LayerDev& D = L[i];
-        const int pb = C.bit_length(i - 1), m = C.max_dad_bit_length(i);
-        D.max_dad_bl = m;
-        D.ci_ru = ci; ci += (uint32_t)max_bl;
-        D.ci_assert = ci; ci += 1;
-        D.ci_rv = ci; if (m != -1) ci += (uint32_t)m;
-        D.ci_sig = ci; ci += (uint32_t)n;
-        D.ci_rliu = ci; ci += (uint32_t)max_bl;
-        D.ci_g = (i == n - 1) ? ci_out : L[i + 1].ci_rliu;
-        D.tr_p1 = ti; ti += 3u * (uint32_t)pb;
-        D.tr_claim_u = ti++;
-        D.tr_p2 = ti;
-        if (m != -1) { ti += 3u * (uint32_t)m; D.tr_claims_v = ti; ti += (uint32_t)i; }
-        D.tr_liu = ti; ti += 3u * (uint32_t)pb;
-        D.tr_claim_liu = ti++;
+        static_cast<LayerLayout&>(L[i]) = lay.layer[i];
+        L[i].ci_g = (i == n - 1) ? lay.ci_out : L[i + 1].ci_rliu;
     }
-    tr_input = ti++;
-    n_chal = ci;
-    n_tr = ti;
     {   // claim chains for k_derive_b (verifier.cpp:150-166, 281-284, 333)
         std::vector<ChainDesc> ch;
         std::vector<ChainSeg> sg;
         std::vector<ChainTerm> tm;
         for (int i = n - 1; i >= 1; --i) {
             const LayerDev& D = L[i];
-            const int pb = C.bit_length(i - 1), m = D.max_dad_bl;
-            ChainDesc c12{(int32_t)(i == n - 1 ? tr_vres : L[i + 1].tr_claim_liu), 0, 0, (uint32_t)sg.size(), 0};
+            const int pb = C.bit_length(i - 1), m = D.m;
+            ChainDesc c12{(int32_t)(i == n - 1 ? lay.tr_vres : L[i + 1].tr_claim_liu), 0, 0, (uint32_t)sg.size(), 0};
             sg.push_back(ChainSeg{D.tr_p1, (uint32_t)pb, D.ci_ru});
             if (m != -1) sg.push_back(ChainSeg{D.tr_p2, (uint32_t)m, D.ci_rv});
             c12.n_segs = (uint32_t)sg.size() - c12.seg_begin;
@@ -1239,7 +1217,7 @@ void Engine::build(const Circuit& circ, int dev, int world_, int rank_, const ui
             ChainDesc c3{-1, (uint32_t)tm.size(), 0, (uint32_t)sg.size(), 1};
             tm.push_back(ChainTerm{D.ci_sig, D.tr_claim_u});
             for (int j = i; j < n; ++j)
-                if (L[j].max_dad_bl != -1) tm.push_back(ChainTerm{D.ci_sig + (uint32_t)(j - (i - 1)), L[j].tr_claims_v + (uint32_t)(i - 1)});
+                if (L[j].m != -1) tm.push_back(ChainTerm{D.ci_sig + (uint32_t)(j - (i - 1)), L[j].tr_claims_v + (uint32_t)(i - 1)});
             c3.n_terms = (uint32_t)tm.size() - c3.term_begin;
             sg.push_back(ChainSeg{D.tr_liu, (uint32_t)pb, D.ci_rliu});
             ch.push_back(c3);
@@ -1274,7 +1252,7 @@ void Engine::build(const Circuit& circ, int dev, int world_, int rank_, const ui
     uint32_t cap0 = 4, cap1 = 4, max_rec = 0;
     size_t max_partial = 2;
     eqb_out = (uint32_t)eq_descs.size();
-    add_eq_build(2, ci_out, C.bit_length(n - 1), -1);
+    add_eq_build(2, lay.ci_out, C.bit_length(n - 1), -1);
     // The per-layer host work (gate arrays, the three CSRs cut into work items, their sorts) is independent between the
     // layers apart from the plan arena, the eq descriptor list and a few running maxima (all under `mu`): worker threads
     // take the layers from a counter, each with its own stream for the uploads. A 65 x 2^20 random circuit took 11 s here
@@ -1361,13 +1339,13 @@ void Engine::build(const Circuit& circ, int dev, int world_, int rank_, const ui
         D.eqb_u2 = (uint32_t)eq_descs.size();
         add_eq_build(5 + (uint32_t)n, D.ci_ru, pb, -1);
         D.eqb_v = (uint32_t)eq_descs.size();
-        add_eq_build(6 + (uint32_t)n, D.ci_rv, std::max(D.max_dad_bl, 0), -1);
+        add_eq_build(6 + (uint32_t)n, D.ci_rv, std::max(D.m, 0), -1);
         D.eqb_rl = (uint32_t)eq_descs.size();
         add_eq_build(7 + (uint32_t)n, D.ci_rliu, pb, -1);
         }
         // phase 2
-        if (D.max_dad_bl != -1) {
-            const int m = D.max_dad_bl;
+        if (D.m != -1) {
+            const int m = D.m;
             // table order: bits descending (stable by l); empty subsets get no table (their claim is 0)
             std::vector<int> order;
             for (int l = 0; l < i; ++l)
@@ -1602,7 +1580,7 @@ void Engine::build(const Circuit& circ, int dev, int world_, int rank_, const ui
     auto alloc_lane = [&](LaneRes& R, int role, size_t eqo) {   // role: 0 phase 1, 1 Liu, 2 phase 2
         uint32_t c0 = 4, c1 = 4;
         for (int i = 1; i < n; ++i) {
-            const PhasePlan* P = role == 0 ? &L[i].ph1 : role == 1 ? &L[i].ph3 : (L[i].max_dad_bl != -1 ? &L[i].ph2 : nullptr);
+            const PhasePlan* P = role == 0 ? &L[i].ph1 : role == 1 ? &L[i].ph3 : (L[i].m != -1 ? &L[i].ph2 : nullptr);
             if (P) { c0 = std::max(c0, P->cap0); c1 = std::max(c1, P->cap1); }
         }
         for (int bb = 0; bb < 2; ++bb) {
@@ -1681,8 +1659,8 @@ void Engine::build(const Circuit& circ, int dev, int world_, int rank_, const ui
             lane2.d_recv.alloc((size_t)std::max<uint32_t>(max_rec, 1) * world);
         }
     }
-    d_chal.alloc(n_chal + 1);
-    d_tr.alloc(n_tr);
+    d_chal.alloc(lay.n_chal + 1);
+    d_tr.alloc(lay.n_tr);
     d_scal.alloc(SC_N);
     d_claims.alloc((size_t)n + 1);
     d_partials.alloc((size_t)12 * (size_t)max_grid);
@@ -1695,8 +1673,8 @@ void Engine::build(const Circuit& circ, int dev, int world_, int rank_, const ui
     d_pcols.upload(arena.pcols, stream);
     d_pdev.upload(arena.pdev, stream);
     d_eqb.upload(eq_descs, stream);
-    CK(cudaMemsetAsync(d_chal.p, 0, (n_chal + 1) * sizeof(F), stream));
-    CK(cudaMemsetAsync(d_tr.p, 0, n_tr * sizeof(F), stream));
+    CK(cudaMemsetAsync(d_chal.p, 0, (lay.n_chal + 1) * sizeof(F), stream));
+    CK(cudaMemsetAsync(d_tr.p, 0, lay.n_tr * sizeof(F), stream));
     CK(cudaMemsetAsync(d_scal.p, 0, SC_N * sizeof(F), stream));
     CK(cudaMemsetAsync(d_claims.p, 0, ((size_t)n + 1) * sizeof(F), stream));
     CK(cudaMemsetAsync(d_counter.p, 0, (4 + 64) * sizeof(unsigned int), stream));
@@ -1886,12 +1864,12 @@ void Engine::run_dot_eq(const F* X, uint32_t S, EqTab eq, F* out, bool local_onl
 
 void Engine::do_vres() {
     run_eq(eqb_out, 2);
-    run_dot_eq(val[n - 1].p, (uint32_t)C.layers[n - 1].size, eqtab(2, C.bit_length(n - 1)), d_tr.p + tr_vres);
+    run_dot_eq(val[n - 1].p, (uint32_t)C.layers[n - 1].size, eqtab(2, C.bit_length(n - 1)), d_tr.p + lay.tr_vres);
 }
 
 void Engine::do_input_mle() {
     run_eq(eqb_in, 2);
-    run_dot_eq(val[0].p, (uint32_t)C.layers[0].size, eqtab(2, C.bit_length(0)), d_tr.p + tr_input);
+    run_dot_eq(val[0].p, (uint32_t)C.layers[0].size, eqtab(2, C.bit_length(0)), d_tr.p + lay.tr_input);
 }
 
 void Engine::do_init_phase1(int i) {
@@ -2401,7 +2379,7 @@ void Engine::verify_sums_async(F* out, F* partial) {
     for (int i = n - 1; i >= 1; --i) {
         LayerDev& D = L[i];
         const uint32_t S_pre = (uint32_t)C.layers[i - 1].size, nb = (uint32_t)D.vf_key.size();
-        const int pb = C.bit_length(i - 1), m = D.max_dad_bl;
+        const int pb = C.bit_length(i - 1), m = D.m;
         run_eq(D.eqb_g, 2);
         run_eq(D.eqb_u, 2);
         if (m != -1) run_eq(D.eqb_v, 2);
@@ -2431,7 +2409,7 @@ int Engine::verify(const F* tr, int* fail_code, int* fail_layer) {
     // Sharded context: a collective call -- every rank passes the same transcript, sums the gates of its own slice of
     // the instances (ko_lo .. ko_hi), and the partial sums of all ranks meet in ONE all-gather before the host checks.
     if (!inputs_loaded) throw CudaError{"vp_verify: inputs not loaded"};
-    if (h_chal.size() < n_chal) throw CudaError{"vp_verify: challenges not set"};
+    if (h_chal.size() < lay.n_chal) throw CudaError{"vp_verify: challenges not set"};
     if (active) throw CudaError{"vp_verify: lanes not joined"};
     // ---- device: all O(#gates) sums, every layer, results in one buffer
     vf_layout();
@@ -2466,27 +2444,28 @@ int Engine::verify_check(const F* tr, const F* out, const F* chal, int* fail_cod
     if (fail_code) *fail_code = 0;
     if (fail_layer) *fail_layer = 0;
     std::vector<std::vector<F>> claims_v(n);
-    size_t ti = 0;
-    F previousSum = tr[ti++];
+    F previousSum = tr[lay.tr_vres];
     for (int i = n - 1; i >= 1; --i) {
         const LayerDev& D = L[i];
-        const int pb = C.bit_length(i - 1), m = D.max_dad_bl;
+        const int pb = D.pb, m = D.m;
         const F* r_u = chal + D.ci_ru;
-        for (int j = 0; j < pb; ++j, ti += 3) {
-            if (!ok_sum(tr + ti, previousSum)) VP_FAIL(1, i);
-            previousSum = ev(tr + ti, r_u[j]);
+        for (int j = 0; j < pb; ++j) {
+            const F* q = tr + D.tr_p1 + 3 * j;
+            if (!ok_sum(q, previousSum)) VP_FAIL(1, i);
+            previousSum = ev(q, r_u[j]);
         }
-        const F claim_u = tr[ti++];
+        const F claim_u = tr[D.tr_claim_u];
         claims_v[i].assign(i, f_zero());
         F bv0 = f_one();
         if (m != -1) {
             const F* r_v = chal + D.ci_rv;
-            for (int j = 0; j < m; ++j, ti += 3) {
-                if (!ok_sum(tr + ti, previousSum)) VP_FAIL(2, i);
-                previousSum = ev(tr + ti, r_v[j]);
+            for (int j = 0; j < m; ++j) {
+                const F* q = tr + D.tr_p2 + 3 * j;
+                if (!ok_sum(q, previousSum)) VP_FAIL(2, i);
+                previousSum = ev(q, r_v[j]);
                 bv0 = f_mul(bv0, f_sub(f_one(), r_v[j]));   // beta_v[0]
             }
-            for (int l = 0; l < i; ++l) claims_v[i][l] = tr[ti++];
+            claims_v[i].assign(tr + D.tr_claims_v, tr + D.tr_claims_v + i);
         }
         // getFinalValue (verifier.cpp:115-132) from the bucket sums
         F cl[4] = {f_zero(), f_zero(), f_zero(), f_zero()}, bias = f_zero(), res = f_zero();
@@ -2531,17 +2510,18 @@ int Engine::verify_check(const F* tr, const F* out, const F* chal, int* fail_cod
         // verifier.cpp:281-284 tests `~dadBitLength`, which is also true for an EMPTY subset (dadBitLength == INT_MIN there,
         // circuit.cpp:73): the claim the prover sent for it (0 if honest) counts, so a non-zero one is caught here
         for (int j = i; j < n; ++j) previousSum = f_add(previousSum, f_mul(sig[j - pre], claims_v[j][pre]));
-        for (int j = 0; j < pb; ++j, ti += 3) {
-            if (!ok_sum(tr + ti, previousSum)) VP_FAIL(4, i);
-            previousSum = ev(tr + ti, r_liu[j]);
+        for (int j = 0; j < pb; ++j) {
+            const F* q = tr + D.tr_liu + 3 * j;
+            if (!ok_sum(q, previousSum)) VP_FAIL(4, i);
+            previousSum = ev(q, r_liu[j]);
         }
-        const F vr = tr[ti++];
+        const F vr = tr[D.tr_claim_liu];
         F gr = f_zero();
         for (uint32_t sg = 0; sg < D.n_vf_liu; ++sg) gr = f_add(gr, o[2 * (D.vf_key.size() + sg)]);
         if (!f_eq(f_mul(vr, gr), previousSum)) VP_FAIL(5, i);
         previousSum = vr;
     }
-    const F acc = out[out_total - 2], claimed = tr[ti++];
+    const F acc = out[out_total - 2], claimed = tr[lay.tr_input];
     if (!f_eq(claimed, acc) || !f_eq(previousSum, claimed)) VP_FAIL(6, 0);
 #undef VP_FAIL
     return 1;
@@ -2550,8 +2530,8 @@ int Engine::verify_check(const F* tr, const F* out, const F* chal, int* fail_cod
 // The whole proof in verifier.cpp:134-189 order, challenges already in d_chal.
 void Engine::prove_all() {
     leave();   // (a previous call may have failed inside a lane)
-    direct_v = use_phase_kernel && use_dfs;   // phase 1 / Liu read V from circuitValue[i-1] (sharded: the rank's rows of it)
-    const bool lane = two_lanes && use_phase_kernel && use_dfs;
+    direct_v = use_dfs;   // phase 1 / Liu read V from circuitValue[i-1] (sharded: the rank's rows of it)
+    const bool lane = two_lanes && use_dfs;
     const bool lane3 = lane && three_lanes;
     const bool lane6 = lane3 && six_lanes;
     evaluate();
@@ -2603,7 +2583,7 @@ void Engine::prove_all() {
     for (const auto& lo : seq) {
         const int i = lo.first;
         LayerDev& D = L[i];
-        const int pb = C.bit_length(i - 1), m = D.max_dad_bl;
+        const int m = D.m;
         const bool odd = lo.second;
         if (extras && i == 1) {   // layer 1's own tables run over layer 0: a block's worth of rows may lie outside the core range
             CK(cudaStreamWaitEvent(stream, ev_extra, 0));
@@ -2613,11 +2593,7 @@ void Engine::prove_all() {
         // ---- phase 1
         if (odd) enter(lane0b, 0);
         do_init_phase1(i);
-        if (use_phase_kernel) do_phase(D.ph1, D.ci_ru, D.tr_p1, lane3 ? d_vu.p + i : scal(SC_VU), nullptr, true, direct_v ? val[i - 1].p : nullptr);
-        else {
-            for (int j = 1; j <= pb; ++j) do_round(D.ph1.planB, j, D.ci_ru + (uint32_t)std::max(0, j - 2), D.tr_p1 + 3u * (uint32_t)(j - 1), nullptr);
-            do_finalize(D.ph1.planB, D.ci_ru + (uint32_t)std::max(0, pb - 1), scal(SC_VU));
-        }
+        do_phase(D.ph1, D.ci_ru, D.tr_p1, lane3 ? d_vu.p + i : scal(SC_VU), nullptr, true, direct_v ? val[i - 1].p : nullptr);
         if (lane3 && m != -1) CK(cudaEventRecord(ev_p1v[i], stream));
         if (odd) leave();
         // ---- phase 2: on its own lane, behind this layer's phase 1
@@ -2629,20 +2605,12 @@ void Engine::prove_all() {
             leave();
         } else if (m != -1) {
             do_init_phase2(i);
-            if (use_phase_kernel) do_phase(D.ph2, D.ci_rv, D.tr_p2, nullptr, scal(SC_UNARY));
-            else {
-                for (int j = 1; j <= m; ++j) do_round(D.ph2.planB, j, D.ci_rv + (uint32_t)std::max(0, j - 2), D.tr_p2 + 3u * (uint32_t)(j - 1), scal(SC_UNARY));
-                do_finalize(D.ph2.planB, D.ci_rv + (uint32_t)std::max(0, m - 1), nullptr);
-            }
+            do_phase(D.ph2, D.ci_rv, D.tr_p2, nullptr, scal(SC_UNARY));
         }
         // ---- Liu
         if (lane) enter(odd ? lane1b : lane1, 1);
-        do_init_liu(i, !(use_phase_kernel && use_dfs));
-        if (use_phase_kernel) do_phase(D.ph3, D.ci_rliu, D.tr_liu, nullptr, nullptr, /*has_a=*/!use_dfs, direct_v ? val[i - 1].p : nullptr);
-        else {
-            for (int j = 1; j <= pb; ++j) do_round(D.ph3.planB, j, D.ci_rliu + (uint32_t)std::max(0, j - 2), D.tr_liu + 3u * (uint32_t)(j - 1), nullptr);
-            do_finalize(D.ph3.planB, D.ci_rliu + (uint32_t)std::max(0, pb - 1), nullptr);
-        }
+        do_init_liu(i, !use_dfs);
+        do_phase(D.ph3, D.ci_rliu, D.tr_liu, nullptr, nullptr, /*has_a=*/!use_dfs, direct_v ? val[i - 1].p : nullptr);
         if (lane) leave();
     }
     if (lane) {   // join: the b coefficients, the input MLE and the transcript copy follow on the main lane
@@ -2654,78 +2622,79 @@ void Engine::prove_all() {
             CK(cudaStreamWaitEvent(stream, R->ev_done, 0));
         }
     }
-    if (use_phase_kernel && use_dfs) derive_b();
+    if (use_dfs) derive_b();
     do_input_mle();
     direct_v = false;
     CK(cudaGetLastError());
 }
 
+// A sumcheck phase of the Fiat-Shamir schedule, the prover's side: its init kernels, its plan, and where its final value
+// goes (keep) and its round-1 scalar comes from (at_init).
+const PhasePlan& Engine::fs_phase_init(int i, int phase, F*& keep, const F*& at_init) {
+    cur_layer = i;
+    LayerDev& D = L[i];
+    keep = nullptr;
+    at_init = nullptr;
+    if (phase == 1) {
+        do_init_phase1(i);
+        keep = scal(SC_VU);
+        return D.ph1;
+    }
+    if (phase == 2) {
+        do_init_phase2(i);
+        at_init = scal(SC_UNARY);
+        return D.ph2;
+    }
+    do_init_liu(i, true);
+    return D.ph3;
+}
+
 // Fiat-Shamir mode (SURVEY 8(f) N4): the whole proof through the one-round-per-launch path, every challenge drawn from
-// the transcript cache right after the message it has to depend on (order: host/fiat_shamir.h). The two-rounds-per-pass
-// kernel cannot be used here: it needs the challenges of a phase before the phase starts.
+// the transcript cache right after the message it has to depend on (fs_schedule). The two-rounds-per-pass kernel cannot
+// be used here: it needs the challenges of a phase before the phase starts.
 void Engine::prove_fs(const uint8_t seed[32], F* tr_out, F* ch_out) {
     leave();
     FsCache fs;
     fs.store(seed, 32);
-    std::vector<F> ch(n_chal, f_zero());
-    auto draw_to = [&](uint32_t idx) {
-        ch[idx] = fs.random();
-        const vp_F v{ch[idx].re, ch[idx].im};
-        set_chal(idx, &v);
-    };
-    auto fetch = [&](uint32_t idx, size_t cnt) {
-        get_tr(idx, reinterpret_cast<vp_F*>(tr_out + idx), cnt);
-        for (size_t k = 0; k < cnt; ++k) fs.store(tr_out[idx + k]);
+    std::vector<F> ch(lay.n_chal, f_zero());
+    auto step = [&](const FsStep& st) {   // the messages from the device into the cache, the challenges back to the device
+        if (st.n_store) get_tr(st.tr_begin, reinterpret_cast<vp_F*>(tr_out + st.tr_begin), st.n_store);
+        for (uint32_t k = 0; k < st.n_store; ++k) fs.store(tr_out[st.tr_begin + k]);
+        for (uint32_t k = 0; k < st.n_draw; ++k) {
+            const uint32_t idx = st.ci_begin + k;
+            ch[idx] = fs.random();
+            const vp_F v{ch[idx].re, ch[idx].im};
+            set_chal(idx, &v);
+        }
     };
     {   // unused challenge slots are zero on the device as well
-        CK(cudaMemsetAsync(d_chal.p, 0, (n_chal + 1) * sizeof(F), stream));
-        h_chal.assign(n_chal, f_zero());
+        CK(cudaMemsetAsync(d_chal.p, 0, (lay.n_chal + 1) * sizeof(F), stream));
+        h_chal.assign(lay.n_chal, f_zero());
     }
     evaluate();
     check_assert_flag();
-    for (int k = 0; k < C.bit_length(n - 1); ++k) draw_to(ci_out + (uint32_t)k);
-    do_vres();
-    fetch(tr_vres, 1);
-    auto run_phase = [&](int i, int phase, const PhasePlan& PP, uint32_t ci, uint32_t tr, const F* at_init) {
-        (void)i;
-        for (int j = 1; j <= PP.rounds; ++j) {
-            const uint32_t t = tr + 3u * (uint32_t)(j - 1);
-            if (PP.sharded) sharded_round(PP, phase, j, ci, t, at_init);
-            else do_round(PP.planB, j, ci + (uint32_t)std::max(0, j - 2), t, at_init);
-            fetch(t, 3);
-            draw_to(ci + (uint32_t)(j - 1));
+    for (const FsEntry& e : fs_sched) {
+        if (!e.phase) {
+            if (e.first.n_store && e.first.tr_begin == lay.tr_vres) do_vres();   // at r_out, drawn by the steps before
+            step(e.first);
+            continue;
         }
-    };
-    for (int i = n - 1; i >= 1; --i) {
-        LayerDev& D = L[i];
-        const int m = D.max_dad_bl;
-        cur_layer = i;
-        draw_to(D.ci_assert);
-        do_init_phase1(i);
-        run_phase(i, 1, D.ph1, D.ci_ru, D.tr_p1, nullptr);
-        do_finalize(D.ph1.planB, D.ci_ru + (uint32_t)std::max(0, D.ph1.rounds - 1), scal(SC_VU));
-        fetch(D.tr_claim_u, 1);
-        if (m != -1) {
-            do_init_phase2(i);
-            run_phase(i, 2, D.ph2, D.ci_rv, D.tr_p2, scal(SC_UNARY));
-            do_finalize(D.ph2.planB, D.ci_rv + (uint32_t)std::max(0, D.ph2.rounds - 1), nullptr);
-            fetch(D.tr_claims_v, (size_t)i);
+        F* keep;
+        const F* at_init;
+        const PhasePlan& PP = fs_phase_init(e.layer, e.phase, keep, at_init);
+        for (uint32_t k = 0; k < e.count; ++k) {
+            const FsStep st = e.step(k);
+            const int j = (int)k + 1;
+            if (PP.sharded) sharded_round(PP, e.phase, j, e.first.ci_begin, st.tr_begin, at_init);
+            else do_round(PP.planB, j, e.first.ci_begin + (uint32_t)std::max(0, j - 2), st.tr_begin, at_init);
+            step(st);
         }
-        for (int k = 0; k < n; ++k) draw_to(D.ci_sig + (uint32_t)k);
-        do_init_liu(i, true);
-        run_phase(i, 3, D.ph3, D.ci_rliu, D.tr_liu, nullptr);
-        do_finalize(D.ph3.planB, D.ci_rliu + (uint32_t)std::max(0, D.ph3.rounds - 1), nullptr);
-        fetch(D.tr_claim_liu, 1);
+        do_finalize(PP.planB, e.first.ci_begin + (uint32_t)std::max(0, (int)e.count - 1), keep);
     }
     do_input_mle();
-    fetch(tr_input, 1);
-    if (ch_out) memcpy(ch_out, ch.data(), n_chal * sizeof(F));
-    proof_size = 0;
-    for (int i = n - 1; i >= 1; --i) {
-        const int pb = C.bit_length(i - 1), m = L[i].max_dad_bl;
-        proof_size += (uint64_t)(2 * pb + (m != -1 ? m : 0)) * 3 * sizeof(F) + sizeof(F);
-        if (m != -1) proof_size += (uint64_t)i * sizeof(F);
-    }
+    get_tr(0, reinterpret_cast<vp_F*>(tr_out), lay.n_tr);   // with what no step stores: the last claim_liu, the input MLE
+    if (ch_out) memcpy(ch_out, ch.data(), lay.n_chal * sizeof(F));
+    proof_size = lay.proof_size;
 }
 
 // ---- Fiat-Shamir mode on the device (fs_device.cuh): the order of prove_fs, with the transcript cache in a device pool;
@@ -2733,17 +2702,15 @@ void Engine::prove_fs(const uint8_t seed[32], F* tr_out, F* ch_out) {
 void Engine::fs_alloc() {
     if (d_fs_pool.p) return;
     d_fs_pool.alloc(1 + 4 + 2 * ((size_t)n + 4));   // the longest run of stores between two draws: claim_u + claims_v
-    size_t rounds = 0;
-    for (int i = 1; i < n; ++i) rounds += (size_t)(2 * C.bit_length(i - 1) + std::max(L[i].max_dad_bl, 0));
-    d_fs_stamps.alloc(4 * std::max<size_t>(rounds, 1));
+    d_fs_stamps.alloc(4 * std::max<size_t>(lay.rounds, 1));
     d_stmt.alloc(16);
     d_circuit_digest = d_stmt.p;
 }
 void Engine::fs_begin() {
     leave();
     fs_alloc();
-    memset_stmts(d_chal.p, (n_chal + 1) * sizeof(F));   // unused challenge slots are zero
-    if (n_stmt == 1) h_chal.assign(n_chal, f_zero());
+    memset_stmts(d_chal.p, (lay.n_chal + 1) * sizeof(F));   // unused challenge slots are zero
+    if (n_stmt == 1) h_chal.assign(lay.n_chal, f_zero());
     evaluate();
     if (n_stmt == 1) {
         check_assert_flag();
@@ -2974,8 +2941,8 @@ void Engine::statement_async(const uint8_t context[32], const F* d_outputs, cons
     ++launches;
 }
 
-// The proof in the order of prove_fs (host/fiat_shamir.h). seed != null: the pool starts with it; null: statement_async
-// seeded it. The transcript and the challenges come back in one copy each.
+// The proof in the order of fs_schedule. seed != null: the pool starts with it; null: statement_async seeded it. The
+// transcript and the challenges come back in one copy each.
 void Engine::prove_fs_device(const uint8_t* seed, F* tr_out, F* ch_out) {
     if (seed) {
         uint64_t h[5] = {4, 0, 0, 0, 0};
@@ -2983,106 +2950,38 @@ void Engine::prove_fs_device(const uint8_t* seed, F* tr_out, F* ch_out) {
         CK(cudaMemcpyAsync(d_fs_pool.p, h, sizeof h, cudaMemcpyHostToDevice, stream));
     }
     size_t sr = 0;   // stamp slot of the next phase's first round
-    fs_absorb_draw(0, 0, ci_out, (uint32_t)C.bit_length(n - 1));
-    do_vres();
-    uint32_t tr_prev = tr_vres;   // the message stored before the next layer's assert_random: Vres, then claim_liu
-    for (int i = n - 1; i >= 1; --i) {
-        LayerDev& D = L[i];
-        const int m = D.max_dad_bl;
-        cur_layer = i;
-        fs_absorb_draw(tr_prev, 1, D.ci_assert, 1);
-        do_init_phase1(i);
-        launch_phase_kernel_fs(D.ph1.planB, D.ci_ru, scal(SC_VU), nullptr, D.tr_p1, sr);
-        sr += (size_t)D.ph1.planB.rounds;
-        if (m != -1) {
-            fs_absorb_draw(D.tr_claim_u, 1, 0, 0);
-            do_init_phase2(i);
-            launch_phase_kernel_fs(D.ph2.planB, D.ci_rv, nullptr, scal(SC_UNARY), D.tr_p2, sr);
-            sr += (size_t)D.ph2.planB.rounds;
-            fs_absorb_draw(D.tr_claims_v, (uint32_t)i, D.ci_sig, (uint32_t)n);
-        } else
-            fs_absorb_draw(D.tr_claim_u, 1, D.ci_sig, (uint32_t)n);
-        do_init_liu(i, true);
-        launch_phase_kernel_fs(D.ph3.planB, D.ci_rliu, nullptr, nullptr, D.tr_liu, sr);
-        sr += (size_t)D.ph3.planB.rounds;
-        tr_prev = D.tr_claim_liu;
+    for (const FsEntry& e : fs_sched) {
+        if (!e.phase) {
+            if (e.first.n_store && e.first.tr_begin == lay.tr_vres) do_vres();   // at r_out, drawn by the steps before
+            fs_absorb_draw(e.first.tr_begin, e.first.n_store, e.first.ci_begin, e.first.n_draw);
+            continue;
+        }
+        F* keep;
+        const F* at_init;
+        const PhasePlan& PP = fs_phase_init(e.layer, e.phase, keep, at_init);
+        launch_phase_kernel_fs(PP.planB, e.first.ci_begin, keep, at_init, e.first.tr_begin, sr);   // stores and draws e.count rounds
+        sr += e.count;
     }
     do_input_mle();
     fs_rounds = sr;
-    std::vector<F> ch((size_t)n_stmt * n_chal);   // statement-major, like the transcripts
-    copy_stmts_to_host(tr_out, n_tr * sizeof(F), d_tr.p, n_tr * sizeof(F));
-    copy_stmts_to_host(ch.data(), n_chal * sizeof(F), d_chal.p, n_chal * sizeof(F));
+    std::vector<F> ch((size_t)n_stmt * lay.n_chal);   // statement-major, like the transcripts
+    copy_stmts_to_host(tr_out, lay.n_tr * sizeof(F), d_tr.p, lay.n_tr * sizeof(F));
+    copy_stmts_to_host(ch.data(), lay.n_chal * sizeof(F), d_chal.p, lay.n_chal * sizeof(F));
     CK(cudaStreamSynchronize(stream));
     CK(cudaGetLastError());
     if (n_stmt == 1) h_chal = ch;   // a later vp_verify / vp_prove on this context sees the challenges the proof used
     if (ch_out) memcpy(ch_out, ch.data(), ch.size() * sizeof(F));
-    proof_size = 0;
-    for (int i = n - 1; i >= 1; --i) {
-        const int pb = C.bit_length(i - 1), m = L[i].max_dad_bl;
-        proof_size += (uint64_t)(2 * pb + (m != -1 ? m : 0)) * 3 * sizeof(F) + sizeof(F);
-        if (m != -1) proof_size += (uint64_t)i * sizeof(F);
-    }
+    proof_size = lay.proof_size;
 }
 
-// The store / draw order of prove_fs_device (and of fs_challenges below) as k_fs_replay's steps, built once per context.
+// fs_schedule as k_fs_replay's steps, one per round of a phase, built once per context.
 void Engine::fs_replay_table() {
     if (d_fs_steps.p) return;
     std::vector<FsStep> st;
-    auto rounds = [&](uint32_t tr0, uint32_t ci0, int cnt) {
-        for (int j = 0; j < cnt; ++j) st.push_back(FsStep{tr0 + 3u * (uint32_t)j, 3, ci0 + (uint32_t)j, 1});
-    };
-    st.push_back(FsStep{0, 0, ci_out, (uint32_t)C.bit_length(n - 1)});
-    uint32_t tr_prev = tr_vres;
-    for (int i = n - 1; i >= 1; --i) {
-        const LayerDev& D = L[i];
-        const int pb = C.bit_length(i - 1), m = D.max_dad_bl;
-        st.push_back(FsStep{tr_prev, 1, D.ci_assert, 1});
-        rounds(D.tr_p1, D.ci_ru, pb);
-        if (m != -1) {
-            st.push_back(FsStep{D.tr_claim_u, 1, 0, 0});
-            rounds(D.tr_p2, D.ci_rv, m);
-            st.push_back(FsStep{D.tr_claims_v, (uint32_t)i, D.ci_sig, (uint32_t)n});
-        } else
-            st.push_back(FsStep{D.tr_claim_u, 1, D.ci_sig, (uint32_t)n});
-        rounds(D.tr_liu, D.ci_rliu, pb);
-        tr_prev = D.tr_claim_liu;
-    }
+    for (const FsEntry& e : fs_sched)
+        for (uint32_t k = 0; k < e.count; ++k) st.push_back(e.step(k));
     d_fs_steps.upload(st, stream);
     CK(cudaStreamSynchronize(stream));   // (the host vector goes out of scope)
-}
-
-// The challenges of a Fiat-Shamir transcript, recomputed from the messages alone (what a verifier does first), in the
-// usual challenge layout (vp_draw_challenges order; unused slots zero).
-static void fs_challenges(const Circuit& C, const uint8_t seed[32], const F* tr, F* ch, size_t n_chal) {
-    const int n = C.n_layers(), mbl = C.max_bit_length();
-    FsCache fs;
-    fs.store(seed, 32);
-    for (size_t k = 0; k < n_chal; ++k) ch[k] = f_zero();
-    size_t ci = 0, ti = 0;
-    for (int k = 0; k < C.bit_length(n - 1); ++k) ch[ci++] = fs.random();
-    fs.store(tr[ti++]);
-    auto rounds = [&](int cnt, size_t ci0) {
-        for (int j = 0; j < cnt; ++j) {
-            for (int q = 0; q < 3; ++q) fs.store(tr[ti++]);
-            ch[ci0 + (size_t)j] = fs.random();
-        }
-    };
-    for (int i = n - 1; i >= 1; --i) {
-        const int pb = C.bit_length(i - 1), m = C.max_dad_bit_length(i);
-        const size_t ci_ru = ci, ci_assert = ci_ru + (size_t)mbl, ci_rv = ci_assert + 1, ci_sig = ci_rv + (m != -1 ? (size_t)m : 0),
-                     ci_rliu = ci_sig + (size_t)n;
-        ch[ci_assert] = fs.random();
-        rounds(pb, ci_ru);
-        fs.store(tr[ti++]);
-        if (m != -1) {
-            rounds(m, ci_rv);
-            for (int l = 0; l < i; ++l) fs.store(tr[ti++]);
-        }
-        for (int k = 0; k < n; ++k) ch[ci_sig + (size_t)k] = fs.random();
-        rounds(pb, ci_rliu);
-        fs.store(tr[ti++]);
-        ci = ci_rliu + (size_t)mbl;
-    }
 }
 
 struct vp_ctx {
@@ -3264,17 +3163,7 @@ extern "C" int vp_circuit_set_inputs(vp_circuit* c, const uint64_t* in) {
     }
     return VP_OK;
 }
-extern "C" size_t vp_challenge_count(const vp_circuit* c) {
-    if (!c) return 0;
-    const Circuit& C = c->c;
-    const int n = C.n_layers(), mbl = C.max_bit_length();
-    size_t t = (size_t)C.bit_length(n - 1);
-    for (int i = n - 1; i >= 1; --i) {
-        int m = C.max_dad_bit_length(i);
-        t += (size_t)mbl + 1 + (m != -1 ? (size_t)m : 0) + (size_t)n + (size_t)mbl;
-    }
-    return t;
-}
+extern "C" size_t vp_challenge_count(const vp_circuit* c) { return c ? proof_layout(c->c).n_chal : 0; }
 extern "C" int vp_draw_challenges(const vp_circuit* c, unsigned seed, vp_F* out) {
     if (!c || !out) return fail(VP_ERR_ARG, "null argument");
     ChallengeStream cs = draw_challenges(c->c, seed);
@@ -3301,18 +3190,7 @@ extern "C" int vp_draw_field(unsigned seed, size_t n, vp_F* out) {
     }
     return VP_OK;
 }
-extern "C" size_t vp_transcript_len(const vp_circuit* c) {
-    if (!c) return 0;
-    const Circuit& C = c->c;
-    size_t t = 1;
-    for (int i = C.n_layers() - 1; i >= 1; --i) {
-        const int pb = C.bit_length(i - 1), m = C.max_dad_bit_length(i);
-        t += 3 * (size_t)pb + 1;
-        if (m != -1) t += 3 * (size_t)m + (size_t)i;
-        t += 3 * (size_t)pb + 1;
-    }
-    return t + 1;
-}
+extern "C" size_t vp_transcript_len(const vp_circuit* c) { return c ? proof_layout(c->c).n_tr : 0; }
 
 // ------------------------------------------------------------------ C ABI: transcript containers
 extern "C" int vp_transcript_to_gkrproof(const vp_circuit* c, const vp_F* transcript, unsigned char* out, size_t cap, size_t* len) {
@@ -3495,9 +3373,9 @@ extern "C" int vp_vres(vp_ctx* ctx, const vp_F* r, int n, vp_F* out) {
     ScopedTimer t(e);
     if (!e.evaluated) return fail(VP_ERR_ARG, "vp_vres before vp_evaluate");
     if (n != e.C.bit_length(e.n - 1)) return fail(VP_ERR_ARG, "vp_vres: n must be the output layer's bit length");
-    if (n) e.set_chal(e.ci_out, r, (size_t)n);
+    if (n) e.set_chal(e.lay.ci_out, r, (size_t)n);
     e.do_vres();
-    e.get_tr(e.tr_vres, out);
+    e.get_tr(e.lay.tr_vres, out);
     return VP_OK;
     API_END
 }
@@ -3507,7 +3385,7 @@ extern "C" int vp_sumcheck_init_all(vp_ctx* ctx, const vp_F* r_last, int n) {
     Engine& e = ctx->e;
     ScopedTimer t(e);
     if (n != e.C.bit_length(e.n - 1)) return fail(VP_ERR_ARG, "sumcheck_init_all: wrong n");
-    if (n) e.set_chal(e.ci_out, r_last, (size_t)n);
+    if (n) e.set_chal(e.lay.ci_out, r_last, (size_t)n);
     e.cur_layer = e.n;
     e.phase = 0;
     CK(cudaStreamSynchronize(e.stream));
@@ -3542,7 +3420,7 @@ extern "C" int vp_init_phase2(vp_ctx* ctx) {
     Engine& e = ctx->e;
     ScopedTimer t(e);
     if (e.cur_layer < 1 || e.cur_layer >= e.n) return fail(VP_ERR_ARG, "init_phase2 outside a layer");
-    if (e.L[e.cur_layer].max_dad_bl == -1) return fail(VP_ERR_ARG, "layer %d has no phase 2", e.cur_layer);
+    if (e.L[e.cur_layer].m == -1) return fail(VP_ERR_ARG, "layer %d has no phase 2", e.cur_layer);
     e.do_init_phase2(e.cur_layer);
     e.phase = 2;
     e.round = 0;
@@ -3656,7 +3534,7 @@ extern "C" int vp_inner_prod(vp_ctx* ctx, const vp_F* pub, size_t n, vp_F* out) 
     if (e.d_pub.n < n) e.d_pub.alloc(n);
     CK(cudaMemcpyAsync(e.d_pub.p, pub, n * sizeof(F), cudaMemcpyHostToDevice, e.stream));
     if (e.world == 1) {
-        k_dot<<<e.grid_for((uint32_t)n, e.cap_dot), 256, 0, e.stream>>>(e.val[0].p, e.d_pub.p, (uint32_t)n, e.d_tr.p + e.tr_input,
+        k_dot<<<e.grid_for((uint32_t)n, e.cap_dot), 256, 0, e.stream>>>(e.val[0].p, e.d_pub.p, (uint32_t)n, e.d_tr.p + e.lay.tr_input,
                                                                e.d_partials.p, e.d_counter.p);
         ++e.launches;
     } else {   // every rank sums its own slice of the instances, one 16-byte-per-rank all-gather (collective call)
@@ -3664,10 +3542,10 @@ extern "C" int vp_inner_prod(vp_ctx* ctx, const vp_F* pub, size_t n, vp_F* out) 
         k_dot<<<e.grid_for((uint32_t)std::max<size_t>(en - b, 1), e.cap_dot), 256, 0, e.stream>>>(e.val[0].p + b, e.d_pub.p + b, (uint32_t)(en - b),
                                                                                               e.d_send.p, e.d_partials.p, e.d_counter.p);
         NCK(g_nccl.AllGather(e.d_send.p, e.d_recv.p, 2, /*ncclUint64*/ 5, e.comm, e.stream));
-        k_sum_ranks<<<1, 32, 0, e.stream>>>(e.d_recv.p, (uint32_t)e.world, 1, e.d_tr.p + e.tr_input);
+        k_sum_ranks<<<1, 32, 0, e.stream>>>(e.d_recv.p, (uint32_t)e.world, 1, e.d_tr.p + e.lay.tr_input);
         e.launches += 3;
     }
-    e.get_tr(e.tr_input, out);
+    e.get_tr(e.lay.tr_input, out);
     return VP_OK;
     API_END
 }
@@ -3682,10 +3560,10 @@ extern "C" int vp_dot_host(vp_ctx* ctx, const vp_F* a, const vp_F* b, size_t n, 
     db.alloc(std::max<size_t>(n, 1));
     CK(cudaMemcpyAsync(da.p, a, n * sizeof(F), cudaMemcpyHostToDevice, e.stream));
     CK(cudaMemcpyAsync(db.p, b, n * sizeof(F), cudaMemcpyHostToDevice, e.stream));
-    k_dot<<<e.grid_for((uint32_t)n, e.cap_dot), 256, 0, e.stream>>>(da.p, db.p, (uint32_t)n, e.d_tr.p + e.tr_input, e.d_partials.p,
+    k_dot<<<e.grid_for((uint32_t)n, e.cap_dot), 256, 0, e.stream>>>(da.p, db.p, (uint32_t)n, e.d_tr.p + e.lay.tr_input, e.d_partials.p,
                                                            e.d_counter.p);
     ++e.launches;
-    e.get_tr(e.tr_input, out);
+    e.get_tr(e.lay.tr_input, out);
     return VP_OK;
     API_END
 }
@@ -3697,7 +3575,7 @@ extern "C" int vp_input_mle(vp_ctx* ctx, const vp_F* r, int n, vp_F* out) {
     if (n != e.C.bit_length(0)) return fail(VP_ERR_ARG, "input_mle: n must be the input layer's bit length");
     if (n) e.set_chal(e.L[1].ci_rliu, r, (size_t)n);
     e.do_input_mle();
-    e.get_tr(e.tr_input, out);
+    e.get_tr(e.lay.tr_input, out);
     return VP_OK;
     API_END
 }
@@ -3709,7 +3587,7 @@ extern "C" int vp_set_challenges(vp_ctx* ctx, const vp_F* challenges, size_t n) 
     API_BEGIN
     Engine& e = ctx->e;
     cudaSetDevice(e.device);
-    if (n != e.n_chal) return fail(VP_ERR_ARG, "expected %zu challenges, got %zu", e.n_chal, n);
+    if (n != e.lay.n_chal) return fail(VP_ERR_ARG, "expected %zu challenges, got %zu", e.lay.n_chal, n);
     e.set_chal(0, challenges, n);
     CK(cudaStreamSynchronize(e.stream));
     return VP_OK;
@@ -3723,8 +3601,8 @@ static int prove_impl(vp_ctx* ctx, int host_io, bool local_inputs, const uint64_
     ScopedTimer t(e);
     if (host_io) {
         if (!inputs || !challenges || !transcript) return fail(VP_ERR_ARG, "host_io needs inputs, challenges and transcript");
-        if (n_challenges != e.n_chal) return fail(VP_ERR_ARG, "expected %zu challenges, got %zu", e.n_chal, n_challenges);
-        if (transcript_cap < e.n_tr) return fail(VP_ERR_ARG, "transcript buffer too small (%zu < %zu)", transcript_cap, e.n_tr);
+        if (n_challenges != e.lay.n_chal) return fail(VP_ERR_ARG, "expected %zu challenges, got %zu", e.lay.n_chal, n_challenges);
+        if (transcript_cap < e.lay.n_tr) return fail(VP_ERR_ARG, "transcript buffer too small (%zu < %zu)", transcript_cap, e.lay.n_tr);
     }
     const uint64_t l0 = e.launches;
     CK(cudaEventRecord(e.ev0, e.stream));
@@ -3733,18 +3611,12 @@ static int prove_impl(vp_ctx* ctx, int host_io, bool local_inputs, const uint64_
         e.load_inputs_chunked(inputs, n_inputs, local_inputs);   // copies overlap evaluate chunk by chunk
     }
     e.prove_all();
-    if (host_io) CK(cudaMemcpyAsync(transcript, e.d_tr.p, e.n_tr * sizeof(F), cudaMemcpyDeviceToHost, e.stream));
+    if (host_io) CK(cudaMemcpyAsync(transcript, e.d_tr.p, e.lay.n_tr * sizeof(F), cudaMemcpyDeviceToHost, e.stream));
     CK(cudaEventRecord(e.ev1, e.stream));
     e.check_assert_flag();  // synchronises the stream
     CK(cudaEventElapsedTime(&e.last_ms, e.ev0, e.ev1));
     e.last_launches = e.launches - l0;
-    // proof-size accounting of the interactive path (prover.cpp:451,500,512)
-    e.proof_size = 0;
-    for (int i = e.n - 1; i >= 1; --i) {
-        const int pb = e.C.bit_length(i - 1), m = e.L[i].max_dad_bl;
-        e.proof_size += (uint64_t)(2 * pb + (m != -1 ? m : 0)) * 3 * sizeof(F) + sizeof(F);
-        if (m != -1) e.proof_size += (uint64_t)i * sizeof(F);
-    }
+    e.proof_size = e.lay.proof_size;
     return VP_OK;
     API_END
 }
@@ -3968,8 +3840,8 @@ extern "C" int vp_prove_fs(vp_ctx* ctx, const uint8_t seed[32], vp_F* transcript
     API_BEGIN
     Engine& e = ctx->e;
     ScopedTimer t(e);
-    if (transcript_cap < e.n_tr) return fail(VP_ERR_ARG, "transcript buffer too small (%zu < %zu)", transcript_cap, e.n_tr);
-    if (challenges && challenges_cap < e.n_chal) return fail(VP_ERR_ARG, "challenge buffer too small (%zu < %zu)", challenges_cap, e.n_chal);
+    if (transcript_cap < e.lay.n_tr) return fail(VP_ERR_ARG, "transcript buffer too small (%zu < %zu)", transcript_cap, e.lay.n_tr);
+    if (challenges && challenges_cap < e.lay.n_chal) return fail(VP_ERR_ARG, "challenge buffer too small (%zu < %zu)", challenges_cap, e.lay.n_chal);
     if (!e.inputs_loaded) return fail(VP_ERR_ARG, "vp_prove_fs: inputs not loaded");
     const uint64_t l0 = e.launches;
     CK(cudaEventRecord(e.ev0, e.stream));
@@ -3988,12 +3860,12 @@ extern "C" int vp_prove_fs(vp_ctx* ctx, const uint8_t seed[32], vp_F* transcript
 extern "C" int vp_fs_challenges(const vp_circuit* c, const uint8_t seed[32], const vp_F* transcript, size_t n, vp_F* challenges, size_t cap) {
     if (!c || !seed || !transcript || !challenges) return fail(VP_ERR_ARG, "null argument");
     API_BEGIN
-    if (n != vp_transcript_len(c)) return fail(VP_ERR_ARG, "expected a transcript of %zu field elements, got %zu", vp_transcript_len(c), n);
-    const size_t nc = vp_challenge_count(c);
-    if (cap < nc) return fail(VP_ERR_ARG, "challenge buffer too small (%zu < %zu)", cap, nc);
+    const ProofLayout lay = proof_layout(c->c);
+    if (n != lay.n_tr) return fail(VP_ERR_ARG, "expected a transcript of %zu field elements, got %zu", lay.n_tr, n);
+    if (cap < lay.n_chal) return fail(VP_ERR_ARG, "challenge buffer too small (%zu < %zu)", cap, lay.n_chal);
     for (size_t i = 0; i < n; ++i)
         if (transcript[i].re >= P || transcript[i].im >= P) return fail(VP_ERR_ARG, "transcript element %zu is not canonical", i);
-    fs_challenges(c->c, seed, reinterpret_cast<const F*>(transcript), reinterpret_cast<F*>(challenges), nc);
+    fs_challenges(lay, fs_schedule(lay), seed, reinterpret_cast<const F*>(transcript), reinterpret_cast<F*>(challenges));
     return VP_OK;
     API_END
 }
@@ -4002,12 +3874,12 @@ extern "C" int vp_verify_fs(vp_ctx* ctx, const uint8_t seed[32], const vp_F* tra
     API_BEGIN
     Engine& e = ctx->e;
     cudaSetDevice(e.device);
-    if (n != e.n_tr) return fail(VP_ERR_ARG, "expected a transcript of %zu field elements, got %zu", e.n_tr, n);
+    if (n != e.lay.n_tr) return fail(VP_ERR_ARG, "expected a transcript of %zu field elements, got %zu", e.lay.n_tr, n);
     for (size_t i = 0; i < n; ++i)
         if (transcript[i].re >= P || transcript[i].im >= P) { *accept = 0; if (fail_code) *fail_code = 7; if (fail_layer) *fail_layer = 0; return VP_OK; }
-    std::vector<F> ch(e.n_chal);
-    fs_challenges(e.C, seed, reinterpret_cast<const F*>(transcript), ch.data(), e.n_chal);
-    e.set_chal(0, reinterpret_cast<const vp_F*>(ch.data()), e.n_chal);
+    std::vector<F> ch(e.lay.n_chal);
+    fs_challenges(e.lay, e.fs_sched, seed, reinterpret_cast<const F*>(transcript), ch.data());
+    e.set_chal(0, reinterpret_cast<const vp_F*>(ch.data()), e.lay.n_chal);
     *accept = e.verify(reinterpret_cast<const F*>(transcript), fail_code, fail_layer);
     return VP_OK;
     API_END
@@ -4048,8 +3920,8 @@ extern "C" int vp_prove_fs_bound(vp_ctx* ctx, const uint8_t context[32], vp_F* t
     Engine& e = ctx->e;
     ScopedTimer t(e);
     if (e.world != 1) return fail(VP_ERR_ARG, "vp_prove_fs_bound: sharded contexts are not supported");
-    if (cap < e.n_tr) return fail(VP_ERR_ARG, "transcript buffer too small (%zu < %zu)", cap, e.n_tr);
-    if (challenges && ch_cap < e.n_chal) return fail(VP_ERR_ARG, "challenge buffer too small (%zu < %zu)", ch_cap, e.n_chal);
+    if (cap < e.lay.n_tr) return fail(VP_ERR_ARG, "transcript buffer too small (%zu < %zu)", cap, e.lay.n_tr);
+    if (challenges && ch_cap < e.lay.n_chal) return fail(VP_ERR_ARG, "challenge buffer too small (%zu < %zu)", ch_cap, e.lay.n_chal);
     if (!e.inputs_loaded) return fail(VP_ERR_ARG, "vp_prove_fs_bound: inputs not loaded");
     const uint64_t l0 = e.launches;
     CK(cudaEventRecord(e.ev0, e.stream));
@@ -4100,8 +3972,8 @@ extern "C" int vp_prove_fs_bound_batch(vp_ctx* ctx, size_t B, const uint64_t* in
     if (B == 0 || B > 65535) return fail(VP_ERR_ARG, "batch size %zu is not in [1, 65535]", B);
     const size_t n_in = e.C.layer_size(0);
     if (n_inputs != B * n_in) return fail(VP_ERR_ARG, "expected %zu inputs (%zu statements of %zu), got %zu", B * n_in, B, n_in, n_inputs);
-    if (cap < B * e.n_tr) return fail(VP_ERR_ARG, "transcript buffer too small (%zu < %zu)", cap, B * e.n_tr);
-    if (challenges && ch_cap < B * e.n_chal) return fail(VP_ERR_ARG, "challenge buffer too small (%zu < %zu)", ch_cap, B * e.n_chal);
+    if (cap < B * e.lay.n_tr) return fail(VP_ERR_ARG, "transcript buffer too small (%zu < %zu)", cap, B * e.lay.n_tr);
+    if (challenges && ch_cap < B * e.lay.n_chal) return fail(VP_ERR_ARG, "challenge buffer too small (%zu < %zu)", ch_cap, B * e.lay.n_chal);
     for (size_t i = 0; i < n_inputs; ++i)
         if (inputs[i] >= P) return fail(VP_ERR_ARG, "input %zu of statement %zu is not < p", i % n_in, i / n_in);
     e.leave();
@@ -4155,8 +4027,8 @@ extern "C" int vp_verify_fs_bound_batch(vp_ctx* ctx, size_t B, const uint64_t* i
     const size_t n_in = e.C.layer_size(0), n_out = e.C.layer_size(e.n - 1);
     if (n_inputs != B * n_in) return fail(VP_ERR_ARG, "expected %zu inputs (%zu statements of %zu), got %zu", B * n_in, B, n_in, n_inputs);
     if (n_outputs != B * n_out) return fail(VP_ERR_ARG, "expected %zu outputs (%zu statements of %zu), got %zu", B * n_out, B, n_out, n_outputs);
-    if (n_tr != B * e.n_tr) return fail(VP_ERR_ARG, "expected %zu transcript elements (%zu statements of %zu), got %zu", B * e.n_tr, B, e.n_tr, n_tr);
-    if (challenges && ch_cap < B * e.n_chal) return fail(VP_ERR_ARG, "challenge buffer too small (%zu < %zu)", ch_cap, B * e.n_chal);
+    if (n_tr != B * e.lay.n_tr) return fail(VP_ERR_ARG, "expected %zu transcript elements (%zu statements of %zu), got %zu", B * e.lay.n_tr, B, e.lay.n_tr, n_tr);
+    if (challenges && ch_cap < B * e.lay.n_chal) return fail(VP_ERR_ARG, "challenge buffer too small (%zu < %zu)", ch_cap, B * e.lay.n_chal);
     for (size_t i = 0; i < n_inputs; ++i)
         if (inputs[i] >= P) return fail(VP_ERR_ARG, "input %zu of statement %zu is not < p", i % n_in, i / n_in);
     for (size_t i = 0; i < n_outputs; ++i)
@@ -4166,11 +4038,11 @@ extern "C" int vp_verify_fs_bound_batch(vp_ctx* ctx, size_t B, const uint64_t* i
     const F* tr = reinterpret_cast<const F*>(transcripts);
     std::vector<uint8_t> bad(B, 0);
     std::vector<F> clean;
-    for (size_t b = 0; b < B; ++b) bad[b] = !fs_canonical(transcripts + b * e.n_tr, e.n_tr);
+    for (size_t b = 0; b < B; ++b) bad[b] = !fs_canonical(transcripts + b * e.lay.n_tr, e.lay.n_tr);
     if (std::find(bad.begin(), bad.end(), 1) != bad.end()) {
         clean.assign(tr, tr + n_tr);
         for (size_t b = 0; b < B; ++b)
-            if (bad[b]) std::fill(clean.begin() + b * e.n_tr, clean.begin() + (b + 1) * e.n_tr, f_zero());
+            if (bad[b]) std::fill(clean.begin() + b * e.lay.n_tr, clean.begin() + (b + 1) * e.lay.n_tr, f_zero());
         tr = clean.data();
     }
     e.leave();
@@ -4181,7 +4053,7 @@ extern "C" int vp_verify_fs_bound_batch(vp_ctx* ctx, size_t B, const uint64_t* i
     e.batch_outputs = 0;
     const uint32_t out_total = e.vf_out_total;
     if (e.d_fs_outputs.n < n_outputs) e.d_fs_outputs.alloc(n_outputs);
-    std::vector<F> sums((size_t)B * out_total), ch((size_t)B * e.n_chal);
+    std::vector<F> sums((size_t)B * out_total), ch((size_t)B * e.lay.n_chal);
     const uint64_t l0 = e.launches;
     {
         FsBatchScope scope(e, (uint32_t)B, (size_t)out_total + (size_t)e.vf_max_b * Engine::VF_GX * 2);
@@ -4191,8 +4063,8 @@ extern "C" int vp_verify_fs_bound_batch(vp_ctx* ctx, size_t B, const uint64_t* i
         CK(cudaMemcpyAsync(e.d_inputs.p, inputs, n_inputs * sizeof(uint64_t), cudaMemcpyHostToDevice, e.stream));
         CK(cudaMemcpyAsync(e.d_fs_outputs.p, outputs, n_outputs * sizeof(F), cudaMemcpyHostToDevice, e.stream));
         CK(cudaMemcpyAsync(e.slab.contexts.p, contexts, 32 * B, cudaMemcpyHostToDevice, e.stream));
-        CK(cudaMemcpy2DAsync(e.d_tr.p, e.sstride, tr, e.n_tr * sizeof(F), e.n_tr * sizeof(F), B, cudaMemcpyHostToDevice, e.stream));
-        e.memset_stmts(e.d_chal.p, (e.n_chal + 1) * sizeof(F));   // unused challenge slots are zero
+        CK(cudaMemcpy2DAsync(e.d_tr.p, e.sstride, tr, e.lay.n_tr * sizeof(F), e.lay.n_tr * sizeof(F), B, cudaMemcpyHostToDevice, e.stream));
+        e.memset_stmts(e.d_chal.p, (e.lay.n_chal + 1) * sizeof(F));   // unused challenge slots are zero
         e.memset_stmts(d_out, (size_t)out_total * sizeof(F));
         const uint32_t n0 = (uint32_t)(B * n_in);   // circuitValue[0] of every statement, instance-major over B * K
         k_load_inputs<<<cdiv(n0, 256), 256, 0, e.stream>>>(e.d_inputs.p, e.val[0].p, 0, n0);
@@ -4206,7 +4078,7 @@ extern "C" int vp_verify_fs_bound_batch(vp_ctx* ctx, size_t B, const uint64_t* i
         e.verify_sums_async(d_out, d_part);
         CK(cudaEventRecord(e.ev1, e.stream));
         e.copy_stmts_to_host(sums.data(), out_total * sizeof(F), d_out, out_total * sizeof(F));
-        e.copy_stmts_to_host(ch.data(), e.n_chal * sizeof(F), e.d_chal.p, e.n_chal * sizeof(F));
+        e.copy_stmts_to_host(ch.data(), e.lay.n_chal * sizeof(F), e.d_chal.p, e.lay.n_chal * sizeof(F));
         CK(cudaStreamSynchronize(e.stream));
         CK(cudaGetLastError());
         CK(cudaEventElapsedTime(&e.last_ms, e.ev0, e.ev1));
@@ -4215,15 +4087,15 @@ extern "C" int vp_verify_fs_bound_batch(vp_ctx* ctx, size_t B, const uint64_t* i
     // the host driver, one statement at a time, in vp_verify_fs_bound's order: code 7, code 8, then vp_verify's checks
     for (size_t b = 0; b < B; ++b) {
         int code = 0, layer = 0, ok = 0;
-        const F* tb = tr + b * e.n_tr;
+        const F* tb = tr + b * e.lay.n_tr;
         const F* sb = sums.data() + b * out_total;
         if (bad[b]) code = 7;
-        else if (!f_eq(sb[out_total - 1], tb[e.tr_vres])) code = 8;
-        else ok = e.verify_check(tb, sb, ch.data() + b * e.n_chal, &code, &layer);
+        else if (!f_eq(sb[out_total - 1], tb[e.lay.tr_vres])) code = 8;
+        else ok = e.verify_check(tb, sb, ch.data() + b * e.lay.n_chal, &code, &layer);
         accept[b] = ok;
         if (fail_code) fail_code[b] = code;
         if (fail_layer) fail_layer[b] = layer;
-        if (bad[b]) std::fill(ch.begin() + b * e.n_chal, ch.begin() + (b + 1) * e.n_chal, f_zero());
+        if (bad[b]) std::fill(ch.begin() + b * e.lay.n_chal, ch.begin() + (b + 1) * e.lay.n_chal, f_zero());
     }
     if (challenges) memcpy(challenges, ch.data(), ch.size() * sizeof(F));
     return VP_OK;
@@ -4237,7 +4109,7 @@ extern "C" int vp_verify_fs_bound(vp_ctx* ctx, const uint8_t context[32], const 
     cudaSetDevice(e.device);
     if (e.world != 1) return fail(VP_ERR_ARG, "vp_verify_fs_bound: sharded contexts are not supported");
     if (!e.inputs_loaded) return fail(VP_ERR_ARG, "vp_verify_fs_bound: inputs not loaded");
-    if (n != e.n_tr) return fail(VP_ERR_ARG, "expected a transcript of %zu field elements, got %zu", e.n_tr, n);
+    if (n != e.lay.n_tr) return fail(VP_ERR_ARG, "expected a transcript of %zu field elements, got %zu", e.lay.n_tr, n);
     const size_t n_out = e.C.layer_size(e.n - 1);
     if (n_outputs != n_out) return fail(VP_ERR_ARG, "expected %zu outputs, got %zu", n_out, n_outputs);
     if (!fs_canonical(outputs, n_outputs)) return fail(VP_ERR_ARG, "an output is not canonical (components must be < p)");
@@ -4258,9 +4130,9 @@ extern "C" int vp_verify_fs_bound(vp_ctx* ctx, const uint8_t context[32], const 
     CK(cudaStreamSynchronize(e.stream));
     uint8_t stmt[32];
     memcpy(stmt, h, 32);
-    std::vector<F> ch(e.n_chal);
-    fs_challenges(e.C, stmt, reinterpret_cast<const F*>(transcript), ch.data(), e.n_chal);
-    e.set_chal(0, reinterpret_cast<const vp_F*>(ch.data()), e.n_chal);
+    std::vector<F> ch(e.lay.n_chal);
+    fs_challenges(e.lay, e.fs_sched, stmt, reinterpret_cast<const F*>(transcript), ch.data());
+    e.set_chal(0, reinterpret_cast<const vp_F*>(ch.data()), e.lay.n_chal);
     // the claim chain starts from Vres: it must be the MLE of the claimed outputs at r_out
     e.run_eq(e.eqb_out, 2);
     if (e.d_vf_out.n < 1) e.d_vf_out.alloc(2);
@@ -4268,7 +4140,7 @@ extern "C" int vp_verify_fs_bound(vp_ctx* ctx, const uint8_t context[32], const 
     F mle;
     CK(cudaMemcpyAsync(&mle, e.d_vf_out.p, sizeof mle, cudaMemcpyDeviceToHost, e.stream));
     CK(cudaStreamSynchronize(e.stream));
-    if (!f_eq(mle, reinterpret_cast<const F*>(transcript)[e.tr_vres])) return reject(8);
+    if (!f_eq(mle, reinterpret_cast<const F*>(transcript)[e.lay.tr_vres])) return reject(8);
     *accept = e.verify(reinterpret_cast<const F*>(transcript), fail_code, fail_layer);
     return VP_OK;
     API_END
@@ -4311,7 +4183,7 @@ extern "C" int vp_verify(vp_ctx* ctx, const vp_F* transcript, size_t n, int* acc
     API_BEGIN
     Engine& e = ctx->e;
     cudaSetDevice(e.device);
-    if (n != e.n_tr) return fail(VP_ERR_ARG, "expected a transcript of %zu field elements, got %zu", e.n_tr, n);
+    if (n != e.lay.n_tr) return fail(VP_ERR_ARG, "expected a transcript of %zu field elements, got %zu", e.lay.n_tr, n);
     *accept = e.verify(reinterpret_cast<const F*>(transcript), fail_code, fail_layer);
     return VP_OK;
     API_END
@@ -4321,8 +4193,8 @@ extern "C" int vp_get_transcript(vp_ctx* ctx, vp_F* transcript, size_t cap) {
     API_BEGIN
     Engine& e = ctx->e;
     cudaSetDevice(e.device);
-    if (cap < e.n_tr) return fail(VP_ERR_ARG, "transcript buffer too small");
-    e.get_tr(0, transcript, e.n_tr);
+    if (cap < e.lay.n_tr) return fail(VP_ERR_ARG, "transcript buffer too small");
+    e.get_tr(0, transcript, e.lay.n_tr);
     return VP_OK;
     API_END
 }

@@ -10,6 +10,7 @@
 // bytes apart (kernels.cuh, stmt_at); statement b runs in blockIdx.z == b: one warp per statement in the kernels between
 // phases, one row of blocks per statement in the phase kernel.
 #pragma once
+#include "../host/fiat_shamir.h"   // FsStep
 #include "kernels.cuh"
 #include "keccak.cuh"
 
@@ -57,10 +58,9 @@ __global__ void k_fs_absorb_draw(uint64_t* pool, const F* __restrict__ transcrip
 }
 
 // The verifier's side (vp_verify_fs_bound_batch): every challenge of a transcript recomputed from its messages, in the
-// store / draw order of host/fiat_shamir.h (fs_challenges). The order is a table of steps built once per context: one per
+// store / draw order of host/fiat_shamir.h (fs_schedule). The order is a table of steps built once per context: one per
 // sumcheck round (store the 3 coefficients, draw the round's challenge) and one per store / draw run between phases.
 // One warp per statement (blockIdx.z), lane 0 hashes; the pool must hold the statement (k_fs_statement).
-struct FsStep { uint32_t tr_begin, n_store, ci_begin, n_draw; };
 __global__ void k_fs_replay(const FsStep* __restrict__ steps, uint32_t n_steps, uint64_t* pool, const F* __restrict__ transcript, F* chal,
                             size_t ss) {
     pool = stmt_at(pool, ss); transcript = stmt_at(transcript, ss); chal = stmt_at(chal, ss);

@@ -1,4 +1,5 @@
-// SHA3-256 for the Fiat-Shamir challenge source (see fiat_shamir.h). FIPS 202: Keccak-f[1600], rate 136, suffix 0x06.
+// The Fiat-Shamir challenge source (see fiat_shamir.h): SHA3-256 (FIPS 202: Keccak-f[1600], rate 136, suffix 0x06) and
+// the order of stores and draws.
 #include "fiat_shamir.h"
 
 #include <string.h>
@@ -60,6 +61,41 @@ void sha3_256(const unsigned char* msg, size_t len, unsigned char out[32]) {
     }
     keccak_f(st);
     memcpy(out, st, 32);
+}
+
+std::vector<FsEntry> fs_schedule(const ProofLayout& P) {
+    std::vector<FsEntry> s;
+    auto run = [&](uint32_t tr, uint32_t n_store, uint32_t ci, uint32_t n_draw) { s.push_back(FsEntry{{tr, n_store, ci, n_draw}, 1, 0, 0}); };
+    auto phase = [&](int i, int ph, uint32_t tr, uint32_t ci, int rounds) { s.push_back(FsEntry{{tr, 3, ci, 1}, (uint32_t)rounds, i, ph}); };
+    const int n = (int)P.layer.size();
+    run(0, 0, P.ci_out, (uint32_t)P.out_bits);
+    uint32_t tr_prev = P.tr_vres;   // the message stored before the next layer's assert_random: Vres, then claim_liu
+    for (int i = n - 1; i >= 1; --i) {
+        const LayerLayout& X = P.layer[i];
+        run(tr_prev, 1, X.ci_assert, 1);
+        phase(i, 1, X.tr_p1, X.ci_ru, X.pb);
+        if (X.m != -1) {
+            run(X.tr_claim_u, 1, 0, 0);
+            phase(i, 2, X.tr_p2, X.ci_rv, X.m);
+            run(X.tr_claims_v, (uint32_t)i, X.ci_sig, (uint32_t)n);
+        } else
+            run(X.tr_claim_u, 1, X.ci_sig, (uint32_t)n);
+        phase(i, 3, X.tr_liu, X.ci_rliu, X.pb);
+        tr_prev = X.tr_claim_liu;
+    }
+    return s;
+}
+
+void fs_challenges(const ProofLayout& P, const std::vector<FsEntry>& schedule, const uint8_t seed[32], const F* tr, F* ch) {
+    FsCache fs;
+    fs.store(seed, 32);
+    for (size_t k = 0; k < P.n_chal; ++k) ch[k] = F{0, 0};
+    for (const FsEntry& e : schedule)
+        for (uint32_t k = 0; k < e.count; ++k) {
+            const FsStep st = e.step(k);
+            for (uint32_t q = 0; q < st.n_store; ++q) fs.store(tr[st.tr_begin + q]);
+            for (uint32_t q = 0; q < st.n_draw; ++q) ch[st.ci_begin + q] = fs.random();
+        }
 }
 
 }  // namespace vp
