@@ -804,7 +804,6 @@ struct Engine {
     bool direct_v = false;   // whole-proof: phase 1 / Liu read V from circuitValue[i-1] instead of a copy
     cudaEvent_t ev_eval = nullptr;
     uint32_t region_u_lane1 = 0;
-    bool use_dfs = true;   // two rounds per pass in vp_prove (k_phase_dfs); false: one round per pass (k_sumcheck_phase)
     int cap_dfs = 0;
     int n = 0;            // layers
     uint32_t K = 1;
@@ -969,11 +968,11 @@ struct Engine {
     int n_sm = 148;
     int cap_p1il = 0, cap_p2v2 = 0;
     int dfs_grid_override = 0;   // VP_DFS_GRID: development knob
-    bool old_p2 = false, getenv_no_hs = false, liu_old = false, p1_old = false, layer_order_by_size = true;
+    bool old_p2 = false;   // VP_OLD_P2 (development knob): every phase-2 init runs the five-products-per-gate k_init_phase2
+    bool getenv_no_hs = false, layer_order_by_size = true;
     DBuf<F> d_hs;   // phase-2 init: products of the second-half eq factors, K * ng * nu entries (k_p2_hs)
     bool values_real = true;   // no gate constant has an imaginary part: every circuit value is in the base field
-    bool lane_init = false;    // base-field values: phase-1 init uses the one-real-product-per-gate kernel
-    int cap_round = 0, cap_round1 = 0, cap_eval = 0, cap_p1 = 0, cap_p2 = 0, cap_un = 0, cap_liu = 0, cap_dot = 0, cap_comb = 0, cap_phase = 0;
+    int cap_round = 0, cap_round1 = 0, cap_eval = 0, cap_p1 = 0, cap_p2 = 0, cap_un = 0, cap_liu = 0, cap_dot = 0, cap_comb = 0;
     template <class Kern>
     int occ_cap(Kern k, int threads = 256, size_t dyn_smem = 0) {  // resident blocks on the whole chip
         int occ = 0;
@@ -1007,6 +1006,8 @@ struct Engine {
     void do_init_phase2(int i);
     void do_round(const SumcheckPlan& P, int j, uint32_t ci_prev, uint32_t tr_out, const F* at_init, bool continues = false, F* poly_out = nullptr);
     void sharded_round(const PhasePlan& PP, int phase, int j, uint32_t ci, uint32_t tr, const F* at_init);
+    void fold_only(const PhasePlan& P, uint32_t fo_begin, int fin_buf, uint32_t ci);
+    MergeArgs merge_args(const PhasePlan& P, uint32_t sc_base, uint32_t n_poly, F* out_poly);
     void do_finalize(const SumcheckPlan& P, uint32_t ci_last, F* keep);
     void do_phase(const PhasePlan& P, uint32_t ci, uint32_t tr_rounds, F* keep, const F* at_init, bool has_a = true,
                   const F* v_first = nullptr);
@@ -1029,8 +1030,6 @@ struct Engine {
     DBuf<ChainSeg> d_chain_segs;
     DBuf<ChainTerm> d_chain_terms;
     int n_chains = 0;
-    void launch_phase_kernel(const SumcheckPlan& P, uint32_t ci, uint32_t round_base, const F* at_init, F* add_term_out,
-                             F* claims, F* out_poly, F* keep);
     uint32_t tail_work = 512;
     void prove_all();
     void prove_fs(const uint8_t seed[32], F* tr_out, F* ch_out);
@@ -1169,31 +1168,25 @@ void Engine::build(const Circuit& circ, int dev, int world_, int rank_, const ui
     cap_liu = occ_cap(k_init_liu);
     cap_dot = occ_cap(k_dot_eq);
     cap_comb = occ_cap(k_combine_phase2);
-    cap_phase = occ_cap(k_sumcheck_phase);
     cap_phase_fs = occ_cap(k_sumcheck_phase_fs);
     dfs_enable_smem();
     cap_dfs = std::min({occ_cap(k_phase_dfs<true, DFS_VREAL>, DFS_THREADS, DFS_DYN_SMEM), occ_cap(k_phase_dfs<false, DFS_VREAL>, DFS_THREADS, DFS_DYN_SMEM),
                         occ_cap(k_phase_dfs<true, DFS_PLAIN>, DFS_THREADS, DFS_DYN_SMEM), occ_cap(k_phase_dfs<false, DFS_PLAIN>, DFS_THREADS, DFS_DYN_SMEM)});
     if (getenv("VP_DFS_GRID")) dfs_grid_override = atoi(getenv("VP_DFS_GRID"));
-    if (getenv("VP_DFS_CAP")) cap_dfs = std::max(2, std::min(cap_dfs, atoi(getenv("VP_DFS_CAP"))));
-    if (getenv("VP_ONE_ROUND_PER_PASS")) use_dfs = false;
     values_real = true;
     for (const Layer& T : C.layers)
         for (size_t g = 0; g < T.c.size() && g < T.ty.size(); ++g)
             if ((T.ty[g] == T_ADDC || T.ty[g] == T_MULC) && T.c[g].im != 0) values_real = false;
-    lane_init = values_real && !getenv("VP_NO_LANE_INIT");
     old_p2 = getenv("VP_OLD_P2") != nullptr;
-    liu_old = getenv("VP_LIU_OLD") != nullptr;
-    p1_old = getenv("VP_P1_OLD") != nullptr;
     layer_order_by_size = getenv("VP_LAYERS_TOP_DOWN") == nullptr;
     getenv_no_hs = getenv("VP_NO_HS") != nullptr;
-    d_hs.alloc((size_t)K * 64);   // development knob: the five-products-per-gate phase-2 init
+    d_hs.alloc((size_t)K * 64);
     {
         int coop = 0;
         CK(cudaDeviceGetAttribute(&coop, cudaDevAttrCooperativeLaunch, dev));
         if (!coop) throw CudaError{"device does not support cooperative launches"};
     }
-    max_grid = std::max({cap_round, cap_round1, cap_un, cap_dot, cap_phase, cap_phase_fs, cap_dfs});  // sizes the block-partials buffer
+    max_grid = std::max({cap_round, cap_round1, cap_un, cap_dot, cap_phase_fs, cap_dfs});  // sizes the block-partials buffer
 
     lay = proof_layout(C);
     fs_sched = fs_schedule(lay);
@@ -1881,13 +1874,13 @@ void Engine::do_init_phase1(int i) {
     const uint32_t k0 = D.ph1.sharded ? D.p1_k0 : 0, k1 = D.ph1.sharded ? D.p1_k1 : K;
     const uint64_t work = (uint64_t)D.p1_items.n * (k1 - k0);
     size_t h = prof_begin(KC_INIT1);
-    if (lane_init && K >= 8 && k1 - k0 >= 4 && n <= 64 && !p1_old) {   // template-major: an item of the template x 4 instances per thread
+    if (values_real && K >= 8 && k1 - k0 >= 4 && n <= 64) {   // template-major: an item of the template x 4 instances per thread
         dim3 grid(cdiv(std::max<uint32_t>((uint32_t)D.p1_items.n, 1), 256), cdiv(k1 - k0, 4), n_stmt);
         k_init_phase1_real_tm<4><<<grid, 256, 0, stream>>>(
             D.p1_items.p, (uint32_t)D.p1_items.n, csr, S_pre, D.S, K, eqtab(0, C.bit_length(i)), d_chal.p + D.ci_assert,
             d_valptr.p, d_sizes.p, D.c.p, val[i - 1].p, bufV[0].p + D.ph1.tab_off[0], bufM[0].p + D.ph1.tab_off[0],
             bufA[0].p + D.ph1.tab_off[0], d_rowpart.p, D.p1_nslots, direct_v ? 0 : 1, (uint32_t)i, D.ph1.maps[0], k0, k1, sstride);
-    } else if (lane_init && work < 0xffffffffull && n <= 64)
+    } else if (values_real && work < 0xffffffffull && n <= 64)
         k_init_phase1_real<<<sgrid(grid_b((uint32_t)std::min<uint64_t>(work, 0xffffffffu), cap_p1il)), 256, 0, stream>>>(
             D.p1_items.p, (uint32_t)D.p1_items.n, csr, S_pre, D.S, K, eqtab(0, C.bit_length(i)), d_chal.p + D.ci_assert,
             d_valptr.p, d_sizes.p, D.c.p, val[i - 1].p, bufV[0].p + D.ph1.tab_off[0], bufM[0].p + D.ph1.tab_off[0],
@@ -1983,7 +1976,7 @@ void Engine::do_init_liu(int i, bool write_a) {
         lk0 = lk1 = 0;
         if (D.ph3.row_hi[0] > D.ph3.row_lo[0]) { lk0 = D.ph3.row_lo[0] / S_pre; lk1 = std::min(K, (D.ph3.row_hi[0] - 1) / S_pre + 1); }
     }
-    if (K >= 8 && lk1 - lk0 >= 8 && !liu_old) {   // template-major: one thread per template entry, a chunk of instances each
+    if (K >= 8 && lk1 - lk0 >= 8) {   // template-major: one thread per template entry, a chunk of instances each
         const uint32_t k_chunk = 8;
         dim3 grid(cdiv(S_pre, 256), cdiv(lk1 - lk0, k_chunk), n_stmt);
         k_init_liu_tm<<<grid, 256, 0, stream>>>(D.liu_off.p, D.liu_perm.p, D.liu_ent.p, eq_off ? D.liu_eqtabs_b.p : D.liu_eqtabs.p, S_pre, K, k_chunk,
@@ -2058,34 +2051,14 @@ void Engine::sharded_round(const PhasePlan& PP, int phase, int j, uint32_t ci, u
     }
     if (j == PP.m + 1) {
         F* rec = d_send.p;
-        const uint32_t n_sc = 1 + PP.n_claims, sc0 = PP.sc_base + PP.n_poly;   // record: table regions, (unused polynomials), add_term, claims
+        const uint32_t sc0 = PP.sc_base + PP.n_poly;   // record: table regions, (unused polynomials), add_term, claims
         CK(cudaMemsetAsync(rec, 0, (size_t)PP.rec_len * sizeof(F), stream));
-        if (PP.n_fo) {
-            const FoldOnlyDesc& f0 = arena.fo[PP.foi_begin];
-            dim3 grid(std::max<uint32_t>(1, std::min<uint32_t>(cdiv(f0.cnt, 128), 64)), PP.n_fo);
-            const int fb = PP.planA.fin_buf;
-            k_fold_only<<<grid, 128, 0, stream>>>(d_fo.p + PP.foi_begin, (int)PP.n_fo, bufV[fb].p, bufM[fb].p, bufA[fb].p,
-                                                 d_chal.p + ci + (uint32_t)(PP.m - 1), rec);
-            ++launches;
-        }
+        fold_only(PP, PP.foi_begin, PP.planA.fin_buf, ci);
         CK(cudaMemcpyAsync(rec + sc0, scal(SC_ADD_TERM), sizeof(F), cudaMemcpyDeviceToDevice, stream));
         CK(cudaMemcpyAsync(rec + sc0 + 1, d_claims.p, (size_t)PP.n_claims * sizeof(F), cudaMemcpyDeviceToDevice, stream));
         NCK(g_nccl.AllGather(rec, d_recv.p, (size_t)PP.rec_len * 2, /*ncclUint64*/ 5, comm, stream));
-        MergeArgs ma;
-        ma.recv = d_recv.p;
-        ma.rec_len = PP.rec_len;
-        ma.G = (uint32_t)world;
-        ma.tabs = d_mt.p + PP.mt_begin;
-        ma.n_tabs = PP.n_mt;
-        ma.sc_base = sc0;          // no polynomials in this record: scalar 0 is add_term, then the claims
-        ma.n_poly = 0;
-        ma.n_claims = PP.n_claims;
-        ma.outV = bufV[0].p; ma.outM = bufM[0].p; ma.outA = bufA[0].p;
-        ma.out_poly = d_send.p;    // unused (n_poly == 0)
-        ma.add_term = scal(SC_ADD_TERM);
-        ma.claims = d_claims.p;
-        (void)n_sc;
-        k_shard_merge<<<8, 256, 0, stream>>>(ma);
+        // no polynomials in this record: scalar 0 is add_term, then the claims (out_poly is not written)
+        k_shard_merge<<<8, 256, 0, stream>>>(merge_args(PP, sc0, 0, d_send.p));
         ++launches;
         do_round(PP.planB, 1, ci + (uint32_t)(PP.m - 1), tr, nullptr, /*continues=*/true);
         return;
@@ -2098,36 +2071,6 @@ void Engine::do_finalize(const SumcheckPlan& P, uint32_t ci_last, F* keep) {
     k_finalize<<<cdiv(P.n_fin, 128), 128, 0, stream>>>(d_fins.p + P.fin_begin, (int)P.n_fin, bufV[fb].p,
                                                         d_chal.p + ci_last, P.rounds >= 1 ? 1 : 0, d_claims.p, d_tr.p,
                                                         keep);
-    ++launches;
-}
-
-// One cooperative launch of k_sumcheck_phase over `P`.
-void Engine::launch_phase_kernel(const SumcheckPlan& P, uint32_t ci, uint32_t round_base, const F* at_init, F* add_term_out,
-                                 F* claims, F* out_poly, F* keep) {
-    PhaseArgs a;
-    for (int b = 0; b < 2; ++b) { a.bufV[b] = bufV[b].p; a.bufM[b] = bufM[b].p; a.bufA[b] = bufA[b].p; }
-    a.rounds = d_rdev.p + P.rdev_begin;
-    a.tabs = d_tabs.p;
-    a.cols = d_cols.p;
-    a.fins = d_fins.p + P.fin_begin;
-    a.n_rounds = (uint32_t)P.rounds;
-    a.n_fin = P.n_fin;
-    a.fin_buf = (uint32_t)P.fin_buf;
-    a.tail_work = tail_work;
-    a.round_base = round_base;
-    a.at_init = at_init;
-    a.chal = d_chal.p + ci;
-    a.add_term = add_term_out;
-    a.claims = claims;
-    a.out_poly = out_poly;
-    a.transcript = d_tr.p;
-    a.keep = keep;
-    a.partials = d_partials.p;
-    const int grid = P.max_work > tail_work ? grid_for(P.max_work, cap_phase) : 1;
-    void* args[] = {&a};
-    size_t h = prof_begin(KC_ROUND_FOLD);
-    CK(cudaLaunchCooperativeKernel((const void*)k_sumcheck_phase, dim3(grid), dim3(256), args, 0, stream));
-    prof_end(h, P.bytes);
     ++launches;
 }
 
@@ -2186,23 +2129,55 @@ void Engine::launch_dfs_kernel(const PassPlan& P, uint32_t ci, uint32_t round_ba
     ++launches;
 }
 
+// The hand-over of a sharded phase over NCCL (sharded_round, do_phase), first step: k_fold_only writes the level-m value of
+// every block of stage A's final buffer fin_buf into the record at d_send, folding a pending pair with r_m.
+void Engine::fold_only(const PhasePlan& P, uint32_t fo_begin, int fin_buf, uint32_t ci) {
+    if (!P.n_fo) return;
+    const FoldOnlyDesc& f0 = arena.fo[fo_begin];
+    dim3 grid(std::max<uint32_t>(1, std::min<uint32_t>(cdiv(f0.cnt, 128), 64)), P.n_fo);
+    k_fold_only<<<grid, 128, 0, stream>>>(d_fo.p + fo_begin, (int)P.n_fo, bufV[fin_buf].p, bufM[fin_buf].p, bufA[fin_buf].p,
+                                         d_chal.p + ci + (uint32_t)(P.m - 1), d_send.p);
+    ++launches;
+}
+
+// The merge of the gathered records of a sharded phase (k_shard_merge, k_xchg): the stage-B tables, and the sums of the
+// record's scalars from sc_base on -- n_poly polynomial coefficients to out_poly, add_term, the claims.
+MergeArgs Engine::merge_args(const PhasePlan& P, uint32_t sc_base, uint32_t n_poly, F* out_poly) {
+    MergeArgs ma;
+    ma.recv = d_recv.p;
+    ma.rec_len = P.rec_len;
+    ma.G = (uint32_t)world;
+    ma.tabs = d_mt.p + P.mt_begin;
+    ma.n_tabs = P.n_mt;
+    ma.sc_base = sc_base;
+    ma.n_poly = n_poly;
+    ma.n_claims = P.n_claims;
+    ma.outV = bufV[0].p; ma.outM = bufM[0].p; ma.outA = bufA[0].p;
+    ma.out_poly = out_poly;
+    ma.add_term = scal(SC_ADD_TERM);
+    ma.claims = d_claims.p;
+    return ma;
+}
+
 // All rounds + the final claims of one sumcheck phase. Unsharded: one cooperative launch. Sharded: the m local
 // rounds on this rank's blocks, fold-only, ONE all-gather of the per-rank records (collapsed blocks + partial
 // round polynomials + partial add_term + claims), merge, then the remaining rounds replicated on every rank.
 void Engine::do_phase(const PhasePlan& P, uint32_t ci, uint32_t tr_rounds, F* keep, const F* at_init, bool has_a,
                       const F* v_first) {
+    const int first = values_real ? DFS_VREAL : DFS_PLAIN;
     if (!P.sharded) {
-        if (use_dfs) launch_dfs_kernel(P.ppB, ci, 0, at_init, scal(SC_ADD_TERM), d_claims.p, d_tr.p + tr_rounds, keep, has_a, values_real ? DFS_VREAL : DFS_PLAIN, v_first);
-        else launch_phase_kernel(P.planB, ci, 0, at_init, scal(SC_ADD_TERM), d_claims.p, d_tr.p + tr_rounds, keep);
+        launch_dfs_kernel(P.ppB, ci, 0, at_init, scal(SC_ADD_TERM), d_claims.p, d_tr.p + tr_rounds, keep, has_a, first, v_first);
         return;
     }
-    const F* v_local_x = (v_first && P.maps.size() == 1 && P.tab_off[0] == 0) ? v_first + P.maps[0].lo : nullptr;
-    if (v_first && !v_local_x) throw CudaError{"direct V: unexpected table layout"};
+    // phase 1 / Liu (one table over layer i-1): the local rows [lo, hi) of V are read straight from circuitValue[i-1]
+    const F* v_local = (v_first && P.maps.size() == 1 && P.tab_off[0] == 0) ? v_first + P.maps[0].lo : nullptr;
+    if (v_first && !v_local) throw CudaError{"direct V: unexpected table layout"};
+    const MergeArgs mg = merge_args(P, P.sc_base, P.n_poly, d_tr.p + tr_rounds);
     if (use_ipc) {
         // stage A leaves its partial scalars in the lane's scalar buffer (zero between phases); ONE kernel pushes the
-        // record to every rank over NVLink, waits for theirs and merges; stage B as below
+        // record to every rank over NVLink, waits for theirs and merges
         F* sc = x.d_sc.p;
-        launch_dfs_kernel(P.ppA, ci, 0, at_init, sc + P.n_poly, sc + P.n_poly + 1, sc, nullptr, has_a, values_real ? DFS_VREAL : DFS_PLAIN, v_local_x);
+        launch_dfs_kernel(P.ppA, ci, 0, at_init, sc + P.n_poly, sc + P.n_poly + 1, sc, nullptr, has_a, first, v_local);
         XchgArgs a;
         memset(&a, 0, sizeof a);
         for (int q = 0; q < world; ++q) a.peer[q] = x.peer[q];
@@ -2224,57 +2199,21 @@ void Engine::do_phase(const PhasePlan& P, uint32_t ci, uint32_t tr_rounds, F* ke
         a.ticket = x.ticket.p;
         a.tag = tr_rounds;
         a.err = d_xerr.p;
-        a.mg.recv = nullptr;
-        a.mg.rec_len = P.rec_len;
-        a.mg.G = (uint32_t)world;
-        a.mg.tabs = d_mt.p + P.mt_begin;
-        a.mg.n_tabs = P.n_mt;
-        a.mg.sc_base = P.sc_base;
-        a.mg.n_poly = P.n_poly;
-        a.mg.n_claims = P.n_claims;
-        a.mg.outV = bufV[0].p; a.mg.outM = bufM[0].p; a.mg.outA = bufA[0].p;
-        a.mg.out_poly = d_tr.p + tr_rounds;
-        a.mg.add_term = scal(SC_ADD_TERM);
-        a.mg.claims = d_claims.p;
+        a.mg = mg;
         const int grid = (int)std::max<uint32_t>(2, std::min<uint32_t>(cdiv(P.rec_len, 512), 32));
         k_xchg<<<grid, 256, 0, stream>>>(a);
         ++launches;
-        launch_dfs_kernel(P.ppB, ci, (uint32_t)P.m, scal(SC_ADD_TERM), scal(SC_ADD_TERM), d_claims.p,
-                          d_tr.p + tr_rounds + 3u * (uint32_t)P.m, keep, has_a, DFS_PLAIN);
-        return;
-    }
-    F* rec = d_send.p;
-    F* sc = rec + P.sc_base;
-    CK(cudaMemsetAsync(sc, 0, (size_t)(P.n_poly + 1 + P.n_claims) * sizeof(F), stream));
-    // stage A: partial polynomials, add_term and claims go straight into the record's scalar region
-    // phase 1 / Liu (one table over layer i-1): the local rows [lo, hi) of V are read straight from circuitValue[i-1]
-    const F* v_local = (v_first && P.maps.size() == 1 && P.tab_off[0] == 0) ? v_first + P.maps[0].lo : nullptr;
-    if (v_first && !v_local) throw CudaError{"direct V: unexpected table layout"};
-    launch_dfs_kernel(P.ppA, ci, 0, at_init, sc + P.n_poly, sc + P.n_poly + 1, sc, nullptr, has_a, values_real ? DFS_VREAL : DFS_PLAIN, v_local);
-    if (P.n_fo) {
-        const FoldOnlyDesc& f0 = arena.fo[P.fo_begin];
-        dim3 grid(std::max<uint32_t>(1, std::min<uint32_t>(cdiv(f0.cnt, 128), 64)), P.n_fo);
-        const int fb = P.ppA.fin_buf;
-        k_fold_only<<<grid, 128, 0, stream>>>(d_fo.p + P.fo_begin, (int)P.n_fo, bufV[fb].p, bufM[fb].p, bufA[fb].p,
-                                             d_chal.p + ci + (uint32_t)(P.m - 1), rec);
+    } else {
+        F* rec = d_send.p;
+        F* sc = rec + P.sc_base;
+        CK(cudaMemsetAsync(sc, 0, (size_t)(P.n_poly + 1 + P.n_claims) * sizeof(F), stream));
+        // stage A: partial polynomials, add_term and claims go straight into the record's scalar region
+        launch_dfs_kernel(P.ppA, ci, 0, at_init, sc + P.n_poly, sc + P.n_poly + 1, sc, nullptr, has_a, first, v_local);
+        fold_only(P, P.fo_begin, P.ppA.fin_buf, ci);
+        NCK(g_nccl.AllGather(rec, d_recv.p, (size_t)P.rec_len * 2, /*ncclUint64*/ 5, comm, stream));
+        k_shard_merge<<<8, 256, 0, stream>>>(mg);
         ++launches;
     }
-    NCK(g_nccl.AllGather(rec, d_recv.p, (size_t)P.rec_len * 2, /*ncclUint64*/ 5, comm, stream));
-    MergeArgs ma;
-    ma.recv = d_recv.p;
-    ma.rec_len = P.rec_len;
-    ma.G = (uint32_t)world;
-    ma.tabs = d_mt.p + P.mt_begin;
-    ma.n_tabs = P.n_mt;
-    ma.sc_base = P.sc_base;
-    ma.n_poly = P.n_poly;
-    ma.n_claims = P.n_claims;
-    ma.outV = bufV[0].p; ma.outM = bufM[0].p; ma.outA = bufA[0].p;
-    ma.out_poly = d_tr.p + tr_rounds;
-    ma.add_term = scal(SC_ADD_TERM);
-    ma.claims = d_claims.p;
-    k_shard_merge<<<8, 256, 0, stream>>>(ma);
-    ++launches;
     // stage B: replicated; starts from the summed add_term
     launch_dfs_kernel(P.ppB, ci, (uint32_t)P.m, scal(SC_ADD_TERM), scal(SC_ADD_TERM), d_claims.p,
                       d_tr.p + tr_rounds + 3u * (uint32_t)P.m, keep, has_a, DFS_PLAIN);
@@ -2530,8 +2469,8 @@ int Engine::verify_check(const F* tr, const F* out, const F* chal, int* fail_cod
 // The whole proof in verifier.cpp:134-189 order, challenges already in d_chal.
 void Engine::prove_all() {
     leave();   // (a previous call may have failed inside a lane)
-    direct_v = use_dfs;   // phase 1 / Liu read V from circuitValue[i-1] (sharded: the rank's rows of it)
-    const bool lane = two_lanes && use_dfs;
+    direct_v = true;   // phase 1 / Liu read V from circuitValue[i-1] (sharded: the rank's rows of it)
+    const bool lane = two_lanes;
     const bool lane3 = lane && three_lanes;
     const bool lane6 = lane3 && six_lanes;
     evaluate();
@@ -2593,7 +2532,7 @@ void Engine::prove_all() {
         // ---- phase 1
         if (odd) enter(lane0b, 0);
         do_init_phase1(i);
-        do_phase(D.ph1, D.ci_ru, D.tr_p1, lane3 ? d_vu.p + i : scal(SC_VU), nullptr, true, direct_v ? val[i - 1].p : nullptr);
+        do_phase(D.ph1, D.ci_ru, D.tr_p1, lane3 ? d_vu.p + i : scal(SC_VU), nullptr, true, val[i - 1].p);
         if (lane3 && m != -1) CK(cudaEventRecord(ev_p1v[i], stream));
         if (odd) leave();
         // ---- phase 2: on its own lane, behind this layer's phase 1
@@ -2609,8 +2548,8 @@ void Engine::prove_all() {
         }
         // ---- Liu
         if (lane) enter(odd ? lane1b : lane1, 1);
-        do_init_liu(i, !use_dfs);
-        do_phase(D.ph3, D.ci_rliu, D.tr_liu, nullptr, nullptr, /*has_a=*/!use_dfs, direct_v ? val[i - 1].p : nullptr);
+        do_init_liu(i, false);   // the Liu add table is zero: the pass kernel runs without it (has_a)
+        do_phase(D.ph3, D.ci_rliu, D.tr_liu, nullptr, nullptr, /*has_a=*/false, val[i - 1].p);
         if (lane) leave();
     }
     if (lane) {   // join: the b coefficients, the input MLE and the transcript copy follow on the main lane
@@ -2622,7 +2561,7 @@ void Engine::prove_all() {
             CK(cudaStreamWaitEvent(stream, R->ev_done, 0));
         }
     }
-    if (use_dfs) derive_b();
+    derive_b();
     do_input_mle();
     direct_v = false;
     CK(cudaGetLastError());
@@ -2842,9 +2781,7 @@ void Engine::launch_phase_kernel_fs(const SumcheckPlan& P, uint32_t ci, F* keep,
     a.n_fin = P.n_fin;
     a.fin_buf = (uint32_t)P.fin_buf;
     a.tail_work = tail_work;
-    a.round_base = 0;
     a.at_init = at_init;
-    a.chal = d_chal.p + ci;
     a.add_term = scal(SC_ADD_TERM);
     a.claims = d_claims.p;
     a.out_poly = d_tr.p + tr_rounds;
@@ -2868,7 +2805,7 @@ void Engine::launch_phase_kernel_fs(const SumcheckPlan& P, uint32_t ci, F* keep,
             const size_t d = s0 * sstride;
             auto sh = [d](auto* q) { return q ? reinterpret_cast<decltype(q)>(reinterpret_cast<uintptr_t>(q) + d) : q; };
             for (int b = 0; b < 2; ++b) { ac.bufV[b] = sh(a.bufV[b]); ac.bufM[b] = sh(a.bufM[b]); ac.bufA[b] = sh(a.bufA[b]); }
-            ac.at_init = sh(a.at_init); ac.chal = sh(a.chal); ac.add_term = sh(a.add_term); ac.claims = sh(a.claims);
+            ac.at_init = sh(a.at_init); ac.add_term = sh(a.add_term); ac.claims = sh(a.claims);
             ac.out_poly = sh(a.out_poly); ac.transcript = sh(a.transcript); ac.keep = sh(a.keep); ac.partials = sh(a.partials);
             fc.pool = sh(f.pool); fc.chal = sh(f.chal); fc.stamps = nullptr;
         }

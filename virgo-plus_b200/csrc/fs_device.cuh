@@ -98,18 +98,20 @@ __global__ void k_fs_statement(const uint64_t* __restrict__ circuit, const uint6
 }
 
 // ------------------------------------------------------------------ K6f: a Fiat-Shamir sumcheck phase in ONE launch
-// k_sumcheck_phase with the challenges drawn inside: after round j's grid barrier block 0 reduces the partials, writes
-// (a, b, c) to the transcript, stores them in the pool and draws the round's challenge into chal[j - 1]; a second grid
-// barrier then releases the other blocks into round j + 1's fold, which needs that challenge. The tail rounds (block 0
-// alone) store and draw the same way behind a block barrier. The final claims are written like k_sumcheck_phase writes
-// them; storing them is the next k_fs_absorb_draw's job.
+// All rounds of one phase (phase 1, phase 2 or Liu of one layer; the plan is PhaseArgs, kernels.cuh), with the challenges
+// drawn inside. A cooperative grid walks the rounds; blocks meet at a grid barrier once per round (the round's tables are
+// written by all blocks and read by all blocks in the next round). After round j's barrier block 0 reduces the per-block
+// partials, writes (a, b, c) to the transcript, stores them in the pool and draws the round's challenge into chal[j - 1];
+// a second grid barrier then releases the other blocks into round j + 1's fold, which needs that challenge. Block 0 keeps
+// add_term in a register. Once a round's work fits one block, block 0 runs the remaining rounds alone, storing and drawing
+// the same way behind block barriers, and writes the final claims; storing them is the next k_fs_absorb_draw's job.
 // stamps (4 per round, block 0, %globaltimer): round start, own fold work done, polynomial reduced (grid rounds: after the
 // barrier), challenge drawn. The next round's start minus "drawn" is the release barrier.
 // A batch runs a gridDim.x x B grid: row blockIdx.z is statement b, its block x == 0 reduces the row's partials and draws
 // the statement's challenge, and one grid barrier serves all rows. Stamps are those of row 0.
 struct FsPhaseArgs {
     uint64_t* pool;
-    F* chal;                     // = PhaseArgs::chal, writable
+    F* chal;                     // chal[j - 1]: the challenge drawn after round j
     unsigned long long* stamps;  // 4 * n_rounds, may be null
     size_t ss;                   // bytes between two statements' working sets (0: one statement)
 };
@@ -118,6 +120,44 @@ VP_D void fs_stamp(unsigned long long* s, uint32_t j, int k) {
     unsigned long long t;
     asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
     s[4 * (j - 1) + k] = t;
+}
+
+// Round j of k_sumcheck_phase_fs on threads t, t + stride, ... (t == 0: thread 0 of block 0): fold the round's tables
+// with the previous challenge and sum them into v. reduce(v, collapse) makes v the round's sums and calls collapse() on
+// thread 0 of block 0 (the tables that collapse in this round join add_term); it returns true on that thread alone, which
+// then writes the round polynomial, stores it in the pool and draws the round's challenge.
+template <class Reduce>
+VP_D void fs_round(const PhaseArgs& p, const RoundDev& R, uint32_t j, uint32_t t, uint32_t stride, size_t ss, uint32_t* s_wend,
+                   uint64_t* pool, F* chal, F* claims, F& at, unsigned long long* stamps, Reduce reduce) {
+    if (t == 0) fs_stamp(stamps, j, 0);
+    __syncthreads();   // (tail rounds: also publishes the previous round's challenge to the block)
+    for (uint32_t i = threadIdx.x; i < R.n_tabs; i += blockDim.x) s_wend[i] = p.tabs[R.tab_begin + i].work_end;
+    __syncthreads();
+    const uint32_t ib = R.in_buf, ob = ib ^ 1;
+    const bool fold = j >= 2;
+    const F prev = fold ? ld_f_cg(chal + j - 2) : f_zero();   // drawn by block 0 in this launch: bypass L1
+    const FoldK rk = make_foldk(prev);
+    F* const inV = stmt_at(p.bufV[ib], ss);
+    F* const inM = stmt_at(p.bufM[ib], ss);
+    F* const inA = stmt_at(p.bufA[ib], ss);
+    RoundAcc acc;
+    racc_init(acc);
+    if (fold) round_work<true, false>(acc, p.tabs + R.tab_begin, R.n_tabs, s_wend, inV, inM, inA, stmt_at(p.bufV[ob], ss),
+                                      stmt_at(p.bufM[ob], ss), stmt_at(p.bufA[ob], ss), rk, t, stride);
+    else round_work<false, false>(acc, p.tabs + R.tab_begin, R.n_tabs, s_wend, inV, inM, inA, stmt_at(p.bufV[ob], ss),
+                                  stmt_at(p.bufM[ob], ss), stmt_at(p.bufA[ob], ss), rk, t, stride);
+    F v[3];
+    racc_finish(acc, v);
+    const auto collapse = [&] {
+        at = collapse_update<false>(at, p.cols + R.col_begin, R.n_cols, inV, inM, inA, fold, /*scale=*/fold, prev, rk, claims);
+    };
+    if (!reduce(v, collapse)) return;
+    const F o[3] = {v[0], f_sub(v[1], at), f_add(v[2], at)};
+    F* out = stmt_at(p.out_poly, ss) + 3 * (j - 1);
+    fs_stamp(stamps, j, 2);
+    for (int k = 0; k < 3; ++k) { st_f(out + k, o[k]); fs_store(pool, o[k]); }
+    st_f(chal + j - 1, fs_draw(pool));
+    fs_stamp(stamps, j, 3);
 }
 
 __global__ void __launch_bounds__(256, 2) k_sumcheck_phase_fs(PhaseArgs p, FsPhaseArgs f) {
@@ -138,91 +178,42 @@ __global__ void __launch_bounds__(256, 2) k_sumcheck_phase_fs(PhaseArgs p, FsPha
     for (; j <= p.n_rounds; ++j) {
         const RoundDev R = p.rounds[j - 1];
         if (R.work <= p.tail_work) break;
-        if (stamp) fs_stamp(stamps, j, 0);
-        const bool fold = j >= 2;
-        __syncthreads();
-        for (uint32_t i = threadIdx.x; i < R.n_tabs; i += blockDim.x) s_wend[i] = p.tabs[R.tab_begin + i].work_end;
-        __syncthreads();
-        const uint32_t ib = R.in_buf, ob = ib ^ 1;
-        const bool scale = j >= 2;
-        const F prev = scale ? ld_f_cg(chal + j - 2) : f_zero();   // drawn by block 0 in this launch: bypass L1
-        const FoldK rk = make_foldk(prev);
-        RoundAcc acc;
-        racc_init(acc);
-        if (fold) round_work<true, false>(acc, p.tabs + R.tab_begin, R.n_tabs, s_wend, stmt_at(p.bufV[ib], ss), stmt_at(p.bufM[ib], ss),
-                                          stmt_at(p.bufA[ib], ss), stmt_at(p.bufV[ob], ss), stmt_at(p.bufM[ob], ss),
-                                          stmt_at(p.bufA[ob], ss), rk, gtid, gstride);
-        else round_work<false, false>(acc, p.tabs + R.tab_begin, R.n_tabs, s_wend, stmt_at(p.bufV[ib], ss), stmt_at(p.bufM[ib], ss),
-                                      stmt_at(p.bufA[ib], ss), stmt_at(p.bufV[ob], ss), stmt_at(p.bufM[ob], ss),
-                                      stmt_at(p.bufA[ob], ss), rk, gtid, gstride);
-        F v[3];
-        racc_finish(acc, v);
-        block_sum<3>(v, smem);
         F* part = stmt_at(p.partials, ss) + (size_t)(j & 1) * gridDim.x * 3;
-        if (threadIdx.x == 0) {
-            st_f(part + (size_t)blockIdx.x * 3 + 0, v[0]);
-            st_f(part + (size_t)blockIdx.x * 3 + 1, v[1]);
-            st_f(part + (size_t)blockIdx.x * 3 + 2, v[2]);
-            if (blockIdx.x == 0)
-                at = collapse_update<false>(at, p.cols + R.col_begin, R.n_cols, stmt_at(p.bufV[ib], ss), stmt_at(p.bufM[ib], ss),
-                                            stmt_at(p.bufA[ib], ss), fold, scale, prev, rk, claims);
-        }
-        if (stamp) fs_stamp(stamps, j, 1);
-        grid.sync();
-        if (blockIdx.x == 0) {
-            F t[3] = {f_zero(), f_zero(), f_zero()};
-            for (uint32_t b = threadIdx.x; b < gridDim.x; b += blockDim.x) {
-                t[0] = f_add(t[0], ld_one<false>(part + (size_t)b * 3 + 0));
-                t[1] = f_add(t[1], ld_one<false>(part + (size_t)b * 3 + 1));
-                t[2] = f_add(t[2], ld_one<false>(part + (size_t)b * 3 + 2));
-            }
-            block_sum<3>(t, smem);
+        fs_round(p, R, j, gtid, gstride, ss, s_wend, pool, chal, claims, at, stamps, [&](F (&v)[3], auto collapse) {
+            block_sum<3>(v, smem);
             if (threadIdx.x == 0) {
-                const F o[3] = {t[0], f_sub(t[1], at), f_add(t[2], at)};
-                F* out = stmt_at(p.out_poly, ss) + 3 * (j - 1);
-                fs_stamp(stamps, j, 2);
-                for (int k = 0; k < 3; ++k) { st_f(out + k, o[k]); fs_store(pool, o[k]); }
-                st_f(chal + j - 1, fs_draw(pool));
-                fs_stamp(stamps, j, 3);
+                st_f(part + (size_t)blockIdx.x * 3 + 0, v[0]);
+                st_f(part + (size_t)blockIdx.x * 3 + 1, v[1]);
+                st_f(part + (size_t)blockIdx.x * 3 + 2, v[2]);
+                // tables collapsing in this round are inputs of this round: read them before the barrier, the next
+                // round may overwrite that buffer
+                if (blockIdx.x == 0) collapse();
             }
-        }
+            if (stamp) fs_stamp(stamps, j, 1);
+            grid.sync();
+            if (blockIdx.x != 0) return false;
+            v[0] = v[1] = v[2] = f_zero();
+            for (uint32_t b = threadIdx.x; b < gridDim.x; b += blockDim.x) {
+                v[0] = f_add(v[0], ld_one<false>(part + (size_t)b * 3 + 0));
+                v[1] = f_add(v[1], ld_one<false>(part + (size_t)b * 3 + 1));
+                v[2] = f_add(v[2], ld_one<false>(part + (size_t)b * 3 + 2));
+            }
+            block_sum<3>(v, smem);
+            return threadIdx.x == 0;
+        });
         grid.sync();   // release: round j + 1 folds with the challenge just drawn
     }
     if (blockIdx.x != 0) return;
     // ---- tail rounds: block 0 alone
     for (; j <= p.n_rounds; ++j) {
         const RoundDev R = p.rounds[j - 1];
-        if (stamp) fs_stamp(stamps, j, 0);
-        const bool fold = j >= 2;
-        __syncthreads();   // (also publishes the previous round's challenge to the block)
-        for (uint32_t i = threadIdx.x; i < R.n_tabs; i += blockDim.x) s_wend[i] = p.tabs[R.tab_begin + i].work_end;
-        __syncthreads();
-        const uint32_t ib = R.in_buf, ob = ib ^ 1;
-        const bool scale = j >= 2;
-        const F prev = scale ? ld_f_cg(chal + j - 2) : f_zero();
-        const FoldK rk = make_foldk(prev);
-        RoundAcc acc;
-        racc_init(acc);
-        if (fold) round_work<true, false>(acc, p.tabs + R.tab_begin, R.n_tabs, s_wend, stmt_at(p.bufV[ib], ss), stmt_at(p.bufM[ib], ss),
-                                          stmt_at(p.bufA[ib], ss), stmt_at(p.bufV[ob], ss), stmt_at(p.bufM[ob], ss),
-                                          stmt_at(p.bufA[ob], ss), rk, threadIdx.x, blockDim.x);
-        else round_work<false, false>(acc, p.tabs + R.tab_begin, R.n_tabs, s_wend, stmt_at(p.bufV[ib], ss), stmt_at(p.bufM[ib], ss),
-                                      stmt_at(p.bufA[ib], ss), stmt_at(p.bufV[ob], ss), stmt_at(p.bufM[ob], ss),
-                                      stmt_at(p.bufA[ob], ss), rk, threadIdx.x, blockDim.x);
-        F v[3];
-        racc_finish(acc, v);
-        if (stamp) fs_stamp(stamps, j, 1);
-        block_sum<3>(v, smem);
-        if (threadIdx.x == 0) {
-            at = collapse_update<false>(at, p.cols + R.col_begin, R.n_cols, stmt_at(p.bufV[ib], ss), stmt_at(p.bufM[ib], ss),
-                                        stmt_at(p.bufA[ib], ss), fold, scale, prev, rk, claims);
-            const F o[3] = {v[0], f_sub(v[1], at), f_add(v[2], at)};
-            F* out = stmt_at(p.out_poly, ss) + 3 * (j - 1);
-            fs_stamp(stamps, j, 2);
-            for (int k = 0; k < 3; ++k) { st_f(out + k, o[k]); fs_store(pool, o[k]); }
-            st_f(chal + j - 1, fs_draw(pool));
-            fs_stamp(stamps, j, 3);
-        }
+        fs_round(p, R, j, threadIdx.x, blockDim.x, ss, s_wend, pool, chal, claims, at, stamps, [&](F (&v)[3], auto collapse) {
+            if (stamp) fs_stamp(stamps, j, 1);
+            block_sum<3>(v, smem);
+            if (threadIdx.x != 0) return false;
+            collapse();
+            return true;
+        });
     }
     __syncthreads();  // the last round's table writes, the claims of collapsed tables and the last challenge
     if (threadIdx.x == 0) st_f(stmt_at(p.add_term, ss), at);

@@ -1137,13 +1137,9 @@ __global__ void k_finalize(const FinDesc* __restrict__ d, int n, const F* __rest
     if (keep && i == 0) st_f(keep, c);   // V_u for phase 2 (prover.cpp:497)
 }
 
-// ------------------------------------------------------------------ K6p: a whole sumcheck phase in ONE launch
-// All rounds of one phase (phase 1, phase 2 or Liu of one layer) when the challenges are already on
-// the device (vp_prove; the reference verifier's challenges do not depend on the prover's messages).
-// A cooperative grid walks the rounds; blocks meet at a grid barrier once per round (the round's
-// tables are written by all blocks and read by all blocks in the next round), block 0 reduces the
-// per-block partials and keeps add_term in a register. Once a round's work fits one block, block 0
-// finishes the remaining rounds alone with block barriers only, and writes the final claims.
+// ------------------------------------------------------------------ K6f: one sumcheck phase in ONE launch, one round per pass
+// The plan of k_sumcheck_phase_fs (fs_device.cuh), which runs all rounds of one phase (phase 1, phase 2 or Liu of one
+// layer) of a Fiat-Shamir proof and draws each round's challenge itself.
 struct RoundDev {
     uint32_t tab_begin, n_tabs, col_begin, n_cols;
     uint32_t work;     // pairs (first round) or quads
@@ -1159,9 +1155,7 @@ struct PhaseArgs {
     const FinDesc* fins;
     uint32_t n_rounds, n_fin, fin_buf;
     uint32_t tail_work;        // rounds with work <= tail_work run on block 0 alone
-    uint32_t round_base;       // rounds already done before this kernel (sharded: the local rounds); global round = base + j
-    const F* at_init;          // initial add_term (phase 2: unary-gate sum; stage B: the summed partial add_terms), may be null
-    const F* chal;             // challenge bound after GLOBAL round g = chal[g-1]; prev of global round g = chal[g-2]
+    const F* at_init;          // initial add_term (phase 2: the unary-gate sum), may be null
     F* add_term;
     F* claims;
     F* out_poly;               // round j -> out_poly[3*(j-1) ..]
@@ -1169,113 +1163,6 @@ struct PhaseArgs {
     F* keep;                   // V_u (phase 1) or null
     F* partials;               // 2 * gridDim.x * 3
 };
-
-__global__ void __launch_bounds__(256, 2) k_sumcheck_phase(PhaseArgs p) {
-    namespace cg = cooperative_groups;
-    cg::grid_group grid = cg::this_grid();
-    __shared__ F smem[3 * 32];
-    __shared__ uint32_t s_wend[128];
-    const uint32_t gtid = blockIdx.x * blockDim.x + threadIdx.x, gstride = gridDim.x * blockDim.x;
-    F at = p.at_init ? *p.at_init : f_zero();  // add_term: meaningful in block 0 / thread 0 only
-    uint32_t j = 1;
-    // ---- grid rounds
-    for (; j <= p.n_rounds; ++j) {
-        const RoundDev R = p.rounds[j - 1];
-        if (R.work <= p.tail_work) break;
-        const bool fold = j >= 2;
-        __syncthreads();
-        for (uint32_t i = threadIdx.x; i < R.n_tabs; i += blockDim.x) s_wend[i] = p.tabs[R.tab_begin + i].work_end;
-        __syncthreads();
-        const uint32_t ib = R.in_buf, ob = ib ^ 1;
-        const bool scale = p.round_base + j >= 2;
-        const F prev = scale ? p.chal[p.round_base + j - 2] : f_zero();
-        const FoldK rk = make_foldk(prev);
-        RoundAcc acc;
-        racc_init(acc);
-        if (fold) round_work<true, false>(acc, p.tabs + R.tab_begin, R.n_tabs, s_wend, p.bufV[ib], p.bufM[ib], p.bufA[ib],
-                                          p.bufV[ob], p.bufM[ob], p.bufA[ob], rk, gtid, gstride);
-        else round_work<false, false>(acc, p.tabs + R.tab_begin, R.n_tabs, s_wend, p.bufV[ib], p.bufM[ib], p.bufA[ib],
-                                      p.bufV[ob], p.bufM[ob], p.bufA[ob], rk, gtid, gstride);
-        F v[3];
-        racc_finish(acc, v);
-        block_sum<3>(v, smem);
-        F* part = p.partials + (size_t)(j & 1) * gridDim.x * 3;
-        if (threadIdx.x == 0) {
-            st_f(part + (size_t)blockIdx.x * 3 + 0, v[0]);
-            st_f(part + (size_t)blockIdx.x * 3 + 1, v[1]);
-            st_f(part + (size_t)blockIdx.x * 3 + 2, v[2]);
-            // tables collapsing in this round are inputs of this round: read them before the barrier, the next
-            // round may overwrite that buffer
-            if (blockIdx.x == 0)
-                at = collapse_update<false>(at, p.cols + R.col_begin, R.n_cols, p.bufV[ib], p.bufM[ib], p.bufA[ib], fold,
-                                            scale, prev, rk, p.claims);
-        }
-        grid.sync();
-        if (blockIdx.x == 0) {
-            F t[3] = {f_zero(), f_zero(), f_zero()};
-            for (uint32_t b = threadIdx.x; b < gridDim.x; b += blockDim.x) {
-                t[0] = f_add(t[0], ld_one<false>(part + (size_t)b * 3 + 0));
-                t[1] = f_add(t[1], ld_one<false>(part + (size_t)b * 3 + 1));
-                t[2] = f_add(t[2], ld_one<false>(part + (size_t)b * 3 + 2));
-            }
-            block_sum<3>(t, smem);
-            if (threadIdx.x == 0) {
-                F* o = p.out_poly + 3 * (j - 1);
-                st_f(o + 0, t[0]);
-                st_f(o + 1, f_sub(t[1], at));
-                st_f(o + 2, f_add(t[2], at));
-            }
-        }
-    }
-    if (blockIdx.x != 0) return;
-    // ---- tail rounds: block 0 alone (everything it reads was written before the last grid barrier, or by itself)
-    for (; j <= p.n_rounds; ++j) {
-        const RoundDev R = p.rounds[j - 1];
-        const bool fold = j >= 2;
-        __syncthreads();
-        for (uint32_t i = threadIdx.x; i < R.n_tabs; i += blockDim.x) s_wend[i] = p.tabs[R.tab_begin + i].work_end;
-        __syncthreads();
-        const uint32_t ib = R.in_buf, ob = ib ^ 1;
-        const bool scale = p.round_base + j >= 2;
-        const F prev = scale ? p.chal[p.round_base + j - 2] : f_zero();
-        const FoldK rk = make_foldk(prev);
-        RoundAcc acc;
-        racc_init(acc);
-        if (fold) round_work<true, false>(acc, p.tabs + R.tab_begin, R.n_tabs, s_wend, p.bufV[ib], p.bufM[ib], p.bufA[ib],
-                                          p.bufV[ob], p.bufM[ob], p.bufA[ob], rk, threadIdx.x, blockDim.x);
-        else round_work<false, false>(acc, p.tabs + R.tab_begin, R.n_tabs, s_wend, p.bufV[ib], p.bufM[ib], p.bufA[ib],
-                                      p.bufV[ob], p.bufM[ob], p.bufA[ob], rk, threadIdx.x, blockDim.x);
-        F v[3];
-        racc_finish(acc, v);
-        block_sum<3>(v, smem);
-        if (threadIdx.x == 0) {
-            at = collapse_update<false>(at, p.cols + R.col_begin, R.n_cols, p.bufV[ib], p.bufM[ib], p.bufA[ib], fold, scale, prev,
-                                        rk, p.claims);
-            F* o = p.out_poly + 3 * (j - 1);
-            st_f(o + 0, v[0]);
-            st_f(o + 1, f_sub(v[1], at));
-            st_f(o + 2, f_add(v[2], at));
-        }
-    }
-    __syncthreads();  // the last round's table writes and the claims of collapsed tables
-    if (threadIdx.x == 0) st_f(p.add_term, at);
-    // ---- final claims (prover.cpp:494-521)
-    const F* V = p.bufV[p.fin_buf];
-    for (uint32_t i = threadIdx.x; i < p.n_fin; i += blockDim.x) {
-        const FinDesc f = p.fins[i];
-        F c;
-        if (f.from_claim >= 0) c = ld_one<false>(p.claims + f.from_claim);
-        else {
-            const F v0 = f.n_vals >= 1 ? ld_one<false>(V + f.in_off) : f_zero();
-            if (p.n_rounds >= 1) {
-                const F v1 = f.n_vals >= 2 ? ld_one<false>(V + f.in_off + 1) : f_zero();
-                c = f_fold(v0, v1, p.chal[p.round_base + p.n_rounds - 1]);
-            } else c = v0;
-        }
-        st_f(p.transcript + f.out_idx, c);
-        if (p.keep && i == 0) st_f(p.keep, c);
-    }
-}
 
 // ------------------------------------------------------------------ K6d: two rounds per pass (whole-proof mode)
 // With the challenges on the device a pass can run TWO rounds on data it holds in registers: a thread reads a
@@ -1333,10 +1220,6 @@ struct DfsArgs {
 // the verifier's check verifier.cpp:209,248,296 identically, so b need not be summed: k_derive_b fills it in from the
 // claim chain once the claims it starts from are known). Two complex products per pair instead of the reference's
 // four (polynomial.cpp:101-110); both sums are LAZY (96-bit partial sums of the limb products, reduced once per pass).
-#ifndef VP_DFS_LAZY1
-#define VP_DFS_LAZY1 1
-#endif
-#if VP_DFS_LAZY1
 struct PassAcc {
     CAcc A, C;
     u64 s0re, s0im;   // sum of a0, folded once per work item
@@ -1354,23 +1237,6 @@ VP_D void pacc_mad_real(CAcc& acc, const F& m, u64 v) { cacc_mad_real(acc, m, v)
 typedef CAcc PassSum;
 VP_D PassSum psum_zero() { return cacc_zero(); }
 VP_D F psum_reduce(const PassSum& s) { return cacc_reduce(s); }
-#else   // build-time variant: weakly canonical running values in round 1 as well (fewer registers, 16 more instructions per product)
-struct PassAcc {
-    F A, C;
-    u64 s0re, s0im;
-};
-VP_D void pacc_init(PassAcc& s) { s.A = f_zero(); s.C = f_zero(); s.s0re = s.s0im = 0; }
-VP_D void pacc_finish(const PassAcc& s, F& a, F& c) {
-    a = f_strict(s.A);
-    c = f_add(f_strict(s.C), F{fp_canon(s.s0re), fp_canon(s.s0im)});
-}
-VP_D F f_mul_add_w(const F& a, const F& b, const F& acc);
-VP_D void pacc_mad(F& acc, const F& m, const F& v) { acc = f_mul_add_w(m, v, acc); }
-VP_D void pacc_mad_real(F& acc, const F& m, u64 v) { acc = f_mad_real_w(acc, m, v); }
-typedef F PassSum;
-VP_D PassSum psum_zero() { return f_zero(); }
-VP_D F psum_reduce(const PassSum& s) { return f_strict(s); }
-#endif
 // Second round of a pass: the same two sums, but as weakly canonical running values that ride in the products'
 // reductions (8 registers instead of 28: the pass kernel is register bound, and the second round is a third of the work)
 struct PassAcc2 {
@@ -1982,7 +1848,7 @@ struct XchgArgs {
     unsigned int* ticket;     // zero at launch, left zero
     uint32_t tag;             // identifies the phase (its transcript offset): every rank must be exchanging the same phase
     unsigned int* err;        // set to 1 if a peer's record carries another tag / sequence number
-    MergeArgs mg;             // recv is filled in by the kernel
+    MergeArgs mg;             // recv is not read: the kernel merges from the exchange buffer
 };
 VP_D void st_f_sys(F* p, const F& v) {   // peer memory: plain 128-bit store, ordered by the release below
     asm volatile("st.global.v2.u64 [%0], {%1,%2};" ::"l"(p), "l"(v.re), "l"(v.im) : "memory");

@@ -144,30 +144,6 @@ __global__ void __launch_bounds__(512) k_pc_ntt_smem(const F* __restrict__ coef,
     }
     (void)n;
 }
-// One global DIT stage s >= 11 over the work buffer ([64 * 32] transforms of size n); the last stage (s == log_n - 1)
-// writes to l_eval[s][32 k + c] instead.
-__global__ void k_pc_dit_stage(F* __restrict__ work, uint32_t log_n, uint32_t s, size_t total_pairs, const F* __restrict__ tw, uint32_t log_N,
-                               F* __restrict__ l_eval, int last) {
-    const uint32_t half = 1u << s;
-    for (size_t w = (size_t)blockIdx.x * blockDim.x + threadIdx.x; w < total_pairs; w += (size_t)gridDim.x * blockDim.x) {
-        const size_t t = w >> (log_n - 1);                       // transform = slice * 32 + coset
-        const uint32_t q = (uint32_t)(w & ((1u << (log_n - 1)) - 1));
-        const uint32_t j = q & (half - 1), p = ((q >> s) << (s + 1)) | j;
-        F* x = work + (t << log_n);
-        const F u = pc_ld(x + p), v = f_mul(pc_ld(x + p + half), pc_ld(tw + ((size_t)j << (log_N - s - 1))));
-        const F r0 = f_add(u, v), r1 = f_sub(u, v);
-        if (last) {
-            const size_t sl = t >> PC_LOG_RATE, c = t & (PC_COSETS - 1);
-            F* o = l_eval + (sl << log_N) + c;
-            pc_st(o + ((size_t)p << PC_LOG_RATE), r0);
-            pc_st(o + ((size_t)(p + half) << PC_LOG_RATE), r1);
-        } else {
-            pc_st(x + p, r0);
-            pc_st(x + p + half, r1);
-        }
-    }
-}
-
 // g <= 6 consecutive global DIT stages s0 .. s0+g-1 in ONE pass over the work buffer. Those stages only couple positions that
 // differ in bits s0 .. s0+g-1, so position p = top << (s0+g) | mid << s0 | lo splits every transform into independent 2^g-point
 // columns of stride 2^s0; a block takes 32 neighbouring columns (32 consecutive lo: 512-byte rows) into shared memory
@@ -519,13 +495,7 @@ static void pc_extend(PcCommit* p, const F* src, size_t slice_stride, uint32_t i
     k_pc_ntt_smem<<<grid, threads, sizeof(F) << log_m, st>>>(src, log_n, log_m, p->tw, log_N, direct ? eval : p->work, direct ? 1 : 0, slice_stride,
                                                             in_stride, in_off);
     ++p->launches;
-    if (!direct && getenv("VP_PC_SINGLE_STAGES")) {                 // one pass per stage (kept for A/B timing)
-        const size_t pairs = ((size_t)PC_SLICES * PC_COSETS << log_n) / 2;
-        for (uint32_t s = log_m; s < log_n; ++s) {
-            k_pc_dit_stage<<<pc_grid(pairs, 256), 256, 0, st>>>(p->work, log_n, s, pairs, p->tw, log_N, eval, s == log_n - 1 ? 1 : 0);
-            ++p->launches;
-        }
-    } else if (!direct) {
+    if (!direct) {
         for (uint32_t s0 = log_m; s0 < log_n;) {                   // up to 6 stages per pass
             const uint32_t g = std::min<uint32_t>(PC_DIT_GROUP, log_n - s0);
             const size_t blocks = ((size_t)PC_SLICES * PC_COSETS) << (log_n - g - PC_DIT_COLS_LOG);
