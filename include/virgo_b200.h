@@ -318,6 +318,36 @@ int vp_verify_fs_bound(vp_ctx* ctx, const uint8_t context[32], const vp_F* outpu
                        int* accept, int* fail_code, int* fail_layer);
 int vp_fs_round_stamps(vp_ctx* ctx, unsigned long long* out, size_t cap, size_t* n_rounds);
 
+/* Aggregate statement-bound proofs: ONE Fiat-Shamir proof that binds B statements of one circuit, each with its own inputs,
+ * outputs and 32-byte context. The context's circuit is replicate(template, N); for 1 <= B <= 65535 with B | N, K = N / B,
+ * statement b covers instances [b K, (b + 1) K) of the resident inputs and of the output layer:
+ *   statement_b = H("VPSTMT01" | circuit digest of template + K (the VPCIRC01 bytes with u64 instances = K) | u64 K * S_0 |
+ *                   R(statement b's slice of circuitValue[0]) | u64 K * S_out | R(its slice of the output layer) | context_b),
+ *   i.e. vp_statement_digest on a context of replicate(template, K) (the template itself when K = 1) holding inputs b, with
+ *   context b: exactly the seed a single bound proof of statement b would use;
+ *   aggregate = H("VPAGGR01" | u64 B | R(statement_0 | ... | statement_{B-1})) (48 bytes hashed; domain-separated from
+ *   VPSTMT01, so the aggregate of one statement is not that statement's seed).
+ * vp_prove_fs_aggregate(ctx, B, contexts) is, by definition, vp_prove_fs(ctx, aggregate): its rounds grow with log B, not
+ * with B. contexts: B * 32 bytes; statements (may be NULL): B * 32 bytes, statement-major; aggregate (may be NULL in the
+ * prover): 32 bytes.
+ * vp_aggregate_digest: the statements and the aggregate of the resident inputs (evaluated first if needed).
+ * vp_prove_fs_aggregate: on the context's own buffers, like vp_prove_fs_bound: the resident challenges are the proof's
+ *   afterwards (a later vp_verify sees them); vp_last_prove_ms / vp_last_prove_launches describe the call; VP_ERR_ASSERT
+ *   when an is_assert gate is non-zero.
+ * vp_verify_fs_aggregate: vp_verify_fs_bound's order and codes with the aggregate as the seed, from the resident inputs and
+ *   the CLAIMED outputs (n_outputs = N * layer_size(n-1) canonical elements): fail_code 7 a non-canonical transcript
+ *   element, 8 Vres != MLE(outputs)(r_out), then vp_verify's checks.
+ * VP_ERR_ARG: B = 0, B > 65535, B not dividing N, short buffers, wrong counts, non-canonical outputs, sharded contexts.
+ * On the device, on the context's stream: the B inputs roots and the B outputs roots in one pc_vector_root pass each, the B
+ * statements by one thread each (k_fs_statements), R over them, then one thread hashes the aggregate into the pool; no
+ * launch per statement and no hashing of statement data on the host. The circuit digest of template + K is kept for the
+ * last K. */
+int vp_aggregate_digest(vp_ctx* ctx, size_t B, const uint8_t* contexts, uint8_t* statements, uint8_t aggregate[32]);
+int vp_prove_fs_aggregate(vp_ctx* ctx, size_t B, const uint8_t* contexts, vp_F* transcript, size_t cap, vp_F* challenges, size_t ch_cap,
+                          uint8_t* statements, uint8_t aggregate[32]);
+int vp_verify_fs_aggregate(vp_ctx* ctx, size_t B, const uint8_t* contexts, const vp_F* outputs, size_t n_outputs, const vp_F* transcript,
+                           size_t n, int* accept, int* fail_code, int* fail_layer);
+
 /* B independent statement-bound proofs over this context's circuit (template + K, as the context was created), in one pass.
  * inputs: B * vp_circuit_num_inputs values, statement-major, read with vp_circuit_set_inputs' rules (0 <= x < p; others VP_ERR_ARG).
  * contexts: B * 32 bytes. transcripts: B * n_tr (cap >= that), statement-major; challenges (may be NULL): B * n_chal;

@@ -139,6 +139,10 @@ def _declare(L):
     L.vp_last_batch_outputs.argtypes = [vp, vp, C.c_size_t]
     L.vp_verify_fs_bound_batch.argtypes = [vp, C.c_size_t, vp, C.c_size_t, vp, vp, C.c_size_t, vp, C.c_size_t, vp, vp, vp, vp,
                                            C.c_size_t]
+    L.vp_aggregate_digest.argtypes = [vp, C.c_size_t, vp, vp, vp]
+    L.vp_prove_fs_aggregate.argtypes = [vp, C.c_size_t, vp, vp, C.c_size_t, vp, C.c_size_t, vp, vp]
+    L.vp_verify_fs_aggregate.argtypes = [vp, C.c_size_t, vp, vp, C.c_size_t, vp, C.c_size_t, C.POINTER(C.c_int), C.POINTER(C.c_int),
+                                         C.POINTER(C.c_int)]
     L.vp_get_transcript.argtypes = [vp, vp, C.c_size_t]
     L.vp_last_prove_ms.argtypes = [vp]
     L.vp_last_prove_ms.restype = C.c_float
@@ -183,6 +187,18 @@ def _context(context):
     if len(context) != 32:
         raise ValueError("a Fiat-Shamir context is 32 bytes")
     return context
+
+
+def _contexts(B, contexts):
+    """B contexts (B `bytes` of 32 or a [B, 32] uint8 array) as one contiguous [B, 32] uint8 array"""
+    if isinstance(contexts, np.ndarray):
+        if contexts.dtype != np.uint8 or contexts.shape != (B, 32):
+            raise ValueError(f"contexts must be a [{B}, 32] uint8 array, got {contexts.dtype} {contexts.shape}")
+        return np.ascontiguousarray(contexts)
+    contexts = list(contexts)
+    if len(contexts) != B:
+        raise ValueError(f"{B} statements need {B} contexts, got {len(contexts)}")
+    return np.frombuffer(b"".join(_context(c) for c in contexts), np.uint8).reshape(B, 32)
 
 
 def fe(re, im=0):
@@ -717,17 +733,7 @@ class Prover:
             raise ValueError(f"inputs must be a [B, {n_in}] array with B >= 1, got shape {inputs.shape}")
         if inputs.dtype.kind not in "ui":
             raise ValueError(f"inputs must be integers, got {inputs.dtype}")
-        B = inputs.shape[0]
-        if isinstance(contexts, np.ndarray):
-            if contexts.dtype != np.uint8 or contexts.shape != (B, 32):
-                raise ValueError(f"contexts must be a [{B}, 32] uint8 array, got {contexts.dtype} {contexts.shape}")
-            ctx = np.ascontiguousarray(contexts)
-        else:
-            contexts = list(contexts)
-            if len(contexts) != B:
-                raise ValueError(f"{B} statements need {B} contexts, got {len(contexts)}")
-            ctx = np.frombuffer(b"".join(_context(c) for c in contexts), np.uint8).reshape(B, 32)
-        return np.ascontiguousarray(inputs, dtype=np.uint64), ctx
+        return np.ascontiguousarray(inputs, dtype=np.uint64), _contexts(inputs.shape[0], contexts)
 
     def _n_outputs(self):
         return self.circuit.layer_size(self.circuit.n_layers - 1) * self.circuit.instances
@@ -777,6 +783,47 @@ class Prover:
         a, c, l = C.c_int(0), C.c_int(0), C.c_int(0)
         _ck(lib().vp_verify_fs_bound(self.h, _context(context), _ptr(out), len(out), _ptr(tr), len(tr), C.byref(a), C.byref(c),
                                      C.byref(l)))
+        return bool(a.value), c.value, l.value
+
+    def _aggregate_contexts(self, B, contexts):
+        """checked contexts [B, 32] uint8 of an aggregate call: 1 <= B <= 65535 statements dividing the instances"""
+        N = self.circuit.instances
+        if not isinstance(B, (int, np.integer)) or isinstance(B, bool) or not 1 <= B <= 65535:
+            raise ValueError(f"B must be an integer in [1, 65535], got {B!r}")
+        if N % B:
+            raise ValueError(f"{B} statements do not divide the {N} instances")
+        return _contexts(B, contexts)
+
+    def aggregate_digest(self, B, contexts):
+        """the B statements of the resident inputs (statement b: instances [b K, (b + 1) K), K = instances / B) and their
+        aggregate (include/virgo_b200.h) -> (statements [B, 32] uint8, aggregate 32 bytes)"""
+        ctx = self._aggregate_contexts(B, contexts)
+        st, agg = np.zeros((B, 32), np.uint8), np.zeros(32, np.uint8)
+        _ck(lib().vp_aggregate_digest(self.h, B, _ptr(ctx), _ptr(st), _ptr(agg)))
+        return st, agg.tobytes()
+
+    def prove_fs_aggregate(self, B, contexts):
+        """one Fiat-Shamir proof of B statements with their own contexts -> (transcript, challenges, statements [B, 32] uint8,
+        aggregate); == prove_fs(aggregate)"""
+        ctx = self._aggregate_contexts(B, contexts)
+        tr = np.zeros(self.circuit.transcript_len, F_DTYPE)
+        ch = np.zeros(self.circuit.challenge_count, F_DTYPE)
+        st, agg = np.zeros((B, 32), np.uint8), np.zeros(32, np.uint8)
+        _ck(lib().vp_prove_fs_aggregate(self.h, B, _ptr(ctx), _ptr(tr), len(tr), _ptr(ch), len(ch), _ptr(st), _ptr(agg)))
+        return tr, ch, st, agg.tobytes()
+
+    def verify_fs_aggregate(self, B, contexts, outputs, transcript):
+        """(accept, fail_code, fail_layer) of an aggregate proof for the claimed outputs [instances * S_out] (statement-major,
+        as the output layer) and this context's inputs"""
+        ctx = self._aggregate_contexts(B, contexts)
+        for name, a, n in (("outputs", outputs, self._n_outputs()), ("transcript", transcript, self.circuit.transcript_len)):
+            if not isinstance(a, np.ndarray) or a.dtype != F_DTYPE or a.shape != (n,):
+                raise ValueError(f"{name} must be a [{n}] field-element array, got "
+                                 f"{getattr(a, 'dtype', type(a))} {getattr(a, 'shape', None)}")
+        out, tr = np.ascontiguousarray(outputs), np.ascontiguousarray(transcript)
+        a, c, l = C.c_int(0), C.c_int(0), C.c_int(0)
+        _ck(lib().vp_verify_fs_aggregate(self.h, B, _ptr(ctx), _ptr(out), out.size, _ptr(tr), tr.size, C.byref(a), C.byref(c),
+                                         C.byref(l)))
         return bool(a.value), c.value, l.value
 
     def fs_round_stamps(self):

@@ -1049,6 +1049,17 @@ struct Engine {
     void fs_begin();
     void statement_async(const uint8_t context[32], const F* d_outputs, const uint64_t* d_contexts = nullptr);
     void circuit_digest_async();
+    void circuit_digest_async(uint64_t instances, uint64_t* out);
+    // Aggregate proofs (vp_prove_fs_aggregate): the circuit digest of template + K for the last K asked for (0: none yet),
+    // and the B statements' {inputs roots, outputs roots, contexts, statements}, 4 * B words each, then the statements'
+    // root and the aggregate (4 words each)
+    DBuf<uint64_t> d_digest_k;
+    uint64_t digest_k = 0;
+    DBuf<uint64_t> d_agg;
+    const uint64_t* circuit_digest_k_async(uint64_t K);
+    void aggregate_async(uint32_t B, const uint8_t* contexts, const F* d_outputs);
+    const uint64_t* agg_statements(uint32_t B) const { return d_agg.p + 12 * (size_t)B; }
+    const uint64_t* agg_digest(uint32_t B) const { return d_agg.p + 16 * (size_t)B + 4; }
     void prove_fs_device(const uint8_t* seed, F* tr_out, F* ch_out);
     void launch_phase_kernel_fs(const SumcheckPlan& P, uint32_t ci, F* keep, const F* at_init, uint32_t tr_rounds, size_t stamp_round);
     // A batch of statements (vp_prove_fs_bound_batch): the Fiat-Shamir path runs n_stmt statements at once, statement b
@@ -2820,6 +2831,21 @@ void Engine::launch_phase_kernel_fs(const SumcheckPlan& P, uint32_t ci, F* keep,
 // The circuit digest R(circuit_bytes) (include/virgo_b200.h), serialised on the host once per context and hashed on the device.
 void Engine::circuit_digest_async() {
     if (circuit_digest_ready) return;
+    circuit_digest_async(C.instances, const_cast<uint64_t*>(d_circuit_digest));
+    circuit_digest_ready = true;
+}
+// ... of template + K, kept for the last K
+const uint64_t* Engine::circuit_digest_k_async(uint64_t K) {
+    if (digest_k != K) {
+        if (!d_digest_k.p) d_digest_k.alloc(4);
+        digest_k = 0;
+        circuit_digest_async(K, d_digest_k.p);
+        digest_k = K;
+    }
+    return d_digest_k.p;
+}
+// R(circuit_bytes) with `instances` as the serialised instance count, to out (4 words, device)
+void Engine::circuit_digest_async(uint64_t instances, uint64_t* out) {
     std::vector<uint8_t> b;
     auto put = [&](const void* q, size_t len) { const uint8_t* c = static_cast<const uint8_t*>(q); b.insert(b.end(), c, c + len); };
     auto u64 = [&](uint64_t x) { put(&x, 8); };
@@ -2831,7 +2857,7 @@ void Engine::circuit_digest_async() {
     b.reserve(total + 64);
     put("VPCIRC01", 8);
     u64((uint64_t)n);
-    u64(C.instances);
+    u64(instances);
     for (int i = 0; i < n; ++i) u64(C.layers[i].size);
     for (int i = 1; i < n; ++i) {
         const Layer& T = C.layers[i];
@@ -2853,9 +2879,37 @@ void Engine::circuit_digest_async() {
     words.alloc(b.size() / 8);
     CK(cudaMemcpyAsync(words.p, b.data(), b.size(), cudaMemcpyHostToDevice, stream));
     scratch.alloc(pc_vector_root_scratch(words.n) / 8);
-    launches += (uint64_t)pc_vector_root(words.p, words.n, scratch.p, reinterpret_cast<uint8_t*>(const_cast<uint64_t*>(d_circuit_digest)), stream);
+    launches += (uint64_t)pc_vector_root(words.p, words.n, scratch.p, reinterpret_cast<uint8_t*>(out), stream);
     CK(cudaStreamSynchronize(stream));   // (the host bytes and the scratch go out of scope)
-    circuit_digest_ready = true;
+}
+
+// The B statements of an aggregate proof and the aggregate (include/virgo_b200.h), which seeds the pool. Statement b covers
+// instances [b K, (b + 1) K) of circuitValue[0] and of the outputs (d_outputs, or circuitValue[n-1]); the values are
+// instance-major, so its slices lie end to end and each kind of root is one pass of pc_vector_root over B vectors.
+// contexts: B * 32 bytes on the host.
+void Engine::aggregate_async(uint32_t B, const uint8_t* contexts, const F* d_outputs) {
+    const uint64_t K = C.instances / B;
+    const uint64_t* circuit = circuit_digest_k_async(K);
+    const size_t n_in = K * C.layers[0].size, n_out = K * C.layers[n - 1].size;
+    const size_t need = std::max({B * pc_vector_root_scratch(2 * n_in), B * pc_vector_root_scratch(2 * n_out),
+                                  pc_vector_root_scratch(4 * (size_t)B)}) / 8;
+    if (d_root_scratch.n < need) d_root_scratch.alloc(need);
+    if (d_agg.n < 16 * (size_t)B + 8) d_agg.alloc(16 * (size_t)B + 8);
+    uint64_t* const in_roots = d_agg.p;
+    uint64_t* const out_roots = in_roots + 4 * (size_t)B;
+    uint64_t* const ctxs = out_roots + 4 * (size_t)B;
+    uint64_t* const stmts = ctxs + 4 * (size_t)B;
+    uint64_t* const root = stmts + 4 * (size_t)B;
+    CK(cudaMemcpyAsync(ctxs, contexts, 32 * (size_t)B, cudaMemcpyHostToDevice, stream));
+    launches += (uint64_t)pc_vector_root(reinterpret_cast<const uint64_t*>(val[0].p), 2 * n_in, d_root_scratch.p,
+                                         reinterpret_cast<uint8_t*>(in_roots), stream, B, 32);
+    launches += (uint64_t)pc_vector_root(reinterpret_cast<const uint64_t*>(d_outputs ? d_outputs : val[n - 1].p), 2 * n_out,
+                                         d_root_scratch.p, reinterpret_cast<uint8_t*>(out_roots), stream, B, 32);
+    k_fs_statements<<<cdiv(B, 128), 128, 0, stream>>>(circuit, in_roots, out_roots, ctxs, (uint64_t)n_in, (uint64_t)n_out, B, stmts);
+    ++launches;
+    launches += (uint64_t)pc_vector_root(stmts, 4 * (size_t)B, d_root_scratch.p, reinterpret_cast<uint8_t*>(root), stream);
+    k_fs_aggregate<<<1, 32, 0, stream>>>(root, (uint64_t)B, d_fs_pool.p, root + 4);
+    ++launches;
 }
 
 // inputs root (circuitValue[0]), outputs root (d_outputs, or circuitValue[n-1]) and the statement, which seeds the pool.
@@ -4038,6 +4092,46 @@ extern "C" int vp_verify_fs_bound_batch(vp_ctx* ctx, size_t B, const uint64_t* i
     return VP_OK;
     API_END
 }
+static int fs_reject(int code, int* accept, int* fail_code, int* fail_layer) {
+    *accept = 0;
+    if (fail_code) *fail_code = code;
+    if (fail_layer) *fail_layer = 0;
+    return VP_OK;
+}
+// The verifier's circuitValue[0] from the resident inputs (it does not evaluate the circuit) and the claimed outputs in
+// d_fs_outputs (layer_size(n-1) canonical elements, checked by the caller), ahead of the seed's roots.
+static void fs_verify_load(Engine& e, const vp_F* outputs) {
+    const size_t n_out = e.C.layer_size(e.n - 1);
+    e.leave();
+    e.fs_alloc();
+    if (e.d_fs_outputs.n < n_out) e.d_fs_outputs.alloc(n_out);
+    CK(cudaMemcpyAsync(e.d_fs_outputs.p, outputs, n_out * sizeof(F), cudaMemcpyHostToDevice, e.stream));
+    const uint32_t S0 = (uint32_t)e.C.layers[0].size, b0 = e.k_lo * S0, e0 = e.k_hi * S0;
+    k_load_inputs<<<cdiv(std::max<uint32_t>(e0 - b0, 1), 256), 256, 0, e.stream>>>(e.d_inputs.p, e.val[0].p, b0, e0);
+    ++e.launches;
+}
+// A statement-bound verifier once its seed (d_seed, 4 words on the device) is queued: the challenges from the seed and the
+// transcript, the start of the claim chain (Vres == the MLE of the claimed outputs in d_fs_outputs at r_out, else fail_code
+// 8), then vp_verify's checks. The challenges stay resident.
+static int fs_verify_seeded(Engine& e, const uint64_t* d_seed, const vp_F* transcript, int* accept, int* fail_code, int* fail_layer) {
+    uint64_t h[4];
+    CK(cudaMemcpyAsync(h, d_seed, sizeof h, cudaMemcpyDeviceToHost, e.stream));
+    CK(cudaStreamSynchronize(e.stream));
+    uint8_t seed[32];
+    memcpy(seed, h, 32);
+    std::vector<F> ch(e.lay.n_chal);
+    fs_challenges(e.lay, e.fs_sched, seed, reinterpret_cast<const F*>(transcript), ch.data());
+    e.set_chal(0, reinterpret_cast<const vp_F*>(ch.data()), e.lay.n_chal);
+    e.run_eq(e.eqb_out, 2);
+    if (e.d_vf_out.n < 1) e.d_vf_out.alloc(2);
+    e.run_dot_eq(e.d_fs_outputs.p, (uint32_t)e.C.layers[e.n - 1].size, e.eqtab(2, e.C.bit_length(e.n - 1)), e.d_vf_out.p);
+    F mle;
+    CK(cudaMemcpyAsync(&mle, e.d_vf_out.p, sizeof mle, cudaMemcpyDeviceToHost, e.stream));
+    CK(cudaStreamSynchronize(e.stream));
+    if (!f_eq(mle, reinterpret_cast<const F*>(transcript)[e.lay.tr_vres])) return fs_reject(8, accept, fail_code, fail_layer);
+    *accept = e.verify(reinterpret_cast<const F*>(transcript), fail_code, fail_layer);
+    return VP_OK;
+}
 extern "C" int vp_verify_fs_bound(vp_ctx* ctx, const uint8_t context[32], const vp_F* outputs, size_t n_outputs, const vp_F* transcript,
                                   size_t n, int* accept, int* fail_code, int* fail_layer) {
     if (!ctx || !context || !outputs || !transcript || !accept) return fail(VP_ERR_ARG, "null argument");
@@ -4050,36 +4144,78 @@ extern "C" int vp_verify_fs_bound(vp_ctx* ctx, const uint8_t context[32], const 
     const size_t n_out = e.C.layer_size(e.n - 1);
     if (n_outputs != n_out) return fail(VP_ERR_ARG, "expected %zu outputs, got %zu", n_out, n_outputs);
     if (!fs_canonical(outputs, n_outputs)) return fail(VP_ERR_ARG, "an output is not canonical (components must be < p)");
-    auto reject = [&](int code) { *accept = 0; if (fail_code) *fail_code = code; if (fail_layer) *fail_layer = 0; return VP_OK; };
-    if (!fs_canonical(transcript, n)) return reject(7);
+    if (!fs_canonical(transcript, n)) return fs_reject(7, accept, fail_code, fail_layer);
+    fs_verify_load(e, outputs);
+    e.statement_async(context, e.d_fs_outputs.p);
+    return fs_verify_seeded(e, e.d_stmt.p + 12, transcript, accept, fail_code, fail_layer);
+    API_END
+}
+// ---- aggregate proofs: one Fiat-Shamir proof of B statements (unsharded contexts)
+static int aggregate_check(const Engine& e, size_t B, const char* fn) {
+    if (e.world != 1) return fail(VP_ERR_ARG, "%s: sharded contexts are not supported", fn);
+    if (B == 0 || B > 65535) return fail(VP_ERR_ARG, "%s: statement count %zu is not in [1, 65535]", fn, B);
+    if (e.C.instances % B) return fail(VP_ERR_ARG, "%s: %zu statements do not divide the %llu instances", fn, B, (unsigned long long)e.C.instances);
+    return VP_OK;
+}
+// after aggregate_async: the statements (B * 32 bytes, may be null) and the aggregate (32 bytes, may be null) to the host
+static void aggregate_read(Engine& e, uint32_t B, uint8_t* statements, uint8_t* aggregate) {
+    if (statements) CK(cudaMemcpyAsync(statements, e.agg_statements(B), 32 * (size_t)B, cudaMemcpyDeviceToHost, e.stream));
+    if (aggregate) CK(cudaMemcpyAsync(aggregate, e.agg_digest(B), 32, cudaMemcpyDeviceToHost, e.stream));
+    CK(cudaStreamSynchronize(e.stream));
+}
+extern "C" int vp_aggregate_digest(vp_ctx* ctx, size_t B, const uint8_t* contexts, uint8_t* statements, uint8_t aggregate[32]) {
+    if (!ctx || !contexts || !aggregate) return fail(VP_ERR_ARG, "null argument");
+    API_BEGIN
+    Engine& e = ctx->e;
+    ScopedTimer t(e);
+    if (const int rc = aggregate_check(e, B, "vp_aggregate_digest")) return rc;
+    if (!e.inputs_loaded) return fail(VP_ERR_ARG, "vp_aggregate_digest: inputs not loaded");
     e.leave();
     e.fs_alloc();
-    if (e.d_fs_outputs.n < n_out) e.d_fs_outputs.alloc(n_out);
-    CK(cudaMemcpyAsync(e.d_fs_outputs.p, outputs, n_out * sizeof(F), cudaMemcpyHostToDevice, e.stream));
-    {   // circuitValue[0] from the resident inputs: the verifier does not evaluate the circuit
-        const uint32_t S0 = (uint32_t)e.C.layers[0].size, b0 = e.k_lo * S0, e0 = e.k_hi * S0;
-        k_load_inputs<<<cdiv(std::max<uint32_t>(e0 - b0, 1), 256), 256, 0, e.stream>>>(e.d_inputs.p, e.val[0].p, b0, e0);
-        ++e.launches;
-    }
-    e.statement_async(context, e.d_fs_outputs.p);
-    uint64_t h[4];
-    CK(cudaMemcpyAsync(h, e.d_stmt.p + 12, sizeof h, cudaMemcpyDeviceToHost, e.stream));
-    CK(cudaStreamSynchronize(e.stream));
-    uint8_t stmt[32];
-    memcpy(stmt, h, 32);
-    std::vector<F> ch(e.lay.n_chal);
-    fs_challenges(e.lay, e.fs_sched, stmt, reinterpret_cast<const F*>(transcript), ch.data());
-    e.set_chal(0, reinterpret_cast<const vp_F*>(ch.data()), e.lay.n_chal);
-    // the claim chain starts from Vres: it must be the MLE of the claimed outputs at r_out
-    e.run_eq(e.eqb_out, 2);
-    if (e.d_vf_out.n < 1) e.d_vf_out.alloc(2);
-    e.run_dot_eq(e.d_fs_outputs.p, (uint32_t)e.C.layers[e.n - 1].size, e.eqtab(2, e.C.bit_length(e.n - 1)), e.d_vf_out.p);
-    F mle;
-    CK(cudaMemcpyAsync(&mle, e.d_vf_out.p, sizeof mle, cudaMemcpyDeviceToHost, e.stream));
-    CK(cudaStreamSynchronize(e.stream));
-    if (!f_eq(mle, reinterpret_cast<const F*>(transcript)[e.lay.tr_vres])) return reject(8);
-    *accept = e.verify(reinterpret_cast<const F*>(transcript), fail_code, fail_layer);
+    if (!e.evaluated) e.evaluate();
+    e.aggregate_async((uint32_t)B, contexts, nullptr);
+    aggregate_read(e, (uint32_t)B, statements, aggregate);
     return VP_OK;
+    API_END
+}
+extern "C" int vp_prove_fs_aggregate(vp_ctx* ctx, size_t B, const uint8_t* contexts, vp_F* transcript, size_t cap, vp_F* challenges,
+                                     size_t ch_cap, uint8_t* statements, uint8_t aggregate[32]) {
+    if (!ctx || !contexts || !transcript) return fail(VP_ERR_ARG, "null argument");
+    API_BEGIN
+    Engine& e = ctx->e;
+    ScopedTimer t(e);
+    if (const int rc = aggregate_check(e, B, "vp_prove_fs_aggregate")) return rc;
+    if (cap < e.lay.n_tr) return fail(VP_ERR_ARG, "transcript buffer too small (%zu < %zu)", cap, e.lay.n_tr);
+    if (challenges && ch_cap < e.lay.n_chal) return fail(VP_ERR_ARG, "challenge buffer too small (%zu < %zu)", ch_cap, e.lay.n_chal);
+    if (!e.inputs_loaded) return fail(VP_ERR_ARG, "vp_prove_fs_aggregate: inputs not loaded");
+    const uint64_t l0 = e.launches;
+    CK(cudaEventRecord(e.ev0, e.stream));
+    e.fs_begin();
+    e.aggregate_async((uint32_t)B, contexts, nullptr);
+    e.prove_fs_device(nullptr, reinterpret_cast<F*>(transcript), reinterpret_cast<F*>(challenges));
+    CK(cudaEventRecord(e.ev1, e.stream));
+    aggregate_read(e, (uint32_t)B, statements, aggregate);
+    CK(cudaEventElapsedTime(&e.last_ms, e.ev0, e.ev1));
+    e.last_launches = e.launches - l0;
+    return VP_OK;
+    API_END
+}
+extern "C" int vp_verify_fs_aggregate(vp_ctx* ctx, size_t B, const uint8_t* contexts, const vp_F* outputs, size_t n_outputs,
+                                      const vp_F* transcript, size_t n, int* accept, int* fail_code, int* fail_layer) {
+    if (!ctx || !contexts || !outputs || !transcript || !accept) return fail(VP_ERR_ARG, "null argument");
+    API_BEGIN
+    Engine& e = ctx->e;
+    cudaSetDevice(e.device);
+    if (const int rc = aggregate_check(e, B, "vp_verify_fs_aggregate")) return rc;
+    if (!e.inputs_loaded) return fail(VP_ERR_ARG, "vp_verify_fs_aggregate: inputs not loaded");
+    if (n != e.lay.n_tr) return fail(VP_ERR_ARG, "expected a transcript of %zu field elements, got %zu", e.lay.n_tr, n);
+    const size_t n_out = e.C.layer_size(e.n - 1);
+    if (n_outputs != n_out) return fail(VP_ERR_ARG, "expected %zu outputs, got %zu", n_out, n_outputs);
+    if (!fs_canonical(outputs, n_outputs)) return fail(VP_ERR_ARG, "an output is not canonical (components must be < p)");
+    if (!fs_canonical(transcript, n)) return fs_reject(7, accept, fail_code, fail_layer);
+    fs_verify_load(e, outputs);
+    e.aggregate_async((uint32_t)B, contexts, e.d_fs_outputs.p);
+    return fs_verify_seeded(e, e.agg_digest((uint32_t)B), transcript, accept, fail_code, fail_layer);
     API_END
 }
 extern "C" int vp_fs_round_stamps(vp_ctx* ctx, unsigned long long* out, size_t cap, size_t* n_rounds) {

@@ -75,6 +75,16 @@ __global__ void k_fs_replay(const FsStep* __restrict__ steps, uint32_t n_steps, 
 // each. The context is `ctx`, or ctxs[4b ..] for statement b when ctxs is not null. Seeds the pool with the statement and
 // copies it to `out` (4 words).
 struct FsContext { uint64_t w[4]; };
+VP_D void fs_statement_digest(const uint64_t* circuit, const uint64_t* in_root, const uint64_t* out_root, uint64_t n_inputs,
+                              uint64_t n_outputs, const uint64_t (&ctx)[4], uint64_t (&d)[4]) {
+    uint64_t m[19];
+    m[0] = 0x3130544d54535056ull;   // "VPSTMT01"
+#pragma unroll
+    for (int k = 0; k < 4; ++k) { m[1 + k] = circuit[k]; m[6 + k] = in_root[k]; m[11 + k] = out_root[k]; m[15 + k] = ctx[k]; }
+    m[5] = n_inputs;
+    m[10] = n_outputs;
+    sha3_256_words(m, 19, d);
+}
 __global__ void k_fs_statement(const uint64_t* __restrict__ circuit, const uint64_t* __restrict__ roots, uint64_t n_inputs,
                                uint64_t n_outputs, FsContext ctx, const uint64_t* __restrict__ ctxs, uint64_t* pool, uint64_t* out,
                                size_t ss) {
@@ -84,14 +94,39 @@ __global__ void k_fs_statement(const uint64_t* __restrict__ circuit, const uint6
 #pragma unroll
         for (int k = 0; k < 4; ++k) ctx.w[k] = ctxs[4 * (size_t)blockIdx.z + k];
     }
-    uint64_t m[19];
-    m[0] = 0x3130544d54535056ull;   // "VPSTMT01"
-#pragma unroll
-    for (int k = 0; k < 4; ++k) { m[1 + k] = circuit[k]; m[6 + k] = roots[4 + k]; m[11 + k] = roots[8 + k]; m[15 + k] = ctx.w[k]; }
-    m[5] = n_inputs;
-    m[10] = n_outputs;
     uint64_t d[4];
-    sha3_256_words(m, 19, d);
+    fs_statement_digest(circuit, roots + 4, roots + 8, n_inputs, n_outputs, ctx.w, d);
+#pragma unroll
+    for (int k = 0; k < 4; ++k) { pool[1 + k] = d[k]; out[k] = d[k]; }
+    pool[0] = 4;
+}
+
+// The statements of an aggregate proof (vp_prove_fs_aggregate), one thread per statement: statement b from in_roots[4b ..],
+// out_roots[4b ..] and ctxs[4b ..] (the roots of its slices, its context) to out[4b ..]. The circuit digest is that of
+// template + K, shared by all B.
+__global__ void k_fs_statements(const uint64_t* __restrict__ circuit, const uint64_t* __restrict__ in_roots,
+                                const uint64_t* __restrict__ out_roots, const uint64_t* __restrict__ ctxs, uint64_t n_inputs,
+                                uint64_t n_outputs, uint32_t B, uint64_t* out) {
+    const uint32_t b = blockIdx.x * blockDim.x + threadIdx.x;
+    if (b >= B) return;
+    uint64_t c[4], d[4];
+#pragma unroll
+    for (int k = 0; k < 4; ++k) c[k] = ctxs[4 * (size_t)b + k];
+    fs_statement_digest(circuit, in_roots + 4 * (size_t)b, out_roots + 4 * (size_t)b, n_inputs, n_outputs, c, d);
+#pragma unroll
+    for (int k = 0; k < 4; ++k) out[4 * (size_t)b + k] = d[k];
+}
+
+// The aggregate H("VPAGGR01" | u64 B | root), root = R over the B statements (48 bytes hashed). Seeds the pool with it, as
+// k_fs_statement does with a statement, and copies it to `out` (4 words).
+__global__ void k_fs_aggregate(const uint64_t* __restrict__ root, uint64_t B, uint64_t* pool, uint64_t* out) {
+    if (threadIdx.x != 0) return;
+    uint64_t m[6], d[4];
+    m[0] = 0x3130524747415056ull;   // "VPAGGR01"
+    m[1] = B;
+#pragma unroll
+    for (int k = 0; k < 4; ++k) m[2 + k] = root[k];
+    sha3_256_words(m, 6, d);
 #pragma unroll
     for (int k = 0; k < 4; ++k) { pool[1 + k] = d[k]; out[k] = d[k]; }
     pool[0] = 4;
