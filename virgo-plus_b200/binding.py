@@ -201,6 +201,13 @@ def _contexts(B, contexts):
     return np.frombuffer(b"".join(_context(c) for c in contexts), np.uint8).reshape(B, 32)
 
 
+def _verdict(call):
+    """call(accept, fail_code, fail_layer) with the three int out-parameters -> (accept, fail_code, fail_layer)"""
+    a, c, l = C.c_int(0), C.c_int(0), C.c_int(0)
+    _ck(call(C.byref(a), C.byref(c), C.byref(l)))
+    return bool(a.value), c.value, l.value
+
+
 def fe(re, im=0):
     """one field element as a 0-d structured array"""
     a = np.zeros((), dtype=F_DTYPE)
@@ -698,18 +705,19 @@ class Prover:
     def last_commit_ms(self):
         return float(lib().vp_last_commit_ms(self.h))
 
+    def _proof_arrays(self, *B):
+        """zeroed transcript and challenge arrays of one proof, or of B proofs ([B, n]) when B is given"""
+        return np.zeros(B + (self.circuit.transcript_len,), F_DTYPE), np.zeros(B + (self.circuit.challenge_count,), F_DTYPE)
+
     def prove_fs(self, seed32):
         """Fiat-Shamir mode: (transcript, challenges) with every challenge hashed from the messages before it"""
-        tr = np.zeros(self.circuit.transcript_len, F_DTYPE)
-        ch = np.zeros(self.circuit.challenge_count, F_DTYPE)
+        tr, ch = self._proof_arrays()
         _ck(lib().vp_prove_fs(self.h, bytes(seed32), _ptr(tr), len(tr), _ptr(ch), len(ch)))
         return tr, ch
 
     def verify_fs(self, seed32, transcript):
         tr = np.ascontiguousarray(transcript, dtype=F_DTYPE)
-        a, c, l = C.c_int(0), C.c_int(0), C.c_int(0)
-        _ck(lib().vp_verify_fs(self.h, bytes(seed32), _ptr(tr), len(tr), C.byref(a), C.byref(c), C.byref(l)))
-        return bool(a.value), c.value, l.value
+        return _verdict(lambda *v: lib().vp_verify_fs(self.h, bytes(seed32), _ptr(tr), len(tr), *v))
 
     def statement_digest(self, context=bytes(32)):
         """the statement of the resident inputs (include/virgo_b200.h) -> dict(circuit, inputs, outputs, statement), 32 bytes each"""
@@ -719,8 +727,7 @@ class Prover:
 
     def prove_fs_bound(self, context=bytes(32)):
         """statement-bound Fiat-Shamir proof -> (transcript, challenges, statement); == prove_fs(statement)"""
-        tr = np.zeros(self.circuit.transcript_len, F_DTYPE)
-        ch = np.zeros(self.circuit.challenge_count, F_DTYPE)
+        tr, ch = self._proof_arrays()
         st = np.zeros(32, np.uint8)
         _ck(lib().vp_prove_fs_bound(self.h, _context(context), _ptr(tr), len(tr), _ptr(ch), len(ch), _ptr(st)))
         return tr, ch, st.tobytes()
@@ -745,9 +752,7 @@ class Prover:
         set_inputs(inputs[b]). The resident inputs and values are not changed."""
         inputs, ctx = self._batch_statements(inputs, contexts)
         B = inputs.shape[0]
-        n_tr, n_ch = self.circuit.transcript_len, self.circuit.challenge_count
-        tr = np.zeros((B, n_tr), F_DTYPE)
-        ch = np.zeros((B, n_ch), F_DTYPE)
+        tr, ch = self._proof_arrays(B)
         st = np.zeros((B, 32), np.uint8)
         _ck(lib().vp_prove_fs_bound_batch(self.h, B, _ptr(inputs), inputs.size, _ptr(ctx), _ptr(tr), tr.size, _ptr(ch), ch.size,
                                           _ptr(st)))
@@ -780,10 +785,7 @@ class Prover:
         """(accept, fail_code, fail_layer) of a statement-bound proof for the claimed outputs and this context's inputs"""
         out = np.ascontiguousarray(outputs, dtype=F_DTYPE)
         tr = np.ascontiguousarray(transcript, dtype=F_DTYPE)
-        a, c, l = C.c_int(0), C.c_int(0), C.c_int(0)
-        _ck(lib().vp_verify_fs_bound(self.h, _context(context), _ptr(out), len(out), _ptr(tr), len(tr), C.byref(a), C.byref(c),
-                                     C.byref(l)))
-        return bool(a.value), c.value, l.value
+        return _verdict(lambda *v: lib().vp_verify_fs_bound(self.h, _context(context), _ptr(out), len(out), _ptr(tr), len(tr), *v))
 
     def _aggregate_contexts(self, B, contexts):
         """checked contexts [B, 32] uint8 of an aggregate call: 1 <= B <= 65535 statements dividing the instances"""
@@ -806,8 +808,7 @@ class Prover:
         """one Fiat-Shamir proof of B statements with their own contexts -> (transcript, challenges, statements [B, 32] uint8,
         aggregate); == prove_fs(aggregate)"""
         ctx = self._aggregate_contexts(B, contexts)
-        tr = np.zeros(self.circuit.transcript_len, F_DTYPE)
-        ch = np.zeros(self.circuit.challenge_count, F_DTYPE)
+        tr, ch = self._proof_arrays()
         st, agg = np.zeros((B, 32), np.uint8), np.zeros(32, np.uint8)
         _ck(lib().vp_prove_fs_aggregate(self.h, B, _ptr(ctx), _ptr(tr), len(tr), _ptr(ch), len(ch), _ptr(st), _ptr(agg)))
         return tr, ch, st, agg.tobytes()
@@ -821,10 +822,7 @@ class Prover:
                 raise ValueError(f"{name} must be a [{n}] field-element array, got "
                                  f"{getattr(a, 'dtype', type(a))} {getattr(a, 'shape', None)}")
         out, tr = np.ascontiguousarray(outputs), np.ascontiguousarray(transcript)
-        a, c, l = C.c_int(0), C.c_int(0), C.c_int(0)
-        _ck(lib().vp_verify_fs_aggregate(self.h, B, _ptr(ctx), _ptr(out), out.size, _ptr(tr), tr.size, C.byref(a), C.byref(c),
-                                         C.byref(l)))
-        return bool(a.value), c.value, l.value
+        return _verdict(lambda *v: lib().vp_verify_fs_aggregate(self.h, B, _ptr(ctx), _ptr(out), out.size, _ptr(tr), tr.size, *v))
 
     def fs_round_stamps(self):
         """block 0's %globaltimer stamps (ns) per round of the last device Fiat-Shamir proof: [rounds, 4] = round start, own
@@ -879,9 +877,7 @@ class Prover:
     def verify(self, transcript):
         """(accept, fail_code, fail_layer) of the device-side verifier on a transcript (inputs + challenges resident)"""
         tr = np.ascontiguousarray(transcript, dtype=F_DTYPE)
-        a, c, l = C.c_int(0), C.c_int(0), C.c_int(0)
-        _ck(lib().vp_verify(self.h, _ptr(tr), len(tr), C.byref(a), C.byref(c), C.byref(l)))
-        return bool(a.value), c.value, l.value
+        return _verdict(lambda *v: lib().vp_verify(self.h, _ptr(tr), len(tr), *v))
 
     def set_lanes(self, lanes):
         return int(lib().vp_set_lanes(self.h, int(lanes)))

@@ -13,6 +13,7 @@
 #include <algorithm>
 #include <atomic>
 #include <chrono>
+#include <functional>
 #include <mutex>
 #include <thread>
 #include <map>
@@ -33,14 +34,25 @@ using namespace vp;
 
 // ------------------------------------------------------------------ error plumbing
 static thread_local std::string g_err;
-static int fail(int code, const char* fmt, ...) {
+static std::string vformat(const char* fmt, va_list ap) {
     char buf[512];
+    vsnprintf(buf, sizeof buf, fmt, ap);
+    return buf;
+}
+static int fail(int code, const char* fmt, ...) {
     va_list ap;
     va_start(ap, fmt);
-    vsnprintf(buf, sizeof buf, fmt, ap);
+    g_err = vformat(fmt, ap);
     va_end(ap);
-    g_err = buf;
     return code;
+}
+// an argument check inside API_BEGIN / API_END: VP_ERR_ARG with this message
+[[noreturn]] static void bad_arg(const char* fmt, ...) {
+    va_list ap;
+    va_start(ap, fmt);
+    std::string msg = vformat(fmt, ap);
+    va_end(ap);
+    throw std::invalid_argument(msg);
 }
 struct CudaError {
     std::string msg;
@@ -1039,6 +1051,10 @@ struct Engine {
     DBuf<unsigned long long> d_fs_stamps;
     size_t fs_rounds = 0;                  // rounds of the last device FS proof (4 stamps each)
     DBuf<uint64_t> d_stmt;                 // {circuit, inputs, outputs, statement} digests, 4 words each
+    uint64_t* stmt_circuit() const { return d_stmt.p; }
+    uint64_t* stmt_inputs() const { return d_stmt.p + 4; }
+    uint64_t* stmt_outputs() const { return d_stmt.p + 8; }
+    uint64_t* stmt_statement() const { return d_stmt.p + 12; }
     DBuf<uint64_t> d_root_scratch;
     DBuf<F> d_fs_outputs;                  // vp_verify_fs_bound(_batch): the claimed outputs, statements end to end
     DBuf<FsStep> d_fs_steps;               // vp_verify_fs_bound_batch: the store / draw order of a transcript (k_fs_replay)
@@ -1060,7 +1076,8 @@ struct Engine {
     void aggregate_async(uint32_t B, const uint8_t* contexts, const F* d_outputs);
     const uint64_t* agg_statements(uint32_t B) const { return d_agg.p + 12 * (size_t)B; }
     const uint64_t* agg_digest(uint32_t B) const { return d_agg.p + 16 * (size_t)B + 4; }
-    void prove_fs_device(const uint8_t* seed, F* tr_out, F* ch_out);
+    void seed_pool(const uint8_t seed[32]);
+    void prove_fs_device(F* tr_out, F* ch_out);
     void launch_phase_kernel_fs(const SumcheckPlan& P, uint32_t ci, F* keep, const F* at_init, uint32_t tr_rounds, size_t stamp_round);
     // A batch of statements (vp_prove_fs_bound_batch): the Fiat-Shamir path runs n_stmt statements at once, statement b
     // in blockIdx.z == b with its working set sstride bytes after statement b - 1's (kernels.cuh, stmt_at). A single proof
@@ -1084,8 +1101,6 @@ struct Engine {
         uint32_t cap = 0;                  // statements it holds
         size_t stride = 0;
         DBuf<uint8_t> mem;
-        size_t o_buf[6] = {0}, o_chal = 0, o_tr = 0, o_scal = 0, o_claims = 0, o_partials = 0, o_counter = 0, o_rowpart = 0, o_eq = 0,
-               o_hs = 0, o_pool = 0, o_stmt = 0;
         size_t o_vf = 0, vf_entries = 0;   // vp_verify_fs_bound_batch: the verifier's sums and partial sums (0: none yet)
         std::vector<DBuf<F>> val;
         DBuf<F*> valptr;
@@ -1098,6 +1113,13 @@ struct Engine {
     uint32_t batch_outputs = 0;   // statements of the last successful vp_prove_fs_bound_batch, whose outputs are in slab.val[n-1]
     void slab_reserve(uint32_t B, size_t vf_entries = 0);
     void slab_swap();   // exchanges the context's buffers with the slab's (an involution)
+    // f(buffer, entries) for every buffer of the Fiat-Shamir path that the slab holds per statement, in slab order
+    template <class Fn> void fs_buffers(Fn f) {
+        for (int b = 0; b < 2; ++b) { f(bufV[b], bufV[b].n); f(bufM[b], bufM[b].n); f(bufA[b], bufA[b].n); }
+        f(d_chal, d_chal.n); f(d_tr, d_tr.n); f(d_scal, d_scal.n); f(d_claims, d_claims.n); f(d_partials, d_partials.n);
+        f(d_counter, d_counter.n); f(d_rowpart, d_rowpart.n); f(d_eq, eq_set_entries); f(d_hs, d_hs.n); f(d_fs_pool, d_fs_pool.n);
+        f(d_stmt, d_stmt.n);
+    }
     void fs_absorb_draw(uint32_t tr_begin, uint32_t n_store, uint32_t ci_begin, uint32_t n_draw) {
         k_fs_absorb_draw<<<sgrid(1), 32, 0, stream>>>(d_fs_pool.p, d_tr.p, tr_begin, n_store, d_chal.p, ci_begin, n_draw, sstride);
         ++launches;
@@ -2674,30 +2696,20 @@ void Engine::fs_begin() {
         if (flags[b]) throw StatementAssert{b, flags[b]};
 }
 
-// Batch slab: per statement a copy of every buffer below, in this order, each 256-byte aligned (slab_swap's order).
+// Batch slab: per statement a copy of every buffer of fs_buffers, in its order, then the verifier's region, each 256-byte
+// aligned.
 void Engine::slab_reserve(uint32_t B, size_t vf_entries) {
     if (slab.cap >= B && slab.vf_entries >= vf_entries) return;
     vf_entries = std::max(vf_entries, slab.vf_entries);
     B = std::max(B, slab.cap);
     batch_outputs = 0;   // (the values are reallocated)
-    size_t off = 0;
+    size_t off = 0, o_eq = 0;
     auto put = [&](size_t bytes) { const size_t o = off; off += (bytes + 255) & ~(size_t)255; return o; };
-    for (int b = 0; b < 2; ++b) {
-        slab.o_buf[3 * b] = put(bufV[b].n * sizeof(F));
-        slab.o_buf[3 * b + 1] = put(bufM[b].n * sizeof(F));
-        slab.o_buf[3 * b + 2] = put(bufA[b].n * sizeof(F));
-    }
-    slab.o_chal = put(d_chal.n * sizeof(F));
-    slab.o_tr = put(d_tr.n * sizeof(F));
-    slab.o_scal = put(d_scal.n * sizeof(F));
-    slab.o_claims = put(d_claims.n * sizeof(F));
-    slab.o_partials = put(d_partials.n * sizeof(F));
-    slab.o_counter = put(d_counter.n * sizeof(unsigned int));
-    slab.o_rowpart = put(d_rowpart.n * sizeof(F));
-    slab.o_eq = put(eq_set_entries * sizeof(F));
-    slab.o_hs = put(d_hs.n * sizeof(F));
-    slab.o_pool = put(d_fs_pool.n * sizeof(uint64_t));
-    slab.o_stmt = put(d_stmt.n * sizeof(uint64_t));
+    std::vector<std::pair<size_t, size_t>> at;   // (offset, entries) of each buffer
+    fs_buffers([&](auto& d, size_t entries) {
+        at.push_back({put(entries * sizeof *d.p), entries});
+        if ((const void*)&d == (const void*)&d_eq) o_eq = at.back().first;
+    });
     slab.o_vf = put(vf_entries * sizeof(F));
     slab.vf_entries = vf_entries;
     slab.cap = 0;
@@ -2716,7 +2728,7 @@ void Engine::slab_reserve(uint32_t B, size_t vf_entries) {
     // descriptors that point into the context's values / eq tables, rebased on the slab's
     slab.p2_tabs.resize(n);
     slab.liu_eqtabs.resize(n);
-    const uintptr_t eq0 = reinterpret_cast<uintptr_t>(d_eq.p), eq1 = reinterpret_cast<uintptr_t>(slab.mem.p + slab.o_eq);
+    const uintptr_t eq0 = reinterpret_cast<uintptr_t>(d_eq.p), eq1 = reinterpret_cast<uintptr_t>(slab.mem.p + o_eq);
     for (int i = 1; i < n; ++i) {
         std::vector<P2Table> t = L[i].h_p2;
         for (P2Table& x : t)
@@ -2731,25 +2743,8 @@ void Engine::slab_reserve(uint32_t B, size_t vf_entries) {
         }
         slab.liu_eqtabs[i].upload(e, stream);
     }
-    // statement 0's views of the slab, in slab_swap's order
-    uint8_t* const m = slab.mem.p;
-    slab.views.clear();
-    for (int b = 0; b < 2; ++b) {
-        slab.views.push_back({m + slab.o_buf[3 * b], bufV[b].n});
-        slab.views.push_back({m + slab.o_buf[3 * b + 1], bufM[b].n});
-        slab.views.push_back({m + slab.o_buf[3 * b + 2], bufA[b].n});
-    }
-    slab.views.push_back({m + slab.o_chal, d_chal.n});
-    slab.views.push_back({m + slab.o_tr, d_tr.n});
-    slab.views.push_back({m + slab.o_scal, d_scal.n});
-    slab.views.push_back({m + slab.o_claims, d_claims.n});
-    slab.views.push_back({m + slab.o_partials, d_partials.n});
-    slab.views.push_back({m + slab.o_counter, d_counter.n});
-    slab.views.push_back({m + slab.o_rowpart, d_rowpart.n});
-    slab.views.push_back({m + slab.o_eq, eq_set_entries});
-    slab.views.push_back({m + slab.o_hs, d_hs.n});
-    slab.views.push_back({m + slab.o_pool, d_fs_pool.n});
-    slab.views.push_back({m + slab.o_stmt, d_stmt.n});
+    slab.views.clear();   // statement 0's
+    for (const auto& [o, entries] : at) slab.views.push_back({slab.mem.p + o, entries});
     CK(cudaStreamSynchronize(stream));   // (the host vectors go out of scope)
     slab.cap = B;
 }
@@ -2758,7 +2753,7 @@ void Engine::slab_reserve(uint32_t B, size_t vf_entries) {
 // twice, it restores the context (FsBatchScope).
 void Engine::slab_swap() {
     size_t k = 0;
-    auto sw = [&](auto& d) {
+    fs_buffers([&](auto& d, size_t) {
         using T = std::remove_reference_t<decltype(*d.p)>;
         std::pair<void*, size_t>& v = slab.views[k++];
         T* const p = d.p;
@@ -2766,10 +2761,7 @@ void Engine::slab_swap() {
         d.p = static_cast<T*>(v.first);
         d.n = v.second;
         v = {p, c};
-    };
-    for (int b = 0; b < 2; ++b) { sw(bufV[b]); sw(bufM[b]); sw(bufA[b]); }
-    sw(d_chal); sw(d_tr); sw(d_scal); sw(d_claims); sw(d_partials); sw(d_counter); sw(d_rowpart); sw(d_eq); sw(d_hs); sw(d_fs_pool);
-    sw(d_stmt);
+    });
     std::swap(val, slab.val);
     std::swap(d_valptr, slab.valptr);
     std::swap(d_inputs, slab.inputs);
@@ -2919,27 +2911,28 @@ void Engine::statement_async(const uint8_t context[32], const F* d_outputs, cons
     const size_t n_in = C.layer_size(0), n_out = C.layer_size(n - 1);
     const size_t need = n_stmt * std::max(pc_vector_root_scratch(2 * n_in), pc_vector_root_scratch(2 * n_out)) / 8;
     if (d_root_scratch.n < need) d_root_scratch.alloc(need);
-    uint8_t* roots = reinterpret_cast<uint8_t*>(d_stmt.p);
-    launches += (uint64_t)pc_vector_root(reinterpret_cast<const uint64_t*>(val[0].p), 2 * n_in, d_root_scratch.p, roots + 32, stream,
-                                         n_stmt, sstride);
+    launches += (uint64_t)pc_vector_root(reinterpret_cast<const uint64_t*>(val[0].p), 2 * n_in, d_root_scratch.p,
+                                         reinterpret_cast<uint8_t*>(stmt_inputs()), stream, n_stmt, sstride);
     launches += (uint64_t)pc_vector_root(reinterpret_cast<const uint64_t*>(d_outputs ? d_outputs : val[n - 1].p), 2 * n_out, d_root_scratch.p,
-                                         roots + 64, stream, n_stmt, sstride);
+                                         reinterpret_cast<uint8_t*>(stmt_outputs()), stream, n_stmt, sstride);
     FsContext cx;
     memset(cx.w, 0, 32);
     if (context) memcpy(cx.w, context, 32);
     k_fs_statement<<<sgrid(1), 32, 0, stream>>>(d_circuit_digest, d_stmt.p, (uint64_t)n_in, (uint64_t)n_out, cx, d_contexts, d_fs_pool.p,
-                                                d_stmt.p + 12, sstride);
+                                                stmt_statement(), sstride);
     ++launches;
 }
 
-// The proof in the order of fs_schedule. seed != null: the pool starts with it; null: statement_async seeded it. The
+// the pool starts with a 32-byte seed from the host
+void Engine::seed_pool(const uint8_t seed[32]) {
+    uint64_t h[5] = {4, 0, 0, 0, 0};
+    memcpy(h + 1, seed, 32);
+    CK(cudaMemcpyAsync(d_fs_pool.p, h, sizeof h, cudaMemcpyHostToDevice, stream));
+}
+
+// The proof in the order of fs_schedule, on a pool seeded by seed_pool, statement_async or aggregate_async. The
 // transcript and the challenges come back in one copy each.
-void Engine::prove_fs_device(const uint8_t* seed, F* tr_out, F* ch_out) {
-    if (seed) {
-        uint64_t h[5] = {4, 0, 0, 0, 0};
-        memcpy(h + 1, seed, 32);
-        CK(cudaMemcpyAsync(d_fs_pool.p, h, sizeof h, cudaMemcpyHostToDevice, stream));
-    }
+void Engine::prove_fs_device(F* tr_out, F* ch_out) {
     size_t sr = 0;   // stamp slot of the next phase's first round
     for (const FsEntry& e : fs_sched) {
         if (!e.phase) {
@@ -2989,6 +2982,7 @@ extern "C" const char* vp_version(void) { return "virgo-plus_b200 0.1 (sm_100a)"
     catch (const CudaError& e) { return fail(VP_ERR_CUDA, "%s", e.msg.c_str()); } \
     catch (const std::bad_alloc&) { return fail(VP_ERR_NOMEM, "out of host memory"); } \
     catch (unsigned int flag) { return fail(VP_ERR_ASSERT, "assert gate violated in layer %u", flag - 1); } \
+    catch (const StatementAssert& a) { return fail(VP_ERR_ASSERT, "statement %u: assert gate violated in layer %u", a.stmt, a.flag - 1); } \
     catch (const std::invalid_argument& e) { return fail(VP_ERR_ARG, "%s", e.what()); } \
     catch (const std::length_error& e) { return fail(VP_ERR_CIRCUIT, "%s", e.what()); } \
     catch (const std::runtime_error& e) { return fail(VP_ERR_CUDA, "%s", e.what()); } \
@@ -3325,6 +3319,19 @@ struct ScopedTimer {
     explicit ScopedTimer(Engine& en) : e(en), t0(std::chrono::steady_clock::now()) { cudaSetDevice(e.device); }
     ~ScopedTimer() { e.prove_seconds += std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count(); }
 };
+// The device window of vp_last_prove_ms and vp_last_prove_launches around body(); read_back() queues the results to the
+// host after it, and one synchronisation ends the call.
+template <class Body, class ReadBack>
+static void device_window(Engine& e, Body body, ReadBack read_back) {
+    const uint64_t l0 = e.launches;
+    CK(cudaEventRecord(e.ev0, e.stream));
+    body();
+    CK(cudaEventRecord(e.ev1, e.stream));
+    read_back();
+    CK(cudaStreamSynchronize(e.stream));
+    CK(cudaEventElapsedTime(&e.last_ms, e.ev0, e.ev1));
+    e.last_launches = e.launches - l0;
+}
 
 extern "C" int vp_set_inputs(vp_ctx* ctx, const uint64_t* inputs, size_t n) {
     if (!ctx || !inputs) return fail(VP_ERR_ARG, "null argument");
@@ -3595,18 +3602,14 @@ static int prove_impl(vp_ctx* ctx, int host_io, bool local_inputs, const uint64_
         if (n_challenges != e.lay.n_chal) return fail(VP_ERR_ARG, "expected %zu challenges, got %zu", e.lay.n_chal, n_challenges);
         if (transcript_cap < e.lay.n_tr) return fail(VP_ERR_ARG, "transcript buffer too small (%zu < %zu)", transcript_cap, e.lay.n_tr);
     }
-    const uint64_t l0 = e.launches;
-    CK(cudaEventRecord(e.ev0, e.stream));
-    if (host_io) {
-        e.set_chal(0, challenges, n_challenges);
-        e.load_inputs_chunked(inputs, n_inputs, local_inputs);   // copies overlap evaluate chunk by chunk
-    }
-    e.prove_all();
-    if (host_io) CK(cudaMemcpyAsync(transcript, e.d_tr.p, e.lay.n_tr * sizeof(F), cudaMemcpyDeviceToHost, e.stream));
-    CK(cudaEventRecord(e.ev1, e.stream));
-    e.check_assert_flag();  // synchronises the stream
-    CK(cudaEventElapsedTime(&e.last_ms, e.ev0, e.ev1));
-    e.last_launches = e.launches - l0;
+    device_window(e, [&] {
+        if (host_io) {
+            e.set_chal(0, challenges, n_challenges);
+            e.load_inputs_chunked(inputs, n_inputs, local_inputs);   // copies overlap evaluate chunk by chunk
+        }
+        e.prove_all();
+        if (host_io) CK(cudaMemcpyAsync(transcript, e.d_tr.p, e.lay.n_tr * sizeof(F), cudaMemcpyDeviceToHost, e.stream));
+    }, [&] { e.check_assert_flag(); });
     e.proof_size = e.lay.proof_size;
     return VP_OK;
     API_END
@@ -3826,25 +3829,68 @@ extern "C" int vp_pc_fri(int device, const vp_F* array, size_t n, const vp_F* pu
     API_END
 }
 // ------------------------------------------------------------------ C ABI: Fiat-Shamir mode (N4)
+// Argument checks shared by the entry points below (VP_ERR_ARG through bad_arg).
+static void check_unsharded(const Engine& e, const char* fn) {
+    if (e.world != 1) bad_arg("%s: sharded contexts are not supported", fn);
+}
+static void check_inputs_loaded(const Engine& e, const char* fn) {
+    if (!e.inputs_loaded) bad_arg("%s: inputs not loaded", fn);
+}
+// room for B transcripts and, when asked for, B challenge vectors
+static void check_capacity(const Engine& e, size_t B, size_t tr_cap, const vp_F* challenges, size_t ch_cap) {
+    if (tr_cap < B * e.lay.n_tr) bad_arg("transcript buffer too small (%zu < %zu)", tr_cap, B * e.lay.n_tr);
+    if (challenges && ch_cap < B * e.lay.n_chal) bad_arg("challenge buffer too small (%zu < %zu)", ch_cap, B * e.lay.n_chal);
+}
+static void check_count(size_t B, const char* fn) {
+    if (B == 0 || B > 65535) bad_arg("%s: statement count %zu is not in [1, 65535]", fn, B);
+}
+// the index of the first non-canonical element of x[0, n), or n
+static size_t first_noncanonical(const vp_F* x, size_t n) {
+    size_t i = 0;
+    while (i < n && x[i].re < P && x[i].im < P) ++i;
+    return i;
+}
+// B statements' inputs (outputs), `per` each, end to end: their count, and every value canonical
+static void check_inputs(const uint64_t* x, size_t n, size_t B, size_t per) {
+    if (n != B * per) bad_arg("expected %zu inputs (%zu statements of %zu), got %zu", B * per, B, per, n);
+    for (size_t i = 0; i < n; ++i)
+        if (x[i] >= P) bad_arg("input %zu of statement %zu is not < p", i % per, i / per);
+}
+static void check_outputs(const vp_F* x, size_t n, size_t B, size_t per) {
+    if (n != B * per) bad_arg("expected %zu outputs (%zu statements of %zu), got %zu", B * per, B, per, n);
+    const size_t i = first_noncanonical(x, n);
+    if (i < n) bad_arg("output %zu of statement %zu is not canonical (components must be < p)", i % per, i / per);
+}
+static void aggregate_check(const Engine& e, size_t B, const char* fn) {
+    check_unsharded(e, fn);
+    check_count(B, fn);
+    if (e.C.instances % B) bad_arg("%s: %zu statements do not divide the %llu instances", fn, B, (unsigned long long)e.C.instances);
+}
+
+// The device Fiat-Shamir prover of vp_prove_fs (unsharded), vp_prove_fs_bound, vp_prove_fs_bound_batch and
+// vp_prove_fs_aggregate, in the window of vp_last_prove_ms: a batch's inputs (null: the resident ones), fs_begin, seed()
+// (queues the pool's seed), the proof; read_back() queues the digests to the host after the window.
+template <class Seed, class ReadBack>
+static void prove_fs_window(Engine& e, const uint64_t* inputs, size_t n_inputs, Seed seed, vp_F* transcript, vp_F* challenges,
+                            ReadBack read_back) {
+    device_window(e, [&] {
+        if (inputs) CK(cudaMemcpyAsync(e.d_inputs.p, inputs, n_inputs * sizeof(uint64_t), cudaMemcpyHostToDevice, e.stream));
+        e.fs_begin();
+        seed();
+        e.prove_fs_device(reinterpret_cast<F*>(transcript), reinterpret_cast<F*>(challenges));
+    }, read_back);
+}
 extern "C" int vp_prove_fs(vp_ctx* ctx, const uint8_t seed[32], vp_F* transcript, size_t transcript_cap, vp_F* challenges, size_t challenges_cap) {
     if (!ctx || !seed || !transcript) return fail(VP_ERR_ARG, "null argument");
     API_BEGIN
     Engine& e = ctx->e;
     ScopedTimer t(e);
-    if (transcript_cap < e.lay.n_tr) return fail(VP_ERR_ARG, "transcript buffer too small (%zu < %zu)", transcript_cap, e.lay.n_tr);
-    if (challenges && challenges_cap < e.lay.n_chal) return fail(VP_ERR_ARG, "challenge buffer too small (%zu < %zu)", challenges_cap, e.lay.n_chal);
-    if (!e.inputs_loaded) return fail(VP_ERR_ARG, "vp_prove_fs: inputs not loaded");
-    const uint64_t l0 = e.launches;
-    CK(cudaEventRecord(e.ev0, e.stream));
-    if (e.world == 1) {   // the whole proof queued on the device; sharded contexts keep the host loop
-        e.fs_begin();
-        e.prove_fs_device(seed, reinterpret_cast<F*>(transcript), reinterpret_cast<F*>(challenges));
-    } else
-        e.prove_fs(seed, reinterpret_cast<F*>(transcript), reinterpret_cast<F*>(challenges));
-    CK(cudaEventRecord(e.ev1, e.stream));
-    CK(cudaStreamSynchronize(e.stream));
-    CK(cudaEventElapsedTime(&e.last_ms, e.ev0, e.ev1));
-    e.last_launches = e.launches - l0;
+    check_capacity(e, 1, transcript_cap, challenges, challenges_cap);
+    check_inputs_loaded(e, "vp_prove_fs");
+    if (e.world == 1)   // the whole proof queued on the device; sharded contexts keep the host loop
+        prove_fs_window(e, nullptr, 0, [&] { e.seed_pool(seed); }, transcript, challenges, [] {});
+    else
+        device_window(e, [&] { e.prove_fs(seed, reinterpret_cast<F*>(transcript), reinterpret_cast<F*>(challenges)); }, [] {});
     return VP_OK;
     API_END
 }
@@ -3854,53 +3900,92 @@ extern "C" int vp_fs_challenges(const vp_circuit* c, const uint8_t seed[32], con
     const ProofLayout lay = proof_layout(c->c);
     if (n != lay.n_tr) return fail(VP_ERR_ARG, "expected a transcript of %zu field elements, got %zu", lay.n_tr, n);
     if (cap < lay.n_chal) return fail(VP_ERR_ARG, "challenge buffer too small (%zu < %zu)", cap, lay.n_chal);
-    for (size_t i = 0; i < n; ++i)
-        if (transcript[i].re >= P || transcript[i].im >= P) return fail(VP_ERR_ARG, "transcript element %zu is not canonical", i);
+    const size_t i = first_noncanonical(transcript, n);
+    if (i < n) return fail(VP_ERR_ARG, "transcript element %zu is not canonical", i);
     fs_challenges(lay, fs_schedule(lay), seed, reinterpret_cast<const F*>(transcript), reinterpret_cast<F*>(challenges));
     return VP_OK;
     API_END
+}
+static int fs_reject(int code, int* accept, int* fail_code, int* fail_layer) {
+    *accept = 0;
+    if (fail_code) *fail_code = code;
+    if (fail_layer) *fail_layer = 0;
+    return VP_OK;
+}
+// The single-transcript Fiat-Shamir verifier of vp_verify_fs, vp_verify_fs_bound and vp_verify_fs_aggregate: code 7 for a
+// non-canonical transcript element; the seed, from the host or, with claimed outputs, read back from where queue_seed()
+// queued it on the device; the challenges replayed on the host; with claimed outputs, code 8 unless Vres is their MLE at
+// r_out; then vp_verify's checks. The challenges stay resident.
+static int fs_verify(Engine& e, const uint8_t* seed, const vp_F* outputs, const std::function<const uint64_t*()>& queue_seed,
+                     const vp_F* transcript, size_t n, int* accept, int* fail_code, int* fail_layer) {
+    if (n != e.lay.n_tr) bad_arg("expected a transcript of %zu field elements, got %zu", e.lay.n_tr, n);
+    if (first_noncanonical(transcript, n) < n) return fs_reject(7, accept, fail_code, fail_layer);
+    uint64_t h[4];
+    if (outputs) {
+        // the verifier's circuitValue[0] from the resident inputs (it does not evaluate the circuit) and the claimed
+        // outputs (the output layer) in d_fs_outputs, ahead of the seed's roots
+        const size_t n_out = e.C.layer_size(e.n - 1);
+        e.leave();
+        e.fs_alloc();
+        if (e.d_fs_outputs.n < n_out) e.d_fs_outputs.alloc(n_out);
+        CK(cudaMemcpyAsync(e.d_fs_outputs.p, outputs, n_out * sizeof(F), cudaMemcpyHostToDevice, e.stream));
+        const uint32_t S0 = (uint32_t)e.C.layers[0].size, b0 = e.k_lo * S0, e0 = e.k_hi * S0;
+        k_load_inputs<<<cdiv(std::max<uint32_t>(e0 - b0, 1), 256), 256, 0, e.stream>>>(e.d_inputs.p, e.val[0].p, b0, e0);
+        ++e.launches;
+        CK(cudaMemcpyAsync(h, queue_seed(), sizeof h, cudaMemcpyDeviceToHost, e.stream));
+        CK(cudaStreamSynchronize(e.stream));
+        seed = reinterpret_cast<const uint8_t*>(h);
+    }
+    std::vector<F> ch(e.lay.n_chal);
+    fs_challenges(e.lay, e.fs_sched, seed, reinterpret_cast<const F*>(transcript), ch.data());
+    e.set_chal(0, reinterpret_cast<const vp_F*>(ch.data()), e.lay.n_chal);
+    if (outputs) {
+        e.run_eq(e.eqb_out, 2);
+        if (e.d_vf_out.n < 1) e.d_vf_out.alloc(2);
+        e.run_dot_eq(e.d_fs_outputs.p, (uint32_t)e.C.layers[e.n - 1].size, e.eqtab(2, e.C.bit_length(e.n - 1)), e.d_vf_out.p);
+        F mle;
+        CK(cudaMemcpyAsync(&mle, e.d_vf_out.p, sizeof mle, cudaMemcpyDeviceToHost, e.stream));
+        CK(cudaStreamSynchronize(e.stream));
+        if (!f_eq(mle, reinterpret_cast<const F*>(transcript)[e.lay.tr_vres])) return fs_reject(8, accept, fail_code, fail_layer);
+    }
+    *accept = e.verify(reinterpret_cast<const F*>(transcript), fail_code, fail_layer);
+    return VP_OK;
 }
 extern "C" int vp_verify_fs(vp_ctx* ctx, const uint8_t seed[32], const vp_F* transcript, size_t n, int* accept, int* fail_code, int* fail_layer) {
     if (!ctx || !seed || !transcript || !accept) return fail(VP_ERR_ARG, "null argument");
     API_BEGIN
     Engine& e = ctx->e;
     cudaSetDevice(e.device);
-    if (n != e.lay.n_tr) return fail(VP_ERR_ARG, "expected a transcript of %zu field elements, got %zu", e.lay.n_tr, n);
-    for (size_t i = 0; i < n; ++i)
-        if (transcript[i].re >= P || transcript[i].im >= P) { *accept = 0; if (fail_code) *fail_code = 7; if (fail_layer) *fail_layer = 0; return VP_OK; }
-    std::vector<F> ch(e.lay.n_chal);
-    fs_challenges(e.lay, e.fs_sched, seed, reinterpret_cast<const F*>(transcript), ch.data());
-    e.set_chal(0, reinterpret_cast<const vp_F*>(ch.data()), e.lay.n_chal);
-    *accept = e.verify(reinterpret_cast<const F*>(transcript), fail_code, fail_layer);
-    return VP_OK;
+    return fs_verify(e, seed, nullptr, nullptr, transcript, n, accept, fail_code, fail_layer);
     API_END
 }
 // ---- statement-bound Fiat-Shamir proofs (unsharded contexts)
-static bool fs_canonical(const vp_F* x, size_t n) {
-    for (size_t i = 0; i < n; ++i)
-        if (x[i].re >= P || x[i].im >= P) return false;
-    return true;
+// vp_statement_digest and vp_aggregate_digest: the context's values (evaluated if needed), then queue() queues the
+// digests and their copies to the host; one synchronisation.
+template <class Queue>
+static void fs_digest(Engine& e, Queue queue) {
+    e.leave();
+    e.fs_alloc();
+    if (!e.evaluated) e.evaluate();
+    queue();
+    CK(cudaStreamSynchronize(e.stream));
 }
-static void copy_digest(const uint64_t* h, uint8_t* out) { if (out) memcpy(out, h, 32); }
 extern "C" int vp_statement_digest(vp_ctx* ctx, const uint8_t context[32], uint8_t circuit[32], uint8_t inputs[32], uint8_t outputs[32],
                                    uint8_t statement[32]) {
     if (!ctx || !context || !statement) return fail(VP_ERR_ARG, "null argument");
     API_BEGIN
     Engine& e = ctx->e;
     ScopedTimer t(e);
-    if (e.world != 1) return fail(VP_ERR_ARG, "vp_statement_digest: sharded contexts are not supported");
-    if (!e.inputs_loaded) return fail(VP_ERR_ARG, "vp_statement_digest: inputs not loaded");
-    e.leave();
-    e.fs_alloc();
-    if (!e.evaluated) e.evaluate();
-    e.statement_async(context, nullptr);
-    uint64_t h[16];
-    CK(cudaMemcpyAsync(h, e.d_stmt.p, sizeof h, cudaMemcpyDeviceToHost, e.stream));
-    CK(cudaStreamSynchronize(e.stream));
-    copy_digest(h, circuit);
-    copy_digest(h + 4, inputs);
-    copy_digest(h + 8, outputs);
-    copy_digest(h + 12, statement);
+    check_unsharded(e, "vp_statement_digest");
+    check_inputs_loaded(e, "vp_statement_digest");
+    uint64_t h[4][4];   // d_stmt: circuit, inputs, outputs, statement
+    fs_digest(e, [&] {
+        e.statement_async(context, nullptr);
+        CK(cudaMemcpyAsync(h, e.stmt_circuit(), sizeof h, cudaMemcpyDeviceToHost, e.stream));
+    });
+    uint8_t* const out[4] = {circuit, inputs, outputs, statement};
+    for (int k = 0; k < 4; ++k)
+        if (out[k]) memcpy(out[k], h[k], 32);
     return VP_OK;
     API_END
 }
@@ -3910,22 +3995,11 @@ extern "C" int vp_prove_fs_bound(vp_ctx* ctx, const uint8_t context[32], vp_F* t
     API_BEGIN
     Engine& e = ctx->e;
     ScopedTimer t(e);
-    if (e.world != 1) return fail(VP_ERR_ARG, "vp_prove_fs_bound: sharded contexts are not supported");
-    if (cap < e.lay.n_tr) return fail(VP_ERR_ARG, "transcript buffer too small (%zu < %zu)", cap, e.lay.n_tr);
-    if (challenges && ch_cap < e.lay.n_chal) return fail(VP_ERR_ARG, "challenge buffer too small (%zu < %zu)", ch_cap, e.lay.n_chal);
-    if (!e.inputs_loaded) return fail(VP_ERR_ARG, "vp_prove_fs_bound: inputs not loaded");
-    const uint64_t l0 = e.launches;
-    CK(cudaEventRecord(e.ev0, e.stream));
-    e.fs_begin();
-    e.statement_async(context, nullptr);
-    e.prove_fs_device(nullptr, reinterpret_cast<F*>(transcript), reinterpret_cast<F*>(challenges));
-    CK(cudaEventRecord(e.ev1, e.stream));
-    uint64_t h[4];
-    CK(cudaMemcpyAsync(h, e.d_stmt.p + 12, sizeof h, cudaMemcpyDeviceToHost, e.stream));
-    CK(cudaStreamSynchronize(e.stream));
-    copy_digest(h, statement);
-    CK(cudaEventElapsedTime(&e.last_ms, e.ev0, e.ev1));
-    e.last_launches = e.launches - l0;
+    check_unsharded(e, "vp_prove_fs_bound");
+    check_capacity(e, 1, cap, challenges, ch_cap);
+    check_inputs_loaded(e, "vp_prove_fs_bound");
+    prove_fs_window(e, nullptr, 0, [&] { e.statement_async(context, nullptr); }, transcript, challenges,
+                    [&] { if (statement) e.copy_stmts_to_host(statement, 32, e.stmt_statement(), 32); });
     return VP_OK;
     API_END
 }
@@ -3959,35 +4033,19 @@ extern "C" int vp_prove_fs_bound_batch(vp_ctx* ctx, size_t B, const uint64_t* in
     API_BEGIN
     Engine& e = ctx->e;
     ScopedTimer t(e);
-    if (e.world != 1) return fail(VP_ERR_ARG, "vp_prove_fs_bound_batch: sharded contexts are not supported");
-    if (B == 0 || B > 65535) return fail(VP_ERR_ARG, "batch size %zu is not in [1, 65535]", B);
-    const size_t n_in = e.C.layer_size(0);
-    if (n_inputs != B * n_in) return fail(VP_ERR_ARG, "expected %zu inputs (%zu statements of %zu), got %zu", B * n_in, B, n_in, n_inputs);
-    if (cap < B * e.lay.n_tr) return fail(VP_ERR_ARG, "transcript buffer too small (%zu < %zu)", cap, B * e.lay.n_tr);
-    if (challenges && ch_cap < B * e.lay.n_chal) return fail(VP_ERR_ARG, "challenge buffer too small (%zu < %zu)", ch_cap, B * e.lay.n_chal);
-    for (size_t i = 0; i < n_inputs; ++i)
-        if (inputs[i] >= P) return fail(VP_ERR_ARG, "input %zu of statement %zu is not < p", i % n_in, i / n_in);
+    check_unsharded(e, "vp_prove_fs_bound_batch");
+    check_count(B, "vp_prove_fs_bound_batch");
+    check_capacity(e, B, cap, challenges, ch_cap);
+    check_inputs(inputs, n_inputs, B, e.C.layer_size(0));
     e.leave();
     e.fs_alloc();
     e.circuit_digest_async();
     e.batch_outputs = 0;
-    const uint64_t l0 = e.launches;
-    try {
-        FsBatchScope scope(e, (uint32_t)B);
-        CK(cudaEventRecord(e.ev0, e.stream));
-        CK(cudaMemcpyAsync(e.d_inputs.p, inputs, n_inputs * sizeof(uint64_t), cudaMemcpyHostToDevice, e.stream));
+    FsBatchScope scope(e, (uint32_t)B);
+    prove_fs_window(e, inputs, n_inputs, [&] {
         CK(cudaMemcpyAsync(e.slab.contexts.p, contexts, 32 * B, cudaMemcpyHostToDevice, e.stream));
-        e.fs_begin();
         e.statement_async(nullptr, nullptr, e.slab.contexts.p);
-        e.prove_fs_device(nullptr, reinterpret_cast<F*>(transcripts), reinterpret_cast<F*>(challenges));
-        CK(cudaEventRecord(e.ev1, e.stream));
-        if (statements) e.copy_stmts_to_host(statements, 32, e.d_stmt.p + 12, 32);
-        CK(cudaStreamSynchronize(e.stream));
-        CK(cudaEventElapsedTime(&e.last_ms, e.ev0, e.ev1));
-    } catch (const StatementAssert& a) {
-        return fail(VP_ERR_ASSERT, "statement %u: assert gate violated in layer %u", a.stmt, a.flag - 1);
-    }
-    e.last_launches = e.launches - l0;
+    }, transcripts, challenges, [&] { if (statements) e.copy_stmts_to_host(statements, 32, e.stmt_statement(), 32); });
     e.batch_outputs = (uint32_t)B;
     return VP_OK;
     API_END
@@ -4013,23 +4071,18 @@ extern "C" int vp_verify_fs_bound_batch(vp_ctx* ctx, size_t B, const uint64_t* i
     API_BEGIN
     Engine& e = ctx->e;
     ScopedTimer t(e);
-    if (e.world != 1) return fail(VP_ERR_ARG, "vp_verify_fs_bound_batch: sharded contexts are not supported");
-    if (B == 0 || B > 65535) return fail(VP_ERR_ARG, "batch size %zu is not in [1, 65535]", B);
+    check_unsharded(e, "vp_verify_fs_bound_batch");
+    check_count(B, "vp_verify_fs_bound_batch");
     const size_t n_in = e.C.layer_size(0), n_out = e.C.layer_size(e.n - 1);
-    if (n_inputs != B * n_in) return fail(VP_ERR_ARG, "expected %zu inputs (%zu statements of %zu), got %zu", B * n_in, B, n_in, n_inputs);
-    if (n_outputs != B * n_out) return fail(VP_ERR_ARG, "expected %zu outputs (%zu statements of %zu), got %zu", B * n_out, B, n_out, n_outputs);
+    check_inputs(inputs, n_inputs, B, n_in);
+    check_outputs(outputs, n_outputs, B, n_out);
     if (n_tr != B * e.lay.n_tr) return fail(VP_ERR_ARG, "expected %zu transcript elements (%zu statements of %zu), got %zu", B * e.lay.n_tr, B, e.lay.n_tr, n_tr);
-    if (challenges && ch_cap < B * e.lay.n_chal) return fail(VP_ERR_ARG, "challenge buffer too small (%zu < %zu)", ch_cap, B * e.lay.n_chal);
-    for (size_t i = 0; i < n_inputs; ++i)
-        if (inputs[i] >= P) return fail(VP_ERR_ARG, "input %zu of statement %zu is not < p", i % n_in, i / n_in);
-    for (size_t i = 0; i < n_outputs; ++i)
-        if (outputs[i].re >= P || outputs[i].im >= P)
-            return fail(VP_ERR_ARG, "output %zu of statement %zu is not canonical (components must be < p)", i % n_out, i / n_out);
+    check_capacity(e, B, n_tr, challenges, ch_cap);
     // a statement with a non-canonical transcript element is rejected (code 7) on its own; its row goes up as zeros
     const F* tr = reinterpret_cast<const F*>(transcripts);
     std::vector<uint8_t> bad(B, 0);
     std::vector<F> clean;
-    for (size_t b = 0; b < B; ++b) bad[b] = !fs_canonical(transcripts + b * e.lay.n_tr, e.lay.n_tr);
+    for (size_t b = 0; b < B; ++b) bad[b] = first_noncanonical(transcripts + b * e.lay.n_tr, e.lay.n_tr) < e.lay.n_tr;
     if (std::find(bad.begin(), bad.end(), 1) != bad.end()) {
         clean.assign(tr, tr + n_tr);
         for (size_t b = 0; b < B; ++b)
@@ -4045,36 +4098,33 @@ extern "C" int vp_verify_fs_bound_batch(vp_ctx* ctx, size_t B, const uint64_t* i
     const uint32_t out_total = e.vf_out_total;
     if (e.d_fs_outputs.n < n_outputs) e.d_fs_outputs.alloc(n_outputs);
     std::vector<F> sums((size_t)B * out_total), ch((size_t)B * e.lay.n_chal);
-    const uint64_t l0 = e.launches;
     {
         FsBatchScope scope(e, (uint32_t)B, (size_t)out_total + (size_t)e.vf_max_b * Engine::VF_GX * 2);
         F* const d_out = reinterpret_cast<F*>(e.slab.mem.p + e.slab.o_vf);
         F* const d_part = d_out + out_total;
-        CK(cudaEventRecord(e.ev0, e.stream));
-        CK(cudaMemcpyAsync(e.d_inputs.p, inputs, n_inputs * sizeof(uint64_t), cudaMemcpyHostToDevice, e.stream));
-        CK(cudaMemcpyAsync(e.d_fs_outputs.p, outputs, n_outputs * sizeof(F), cudaMemcpyHostToDevice, e.stream));
-        CK(cudaMemcpyAsync(e.slab.contexts.p, contexts, 32 * B, cudaMemcpyHostToDevice, e.stream));
-        CK(cudaMemcpy2DAsync(e.d_tr.p, e.sstride, tr, e.lay.n_tr * sizeof(F), e.lay.n_tr * sizeof(F), B, cudaMemcpyHostToDevice, e.stream));
-        e.memset_stmts(e.d_chal.p, (e.lay.n_chal + 1) * sizeof(F));   // unused challenge slots are zero
-        e.memset_stmts(d_out, (size_t)out_total * sizeof(F));
-        const uint32_t n0 = (uint32_t)(B * n_in);   // circuitValue[0] of every statement, instance-major over B * K
-        k_load_inputs<<<cdiv(n0, 256), 256, 0, e.stream>>>(e.d_inputs.p, e.val[0].p, 0, n0);
-        ++e.launches;
-        e.statement_async(nullptr, e.d_fs_outputs.p, e.slab.contexts.p);
-        k_fs_replay<<<e.sgrid(1), 32, 0, e.stream>>>(e.d_fs_steps.p, (uint32_t)e.d_fs_steps.n, e.d_fs_pool.p, e.d_tr.p, e.d_chal.p, e.sstride);
-        ++e.launches;
-        // the claim chain starts from Vres: the MLE of the claimed outputs at r_out, next to the input MLE
-        e.run_eq(e.eqb_out, 2);
-        e.run_dot_eq(e.d_fs_outputs.p, (uint32_t)e.C.layers[e.n - 1].size, e.eqtab(2, e.C.bit_length(e.n - 1)), d_out + out_total - 1);
-        e.verify_sums_async(d_out, d_part);
-        CK(cudaEventRecord(e.ev1, e.stream));
-        e.copy_stmts_to_host(sums.data(), out_total * sizeof(F), d_out, out_total * sizeof(F));
-        e.copy_stmts_to_host(ch.data(), e.lay.n_chal * sizeof(F), e.d_chal.p, e.lay.n_chal * sizeof(F));
-        CK(cudaStreamSynchronize(e.stream));
-        CK(cudaGetLastError());
-        CK(cudaEventElapsedTime(&e.last_ms, e.ev0, e.ev1));
+        device_window(e, [&] {
+            CK(cudaMemcpyAsync(e.d_inputs.p, inputs, n_inputs * sizeof(uint64_t), cudaMemcpyHostToDevice, e.stream));
+            CK(cudaMemcpyAsync(e.d_fs_outputs.p, outputs, n_outputs * sizeof(F), cudaMemcpyHostToDevice, e.stream));
+            CK(cudaMemcpyAsync(e.slab.contexts.p, contexts, 32 * B, cudaMemcpyHostToDevice, e.stream));
+            CK(cudaMemcpy2DAsync(e.d_tr.p, e.sstride, tr, e.lay.n_tr * sizeof(F), e.lay.n_tr * sizeof(F), B, cudaMemcpyHostToDevice, e.stream));
+            e.memset_stmts(e.d_chal.p, (e.lay.n_chal + 1) * sizeof(F));   // unused challenge slots are zero
+            e.memset_stmts(d_out, (size_t)out_total * sizeof(F));
+            const uint32_t n0 = (uint32_t)(B * n_in);   // circuitValue[0] of every statement, instance-major over B * K
+            k_load_inputs<<<cdiv(n0, 256), 256, 0, e.stream>>>(e.d_inputs.p, e.val[0].p, 0, n0);
+            ++e.launches;
+            e.statement_async(nullptr, e.d_fs_outputs.p, e.slab.contexts.p);
+            k_fs_replay<<<e.sgrid(1), 32, 0, e.stream>>>(e.d_fs_steps.p, (uint32_t)e.d_fs_steps.n, e.d_fs_pool.p, e.d_tr.p, e.d_chal.p, e.sstride);
+            ++e.launches;
+            // the claim chain starts from Vres: the MLE of the claimed outputs at r_out, next to the input MLE
+            e.run_eq(e.eqb_out, 2);
+            e.run_dot_eq(e.d_fs_outputs.p, (uint32_t)e.C.layers[e.n - 1].size, e.eqtab(2, e.C.bit_length(e.n - 1)), d_out + out_total - 1);
+            e.verify_sums_async(d_out, d_part);
+        }, [&] {
+            e.copy_stmts_to_host(sums.data(), out_total * sizeof(F), d_out, out_total * sizeof(F));
+            e.copy_stmts_to_host(ch.data(), e.lay.n_chal * sizeof(F), e.d_chal.p, e.lay.n_chal * sizeof(F));
+            CK(cudaGetLastError());
+        });
     }
-    e.last_launches = e.launches - l0;
     // the host driver, one statement at a time, in vp_verify_fs_bound's order: code 7, code 8, then vp_verify's checks
     for (size_t b = 0; b < B; ++b) {
         int code = 0, layer = 0, ok = 0;
@@ -4092,89 +4142,36 @@ extern "C" int vp_verify_fs_bound_batch(vp_ctx* ctx, size_t B, const uint64_t* i
     return VP_OK;
     API_END
 }
-static int fs_reject(int code, int* accept, int* fail_code, int* fail_layer) {
-    *accept = 0;
-    if (fail_code) *fail_code = code;
-    if (fail_layer) *fail_layer = 0;
-    return VP_OK;
-}
-// The verifier's circuitValue[0] from the resident inputs (it does not evaluate the circuit) and the claimed outputs in
-// d_fs_outputs (layer_size(n-1) canonical elements, checked by the caller), ahead of the seed's roots.
-static void fs_verify_load(Engine& e, const vp_F* outputs) {
-    const size_t n_out = e.C.layer_size(e.n - 1);
-    e.leave();
-    e.fs_alloc();
-    if (e.d_fs_outputs.n < n_out) e.d_fs_outputs.alloc(n_out);
-    CK(cudaMemcpyAsync(e.d_fs_outputs.p, outputs, n_out * sizeof(F), cudaMemcpyHostToDevice, e.stream));
-    const uint32_t S0 = (uint32_t)e.C.layers[0].size, b0 = e.k_lo * S0, e0 = e.k_hi * S0;
-    k_load_inputs<<<cdiv(std::max<uint32_t>(e0 - b0, 1), 256), 256, 0, e.stream>>>(e.d_inputs.p, e.val[0].p, b0, e0);
-    ++e.launches;
-}
-// A statement-bound verifier once its seed (d_seed, 4 words on the device) is queued: the challenges from the seed and the
-// transcript, the start of the claim chain (Vres == the MLE of the claimed outputs in d_fs_outputs at r_out, else fail_code
-// 8), then vp_verify's checks. The challenges stay resident.
-static int fs_verify_seeded(Engine& e, const uint64_t* d_seed, const vp_F* transcript, int* accept, int* fail_code, int* fail_layer) {
-    uint64_t h[4];
-    CK(cudaMemcpyAsync(h, d_seed, sizeof h, cudaMemcpyDeviceToHost, e.stream));
-    CK(cudaStreamSynchronize(e.stream));
-    uint8_t seed[32];
-    memcpy(seed, h, 32);
-    std::vector<F> ch(e.lay.n_chal);
-    fs_challenges(e.lay, e.fs_sched, seed, reinterpret_cast<const F*>(transcript), ch.data());
-    e.set_chal(0, reinterpret_cast<const vp_F*>(ch.data()), e.lay.n_chal);
-    e.run_eq(e.eqb_out, 2);
-    if (e.d_vf_out.n < 1) e.d_vf_out.alloc(2);
-    e.run_dot_eq(e.d_fs_outputs.p, (uint32_t)e.C.layers[e.n - 1].size, e.eqtab(2, e.C.bit_length(e.n - 1)), e.d_vf_out.p);
-    F mle;
-    CK(cudaMemcpyAsync(&mle, e.d_vf_out.p, sizeof mle, cudaMemcpyDeviceToHost, e.stream));
-    CK(cudaStreamSynchronize(e.stream));
-    if (!f_eq(mle, reinterpret_cast<const F*>(transcript)[e.lay.tr_vres])) return fs_reject(8, accept, fail_code, fail_layer);
-    *accept = e.verify(reinterpret_cast<const F*>(transcript), fail_code, fail_layer);
-    return VP_OK;
-}
 extern "C" int vp_verify_fs_bound(vp_ctx* ctx, const uint8_t context[32], const vp_F* outputs, size_t n_outputs, const vp_F* transcript,
                                   size_t n, int* accept, int* fail_code, int* fail_layer) {
     if (!ctx || !context || !outputs || !transcript || !accept) return fail(VP_ERR_ARG, "null argument");
     API_BEGIN
     Engine& e = ctx->e;
     cudaSetDevice(e.device);
-    if (e.world != 1) return fail(VP_ERR_ARG, "vp_verify_fs_bound: sharded contexts are not supported");
-    if (!e.inputs_loaded) return fail(VP_ERR_ARG, "vp_verify_fs_bound: inputs not loaded");
-    if (n != e.lay.n_tr) return fail(VP_ERR_ARG, "expected a transcript of %zu field elements, got %zu", e.lay.n_tr, n);
-    const size_t n_out = e.C.layer_size(e.n - 1);
-    if (n_outputs != n_out) return fail(VP_ERR_ARG, "expected %zu outputs, got %zu", n_out, n_outputs);
-    if (!fs_canonical(outputs, n_outputs)) return fail(VP_ERR_ARG, "an output is not canonical (components must be < p)");
-    if (!fs_canonical(transcript, n)) return fs_reject(7, accept, fail_code, fail_layer);
-    fs_verify_load(e, outputs);
-    e.statement_async(context, e.d_fs_outputs.p);
-    return fs_verify_seeded(e, e.d_stmt.p + 12, transcript, accept, fail_code, fail_layer);
+    check_unsharded(e, "vp_verify_fs_bound");
+    check_inputs_loaded(e, "vp_verify_fs_bound");
+    check_outputs(outputs, n_outputs, 1, e.C.layer_size(e.n - 1));
+    return fs_verify(e, nullptr, outputs, [&] { e.statement_async(context, e.d_fs_outputs.p); return e.stmt_statement(); }, transcript, n,
+                     accept, fail_code, fail_layer);
     API_END
 }
 // ---- aggregate proofs: one Fiat-Shamir proof of B statements (unsharded contexts)
-static int aggregate_check(const Engine& e, size_t B, const char* fn) {
-    if (e.world != 1) return fail(VP_ERR_ARG, "%s: sharded contexts are not supported", fn);
-    if (B == 0 || B > 65535) return fail(VP_ERR_ARG, "%s: statement count %zu is not in [1, 65535]", fn, B);
-    if (e.C.instances % B) return fail(VP_ERR_ARG, "%s: %zu statements do not divide the %llu instances", fn, B, (unsigned long long)e.C.instances);
-    return VP_OK;
-}
 // after aggregate_async: the statements (B * 32 bytes, may be null) and the aggregate (32 bytes, may be null) to the host
 static void aggregate_read(Engine& e, uint32_t B, uint8_t* statements, uint8_t* aggregate) {
     if (statements) CK(cudaMemcpyAsync(statements, e.agg_statements(B), 32 * (size_t)B, cudaMemcpyDeviceToHost, e.stream));
     if (aggregate) CK(cudaMemcpyAsync(aggregate, e.agg_digest(B), 32, cudaMemcpyDeviceToHost, e.stream));
-    CK(cudaStreamSynchronize(e.stream));
 }
 extern "C" int vp_aggregate_digest(vp_ctx* ctx, size_t B, const uint8_t* contexts, uint8_t* statements, uint8_t aggregate[32]) {
     if (!ctx || !contexts || !aggregate) return fail(VP_ERR_ARG, "null argument");
     API_BEGIN
     Engine& e = ctx->e;
     ScopedTimer t(e);
-    if (const int rc = aggregate_check(e, B, "vp_aggregate_digest")) return rc;
-    if (!e.inputs_loaded) return fail(VP_ERR_ARG, "vp_aggregate_digest: inputs not loaded");
-    e.leave();
-    e.fs_alloc();
-    if (!e.evaluated) e.evaluate();
-    e.aggregate_async((uint32_t)B, contexts, nullptr);
-    aggregate_read(e, (uint32_t)B, statements, aggregate);
+    aggregate_check(e, B, "vp_aggregate_digest");
+    check_inputs_loaded(e, "vp_aggregate_digest");
+    fs_digest(e, [&] {
+        e.aggregate_async((uint32_t)B, contexts, nullptr);
+        aggregate_read(e, (uint32_t)B, statements, aggregate);
+    });
     return VP_OK;
     API_END
 }
@@ -4184,19 +4181,11 @@ extern "C" int vp_prove_fs_aggregate(vp_ctx* ctx, size_t B, const uint8_t* conte
     API_BEGIN
     Engine& e = ctx->e;
     ScopedTimer t(e);
-    if (const int rc = aggregate_check(e, B, "vp_prove_fs_aggregate")) return rc;
-    if (cap < e.lay.n_tr) return fail(VP_ERR_ARG, "transcript buffer too small (%zu < %zu)", cap, e.lay.n_tr);
-    if (challenges && ch_cap < e.lay.n_chal) return fail(VP_ERR_ARG, "challenge buffer too small (%zu < %zu)", ch_cap, e.lay.n_chal);
-    if (!e.inputs_loaded) return fail(VP_ERR_ARG, "vp_prove_fs_aggregate: inputs not loaded");
-    const uint64_t l0 = e.launches;
-    CK(cudaEventRecord(e.ev0, e.stream));
-    e.fs_begin();
-    e.aggregate_async((uint32_t)B, contexts, nullptr);
-    e.prove_fs_device(nullptr, reinterpret_cast<F*>(transcript), reinterpret_cast<F*>(challenges));
-    CK(cudaEventRecord(e.ev1, e.stream));
-    aggregate_read(e, (uint32_t)B, statements, aggregate);
-    CK(cudaEventElapsedTime(&e.last_ms, e.ev0, e.ev1));
-    e.last_launches = e.launches - l0;
+    aggregate_check(e, B, "vp_prove_fs_aggregate");
+    check_capacity(e, 1, cap, challenges, ch_cap);
+    check_inputs_loaded(e, "vp_prove_fs_aggregate");
+    prove_fs_window(e, nullptr, 0, [&] { e.aggregate_async((uint32_t)B, contexts, nullptr); }, transcript, challenges,
+                    [&] { aggregate_read(e, (uint32_t)B, statements, aggregate); });
     return VP_OK;
     API_END
 }
@@ -4206,16 +4195,11 @@ extern "C" int vp_verify_fs_aggregate(vp_ctx* ctx, size_t B, const uint8_t* cont
     API_BEGIN
     Engine& e = ctx->e;
     cudaSetDevice(e.device);
-    if (const int rc = aggregate_check(e, B, "vp_verify_fs_aggregate")) return rc;
-    if (!e.inputs_loaded) return fail(VP_ERR_ARG, "vp_verify_fs_aggregate: inputs not loaded");
-    if (n != e.lay.n_tr) return fail(VP_ERR_ARG, "expected a transcript of %zu field elements, got %zu", e.lay.n_tr, n);
-    const size_t n_out = e.C.layer_size(e.n - 1);
-    if (n_outputs != n_out) return fail(VP_ERR_ARG, "expected %zu outputs, got %zu", n_out, n_outputs);
-    if (!fs_canonical(outputs, n_outputs)) return fail(VP_ERR_ARG, "an output is not canonical (components must be < p)");
-    if (!fs_canonical(transcript, n)) return fs_reject(7, accept, fail_code, fail_layer);
-    fs_verify_load(e, outputs);
-    e.aggregate_async((uint32_t)B, contexts, e.d_fs_outputs.p);
-    return fs_verify_seeded(e, e.agg_digest((uint32_t)B), transcript, accept, fail_code, fail_layer);
+    aggregate_check(e, B, "vp_verify_fs_aggregate");
+    check_inputs_loaded(e, "vp_verify_fs_aggregate");
+    check_outputs(outputs, n_outputs, B, e.C.layer_size(e.n - 1) / B);
+    return fs_verify(e, nullptr, outputs, [&] { e.aggregate_async((uint32_t)B, contexts, e.d_fs_outputs.p); return e.agg_digest((uint32_t)B); },
+                     transcript, n, accept, fail_code, fail_layer);
     API_END
 }
 extern "C" int vp_fs_round_stamps(vp_ctx* ctx, unsigned long long* out, size_t cap, size_t* n_rounds) {
