@@ -388,6 +388,37 @@ int vp_last_batch_outputs(vp_ctx* ctx, vp_F* out, size_t cap);
 int vp_verify_fs_bound_batch(vp_ctx* ctx, size_t B, const uint64_t* inputs, size_t n_inputs, const uint8_t* contexts,
                              const vp_F* outputs, size_t n_outputs, const vp_F* transcripts, size_t n_tr,
                              int* accept, int* fail_code, int* fail_layer, vp_F* challenges, size_t ch_cap);
+/* The two batch calls above on arrays in DEVICE memory, as one stage of a GPU pipeline: every array is device (or managed)
+ * memory of the context's device, statement-major in the layout of its host counterpart: inputs B * num_inputs (u64),
+ * contexts B * 32 bytes, transcripts B * n_tr, challenges B * n_chal, outputs B * (instances * layer_size(n-1)),
+ * statements B * 32 bytes, status / accept / code / layer B int32 each. May be NULL: the prover's challenges, outputs and
+ * statements; the verifier's code, layer and challenges. The library cannot see the arrays' sizes: the caller guarantees
+ * them.
+ * Ordering: the work is queued on the context's stream (vp_set_stream) after whatever was queued there before, and the call
+ * returns once it is queued; the results are in the caller's arrays once the stream has passed the call.
+ * Checked when called (VP_ERR_ARG): 1 <= B <= 65535, every non-NULL array device or managed memory of the context's device
+ * (cudaPointerGetAttributes), vp_F arrays 16-byte aligned and the others 8-byte aligned, an unsharded context.
+ * A failing statement never fails the call and changes no other statement's results; every failing statement is reported.
+ * Prover: status[b] = 0 proved (transcript, challenges, outputs and statement b are bit for bit vp_prove_fs_bound_batch's,
+ *   so vp_prove_fs_bound's, for inputs b and context b); 1 an input of statement b is not < p (its inputs are proved as
+ *   zeros, the caller's array is not touched); 2 + l an is_assert gate of layer l is non-zero in statement b (the layer
+ *   VP_ERR_ASSERT names). When status[b] != 0 all four of b's result rows are zero.
+ * Verifier: (accept, code, layer)[b], checked in this order: code 9 an input or claimed output of statement b is not
+ *   canonical (layer 0; the host-memory call fails with VP_ERR_ARG instead), 7 a non-canonical transcript element, 8 Vres
+ *   is not the claimed outputs' MLE at r_out, then vp_verify's codes 1-6. Apart from code 9 the verdicts and the challenges
+ *   are vp_verify_fs_bound_batch's; a statement with code 7 or 9 has zero challenges. The claim chain runs on the device,
+ *   one thread per statement (vp_verify_fs_bound_batch keeps its host loop).
+ * After one call of a kind with B statements (warm-up: the slab, the circuit digest and the per-context tables), a call of
+ * the same kind with at most B statements allocates nothing and does not synchronise with the host. vp_last_prove_launches
+ * describes the call; vp_last_prove_ms waits for the call's end when it is read. The context's resident inputs, values,
+ * transcript and challenges are not changed; vp_last_batch_outputs has nothing after a device call (use the outputs
+ * array). CUDA graph capture is not supported. */
+int vp_prove_fs_bound_batch_dev(vp_ctx* ctx, size_t B, const uint64_t* d_inputs, const uint8_t* d_contexts,
+                                vp_F* d_transcripts, vp_F* d_challenges, vp_F* d_outputs, uint8_t* d_statements,
+                                int32_t* d_status);
+int vp_verify_fs_bound_batch_dev(vp_ctx* ctx, size_t B, const uint64_t* d_inputs, const uint8_t* d_contexts,
+                                 const vp_F* d_outputs, const vp_F* d_transcripts,
+                                 int32_t* d_accept, int32_t* d_code, int32_t* d_layer, vp_F* d_challenges);
 
 /* Self-test of the device-only arithmetic paths of csrc/field.cuh (inline-PTX carry chains, mul.wide / mad.wide):
    runs one routine on n caller-provided operand triples and returns the results, so that tests can feed edge values

@@ -139,6 +139,8 @@ def _declare(L):
     L.vp_last_batch_outputs.argtypes = [vp, vp, C.c_size_t]
     L.vp_verify_fs_bound_batch.argtypes = [vp, C.c_size_t, vp, C.c_size_t, vp, vp, C.c_size_t, vp, C.c_size_t, vp, vp, vp, vp,
                                            C.c_size_t]
+    L.vp_prove_fs_bound_batch_dev.argtypes = [vp, C.c_size_t] + [vp] * 7
+    L.vp_verify_fs_bound_batch_dev.argtypes = [vp, C.c_size_t] + [vp] * 8
     L.vp_aggregate_digest.argtypes = [vp, C.c_size_t, vp, vp, vp]
     L.vp_prove_fs_aggregate.argtypes = [vp, C.c_size_t, vp, vp, C.c_size_t, vp, C.c_size_t, vp, vp]
     L.vp_verify_fs_aggregate.argtypes = [vp, C.c_size_t, vp, vp, C.c_size_t, vp, C.c_size_t, C.POINTER(C.c_int), C.POINTER(C.c_int),
@@ -529,6 +531,7 @@ class Prover:
 
     def __init__(self, circuit, device=0, rank=0, world=1, nccl_id=None):
         self.circuit = circuit
+        self.device = device
         h = C.c_void_p()
         if world == 1:
             _ck(lib().vp_create(circuit.h, device, C.byref(h)))
@@ -780,6 +783,80 @@ class Prover:
                                            _ptr(acc), _ptr(code), _ptr(layer), _ptr(ch), 0 if ch is None else ch.size))
         res = (acc.astype(bool), code, layer)
         return res + (ch,) if return_challenges else res
+
+    # ---- batches in device memory (torch CUDA tensors)
+    def _cuda_batch(self, arrays):
+        """checks (name, tensor, dtype, shape) of a device-memory batch call: a contiguous CUDA tensor on this context's
+        device with that dtype and shape (B taken from the first) -> B; then runs the next call on the current torch stream"""
+        import torch
+        dev = getattr(self, "device", 0)
+        B = None
+        for name, t, dtype, shape in arrays:
+            if not isinstance(t, torch.Tensor):
+                raise ValueError(f"{name} must be a torch tensor, got {type(t)}")
+            if t.dtype != dtype:
+                raise ValueError(f"{name} must be {dtype}, got {t.dtype}")
+            if B is None:
+                B = t.shape[0] if t.dim() >= 1 else 0
+                if not 1 <= B <= 65535:
+                    raise ValueError(f"{name} must hold 1 to 65535 statements, got shape {tuple(t.shape)}")
+            want = (B,) + shape
+            if tuple(t.shape) != want:
+                raise ValueError(f"{name} must have shape {list(want)}, got {list(t.shape)}")
+            if not t.is_contiguous():
+                raise ValueError(f"{name} must be contiguous")
+        for name, t, _, _ in arrays:
+            if t.device.type != "cuda" or (t.device.index or 0) != dev:
+                raise ValueError(f"{name} must be on cuda:{dev}, got {t.device}")
+        # the context runs on the current stream; vp_set_stream waits for the context's previous stream, so it is called only
+        # when the context's actual stream (vp_stream) is another one. torch's default stream is the legacy NULL stream,
+        # cudaStreamLegacy (1) to the runtime.
+        s = torch.cuda.current_stream(dev).cuda_stream or 1
+        if (self.stream or 0) != s:
+            self.set_stream(s)
+        return B
+
+    def _field_tensors(self, B, *counts):
+        import torch
+        return [torch.empty((B, n, 2), dtype=torch.int64, device=f"cuda:{self.device}") for n in counts]
+
+    def prove_fs_bound_batch_cuda(self, inputs, contexts, challenges=False, outputs=False):
+        """prove_fs_bound_batch on CUDA tensors, queued on torch.cuda.current_stream() without waiting for it. The context
+        moves onto that stream, so later calls of this Prover (host-memory ones too) run there until the next set_stream;
+        a change of the current stream costs one host synchronisation (of the context's previous stream). inputs int64
+        [B, n_inputs], contexts uint8 [B, 32] -> (transcripts int64 [B, n_tr, 2] as (re, im), challenges [B, n_chal, 2] or
+        None, statements uint8 [B, 32], outputs [B, n_outputs, 2] or None, status int32 [B]). status b: 0 proved, 1 an input
+        >= p, 2 + l an assert gate of layer l is non-zero; the rows of a failed statement are zero."""
+        import torch
+        n_in = self.circuit.layer_size(0) * self.circuit.instances
+        B = self._cuda_batch([("inputs", inputs, torch.int64, (n_in,)), ("contexts", contexts, torch.uint8, (32,))])
+        tr, ch, out = self._field_tensors(B, self.circuit.transcript_len, self.circuit.challenge_count if challenges else 0,
+                                          self._n_outputs() if outputs else 0)
+        st = torch.empty((B, 32), dtype=torch.uint8, device=tr.device)
+        status = torch.empty(B, dtype=torch.int32, device=tr.device)
+        ch, out = (ch if challenges else None), (out if outputs else None)
+        _ck(lib().vp_prove_fs_bound_batch_dev(self.h, B, inputs.data_ptr(), contexts.data_ptr(), tr.data_ptr(),
+                                              None if ch is None else ch.data_ptr(), None if out is None else out.data_ptr(),
+                                              st.data_ptr(), status.data_ptr()))
+        return tr, ch, st, out, status
+
+    def verify_fs_bound_batch_cuda(self, inputs, contexts, outputs, transcripts, challenges=False):
+        """verify_fs_bound_batch on CUDA tensors, queued on torch.cuda.current_stream() without waiting for it (the context
+        moves onto that stream, as in prove_fs_bound_batch_cuda): inputs int64
+        [B, n_inputs], contexts uint8 [B, 32], outputs int64 [B, n_outputs, 2], transcripts int64 [B, n_tr, 2] -> (accept,
+        fail_code, fail_layer int32 [B], challenges [B, n_chal, 2] or None). fail_code 9: an input or output of the statement
+        is not canonical."""
+        import torch
+        n_in = self.circuit.layer_size(0) * self.circuit.instances
+        B = self._cuda_batch([("inputs", inputs, torch.int64, (n_in,)), ("contexts", contexts, torch.uint8, (32,)),
+                              ("outputs", outputs, torch.int64, (self._n_outputs(), 2)),
+                              ("transcripts", transcripts, torch.int64, (self.circuit.transcript_len, 2))])
+        acc, code, layer = (torch.empty(B, dtype=torch.int32, device=inputs.device) for _ in range(3))
+        ch = self._field_tensors(B, self.circuit.challenge_count)[0] if challenges else None
+        _ck(lib().vp_verify_fs_bound_batch_dev(self.h, B, inputs.data_ptr(), contexts.data_ptr(), outputs.data_ptr(),
+                                               transcripts.data_ptr(), acc.data_ptr(), code.data_ptr(), layer.data_ptr(),
+                                               None if ch is None else ch.data_ptr()))
+        return acc, code, layer, ch
 
     def verify_fs_bound(self, context, outputs, transcript):
         """(accept, fail_code, fail_layer) of a statement-bound proof for the claimed outputs and this context's inputs"""

@@ -1059,6 +1059,11 @@ struct Engine {
     DBuf<F> d_fs_outputs;                  // vp_verify_fs_bound(_batch): the claimed outputs, statements end to end
     DBuf<FsStep> d_fs_steps;               // vp_verify_fs_bound_batch: the store / draw order of a transcript (k_fs_replay)
     void fs_replay_table();
+    // vp_verify_fs_bound_batch_dev: the claim chain's per-layer table (k_verify_check), built once per context after vf_layout
+    DBuf<VfLayerDesc> d_vf_desc;
+    DBuf<uint32_t> d_vf_keys;
+    VfCheckArgs vf_check_table();
+    void load_batch_inputs(const uint64_t* src, size_t cnt);
     bool circuit_digest_ready = false;
     int cap_phase_fs = 0;
     void fs_alloc();
@@ -1090,9 +1095,14 @@ struct Engine {
         if (n_stmt == 1) CK(cudaMemsetAsync(p, 0, bytes, stream));
         else CK(cudaMemset2DAsync(p, sstride, 0, bytes, n_stmt, stream));
     }
-    void copy_stmts_to_host(void* dst, size_t dpitch, const void* src, size_t bytes) {   // statement b's bytes to dst + b * dpitch
-        if (n_stmt == 1) CK(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToHost, stream));
-        else CK(cudaMemcpy2DAsync(dst, dpitch, src, sstride, bytes, n_stmt, cudaMemcpyDeviceToHost, stream));
+    // A batch whose arrays are in device memory (vp_*_fs_bound_batch_dev): statuses instead of errors, copies device to
+    // device, and no host synchronisation once the buffers are warm.
+    bool dev_io = false;
+    bool ms_pending = false;   // last_ms is that of a device-memory batch still in flight (vp_last_prove_ms waits for ev1)
+    void copy_stmts_out(void* dst, size_t dpitch, const void* src, size_t bytes) {   // statement b's bytes to dst + b * dpitch
+        const cudaMemcpyKind k = dev_io ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost;
+        if (n_stmt == 1) CK(cudaMemcpyAsync(dst, src, bytes, k, stream));
+        else CK(cudaMemcpy2DAsync(dst, dpitch, src, sstride, bytes, n_stmt, k, stream));
     }
     // The batch's own buffers, kept for the next batch and grown when needed: per statement a copy of every buffer the
     // Fiat-Shamir path writes (one slab, `stride` bytes per statement), and the layer values, inputs and the descriptors that
@@ -1105,6 +1115,7 @@ struct Engine {
         std::vector<DBuf<F>> val;
         DBuf<F*> valptr;
         DBuf<uint64_t> inputs, contexts, root_scratch;
+        DBuf<int32_t> status;              // device-memory batches: the statements' statuses (k_batch_screen)
         std::vector<DBuf<P2Table>> p2_tabs;
         std::vector<DBuf<EqTab>> liu_eqtabs;
         std::vector<std::pair<void*, size_t>> views;   // statement 0's buffers in the slab (the context's while swapped)
@@ -2684,13 +2695,18 @@ void Engine::fs_begin() {
     memset_stmts(d_chal.p, (lay.n_chal + 1) * sizeof(F));   // unused challenge slots are zero
     if (n_stmt == 1) h_chal.assign(lay.n_chal, f_zero());
     evaluate();
+    if (dev_io) {   // every statement's assert flag becomes its status on the device
+        k_batch_assert_status<<<cdiv(n_stmt, 128), 128, 0, stream>>>(d_counter.p + 1, sstride, n_stmt, slab.status.p);
+        ++launches;
+        return;
+    }
     if (n_stmt == 1) {
         check_assert_flag();
         return;
     }
     // the first statement with a failed assert gate
     std::vector<unsigned int> flags(n_stmt);
-    copy_stmts_to_host(flags.data(), sizeof(unsigned int), d_counter.p + 1, sizeof(unsigned int));
+    copy_stmts_out(flags.data(), sizeof(unsigned int), d_counter.p + 1, sizeof(unsigned int));
     CK(cudaStreamSynchronize(stream));
     for (uint32_t b = 0; b < n_stmt; ++b)
         if (flags[b]) throw StatementAssert{b, flags[b]};
@@ -2725,6 +2741,7 @@ void Engine::slab_reserve(uint32_t B, size_t vf_entries) {
     slab.valptr.upload(h_ptr, stream);
     slab.inputs.alloc((size_t)B * C.layer_size(0));
     slab.contexts.alloc((size_t)4 * B);
+    slab.status.alloc(B);
     // descriptors that point into the context's values / eq tables, rebased on the slab's
     slab.p2_tabs.resize(n);
     slab.liu_eqtabs.resize(n);
@@ -2948,14 +2965,20 @@ void Engine::prove_fs_device(F* tr_out, F* ch_out) {
     }
     do_input_mle();
     fs_rounds = sr;
+    proof_size = lay.proof_size;
+    if (dev_io) {   // into the caller's device arrays; nothing waits for them
+        copy_stmts_out(tr_out, lay.n_tr * sizeof(F), d_tr.p, lay.n_tr * sizeof(F));
+        if (ch_out) copy_stmts_out(ch_out, lay.n_chal * sizeof(F), d_chal.p, lay.n_chal * sizeof(F));
+        CK(cudaGetLastError());
+        return;
+    }
     std::vector<F> ch((size_t)n_stmt * lay.n_chal);   // statement-major, like the transcripts
-    copy_stmts_to_host(tr_out, lay.n_tr * sizeof(F), d_tr.p, lay.n_tr * sizeof(F));
-    copy_stmts_to_host(ch.data(), lay.n_chal * sizeof(F), d_chal.p, lay.n_chal * sizeof(F));
+    copy_stmts_out(tr_out, lay.n_tr * sizeof(F), d_tr.p, lay.n_tr * sizeof(F));
+    copy_stmts_out(ch.data(), lay.n_chal * sizeof(F), d_chal.p, lay.n_chal * sizeof(F));
     CK(cudaStreamSynchronize(stream));
     CK(cudaGetLastError());
     if (n_stmt == 1) h_chal = ch;   // a later vp_verify / vp_prove on this context sees the challenges the proof used
     if (ch_out) memcpy(ch_out, ch.data(), ch.size() * sizeof(F));
-    proof_size = lay.proof_size;
 }
 
 // fs_schedule as k_fs_replay's steps, one per round of a phase, built once per context.
@@ -2966,6 +2989,37 @@ void Engine::fs_replay_table() {
         for (uint32_t k = 0; k < e.count; ++k) st.push_back(e.step(k));
     d_fs_steps.upload(st, stream);
     CK(cudaStreamSynchronize(stream));   // (the host vector goes out of scope)
+}
+
+// verify_check's view of the proof layout and of the bucket keys for k_verify_check, built once per context (after
+// vf_layout, which places every layer's sums).
+VfCheckArgs Engine::vf_check_table() {
+    if (!d_vf_desc.p) {
+        std::vector<VfLayerDesc> t(n);
+        std::vector<uint32_t> keys;
+        for (int i = 1; i < n; ++i) {
+            const LayerDev& D = L[i];
+            t[i] = VfLayerDesc{D.pb, D.m, D.tr_p1, D.tr_claim_u, D.tr_p2, D.tr_claims_v, D.tr_liu, D.tr_claim_liu, D.ci_ru, D.ci_rv,
+                               D.ci_sig, D.ci_rliu, D.vf_out, (uint32_t)keys.size(), (uint32_t)D.vf_key.size(), D.n_vf_liu};
+            keys.insert(keys.end(), D.vf_key.begin(), D.vf_key.end());
+        }
+        d_vf_desc.upload(t, stream);
+        d_vf_keys.upload(keys, stream);
+        CK(cudaStreamSynchronize(stream));   // (the host vectors go out of scope)
+    }
+    return VfCheckArgs{d_vf_desc.p, d_vf_keys.p, n, lay.tr_vres, lay.tr_input, vf_out_total};
+}
+
+// A batch's inputs (cnt, statement-major) into d_inputs: from the host (checked before the call), or from the caller's
+// device array through k_batch_screen (status 1 and zeros for a statement with an input >= p).
+void Engine::load_batch_inputs(const uint64_t* src, size_t cnt) {
+    if (!dev_io) {
+        CK(cudaMemcpyAsync(d_inputs.p, src, cnt * sizeof(uint64_t), cudaMemcpyHostToDevice, stream));
+        return;
+    }
+    k_batch_screen<<<sgrid(1), 256, 0, stream>>>(src, d_inputs.p, (uint32_t)(cnt / n_stmt), nullptr, nullptr, 0, nullptr, 0, sstride, 1,
+                                                 slab.status.p);
+    ++launches;
 }
 
 struct vp_ctx {
@@ -3320,17 +3374,24 @@ struct ScopedTimer {
     ~ScopedTimer() { e.prove_seconds += std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count(); }
 };
 // The device window of vp_last_prove_ms and vp_last_prove_launches around body(); read_back() queues the results to the
-// host after it, and one synchronisation ends the call.
+// host after it, and one synchronisation ends the call. A device-memory batch (e.dev_io) does not wait: its window covers
+// the whole call, read_back() included, and vp_last_prove_ms waits for the window's end when it is read.
 template <class Body, class ReadBack>
 static void device_window(Engine& e, Body body, ReadBack read_back) {
     const uint64_t l0 = e.launches;
+    e.ms_pending = false;
     CK(cudaEventRecord(e.ev0, e.stream));
     body();
+    if (e.dev_io) read_back();
     CK(cudaEventRecord(e.ev1, e.stream));
-    read_back();
+    if (!e.dev_io) read_back();
+    e.last_launches = e.launches - l0;
+    if (e.dev_io) {
+        e.ms_pending = true;
+        return;
+    }
     CK(cudaStreamSynchronize(e.stream));
     CK(cudaEventElapsedTime(&e.last_ms, e.ev0, e.ev1));
-    e.last_launches = e.launches - l0;
 }
 
 extern "C" int vp_set_inputs(vp_ctx* ctx, const uint64_t* inputs, size_t n) {
@@ -3874,7 +3935,7 @@ template <class Seed, class ReadBack>
 static void prove_fs_window(Engine& e, const uint64_t* inputs, size_t n_inputs, Seed seed, vp_F* transcript, vp_F* challenges,
                             ReadBack read_back) {
     device_window(e, [&] {
-        if (inputs) CK(cudaMemcpyAsync(e.d_inputs.p, inputs, n_inputs * sizeof(uint64_t), cudaMemcpyHostToDevice, e.stream));
+        if (inputs) e.load_batch_inputs(inputs, n_inputs);
         e.fs_begin();
         seed();
         e.prove_fs_device(reinterpret_cast<F*>(transcript), reinterpret_cast<F*>(challenges));
@@ -3999,24 +4060,26 @@ extern "C" int vp_prove_fs_bound(vp_ctx* ctx, const uint8_t context[32], vp_F* t
     check_capacity(e, 1, cap, challenges, ch_cap);
     check_inputs_loaded(e, "vp_prove_fs_bound");
     prove_fs_window(e, nullptr, 0, [&] { e.statement_async(context, nullptr); }, transcript, challenges,
-                    [&] { if (statement) e.copy_stmts_to_host(statement, 32, e.stmt_statement(), 32); });
+                    [&] { if (statement) e.copy_stmts_out(statement, 32, e.stmt_statement(), 32); });
     return VP_OK;
     API_END
 }
 // A batch runs on the context's slab (Engine::FsSlab): the scope swaps the slab in and, on every exit, the context's own
-// buffers and host state back, so that the context's inputs, values, transcript and challenges are untouched.
+// buffers and host state back, so that the context's inputs, values, transcript and challenges are untouched. dev: the
+// batch's arrays are in device memory (Engine::dev_io).
 struct FsBatchScope {
     Engine& e;
     std::vector<F> h_chal;
     bool evaluated;
     int pending_chunks;
-    FsBatchScope(Engine& e_, uint32_t B, size_t vf_entries = 0)
+    FsBatchScope(Engine& e_, uint32_t B, bool dev, size_t vf_entries = 0)
         : e(e_), h_chal(e_.h_chal), evaluated(e_.evaluated), pending_chunks(e_.pending_chunks) {
         e.slab_reserve(B, vf_entries);
         e.slab_swap();
         e.n_stmt = B;
         e.sstride = e.slab.stride;
         e.pending_chunks = 0;
+        e.dev_io = dev;
     }
     ~FsBatchScope() {
         e.slab_swap();
@@ -4025,8 +4088,57 @@ struct FsBatchScope {
         e.h_chal.swap(h_chal);
         e.evaluated = evaluated;
         e.pending_chunks = pending_chunks;
+        e.dev_io = false;
     }
 };
+// Argument checks of the device-memory batches: every non-null array is device or managed memory of the context's device,
+// aligned to `align` bytes (the library cannot see their sizes; the binding checks them from tensor shapes).
+struct DevArray {
+    const void* p;
+    size_t align;
+    const char* name;
+};
+static void check_device_arrays(const Engine& e, const char* fn, std::initializer_list<DevArray> arrays) {
+    for (const DevArray& a : arrays) {
+        if (!a.p) continue;
+        cudaPointerAttributes at;
+        if (cudaPointerGetAttributes(&at, a.p) != cudaSuccess) {
+            cudaGetLastError();
+            bad_arg("%s: %s is not a CUDA pointer", fn, a.name);
+        }
+        if ((at.type != cudaMemoryTypeDevice && at.type != cudaMemoryTypeManaged) || at.device != e.device)
+            bad_arg("%s: %s is not device memory of device %d", fn, a.name, e.device);
+        if (reinterpret_cast<uintptr_t>(a.p) % a.align) bad_arg("%s: %s is not %zu-byte aligned", fn, a.name, a.align);
+    }
+}
+// The batch prover of vp_prove_fs_bound_batch (host arrays, checked by the caller; a failed assert gate throws) and
+// vp_prove_fs_bound_batch_dev (device arrays: status[b] per statement, the rows of a failed statement zeroed, nothing
+// waited for). outputs and status: device arrays only.
+static void prove_batch(Engine& e, uint32_t B, bool dev, const uint64_t* inputs, const uint8_t* contexts, vp_F* transcripts,
+                        vp_F* challenges, vp_F* outputs, uint8_t* statements, int32_t* status) {
+    e.leave();
+    e.fs_alloc();
+    e.circuit_digest_async();
+    e.batch_outputs = 0;
+    FsBatchScope scope(e, B, dev);
+    prove_fs_window(e, inputs, (size_t)B * e.C.layer_size(0), [&] {
+        CK(cudaMemcpyAsync(e.slab.contexts.p, contexts, 32 * (size_t)B, dev ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice, e.stream));
+        e.statement_async(nullptr, nullptr, e.slab.contexts.p);
+    }, transcripts, challenges, [&] {
+        if (statements) e.copy_stmts_out(statements, 32, e.stmt_statement(), 32);
+        if (!dev) return;
+        const size_t n_out = e.C.layer_size(e.n - 1);
+        if (outputs) CK(cudaMemcpyAsync(outputs, e.val[e.n - 1].p, B * n_out * sizeof(F), cudaMemcpyDeviceToDevice, e.stream));
+        k_batch_zero_failed<<<e.sgrid(1), 256, 0, e.stream>>>(e.slab.status.p, reinterpret_cast<F*>(transcripts), (uint32_t)e.lay.n_tr,
+                                                             reinterpret_cast<F*>(challenges), (uint32_t)e.lay.n_chal,
+                                                             reinterpret_cast<F*>(outputs), (uint32_t)n_out,
+                                                             reinterpret_cast<uint64_t*>(statements), 4);
+        ++e.launches;
+        CK(cudaMemcpyAsync(status, e.slab.status.p, B * sizeof(int32_t), cudaMemcpyDeviceToDevice, e.stream));
+        CK(cudaGetLastError());
+    });
+    if (!dev) e.batch_outputs = B;
+}
 extern "C" int vp_prove_fs_bound_batch(vp_ctx* ctx, size_t B, const uint64_t* inputs, size_t n_inputs, const uint8_t* contexts,
                                        vp_F* transcripts, size_t cap, vp_F* challenges, size_t ch_cap, uint8_t* statements) {
     if (!ctx || !inputs || !contexts || !transcripts) return fail(VP_ERR_ARG, "null argument");
@@ -4037,16 +4149,24 @@ extern "C" int vp_prove_fs_bound_batch(vp_ctx* ctx, size_t B, const uint64_t* in
     check_count(B, "vp_prove_fs_bound_batch");
     check_capacity(e, B, cap, challenges, ch_cap);
     check_inputs(inputs, n_inputs, B, e.C.layer_size(0));
-    e.leave();
-    e.fs_alloc();
-    e.circuit_digest_async();
-    e.batch_outputs = 0;
-    FsBatchScope scope(e, (uint32_t)B);
-    prove_fs_window(e, inputs, n_inputs, [&] {
-        CK(cudaMemcpyAsync(e.slab.contexts.p, contexts, 32 * B, cudaMemcpyHostToDevice, e.stream));
-        e.statement_async(nullptr, nullptr, e.slab.contexts.p);
-    }, transcripts, challenges, [&] { if (statements) e.copy_stmts_to_host(statements, 32, e.stmt_statement(), 32); });
-    e.batch_outputs = (uint32_t)B;
+    prove_batch(e, (uint32_t)B, false, inputs, contexts, transcripts, challenges, nullptr, statements, nullptr);
+    return VP_OK;
+    API_END
+}
+extern "C" int vp_prove_fs_bound_batch_dev(vp_ctx* ctx, size_t B, const uint64_t* d_inputs, const uint8_t* d_contexts,
+                                           vp_F* d_transcripts, vp_F* d_challenges, vp_F* d_outputs, uint8_t* d_statements,
+                                           int32_t* d_status) {
+    if (!ctx || !d_inputs || !d_contexts || !d_transcripts || !d_status) return fail(VP_ERR_ARG, "null argument");
+    API_BEGIN
+    Engine& e = ctx->e;
+    ScopedTimer t(e);
+    const char* fn = "vp_prove_fs_bound_batch_dev";
+    check_unsharded(e, fn);
+    check_count(B, fn);
+    check_device_arrays(e, fn, {{d_inputs, 8, "inputs"}, {d_contexts, 8, "contexts"}, {d_transcripts, 16, "transcripts"},
+                                {d_challenges, 16, "challenges"}, {d_outputs, 16, "outputs"}, {d_statements, 8, "statements"},
+                                {d_status, 8, "status"}});
+    prove_batch(e, (uint32_t)B, true, d_inputs, d_contexts, d_transcripts, d_challenges, d_outputs, d_statements, d_status);
     return VP_OK;
     API_END
 }
@@ -4063,6 +4183,54 @@ extern "C" int vp_last_batch_outputs(vp_ctx* ctx, vp_F* out, size_t cap) {
     CK(cudaStreamSynchronize(e.stream));
     return VP_OK;
     API_END
+}
+// The batch verifier of vp_verify_fs_bound_batch (host arrays, checked by the caller, whose non-canonical transcripts come
+// as zero rows) and vp_verify_fs_bound_batch_dev (device arrays, screened on the device: codes 9 and 7 in slab.status).
+// Queues the upload, the roots and statements, the challenge replay and every sum of all B statements; read_back(sums)
+// then queues what follows them (sums: statement 0's vf_out_total sums in the slab, sstride bytes per statement).
+template <class ReadBack>
+static void verify_batch(Engine& e, uint32_t B, bool dev, const uint64_t* inputs, const uint8_t* contexts, const vp_F* outputs,
+                         const vp_F* transcripts, ReadBack read_back) {
+    const size_t n_in = e.C.layer_size(0), n_out = e.C.layer_size(e.n - 1), n_outputs = (size_t)B * n_out;
+    e.leave();
+    e.fs_alloc();
+    e.circuit_digest_async();
+    e.fs_replay_table();
+    e.vf_layout();
+    if (dev) e.vf_check_table();   // (built once per context: k_verify_check's table)
+    e.batch_outputs = 0;
+    const uint32_t out_total = e.vf_out_total;
+    if (e.d_fs_outputs.n < n_outputs) e.d_fs_outputs.alloc(n_outputs);
+    FsBatchScope scope(e, B, dev, (size_t)out_total + (size_t)e.vf_max_b * Engine::VF_GX * 2);
+    F* const d_out = reinterpret_cast<F*>(e.slab.mem.p + e.slab.o_vf);
+    F* const d_part = d_out + out_total;
+    const size_t tr_bytes = e.lay.n_tr * sizeof(F);
+    device_window(e, [&] {
+        if (dev) {
+            CK(cudaMemcpy2DAsync(e.d_tr.p, e.sstride, transcripts, tr_bytes, tr_bytes, B, cudaMemcpyDeviceToDevice, e.stream));
+            k_batch_screen<<<e.sgrid(1), 256, 0, e.stream>>>(inputs, e.d_inputs.p, (uint32_t)n_in, reinterpret_cast<const F*>(outputs),
+                                                            e.d_fs_outputs.p, (uint32_t)n_out, e.d_tr.p, (uint32_t)e.lay.n_tr, e.sstride, 9,
+                                                            e.slab.status.p);
+            ++e.launches;
+        } else {
+            CK(cudaMemcpyAsync(e.d_inputs.p, inputs, B * n_in * sizeof(uint64_t), cudaMemcpyHostToDevice, e.stream));
+            CK(cudaMemcpyAsync(e.d_fs_outputs.p, outputs, n_outputs * sizeof(F), cudaMemcpyHostToDevice, e.stream));
+            CK(cudaMemcpy2DAsync(e.d_tr.p, e.sstride, transcripts, tr_bytes, tr_bytes, B, cudaMemcpyHostToDevice, e.stream));
+        }
+        CK(cudaMemcpyAsync(e.slab.contexts.p, contexts, 32 * (size_t)B, dev ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice, e.stream));
+        e.memset_stmts(e.d_chal.p, (e.lay.n_chal + 1) * sizeof(F));   // unused challenge slots are zero
+        e.memset_stmts(d_out, (size_t)out_total * sizeof(F));
+        const uint32_t n0 = (uint32_t)(B * n_in);   // circuitValue[0] of every statement, instance-major over B * K
+        k_load_inputs<<<cdiv(n0, 256), 256, 0, e.stream>>>(e.d_inputs.p, e.val[0].p, 0, n0);
+        ++e.launches;
+        e.statement_async(nullptr, e.d_fs_outputs.p, e.slab.contexts.p);
+        k_fs_replay<<<e.sgrid(1), 32, 0, e.stream>>>(e.d_fs_steps.p, (uint32_t)e.d_fs_steps.n, e.d_fs_pool.p, e.d_tr.p, e.d_chal.p, e.sstride);
+        ++e.launches;
+        // the claim chain starts from Vres: the MLE of the claimed outputs at r_out, next to the input MLE
+        e.run_eq(e.eqb_out, 2);
+        e.run_dot_eq(e.d_fs_outputs.p, (uint32_t)e.C.layers[e.n - 1].size, e.eqtab(2, e.C.bit_length(e.n - 1)), d_out + out_total - 1);
+        e.verify_sums_async(d_out, d_part);
+    }, [&] { read_back(static_cast<const F*>(d_out)); });
 }
 extern "C" int vp_verify_fs_bound_batch(vp_ctx* ctx, size_t B, const uint64_t* inputs, size_t n_inputs, const uint8_t* contexts,
                                         const vp_F* outputs, size_t n_outputs, const vp_F* transcripts, size_t n_tr, int* accept,
@@ -4089,42 +4257,15 @@ extern "C" int vp_verify_fs_bound_batch(vp_ctx* ctx, size_t B, const uint64_t* i
             if (bad[b]) std::fill(clean.begin() + b * e.lay.n_tr, clean.begin() + (b + 1) * e.lay.n_tr, f_zero());
         tr = clean.data();
     }
-    e.leave();
-    e.fs_alloc();
-    e.circuit_digest_async();
-    e.fs_replay_table();
-    e.vf_layout();
-    e.batch_outputs = 0;
-    const uint32_t out_total = e.vf_out_total;
-    if (e.d_fs_outputs.n < n_outputs) e.d_fs_outputs.alloc(n_outputs);
-    std::vector<F> sums((size_t)B * out_total), ch((size_t)B * e.lay.n_chal);
-    {
-        FsBatchScope scope(e, (uint32_t)B, (size_t)out_total + (size_t)e.vf_max_b * Engine::VF_GX * 2);
-        F* const d_out = reinterpret_cast<F*>(e.slab.mem.p + e.slab.o_vf);
-        F* const d_part = d_out + out_total;
-        device_window(e, [&] {
-            CK(cudaMemcpyAsync(e.d_inputs.p, inputs, n_inputs * sizeof(uint64_t), cudaMemcpyHostToDevice, e.stream));
-            CK(cudaMemcpyAsync(e.d_fs_outputs.p, outputs, n_outputs * sizeof(F), cudaMemcpyHostToDevice, e.stream));
-            CK(cudaMemcpyAsync(e.slab.contexts.p, contexts, 32 * B, cudaMemcpyHostToDevice, e.stream));
-            CK(cudaMemcpy2DAsync(e.d_tr.p, e.sstride, tr, e.lay.n_tr * sizeof(F), e.lay.n_tr * sizeof(F), B, cudaMemcpyHostToDevice, e.stream));
-            e.memset_stmts(e.d_chal.p, (e.lay.n_chal + 1) * sizeof(F));   // unused challenge slots are zero
-            e.memset_stmts(d_out, (size_t)out_total * sizeof(F));
-            const uint32_t n0 = (uint32_t)(B * n_in);   // circuitValue[0] of every statement, instance-major over B * K
-            k_load_inputs<<<cdiv(n0, 256), 256, 0, e.stream>>>(e.d_inputs.p, e.val[0].p, 0, n0);
-            ++e.launches;
-            e.statement_async(nullptr, e.d_fs_outputs.p, e.slab.contexts.p);
-            k_fs_replay<<<e.sgrid(1), 32, 0, e.stream>>>(e.d_fs_steps.p, (uint32_t)e.d_fs_steps.n, e.d_fs_pool.p, e.d_tr.p, e.d_chal.p, e.sstride);
-            ++e.launches;
-            // the claim chain starts from Vres: the MLE of the claimed outputs at r_out, next to the input MLE
-            e.run_eq(e.eqb_out, 2);
-            e.run_dot_eq(e.d_fs_outputs.p, (uint32_t)e.C.layers[e.n - 1].size, e.eqtab(2, e.C.bit_length(e.n - 1)), d_out + out_total - 1);
-            e.verify_sums_async(d_out, d_part);
-        }, [&] {
-            e.copy_stmts_to_host(sums.data(), out_total * sizeof(F), d_out, out_total * sizeof(F));
-            e.copy_stmts_to_host(ch.data(), e.lay.n_chal * sizeof(F), e.d_chal.p, e.lay.n_chal * sizeof(F));
-            CK(cudaGetLastError());
-        });
-    }
+    std::vector<F> sums, ch((size_t)B * e.lay.n_chal);
+    uint32_t out_total = 0;
+    verify_batch(e, (uint32_t)B, false, inputs, contexts, outputs, reinterpret_cast<const vp_F*>(tr), [&](const F* d_out) {
+        out_total = e.vf_out_total;
+        sums.resize((size_t)B * out_total);
+        e.copy_stmts_out(sums.data(), out_total * sizeof(F), d_out, out_total * sizeof(F));
+        e.copy_stmts_out(ch.data(), e.lay.n_chal * sizeof(F), e.d_chal.p, e.lay.n_chal * sizeof(F));
+        CK(cudaGetLastError());
+    });
     // the host driver, one statement at a time, in vp_verify_fs_bound's order: code 7, code 8, then vp_verify's checks
     for (size_t b = 0; b < B; ++b) {
         int code = 0, layer = 0, ok = 0;
@@ -4139,6 +4280,35 @@ extern "C" int vp_verify_fs_bound_batch(vp_ctx* ctx, size_t B, const uint64_t* i
         if (bad[b]) std::fill(ch.begin() + b * e.lay.n_chal, ch.begin() + (b + 1) * e.lay.n_chal, f_zero());
     }
     if (challenges) memcpy(challenges, ch.data(), ch.size() * sizeof(F));
+    return VP_OK;
+    API_END
+}
+extern "C" int vp_verify_fs_bound_batch_dev(vp_ctx* ctx, size_t B, const uint64_t* d_inputs, const uint8_t* d_contexts,
+                                            const vp_F* d_outputs, const vp_F* d_transcripts, int32_t* d_accept, int32_t* d_code,
+                                            int32_t* d_layer, vp_F* d_challenges) {
+    if (!ctx || !d_inputs || !d_contexts || !d_outputs || !d_transcripts || !d_accept) return fail(VP_ERR_ARG, "null argument");
+    API_BEGIN
+    Engine& e = ctx->e;
+    ScopedTimer t(e);
+    const char* fn = "vp_verify_fs_bound_batch_dev";
+    check_unsharded(e, fn);
+    check_count(B, fn);
+    check_device_arrays(e, fn, {{d_inputs, 8, "inputs"}, {d_contexts, 8, "contexts"}, {d_outputs, 16, "outputs"},
+                                {d_transcripts, 16, "transcripts"}, {d_accept, 8, "accept"}, {d_code, 8, "code"}, {d_layer, 8, "layer"},
+                                {d_challenges, 16, "challenges"}});
+    verify_batch(e, (uint32_t)B, true, d_inputs, d_contexts, d_outputs, d_transcripts, [&](const F* d_out) {
+        // the claim chain on the device, one thread per statement, then the challenges (zero for codes 7 and 9)
+        k_verify_check<<<cdiv((uint32_t)B, 128), 128, 0, e.stream>>>(e.vf_check_table(), e.d_tr.p, e.d_chal.p, d_out, e.sstride,
+                                                                    (uint32_t)B, e.slab.status.p, d_accept, d_code, d_layer);
+        ++e.launches;
+        if (d_challenges) {
+            e.copy_stmts_out(d_challenges, e.lay.n_chal * sizeof(F), e.d_chal.p, e.lay.n_chal * sizeof(F));
+            k_batch_zero_failed<<<e.sgrid(1), 256, 0, e.stream>>>(e.slab.status.p, reinterpret_cast<F*>(d_challenges), (uint32_t)e.lay.n_chal, nullptr, 0,
+                                                                 nullptr, 0, nullptr, 0);
+            ++e.launches;
+        }
+        CK(cudaGetLastError());
+    });
     return VP_OK;
     API_END
 }
@@ -4306,7 +4476,19 @@ extern "C" int vp_get_profile(vp_ctx* ctx, double* ms, double* bytes, uint64_t* 
     return VP_OK;
     API_END
 }
-extern "C" float vp_last_prove_ms(const vp_ctx* ctx) { return ctx ? ctx->e.last_ms : 0.f; }
+extern "C" float vp_last_prove_ms(const vp_ctx* ctx) {
+    if (!ctx) return 0.f;
+    Engine& e = const_cast<vp_ctx*>(ctx)->e;
+    if (e.ms_pending) {   // a device-memory batch: wait for its window's end
+        e.ms_pending = false;
+        cudaSetDevice(e.device);
+        if (cudaEventSynchronize(e.ev1) != cudaSuccess || cudaEventElapsedTime(&e.last_ms, e.ev0, e.ev1) != cudaSuccess) {
+            cudaGetLastError();
+            e.last_ms = 0.f;
+        }
+    }
+    return e.last_ms;
+}
 extern "C" uint64_t vp_last_prove_launches(const vp_ctx* ctx) { return ctx ? ctx->e.last_launches : 0; }
 extern "C" void* vp_stream(vp_ctx* ctx) { return ctx ? (void*)ctx->e.stream : nullptr; }
 

@@ -271,4 +271,180 @@ __global__ void __launch_bounds__(256, 2) k_sumcheck_phase_fs(PhaseArgs p, FsPha
     }
 }
 
+// ------------------------------------------------------------------ batches in device memory (vp_*_fs_bound_batch_dev)
+// A statement that fails is reported in status[b] (one int32 per statement) and must not change any other statement's
+// results, so nothing non-canonical it holds reaches the arithmetic.
+VP_D bool f_canonical(const F& x) { return x.re < P && x.im < P; }
+
+// One block per statement (blockIdx.z == b): statement b's inputs (and, in the verifier, its claimed outputs) from the
+// caller's packed arrays into the batch's buffers -- as zeros when one of them is not canonical -- and its transcript,
+// already in its working set (tr, ss bytes per statement; may be null), zeroed when one of its elements is not canonical.
+// status[b] = io_code (prover 1, verifier 9) for an input or output, else 7 for a transcript element, else 0.
+__global__ void k_batch_screen(const uint64_t* __restrict__ in_src, uint64_t* __restrict__ in_dst, uint32_t n_in,
+                               const F* __restrict__ out_src, F* __restrict__ out_dst, uint32_t n_out, F* tr, uint32_t n_tr,
+                               size_t ss, int32_t io_code, int32_t* __restrict__ status) {
+    const size_t b = blockIdx.z;
+    in_src += b * n_in;
+    in_dst += b * n_in;
+    if (out_src) { out_src += b * n_out; out_dst += b * n_out; }
+    if (tr) tr = stmt_at(tr, ss);
+    int bad_io = 0, bad_tr = 0;
+    for (uint32_t i = threadIdx.x; i < n_in; i += blockDim.x) bad_io |= in_src[i] >= P;
+    if (out_src)
+        for (uint32_t i = threadIdx.x; i < n_out; i += blockDim.x) bad_io |= !f_canonical(ld_f(out_src + i));
+    if (tr)
+        for (uint32_t i = threadIdx.x; i < n_tr; i += blockDim.x) bad_tr |= !f_canonical(tr[i]);
+    bad_io = __syncthreads_or(bad_io);
+    bad_tr = __syncthreads_or(bad_tr);
+    for (uint32_t i = threadIdx.x; i < n_in; i += blockDim.x) in_dst[i] = bad_io ? 0 : in_src[i];
+    if (out_src)
+        for (uint32_t i = threadIdx.x; i < n_out; i += blockDim.x) st_f(out_dst + i, bad_io ? f_zero() : ld_f(out_src + i));
+    if (bad_tr)
+        for (uint32_t i = threadIdx.x; i < n_tr; i += blockDim.x) st_f(tr + i, f_zero());
+    if (threadIdx.x == 0) status[b] = bad_io ? io_code : bad_tr ? 7 : 0;
+}
+
+// The prover's assert flags (statement b's copy of d_counter[1], ss bytes apart: 1 + the layer of a non-zero is_assert
+// gate, k_eval_layer) as statuses 2 + layer, one thread per statement; a status already set stays.
+__global__ void k_batch_assert_status(const unsigned int* __restrict__ flag, size_t ss, uint32_t B, int32_t* __restrict__ status) {
+    const uint32_t b = blockIdx.x * blockDim.x + threadIdx.x;
+    if (b >= B) return;
+    const unsigned int f = *reinterpret_cast<const unsigned int*>(reinterpret_cast<uintptr_t>(flag) + (size_t)b * ss);
+    if (status[b] == 0 && f) status[b] = (int32_t)f + 1;
+}
+
+// One block per statement (blockIdx.z == b): when status[b] != 0, zero its row of each packed array (null: none).
+__global__ void k_batch_zero_failed(const int32_t* __restrict__ status, F* a, uint32_t na, F* c, uint32_t nc, F* o, uint32_t no,
+                                    uint64_t* w, uint32_t nw) {
+    const size_t b = blockIdx.z;
+    if (!status[b]) return;
+    if (a) for (uint32_t i = threadIdx.x; i < na; i += blockDim.x) st_f(a + b * na + i, f_zero());
+    if (c) for (uint32_t i = threadIdx.x; i < nc; i += blockDim.x) st_f(c + b * nc + i, f_zero());
+    if (o) for (uint32_t i = threadIdx.x; i < no; i += blockDim.x) st_f(o + b * no + i, f_zero());
+    if (w) for (uint32_t i = threadIdx.x; i < nw; i += blockDim.x) w[b * nw + i] = 0;
+}
+
+// The verifier's claim chain (Engine::verify_check, verifier.cpp:134-337) on the device. Per layer: its rounds, where its
+// messages and challenges sit, where its sums sit among the statement's vf_out_total sums and its bucket keys (keys[key_begin
+// .. + n_keys): 0 Copy, 1 Not, 2 Addc, 3 Mulc, 4 + 7 l + binary type index).
+struct VfLayerDesc {
+    int32_t pb, m;
+    uint32_t tr_p1, tr_claim_u, tr_p2, tr_claims_v, tr_liu, tr_claim_liu;
+    uint32_t ci_ru, ci_rv, ci_sig, ci_rliu;
+    uint32_t vf_out, key_begin, n_keys, n_vf_liu;
+};
+struct VfCheckArgs {
+    const VfLayerDesc* layers;   // by layer id; entry 0 is unused
+    const uint32_t* keys;
+    int32_t n;
+    uint32_t tr_vres, tr_input, out_total;
+};
+// claims_v[j][l] of verify_check: layer j's claims on layers l < j, zero when layer j has no phase 2
+VP_D F vf_claim_v(const VfCheckArgs& a, const F* tr, int j, int l) {
+    const VfLayerDesc& J = a.layers[j];
+    return J.m != -1 ? tr[J.tr_claims_v + l] : f_zero();
+}
+// 0 (accept) or verify_check's fail code, with its layer in *fail_layer; canonical field routines only (as k_verify_sums)
+VP_D int vf_chain(const VfCheckArgs& a, const F* tr, const F* out, const F* chal, int* fail_layer) {
+    auto ev = [](const F* q, const F& x) { return f_mul_add(f_mul_add(q[0], x, q[1]), x, q[2]); };   // a x^2 + b x + c
+    auto ok_sum = [](const F* q, const F& claim) { return f_eq(f_add(q[2], f_add(f_add(q[0], q[1]), q[2])), claim); };
+    *fail_layer = 0;
+    F prev = tr[a.tr_vres];
+    for (int i = a.n - 1; i >= 1; --i) {
+        const VfLayerDesc D = a.layers[i];
+        *fail_layer = i;
+        for (int j = 0; j < D.pb; ++j) {
+            const F* q = tr + D.tr_p1 + 3 * j;
+            if (!ok_sum(q, prev)) return 1;
+            prev = ev(q, chal[D.ci_ru + j]);
+        }
+        const F claim_u = tr[D.tr_claim_u];
+        F bv0 = f_one();
+        for (int j = 0; j < D.m; ++j) {   // (m == -1: no phase 2)
+            const F* q = tr + D.tr_p2 + 3 * j;
+            if (!ok_sum(q, prev)) return 2;
+            const F r = chal[D.ci_rv + j];
+            prev = ev(q, r);
+            bv0 = f_mul(bv0, f_sub(f_one(), r));
+        }
+        // getFinalValue (verifier.cpp:115-132) from the bucket sums
+        F cl[4] = {f_zero(), f_zero(), f_zero(), f_zero()}, bias = f_zero();
+        const F* o = out + D.vf_out;
+        for (uint32_t b = 0; b < D.n_keys; ++b) {
+            const uint32_t key = a.keys[D.key_begin + b];
+            if (key < 4) {
+                cl[key] = o[2 * b];
+                if (key == 2) bias = o[2 * b + 1];
+            }
+        }
+        if (D.m != -1) {
+            for (int k = 0; k < 4; ++k) cl[k] = f_mul(cl[k], bv0);
+            bias = f_mul(bias, bv0);
+        }
+        F res = f_mul(cl[1], f_sub(f_one(), claim_u));
+        res = f_add(res, f_mul(cl[0], claim_u));
+        res = f_add(f_add(res, f_mul(cl[2], claim_u)), bias);
+        res = f_add(res, f_mul(cl[3], claim_u));
+        if (D.m != -1)
+            for (uint32_t b = 0; b < D.n_keys; ++b) {
+                const uint32_t key = a.keys[D.key_begin + b];
+                if (key < 4) continue;
+                const int l = (int)((key - 4) / 7), bi = (int)((key - 4) % 7);
+                const F cu = claim_u, cv = tr[D.tr_claims_v + l], uv = f_mul(cu, cv);
+                F w;
+                switch (bi) {
+                    case 0: w = f_add(cu, cv); break;
+                    case 1: w = f_sub(cu, cv); break;
+                    case 2: w = f_sub(cv, cu); break;
+                    case 3: w = uv; break;
+                    case 4: w = f_sub(cv, uv); break;
+                    case 5: w = f_sub(cu, uv); break;
+                    default: w = f_sub(f_add(cu, cv), f_dbl(uv)); break;
+                }
+                res = f_add(res, f_mul(o[2 * b], w));
+            }
+        if (!f_eq(prev, res)) return 3;
+        // verifyLiu (an EMPTY subset's claim counts as well, as in verify_check)
+        const int pre = i - 1;
+        const F* sig = chal + D.ci_sig;
+        prev = f_mul(sig[0], claim_u);
+        for (int j = i; j < a.n; ++j) prev = f_add(prev, f_mul(sig[j - pre], vf_claim_v(a, tr, j, pre)));
+        for (int j = 0; j < D.pb; ++j) {
+            const F* q = tr + D.tr_liu + 3 * j;
+            if (!ok_sum(q, prev)) return 4;
+            prev = ev(q, chal[D.ci_rliu + j]);
+        }
+        const F vr = tr[D.tr_claim_liu];
+        F gr = f_zero();
+        for (uint32_t sg = 0; sg < D.n_vf_liu; ++sg) gr = f_add(gr, o[2 * (D.n_keys + sg)]);
+        if (!f_eq(f_mul(vr, gr), prev)) return 5;
+        prev = vr;
+    }
+    *fail_layer = 0;
+    const F acc = out[a.out_total - 2], claimed = tr[a.tr_input];
+    if (!f_eq(claimed, acc) || !f_eq(prev, claimed)) return 6;
+    return 0;
+}
+// One thread per statement: its verdict from its screening status (7 or 9), else code 8 when Vres is not the claimed
+// outputs' MLE at r_out (the statement's last sum), else the claim chain. tr / chal / sums: statement 0's, ss bytes apart.
+// code and layer may be null.
+__global__ void k_verify_check(VfCheckArgs a, const F* __restrict__ tr, const F* __restrict__ chal, const F* __restrict__ sums,
+                               size_t ss, uint32_t B, const int32_t* __restrict__ status, int32_t* accept, int32_t* code,
+                               int32_t* layer) {
+    const uint32_t b = blockIdx.x * blockDim.x + threadIdx.x;
+    if (b >= B) return;
+    const size_t d = (size_t)b * ss;
+    tr = reinterpret_cast<const F*>(reinterpret_cast<uintptr_t>(tr) + d);
+    chal = reinterpret_cast<const F*>(reinterpret_cast<uintptr_t>(chal) + d);
+    sums = reinterpret_cast<const F*>(reinterpret_cast<uintptr_t>(sums) + d);
+    int cd = status[b], ly = 0;
+    if (!cd) {
+        if (!f_eq(sums[a.out_total - 1], tr[a.tr_vres])) cd = 8;
+        else cd = vf_chain(a, tr, sums, chal, &ly);
+    }
+    accept[b] = cd == 0;
+    if (code) code[b] = cd;
+    if (layer) layer[b] = ly;
+}
+
 }  // namespace vp
